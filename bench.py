@@ -17,11 +17,17 @@ GPU's share each, with their own roofline fraction and parity; `cpu_baseline` is
 the oracle (the reference's CPU arithmetic restated, see oracle/) timed on this
 box's host cores on a bounded sample.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU); the clips shard across ranks
 with no data-path collective (weak scaling: 1024 clips per GPU), NCCL carries
 only the barrier and the max-over-ranks of the timing.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step
+returned to DIR/mel_spectrogram.npy, float32: a fixed, seeded sample of rank 0's
+clips (dump_sample below), or with --impl reference the oracle's output for that
+arm's 64 clips (clips 0-63).  The inputs are synthesised from a fixed seed, so
+two builds run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -49,6 +55,8 @@ WORKLOAD = ("mel_spectrogram 128 bands, 1024 x 10 s 22.05 kHz f32 clips per GPU,
 BYTES_PER_CLIP = N * 4 + N_MELS * FRAMES * 4       # 1 102 672
 ALGO_BYTES = BATCH * BYTES_PER_CLIP                # 1 129 136 128 per launch
 FALLBACK_HBM_GBS = 6650.0
+# --dump-outputs: 128 of the 1024 clips, 128 x [128, 431] f32 = 28 MB of the 226 MB output
+DUMP_CLIPS, DUMP_SEED = 128, 0
 
 
 def load_synth():
@@ -170,7 +178,7 @@ def run_reference(args, rank, world):
         return
     cores = os.cpu_count() or 1
     clips = 64
-    steps = max(1, args.steps)
+    steps = args.steps
     # torchrun exports OMP_NUM_THREADS=1 to every rank; scipy.fft's worker pool and
     # the BLAS behind the oracle's matmul both size themselves from it.  This arm
     # is the CPU path on all host threads at every N: undo the cap before either
@@ -183,14 +191,15 @@ def run_reference(args, rank, world):
     mc = mel_oracle.MelConfig(N_MELS, SR, FFT)
     for _ in range(max(1, min(args.warmup, 3))):
         cpu_reference_pass(x[:8], sc, mc, cores)
-    steps = min(steps, 20)
     # a BLAS that was loaded before the line above keeps its one thread otherwise
     from threadpoolctl import threadpool_limits
     with threadpool_limits(limits=cores):
         t0 = time.perf_counter()
         for _ in range(steps):
-            cpu_reference_pass(x, sc, mc, cores)
+            y = cpu_reference_pass(x, sc, mc, cores)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y)
     value = clips * CLIP_SECONDS * steps / dt
     sample = (f"{clips} of {BATCH} clips per step (same signal recipe), {steps} steps, clips dealt "
               f"to {cores} threads")
@@ -206,6 +215,23 @@ def run_reference(args, rank, world):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+
+
+def dump_sample(out):
+    """The GPU arm's share of --dump-outputs: float32 [DUMP_CLIPS, N_MELS, FRAMES],
+    the clips of `out` at the sorted indices
+    default_rng(DUMP_SEED).choice(BATCH, DUMP_CLIPS, replace=False)."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(out.shape[0], DUMP_CLIPS, replace=False))
+    return out[torch.from_numpy(idx).to(out.device)].cpu().numpy()
+
+
+def dump_outputs(path, mel):
+    """Write the last timed step's mel spectrograms to DIR/mel_spectrogram.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "mel_spectrogram.npy"), mel)
 
 
 def timed_ms(fn, steps, warmup, barrier, dev):
@@ -346,7 +372,13 @@ def main():
                     help="which fused fft-2048 kernel: auto (the library's choice: the frame-pair "
                          "kernel), the frame-pair kernel (pair), the one-frame-per-warp register FFT "
                          "(fast) or the tcgen05 one (tensor)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's mel spectrograms to "
+                         f"DIR/mel_spectrogram.npy (a fixed, seeded sample of {DUMP_CLIPS} clips; "
+                         "with --impl reference, that arm's 64 clips)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(3, args.warmup)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -406,6 +438,8 @@ def main():
     ms = max_over_ranks(start.elapsed_time(end), device=dev)   # the slowest rank defines the step
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     ms_per_step = ms / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dump_sample(out))
     value = world * BATCH * CLIP_SECONDS / (ms_per_step * 1e-3)
 
     # ---- end to end: pinned host buffers through the same public call
