@@ -255,10 +255,31 @@ int smb_resample_plan_set_stream(smb_resample_plan* plan, void* cuda_stream);
 int smb_resample_plan_sync(smb_resample_plan* plan);
 /* Which kernel runs the stages: SMB_EXEC_PLANNED (default) follows the planner's
  * tags -- overlap-save FFT blocks for "ols" stages (power-of-two lengths), the
- * tcgen05 banded product for "gemm" stages (L <= 160), the direct polyphase
+ * tcgen05 banded product for "gemm" stages (L <= 1024; stages wider than 160
+ * phases run as column groups of <= 160, one launch each), the direct polyphase
  * kernel for everything else; SMB_EXEC_DIRECT forces the direct kernel
  * everywhere.  Same designed filter either way. */
 int smb_resample_plan_set_executor(smb_resample_plan* plan, int exec);
+/* Which kernel smb_resample_apply runs for one stage (float32 audio), and how its
+ * device tables are laid out.  Read-only; the device tables are built first if no
+ * apply has built them yet, so the SMB_ROWS_* and SMB_GEMM_WINDOWS environment
+ * switches set at that moment take effect, as they would for a first apply. */
+enum { SMB_FORM_DIRECT = 0, SMB_FORM_OLS = 1, SMB_FORM_WINDOW = 2, SMB_FORM_ROW = 3 };
+typedef struct smb_resample_layout {
+  int form;          /* SMB_FORM_*: direct kernel, overlap-save, tcgen05 window or row form */
+  int groups;        /* column groups (launches) of the stage's form; 1 for direct and OLS */
+  int columns;       /* phases (output columns) of group `group` */
+  int col_begin;     /* its first phase */
+  /* row form only (0 otherwise; chunks is also set for the window form): */
+  int two_issuers;   /* the main shift's small terms split off, two MMA-issuing threads */
+  int a_tmem;        /* A tiles in tensor memory (else shared memory) */
+  int a_stages, b_stages;
+  int shifts;        /* input-row shifts, one accumulator each */
+  int chunks;        /* K-chunks of 32 inputs per tile */
+  int slices;        /* products per tile (runs of accumulator columns, times two for split runs) */
+} smb_resample_layout;
+int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
+                              smb_resample_layout* out);
 /* Config.pp one-liner, e.g. "resample(44100 -> 16000 Hz, quality=high, ...)". */
 int smb_resample_describe(const smb_resample_plan* plan, char* buf, size_t cap);
 int64_t smb_resample_l(const smb_resample_plan* plan);

@@ -50,6 +50,16 @@ _pd = C.POINTER(C.c_double)
 _pi64 = C.POINTER(C.c_int64)
 _pint = C.POINTER(C.c_int)
 
+
+class ResampleLayout(C.Structure):
+    """``smb_resample_layout`` (include/soundml_b200.h)."""
+    _fields_ = [(name, C.c_int) for name in (
+        "form", "groups", "columns", "col_begin", "two_issuers", "a_tmem", "a_stages",
+        "b_stages", "shifts", "chunks", "slices")]
+
+
+FORMS = {0: "direct", 1: "ols", 2: "window", 3: "row"}
+
 SIGNATURES = {
     "smb_last_error": (C.c_char_p, []),
     "smb_version": (C.c_char_p, []),
@@ -105,6 +115,7 @@ SIGNATURES = {
     "smb_resample_plan_set_stream": (_int, [_vp, _vp]),
     "smb_resample_plan_sync": (_int, [_vp]),
     "smb_resample_plan_set_executor": (_int, [_vp, _int]),
+    "smb_resample_stage_layout": (_int, [_vp, _int, _int, C.POINTER(ResampleLayout)]),
     "smb_resample_describe": (_int, [_vp, C.c_char_p, _sz]),
     "smb_resample_l": (_i64, [_vp]),
     "smb_resample_m": (_i64, [_vp]),

@@ -929,7 +929,9 @@ struct GemmDevice {
     a.a_tmem_col = total_cols;
     if (a_tmem) {
       a.a_stages = 2;
-      a.b_stages = 4;
+      // no more B stages than chunks: the B loader takes back the stage the epilogue borrowed
+      // at chunk b_stages - 1 of the next tile, a chunk a 3-chunk tile does not have
+      a.b_stages = std::min(4, chunks);
       const size_t turn = 8 * 32 * 17 * 4;                      // the producers' transposition tiles
       while (a.b_stages > 2 && smb::resample_rows_smem_bytes(0, a.b_stages, stage_bytes) + turn > budget) --a.b_stages;
       if (smb::resample_rows_smem_bytes(0, a.b_stages, stage_bytes) + turn > budget) return false;
@@ -1119,16 +1121,25 @@ struct smb_resample_plan {
     }
     device_ready = true;
   }
+  // The kernel run_stage picks for stage i (SMB_FORM_*).
+  int form(size_t i) const {
+    if (executor == SMB_EXEC_DIRECT) return SMB_FORM_DIRECT;
+    if (ols[i].plan.ok) return SMB_FORM_OLS;
+    // (SMB_GEMM_WINDOWS=1: the overlapping-window form, for A/B measurement)
+    if (gemm[i].rows_ok && !getenv("SMB_GEMM_WINDOWS")) return SMB_FORM_ROW;
+    if (gemm[i].ok) return SMB_FORM_WINDOW;
+    return SMB_FORM_DIRECT;
+  }
   // One stage over device buffers: overlap-save where the planner tagged it and
   // the GPU plan exists, the direct polyphase kernel otherwise -- the same
   // designed filter either way (resample.ml:495-497).
   void run_stage(size_t i, const float* x, int64_t batch, int64_t n, int64_t n_out, float* out,
                  cudaStream_t st) {
     const smb::ResampleStage& s = plan.stages[i];
-    if (executor != SMB_EXEC_DIRECT && ols[i].plan.ok) {
+    const int f = form(i);
+    if (f == SMB_FORM_OLS) {
       ols[i].run(x, batch, n, n_out, out, st);
-    } else if (executor != SMB_EXEC_DIRECT && gemm[i].rows_ok && !getenv("SMB_GEMM_WINDOWS")) {
-      // (SMB_GEMM_WINDOWS=1: the overlapping-window form below, for A/B measurement)
+    } else if (f == SMB_FORM_ROW) {
       for (const GemmDevice::RowsGroup& g : gemm[i].rows_groups) {
         smb::GemmRowsArgs a = g.a;
         a.x = x;
@@ -1137,7 +1148,7 @@ struct smb_resample_plan {
         a.n_out = n_out;
         CK(smb::launch_resample_rows(a, batch, gemm[i].rows_sm_count, st));
       }
-    } else if (executor != SMB_EXEC_DIRECT && gemm[i].ok) {
+    } else if (f == SMB_FORM_WINDOW) {
       for (const GemmDevice::Group& g : gemm[i].groups) {
         smb::GemmResampleArgs a{};
         a.x = x;
@@ -2140,6 +2151,39 @@ int smb_resample_plan_set_executor(smb_resample_plan* plan, int exec) {
     if (exec != SMB_EXEC_DIRECT && exec != SMB_EXEC_PLANNED)
       throw smb::invalid_argument("set_executor: SMB_EXEC_DIRECT or SMB_EXEC_PLANNED");
     plan->executor = exec;
+  });
+}
+int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
+                              smb_resample_layout* out) {
+  return guarded([&] {
+    if (stage < 0 || stage >= (int)plan->plan.stages.size())
+      throw smb::invalid_argument("stage_layout: no such stage");
+    plan->ensure_device();
+    const GemmDevice& gd = plan->gemm[(size_t)stage];
+    smb_resample_layout r{};
+    r.form = plan->form((size_t)stage);
+    r.groups = r.form == SMB_FORM_ROW ? (int)gd.rows_groups.size()
+             : r.form == SMB_FORM_WINDOW ? (int)gd.groups.size() : 1;
+    if (group < 0 || group >= r.groups) throw smb::invalid_argument("stage_layout: no such column group");
+    if (r.form == SMB_FORM_ROW) {
+      const smb::GemmRowsArgs& a = gd.rows_groups[(size_t)group].a;
+      r.columns = a.l;
+      r.col_begin = a.col_begin;
+      r.two_issuers = a.two_issuers;
+      r.a_tmem = a.a_tmem;
+      r.a_stages = a.a_stages;
+      r.b_stages = a.b_stages;
+      r.shifts = a.shifts;
+      r.chunks = a.chunks;
+      r.slices = a.slices;
+    } else if (r.form == SMB_FORM_WINDOW) {
+      r.columns = gd.groups[(size_t)group].width;
+      r.col_begin = gd.groups[(size_t)group].col_begin;
+      r.chunks = gd.groups[(size_t)group].chunks;
+    } else {
+      r.columns = (int)plan->plan.stages[(size_t)stage].l;
+    }
+    *out = r;
   });
 }
 int smb_resample_describe(const smb_resample_plan* plan, char* buf, size_t cap) {

@@ -78,6 +78,23 @@ class Config:
                             fc=fc.value, beta=beta.value))
         return out
 
+    def layout(self, i):
+        """How ``apply`` runs stage ``i`` on float32 audio: one dict per column group
+        (launch) with the kernel ``form`` ("row", "window", "ols" or "direct") and the
+        tcgen05 layout fields of ``smb_resample_layout``.  Builds the plan's device
+        tables if no ``apply`` has yet (the ``SMB_ROWS_*`` / ``SMB_GEMM_WINDOWS``
+        switches are read then)."""
+        out, g, groups = [], 0, 1
+        while g < groups:
+            r = _lib.ResampleLayout()
+            _lib.check(_lib.lib.smb_resample_stage_layout(self._h, i, g, C.byref(r)))
+            d = {name: getattr(r, name) for name, _ in r._fields_}
+            d["form"] = _lib.FORMS[r.form]
+            d["two_issuers"], d["a_tmem"] = bool(r.two_issuers), bool(r.a_tmem)
+            out.append(d)
+            groups, g = r.groups, g + 1
+        return out
+
     def stage_prototype(self, i):
         n = C.c_int64()
         _lib.check(_lib.lib.smb_resample_stage_prototype(self._h, i, None, C.byref(n)))
