@@ -866,7 +866,7 @@ struct GemmDevice {
                         (single_group || getenv("SMB_ROWS_TMEM_A"));
     int tmem_alloc = 32;
     while (tmem_alloc < total_cols + (a_tmem ? 128 : 0)) tmem_alloc *= 2;
-    const int kSliceAlign = getenv("SMB_ROWS_ALIGN") ? atoi(getenv("SMB_ROWS_ALIGN")) : 8;
+    const int kSliceAlign = 8;
     std::vector<int4> chunk_meta((size_t)chunks), slice_meta;
     struct Run { int bytes_at, start, width; };                  // a chunk's stored rows: [hi | lo][width][32]
     std::vector<Run> runs;

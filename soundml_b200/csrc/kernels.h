@@ -241,7 +241,6 @@ struct GemmRowsArgs {
                            //  three products, 1: hi x hi only, 2: the two small terms only; owner: which of the
                            //  two issuing threads takes the slice
   int two_issuers;         // slices are dealt to two MMA-issuing threads (every accumulator to one of them)
-  int debug;               // measurement only (SMB_ROWS_DEBUG): 1 no MMAs, 2 no B loads, 4 no A gather, 8 no epilogue
 };
 size_t resample_rows_smem_bytes(int a_stages, int b_stages, int b_stage_bytes);
 cudaError_t launch_resample_rows(const GemmRowsArgs& a, long long batch, int sm_count, cudaStream_t st);

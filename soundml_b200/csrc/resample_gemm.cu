@@ -32,7 +32,6 @@
 
 #include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 
 namespace smb {
 
@@ -498,7 +497,7 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
           const uint64_t a_hi = umma_desc(smem_u32(smem + sa * 2 * kABytes));
           const uint64_t a_lo = a_hi + (uint64_t)(kABytes >> 4);
           const uint32_t b_base = smem_u32(b_smem + (size_t)sb * a.b_stage_bytes);
-          for (int sl = meta.z; sl < meta.z + ((a.debug & 1) ? 0 : meta.w); ++sl) {
+          for (int sl = meta.z; sl < meta.z + meta.w; ++sl) {
             const int4 sm = s_slice[sl];
             if (((sm.w >> 2) & 1) != owner) continue;
             const uint32_t idesc = idesc0 | ((uint32_t)(sm.z >> 3) << 17);
@@ -550,13 +549,9 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
         // scratch; it comes round again for chunk kBStages - 1 of the next tile
         if (ch == kBStages - 1 && g >= a.chunks) mbar_wait(bar_scratch, (uint32_t)((g / a.chunks - 1) & 1));
         const int4 meta = s_chunk[ch];
-        if (a.debug & 2) {
-          mbar_arrive(bar_b + 8 * stage);
-        } else {
-          mbar_expect_tx(bar_b + 8 * stage, (uint32_t)meta.y);
-          bulk_g2s(smem_u32(b_smem + (size_t)stage * a.b_stage_bytes), images + meta.x, (uint32_t)meta.y,
-                   bar_b + 8 * stage);
-        }
+        mbar_expect_tx(bar_b + 8 * stage, (uint32_t)meta.y);
+        bulk_g2s(smem_u32(b_smem + (size_t)stage * a.b_stage_bytes), images + meta.x, (uint32_t)meta.y,
+                 bar_b + 8 * stage);
         if (++stage == kBStages) { stage = 0; parity ^= 1; }
         if (++ch == a.chunks) ch = 0;
       }
@@ -577,23 +572,21 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
     int ld_it = 0, ld_ch = 0;
     auto load_chunk = [&](float (&v)[16]) {
       if (ld_it >= my_tiles) return;
-      if (!(a.debug & 4)) {
-        const int tile = (int)blockIdx.x + ld_it * (int)gridDim.x;
-        const int c = tile / tiles_per_clip;
-        const long long row = (long long)(tile - c * tiles_per_clip) * rows_out + group_rows * w4 + sub;
-        const float* xs = a.x + (long long)c * a.n;
-        const long long b0 = row * a.m - a.k + (long long)ld_ch * kChunk + 16 * kh + cc;   // row `sub` of the block
-        const long long first = b0 - cc - (long long)sub * a.m;                          // the block's first sample
-        if (first >= 0 && first + 31LL * a.m + 16 <= a.n) {
-          const float* p = xs + b0;
+      const int tile = (int)blockIdx.x + ld_it * (int)gridDim.x;
+      const int c = tile / tiles_per_clip;
+      const long long row = (long long)(tile - c * tiles_per_clip) * rows_out + group_rows * w4 + sub;
+      const float* xs = a.x + (long long)c * a.n;
+      const long long b0 = row * a.m - a.k + (long long)ld_ch * kChunk + 16 * kh + cc;   // row `sub` of the block
+      const long long first = b0 - cc - (long long)sub * a.m;                          // the block's first sample
+      if (first >= 0 && first + 31LL * a.m + 16 <= a.n) {
+        const float* p = xs + b0;
 #pragma unroll
-          for (int i = 0; i < 16; ++i) v[i] = __ldg(p + 2 * i * a.m);
-        } else {
+        for (int i = 0; i < 16; ++i) v[i] = __ldg(p + 2 * i * a.m);
+      } else {
 #pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            const long long si = b0 + 2LL * i * a.m;
-            v[i] = (si >= 0 && si < a.n) ? __ldg(xs + si) : 0.0f;
-          }
+        for (int i = 0; i < 16; ++i) {
+          const long long si = b0 + 2LL * i * a.m;
+          v[i] = (si >= 0 && si < a.n) ? __ldg(xs + si) : 0.0f;
         }
       }
       if (++ld_ch == a.chunks) { ld_ch = 0; ++ld_it; }
@@ -647,23 +640,21 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
     int ld_it = 0, ld_ch = 0;                                // next chunk to load: tile iteration, chunk
     auto load_chunk = [&](float (&v)[kRowsPerWarp]) {
       if (ld_it >= my_tiles) return;
-      if (!(a.debug & 4)) {
-        const int tile = (int)blockIdx.x + ld_it * (int)gridDim.x;
-        const int c = tile / tiles_per_clip;
-        const long long first_row = (long long)(tile - c * tiles_per_clip) * rows_out + row_in_tile;
-        const float* xs = a.x + (long long)c * a.n;
-        const long long b0 = first_row * a.m + lane - a.k + (long long)ld_ch * kChunk;
-        // the warp's rows of this chunk are interior for most tiles: no bounds checks then
-        if (b0 - lane >= 0 && b0 - lane + (long long)(kRowsPerWarp - 1) * a.m + kChunk <= a.n) {
-          const float* p = xs + b0;
+      const int tile = (int)blockIdx.x + ld_it * (int)gridDim.x;
+      const int c = tile / tiles_per_clip;
+      const long long first_row = (long long)(tile - c * tiles_per_clip) * rows_out + row_in_tile;
+      const float* xs = a.x + (long long)c * a.n;
+      const long long b0 = first_row * a.m + lane - a.k + (long long)ld_ch * kChunk;
+      // the warp's rows of this chunk are interior for most tiles: no bounds checks then
+      if (b0 - lane >= 0 && b0 - lane + (long long)(kRowsPerWarp - 1) * a.m + kChunk <= a.n) {
+        const float* p = xs + b0;
 #pragma unroll
-          for (int rr = 0; rr < kRowsPerWarp; ++rr) v[rr] = __ldg(p + rr * a.m);
-        } else {
+        for (int rr = 0; rr < kRowsPerWarp; ++rr) v[rr] = __ldg(p + rr * a.m);
+      } else {
 #pragma unroll
-          for (int rr = 0; rr < kRowsPerWarp; ++rr) {
-            const long long si = b0 + (long long)rr * a.m;
-            v[rr] = (si >= 0 && si < a.n) ? __ldg(xs + si) : 0.0f;
-          }
+        for (int rr = 0; rr < kRowsPerWarp; ++rr) {
+          const long long si = b0 + (long long)rr * a.m;
+          v[rr] = (si >= 0 && si < a.n) ? __ldg(xs + si) : 0.0f;
         }
       }
       if (++ld_ch == a.chunks) { ld_ch = 0; ++ld_it; }
@@ -725,86 +716,84 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
       const long long out_row = (long long)(tile - c * tiles_per_clip) * rows_out + group_rows * w4 + lane;
       mbar_wait(bar_acc_full, (uint32_t)(it & 1));
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      if (!(a.debug & 8)) {
-        // out[row] = (D_0[row] + D_1[row + 1]) + D_2[row + 2] ..., 16 columns at a time.
-        // When L is not a multiple of 4 (no aligned 16-byte stores) the block is turned
-        // through a [32][17] tile so that a store instruction writes two whole 64-byte
-        // runs instead of 32 words of 32 different rows (48 -> 44.1 kHz: 1.22 -> 0.97 ms).
-        // The tile lives in the B stage of the tile's last chunk (drained: acc_full has
-        // completed).
-        float* obase = a.out + (long long)c * a.n_out;
-        const long long base_row = out_row - lane;              // the warp's first output row
-        const bool vec = ((a.l | a.l_total | a.col_begin) & 3) == 0 && (reinterpret_cast<size_t>(obase) & 15) == 0;
-        const int last_stage = (int)(((long long)it * a.chunks + a.chunks - 1) % kBStages);
-        float* tr = reinterpret_cast<float*>(b_smem + (size_t)last_stage * a.b_stage_bytes) +
-                    (warp - kEpiWarp0) * (32 * 17);
-        for (int col = 16 * half; col < a.n_pad; col += 16 * kEpiPerQuarter) {
-          // every accumulator that holds these 16 columns, in a fixed order
-          // ((acc0 + acc1) + acc2) + ..., three loads in flight at a time (registers)
-          float o[16];
+      // out[row] = (D_0[row] + D_1[row + 1]) + D_2[row + 2] ..., 16 columns at a time.
+      // When L is not a multiple of 4 (no aligned 16-byte stores) the block is turned
+      // through a [32][17] tile so that a store instruction writes two whole 64-byte
+      // runs instead of 32 words of 32 different rows (48 -> 44.1 kHz: 1.22 -> 0.97 ms).
+      // The tile lives in the B stage of the tile's last chunk (drained: acc_full has
+      // completed).
+      float* obase = a.out + (long long)c * a.n_out;
+      const long long base_row = out_row - lane;              // the warp's first output row
+      const bool vec = ((a.l | a.l_total | a.col_begin) & 3) == 0 && (reinterpret_cast<size_t>(obase) & 15) == 0;
+      const int last_stage = (int)(((long long)it * a.chunks + a.chunks - 1) % kBStages);
+      float* tr = reinterpret_cast<float*>(b_smem + (size_t)last_stage * a.b_stage_bytes) +
+                  (warp - kEpiWarp0) * (32 * 17);
+      for (int col = 16 * half; col < a.n_pad; col += 16 * kEpiPerQuarter) {
+        // every accumulator that holds these 16 columns, in a fixed order
+        // ((acc0 + acc1) + acc2) + ..., three loads in flight at a time (registers)
+        float o[16];
 #pragma unroll
-          for (int e = 0; e < 16; ++e) o[e] = 0.0f;
+        for (int e = 0; e < 16; ++e) o[e] = 0.0f;
 #pragma unroll
-          for (int q0 = 0; q0 < 6; q0 += 3) {
-            if (q0 >= a.n_acc) break;
-            uint32_t d[3][16];
-            bool have[3];
+        for (int q0 = 0; q0 < 6; q0 += 3) {
+          if (q0 >= a.n_acc) break;
+          uint32_t d[3][16];
+          bool have[3];
 #pragma unroll
-            for (int u = 0; u < 3; ++u) {
-              const int q = q0 + u;
-              have[u] = q < a.n_acc && col >= a.acc_lo[q < 5 ? q : 4] && col < a.acc_lo[q < 5 ? q : 4] + a.acc_w[q < 5 ? q : 4];
-              if (have[u]) tmem_ld16_async(tmem + lane_base + (uint32_t)(a.acc_col[q < 5 ? q : 4] + col - a.acc_lo[q < 5 ? q : 4]), d[u]);
-            }
-            tmem_ld_wait();
-#pragma unroll
-            for (int u = 0; u < 3; ++u) {
-              const int q = q0 + u < 5 ? q0 + u : 4;
-              if (have[u]) {                                       // (uniform)
-                tmem_st16_zero(tmem + lane_base + (uint32_t)(a.acc_col[q] + col - a.acc_lo[q]));
-                const int sh = a.acc_shift[q];
-#pragma unroll
-                for (int e = 0; e < 16; ++e) o[e] += __shfl_down_sync(0xffffffffu, __uint_as_float(d[u][e]), sh);
-              }
-            }
+          for (int u = 0; u < 3; ++u) {
+            const int q = q0 + u;
+            have[u] = q < a.n_acc && col >= a.acc_lo[q < 5 ? q : 4] && col < a.acc_lo[q < 5 ? q : 4] + a.acc_w[q < 5 ? q : 4];
+            if (have[u]) tmem_ld16_async(tmem + lane_base + (uint32_t)(a.acc_col[q < 5 ? q : 4] + col - a.acc_lo[q < 5 ? q : 4]), d[u]);
           }
-          __syncwarp();                                            // the previous group has been read out
-          const long long idx0 = base_row * a.l_total + a.col_begin + col;   // index of (the warp's row 0, col) in the clip
-          const int rows_ok = (int)min((long long)group_rows, rows_total - base_row);
-          if (vec && col + 16 <= a.l) {
-            // L a multiple of 4: a lane writes its row's 64 bytes itself, four 16-byte
-            // stores (measured faster than turning the block through shared memory:
-            // 1.97 against 2.14 ms on the 44.1 -> 16 kHz workload -- the tensor core waits
-            // for the epilogue, so its latency counts more than its sector efficiency)
-            const long long idx = idx0 + lane * a.l_total;
-            if (lane < rows_ok) {
-              if (idx + 16 <= a.n_out) {
-                float4* dst = reinterpret_cast<float4*>(obase + idx);
+          tmem_ld_wait();
 #pragma unroll
-                for (int e = 0; e < 16; e += 4) dst[e >> 2] = make_float4(o[e], o[e + 1], o[e + 2], o[e + 3]);
-              } else {
+          for (int u = 0; u < 3; ++u) {
+            const int q = q0 + u < 5 ? q0 + u : 4;
+            if (have[u]) {                                       // (uniform)
+              tmem_st16_zero(tmem + lane_base + (uint32_t)(a.acc_col[q] + col - a.acc_lo[q]));
+              const int sh = a.acc_shift[q];
 #pragma unroll
-                for (int e = 0; e < 16; ++e)
-                  if (idx + e < a.n_out) obase[idx + e] = o[e];
-              }
-            }
-          } else {
-#pragma unroll
-            for (int e = 0; e < 16; ++e) tr[lane * 17 + e] = o[e];
-            __syncwarp();
-            const int cc = lane & 15;
-            if (col + cc < a.l) {
-#pragma unroll
-              for (int i = 0; i < 16; ++i) {
-                const int r = 2 * i + (lane >> 4);
-                const long long idx = idx0 + r * a.l_total + cc;
-                if (r < rows_ok && idx < a.n_out) obase[idx] = tr[r * 17 + cc];
-              }
+              for (int e = 0; e < 16; ++e) o[e] += __shfl_down_sync(0xffffffffu, __uint_as_float(d[u][e]), sh);
             }
           }
         }
-        __syncwarp();
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic accesses before the next bulk copy
+        __syncwarp();                                            // the previous group has been read out
+        const long long idx0 = base_row * a.l_total + a.col_begin + col;   // index of (the warp's row 0, col) in the clip
+        const int rows_ok = (int)min((long long)group_rows, rows_total - base_row);
+        if (vec && col + 16 <= a.l) {
+          // L a multiple of 4: a lane writes its row's 64 bytes itself, four 16-byte
+          // stores (measured faster than turning the block through shared memory:
+          // 1.97 against 2.14 ms on the 44.1 -> 16 kHz workload -- the tensor core waits
+          // for the epilogue, so its latency counts more than its sector efficiency)
+          const long long idx = idx0 + lane * a.l_total;
+          if (lane < rows_ok) {
+            if (idx + 16 <= a.n_out) {
+              float4* dst = reinterpret_cast<float4*>(obase + idx);
+#pragma unroll
+              for (int e = 0; e < 16; e += 4) dst[e >> 2] = make_float4(o[e], o[e + 1], o[e + 2], o[e + 3]);
+            } else {
+#pragma unroll
+              for (int e = 0; e < 16; ++e)
+                if (idx + e < a.n_out) obase[idx + e] = o[e];
+            }
+          }
+        } else {
+#pragma unroll
+          for (int e = 0; e < 16; ++e) tr[lane * 17 + e] = o[e];
+          __syncwarp();
+          const int cc = lane & 15;
+          if (col + cc < a.l) {
+#pragma unroll
+            for (int i = 0; i < 16; ++i) {
+              const int r = 2 * i + (lane >> 4);
+              const long long idx = idx0 + r * a.l_total + cc;
+              if (r < rows_ok && idx < a.n_out) obase[idx] = tr[r * 17 + cc];
+            }
+          }
+        }
       }
+      __syncwarp();
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic accesses before the next bulk copy
       if (lane == 0) mbar_arrive(bar_scratch);
       release_accumulators();
     }
@@ -844,7 +833,6 @@ cudaError_t launch_resample_rows(const GemmRowsArgs& a, long long batch, int sm_
     GemmRowsArgs s = a;
     s.x = a.x + b0 * a.n;
     s.out = a.out + b0 * a.n_out;
-    s.debug = getenv("SMB_ROWS_DEBUG") ? atoi(getenv("SMB_ROWS_DEBUG")) : 0;
     const long long total = tiles * nb;
     const int grid = (int)(total < sm_count ? total : sm_count);
     resample_rows_kernel<<<grid, kRowsThreads, smem, st>>>(s, (int)tiles, (int)total);

@@ -9,7 +9,6 @@
 // with xz = x extended by zeros on both sides (resample_stubs.c:127-143;
 // independent evaluator soundml/test/resample/resample_kernel.ml:144-163).
 // Phase and window start are exact integers -- no float time accumulator.
-#include <cstdlib>
 
 #include "kernels.h"
 
@@ -201,7 +200,6 @@ static cudaError_t launch_block(const T* x, long long batch, long long n, const 
 template <typename T>
 static bool try_block(const T* x, long long batch, long long n, const T* bank, int l, int m, int k,
                       long long n_out, T* out, cudaStream_t st, cudaError_t* err) {
-  if (getenv("SMB_NO_BLOCKED_DIRECT")) return false;            // measurement switch: the one-output-per-thread kernel
 #define SMB_TRY(LL, MM)                                                                    \
   if (l == LL && m == MM) {                                                                \
     if (BlockShape<T, LL, MM>::smem(k) > 200 * 1024) return false;                         \

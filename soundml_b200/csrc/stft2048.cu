@@ -130,7 +130,7 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
 
 struct Params {
   Stft2048Args a;
-  // interior tiles by one bulk copy (SMB_NO_BULK=1 turns it off): tiles t in
+  // interior tiles by one bulk copy: tiles t in
   // [bulk_t_lo, bulk_t_hi] of a clip b with (b * bulk_nmod + bulk_c0) % 4 == 0
   int bulk_t_lo, bulk_t_hi;
   unsigned bulk_nmod, bulk_c0;
@@ -612,7 +612,7 @@ cudaError_t launch_stft2048(const Stft2048Args& a, int out_kind, int sm_count, c
   p.bulk_t_lo = 0;
   p.bulk_t_hi = -1;
   p.bulk_nmod = p.bulk_c0 = 0;
-  if (!getenv("SMB_NO_BULK") && (a.g.hop & 3) == 0 && (reinterpret_cast<size_t>(a.x) & 3) == 0) {
+  if ((a.g.hop & 3) == 0 && (reinterpret_cast<size_t>(a.x) & 3) == 0) {
     // full tile t reads source samples [t*T*hop - left, ... + span): inside the clip, and
     // 16-byte aligned when (x/4 + b*n - left) % 4 == 0 (T*hop is a multiple of 4)
     const long long th = (long long)kTile * a.g.hop, span = (long long)(kTile - 1) * a.g.hop + kFft;

@@ -34,7 +34,6 @@
 // frames overwrite its own transposition buffer, [bin][2 frames].
 #include <algorithm>
 #include <cstdint>
-#include <cstdlib>
 
 #include "fft32x2.cuh"
 #include "kernels.h"
@@ -59,10 +58,7 @@ constexpr int kWarpBuf = 32 * kExPitch * 16;   // bytes: [32][33] x (re A, re B,
 constexpr int kPowerBins = 1032;            // bins per power row incl. the zeroed tail the mel steps may read
 static_assert(32 * (kGroupWarps - 1) + kPowerBins * 8 <= kWarpBuf, "power rows fit the transposition buffer");
 
-// kModeFree: the ceiling with its warps running free -- the first tile's samples are
-// staged once and re-read, no group barrier, no staging inside the loop (what the
-// transform skeleton does when nothing couples the warps; measurement only)
-enum Mode { kModeMel = 0, kModeCeiling = 1, kModeFree = 2 };
+enum Mode { kModeMel = 0, kModeCeiling = 1 };
 
 // W_64^k2 = exp(-2 pi i k2 / 64), k2 < 16: the split twiddle W_2048^(l + 32 k2) is the
 // lane's W_2048^l times one of these constants.
@@ -81,9 +77,8 @@ struct Params {
   Stft2048PairArgs a;
   stage::BulkRule bulk;
   int span_bytes;            // bytes reserved per group for samples (multiple of 128)
-  int tables_bytes;          // window, twiddles, mel tables (multiple of 128)
+  int tables_bytes;          // reserved bytes, split twiddles, mel tables (multiple of 128)
   int tiles_per_signal, total_tiles;
-  int skip_b;                // measurement only (SMB_PAIR_NO_B=1): no group barrier before the mel phase (results are wrong)
 };
 
 // ---- TMEM as a per-lane table store.  The window and the inter-pass twiddles are
@@ -142,15 +137,12 @@ __device__ __forceinline__ pk_t power_of(CP x, float power) {
 // starts hop samples = ROWS rows of 32 complex points after frame A, so row n1 of B
 // is row n1 + ROWS of A in the same lane: the pair needs 32 + ROWS sample loads
 // instead of 64.
-// TT: window and twiddle tables in tensor memory (else in shared memory).
-template <bool SQUARE, int MODE, int ROWS, bool TT>
+template <bool SQUARE, int MODE, int ROWS>
 __global__ void __launch_bounds__(kGroups * kGroupThreads, 1)
 stft2048p_kernel(const Params p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  // tables: window [16][32] x float4 {w(n1).re, w(n1).im, w(n1+1).re, w(n1+1).im} x 1/2;
-  // inter-pass twiddles [16][32] x float4 {W(k1), W(k1+1)}; split twiddles [32] float2
-  float* sWindow = reinterpret_cast<float*>(smem_raw);
-  float4* sTwPass = reinterpret_cast<float4*>(smem_raw + 8192);
+  // tables: [0, 16384) unused (see tables_bytes_needed); split twiddles [32] float2;
+  // mel weights; mel items
   float2* sTwPost = reinterpret_cast<float2*>(smem_raw + 16384);
   float* sMelW = reinterpret_cast<float*>(smem_raw + 16640);
   PairMelItem* sItems = reinterpret_cast<PairMelItem*>(sMelW + p.a.mel_w_floats);
@@ -169,49 +161,37 @@ stft2048p_kernel(const Params p) {
   unsigned char* ex = sBufs + warp * kWarpBuf;                 // this warp's
   float* prow = reinterpret_cast<float*>(ex + 32 * warp);      // its power rows, [bin][2]
 
-  uint32_t ttab = 0;                     // tensor-memory address of this warp's table rows
-  if (TT) {
-    if (tid < 32) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                   ::"r"(smem_u32(&tmem_slot)), "r"(kTmemCols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    ttab = tmem_slot + ((uint32_t)(((tid >> 5) & 3) * 32) << 16);
-    if (tid < 128) {                     // one warp per 32-lane quarter fills it
-      uint32_t v[16];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-#pragma unroll
-        for (int e = 0; e < 16; ++e)     // column 2 n1 + c: w[64 n1 + 2 lane + c] / 2
-          v[e] = __float_as_uint(p.a.window[64 * (8 * q + (e >> 1)) + 2 * lane + (e & 1)] * 0.5f);
-        tmem_st16(ttab + 16 * q, v);
-      }
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-#pragma unroll
-        for (int e = 0; e < 16; ++e) {   // column 64 + 2 k1 + c: W1024^(k1 lane)
-          const float2 t = p.a.tw_pass[(8 * q + (e >> 1)) * 32 + lane];
-          v[e] = __float_as_uint((e & 1) ? t.y : t.x);
-        }
-        tmem_st16(ttab + 64 + 16 * q, v);
-      }
-      asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");   // ordered by the barrier below
-  } else {
-    for (int i = tid; i < 2048; i += blockDim.x) {
-      // source index j = 2 (32 n1 + l) + c  ->  ((n1/2) * 32 + l) * 4 + (n1 & 1) * 2 + c
-      const int c = i & 1, l = (i >> 1) & 31, n1 = i >> 6;
-      sWindow[(((n1 >> 1) * 32 + l) << 2) + ((n1 & 1) << 1) + c] = p.a.window[i] * 0.5f;
-    }
-    for (int i = tid; i < 1024; i += blockDim.x) {
-      const int l = i & 31, k1 = i >> 5;
-      reinterpret_cast<float2*>(sTwPass)[(((k1 >> 1) * 32 + l) << 1) + (k1 & 1)] = p.a.tw_pass[i];
-    }
+  if (tid < 32) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                 ::"r"(smem_u32(&tmem_slot)), "r"(kTmemCols) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  // tensor-memory address of this warp's table rows
+  const uint32_t ttab = tmem_slot + ((uint32_t)(((tid >> 5) & 3) * 32) << 16);
+  if (tid < 128) {                       // one warp per 32-lane quarter fills it
+    uint32_t v[16];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+#pragma unroll
+      for (int e = 0; e < 16; ++e)       // column 2 n1 + c: w[64 n1 + 2 lane + c] / 2
+        v[e] = __float_as_uint(p.a.window[64 * (8 * q + (e >> 1)) + 2 * lane + (e & 1)] * 0.5f);
+      tmem_st16(ttab + 16 * q, v);
+    }
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+#pragma unroll
+      for (int e = 0; e < 16; ++e) {     // column 64 + 2 k1 + c: W1024^(k1 lane)
+        const float2 t = p.a.tw_pass[(8 * q + (e >> 1)) * 32 + lane];
+        v[e] = __float_as_uint((e & 1) ? t.y : t.x);
+      }
+      tmem_st16(ttab + 64 + 16 * q, v);
+    }
+    asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");   // ordered by the barrier below
   if (tid < 32) sTwPost[tid] = p.a.tw_post[tid];
   if (MODE == kModeMel) {
     for (int i = tid; i < p.a.mel_w_floats; i += blockDim.x) sMelW[i] = p.a.mel_w[i];
@@ -225,7 +205,7 @@ stft2048p_kernel(const Params p) {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncthreads();
-  if (TT) asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t sbar = smem_u32(&sbars[group]);
   const uint32_t fbar = smem_u32(&sfree[group]);
   uint32_t sphase = 0, tiles_done = 0;
@@ -252,18 +232,16 @@ stft2048p_kernel(const Params p) {
     const int nf = (int)min((long long)kTile, g.frames - p0);
 
     // ---- the tile's samples were requested one iteration ago
-    if (MODE != kModeFree || tile == slot) {
-      // no group barrier here when the tile came by bulk copy: every thread sees the
-      // samples through the mbarrier, and the only other thing the barrier ordered -- the
-      // previous tile's mel reads of the power rows against this tile's transposition
-      // stores -- is waited for where it matters, just before those stores (sfree)
-      if (bulk) {
-        stage::mbar_wait(sbar, sphase & 1);
-        ++sphase;
-      } else {
-        asm volatile("cp.async.wait_all;" ::: "memory");
-        named_sync(group + 1, kGroupThreads);
-      }
+    // no group barrier here when the tile came by bulk copy: every thread sees the
+    // samples through the mbarrier, and the only other thing the barrier ordered -- the
+    // previous tile's mel reads of the power rows against this tile's transposition
+    // stores -- is waited for where it matters, just before those stores (sfree)
+    if (bulk) {
+      stage::mbar_wait(sbar, sphase & 1);
+      ++sphase;
+    } else {
+      asm volatile("cp.async.wait_all;" ::: "memory");
+      named_sync(group + 1, kGroupThreads);
     }
 
     {
@@ -274,82 +252,53 @@ stft2048p_kernel(const Params p) {
       CP a[32];
       if (ROWS > 0) {
         const float2* sA = reinterpret_cast<const float2*>(sSamples + 2 * warp * g.hop) + lane;
-        const float4* w4 = reinterpret_cast<const float4*>(sWindow) + lane;
         float2 raw[32 + ROWS];
 #pragma unroll
         for (int r = 0; r < 32 + ROWS; ++r) raw[r] = sA[32 * r];
-        if (TT) {
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            uint32_t wv[16];
-            tmem_ld16(ttab + 16 * q, wv);
-            tmem_wait16(wv);
+        for (int q = 0; q < 4; ++q) {
+          uint32_t wv[16];
+          tmem_ld16(ttab + 16 * q, wv);
+          tmem_wait16(wv);
 #pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              const int n1 = 8 * q + e;
-              const float wx = __uint_as_float(wv[2 * e]), wy = __uint_as_float(wv[2 * e + 1]);
-              a[n1] = CP{pk(raw[n1].x * wx, raw[n1 + ROWS].x * wx), pk(raw[n1].y * wy, raw[n1 + ROWS].y * wy)};
-            }
-          }
-        } else {
-#pragma unroll
-          for (int n1 = 0; n1 < 32; n1 += 2) {
-            const float4 w = w4[(n1 >> 1) * 32];
-            a[n1] = CP{pk(raw[n1].x * w.x, raw[n1 + ROWS].x * w.x), pk(raw[n1].y * w.y, raw[n1 + ROWS].y * w.y)};
-            a[n1 + 1] = CP{pk(raw[n1 + 1].x * w.z, raw[n1 + 1 + ROWS].x * w.z),
-                           pk(raw[n1 + 1].y * w.w, raw[n1 + 1 + ROWS].y * w.w)};
+          for (int e = 0; e < 8; ++e) {
+            const int n1 = 8 * q + e;
+            const float wx = __uint_as_float(wv[2 * e]), wy = __uint_as_float(wv[2 * e + 1]);
+            a[n1] = CP{pk(raw[n1].x * wx, raw[n1 + ROWS].x * wx), pk(raw[n1].y * wy, raw[n1 + ROWS].y * wy)};
           }
         }
       } else {
         const float2* sA = reinterpret_cast<const float2*>(sSamples + 2 * warp * g.hop) + lane;
         const float2* sB = reinterpret_cast<const float2*>(sSamples + (2 * warp + 1) * g.hop) + lane;
-        const float4* w4 = reinterpret_cast<const float4*>(sWindow) + lane;
-        if (TT) {
 #pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            uint32_t wv[16];
-            tmem_ld16(ttab + 16 * q, wv);
-            tmem_wait16(wv);
+        for (int q = 0; q < 4; ++q) {
+          uint32_t wv[16];
+          tmem_ld16(ttab + 16 * q, wv);
+          tmem_wait16(wv);
 #pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              const int n1 = 8 * q + e;
-              const float2 a0 = sA[32 * n1], b0 = sB[32 * n1];
-              const float wx = __uint_as_float(wv[2 * e]), wy = __uint_as_float(wv[2 * e + 1]);
-              a[n1] = CP{pk(a0.x * wx, b0.x * wx), pk(a0.y * wy, b0.y * wy)};
-            }
-          }
-        } else {
-#pragma unroll
-          for (int n1 = 0; n1 < 32; n1 += 2) {
-            const float2 a0 = sA[32 * n1], a1 = sA[32 * (n1 + 1)];
-            const float2 b0 = sB[32 * n1], b1 = sB[32 * (n1 + 1)];
-            const float4 w = w4[(n1 >> 1) * 32];
-            a[n1] = CP{pk(a0.x * w.x, b0.x * w.x), pk(a0.y * w.y, b0.y * w.y)};
-            a[n1 + 1] = CP{pk(a1.x * w.z, b1.x * w.z), pk(a1.y * w.w, b1.y * w.w)};
+          for (int e = 0; e < 8; ++e) {
+            const int n1 = 8 * q + e;
+            const float2 a0 = sA[32 * n1], b0 = sB[32 * n1];
+            const float wx = __uint_as_float(wv[2 * e]), wy = __uint_as_float(wv[2 * e + 1]);
+            a[n1] = CP{pk(a0.x * wx, b0.x * wx), pk(a0.y * wy, b0.y * wy)};
           }
         }
       }
       fft32(a);                                   // a[k1] = Y[n2 = lane][k1]
       // ---- the previous tile's power rows (this buffer) have been read by all four warps
-      if (MODE != kModeFree && tiles_done > 0) stage::mbar_wait(fbar, (tiles_done - 1) & 1);
+      if (tiles_done > 0) stage::mbar_wait(fbar, (tiles_done - 1) & 1);
       // ---- twiddle W1024^(k1 n2), transpose through the warp's padded buffer
       {
-        const float4* t4 = sTwPass + lane;
         ulonglong2* st = reinterpret_cast<ulonglong2*>(ex) + lane;
         uint32_t tv[16];
 #pragma unroll
         for (int k1 = 0; k1 < 32; k1 += 2) {
-          float4 t;
-          if (TT) {
-            if ((k1 & 7) == 0) {
-              tmem_ld16(ttab + 64 + 2 * k1, tv);
-              tmem_wait16(tv);
-            }
-            t = make_float4(__uint_as_float(tv[2 * (k1 & 7)]), __uint_as_float(tv[2 * (k1 & 7) + 1]),
-                            __uint_as_float(tv[2 * (k1 & 7) + 2]), __uint_as_float(tv[2 * (k1 & 7) + 3]));
-          } else {
-            t = t4[(k1 >> 1) * 32];
+          if ((k1 & 7) == 0) {
+            tmem_ld16(ttab + 64 + 2 * k1, tv);
+            tmem_wait16(tv);
           }
+          const float4 t = make_float4(__uint_as_float(tv[2 * (k1 & 7)]), __uint_as_float(tv[2 * (k1 & 7) + 1]),
+                                       __uint_as_float(tv[2 * (k1 & 7) + 2]), __uint_as_float(tv[2 * (k1 & 7) + 3]));
           const CP v0 = k1 == 0 ? a[0]
                                 : CP{pfmas(a[k1].im, -t.y, pmuls(a[k1].re, t.x)),
                                      pfmas(a[k1].im, t.x, pmuls(a[k1].re, t.y))};
@@ -412,12 +361,10 @@ stft2048p_kernel(const Params p) {
         }
       }
     }
-    if (MODE != kModeFree) {
-      if (!p.skip_b) named_sync(group + 1, kGroupThreads);
-      // ---- the sample buffer is free: fetch the next tile under the mel phase
-      if (tile + stride < total_tiles)
-        bulk = stage::stage_tile<kTile, kGroupThreads>(g, p.a.x, p.bulk, nb, nt, sSamples, gtid, sbar);
-    }
+    named_sync(group + 1, kGroupThreads);
+    // ---- the sample buffer is free: fetch the next tile under the mel phase
+    if (tile + stride < total_tiles)
+      bulk = stage::stage_tile<kTile, kGroupThreads>(g, p.a.x, p.bulk, nb, nt, sSamples, gtid, sbar);
 
     if (MODE == kModeMel) {
       // ---- mel projection.  lane = (filter i of the round's eight, frame pair j): one
@@ -481,13 +428,11 @@ stft2048p_kernel(const Params p) {
     ++tiles_done;
   }
   if (MODE == kModeMel && p.a.max_slot) warp_max_to((double)vmax, p.a.max_slot);
-  if (TT) {
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    if (tid < 32)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_slot), "r"(kTmemCols)
-                   : "memory");
-  }
+  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  __syncthreads();
+  if (tid < 32)
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_slot), "r"(kTmemCols)
+                 : "memory");
 }
 
 }  // namespace
@@ -497,6 +442,10 @@ static const size_t kSmemLimit = 232448;   // 227 KB opt-in maximum per CTA
 static int span_bytes_needed(const FrameGeom& g) {
   return ((((kTile - 1) * g.hop + 2048) * 4) + 127) & ~127;
 }
+// The first 16384 bytes are not read: the window and the inter-pass twiddles live in
+// tensor memory.  They stay reserved because this size decides, through
+// stft2048p_supports, which geometries SMB_PATH_AUTO sends to this kernel; reclaiming
+// them would move geometries between kernels.
 static int tables_bytes_needed(int mel_w_floats, int mel_rounds) {
   return (16640 + mel_w_floats * 4 + kGroupWarps * mel_rounds * kF * (int)sizeof(PairMelItem) + 127) & ~127;
 }
@@ -531,41 +480,31 @@ cudaError_t launch_stft2048p(const Stft2048PairArgs& a, bool ceiling, int sm_cou
   Params p;
   p.a = a;
   if (ceiling) { p.a.mel_w_floats = 0; p.a.mel_rounds = 0; }
-  if (getenv("SMB_PAIR_SKIP_MEL")) p.a.mel_rounds = 0;   // measurement: everything but the mel phase (no output)
-  p.bulk = stage::bulk_rule(a.x, a.g, kTile, !getenv("SMB_NO_BULK"));
+  p.bulk = stage::bulk_rule(a.x, a.g, kTile);
   p.span_bytes = span_bytes_needed(a.g);
   p.tables_bytes = tables_bytes_needed(p.a.mel_w_floats, p.a.mel_rounds);
   p.tiles_per_signal = (int)tiles_per_signal;
   p.total_tiles = (int)(tiles_per_signal * a.batch);
-  p.skip_b = getenv("SMB_PAIR_NO_B") ? 1 : 0;
   const size_t smem = smem_needed(a.g, p.a.mel_w_floats, p.a.mel_rounds);
   if (smem + 64 > kSmemLimit) return cudaErrorInvalidConfiguration;
   const long long want = (p.total_tiles + kGroups - 1) / kGroups;
   const int grid = (int)(want < sm_count ? want : sm_count);
   cudaError_t e;
-#define SMB_LAUNCH2048P_RT(SQ, MODE, R, T)                                                     \
-  e = cudaFuncSetAttribute(stft2048p_kernel<SQ, MODE, R, T>,                                   \
+#define SMB_LAUNCH2048P_R(SQ, MODE, R)                                                         \
+  e = cudaFuncSetAttribute(stft2048p_kernel<SQ, MODE, R>,                                      \
                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);            \
   if (e != cudaSuccess) return e;                                                              \
-  stft2048p_kernel<SQ, MODE, R, T><<<grid, kGroups * kGroupThreads, smem, st>>>(p);
-  // SMB_NO_TMEM_TABLES=1: window and twiddles from shared memory instead of tensor
-  // memory (A/B measurement: 64 more shared-memory wavefronts per frame, 0.941 against
-  // 0.937 ms on the headline workload)
-  const bool tmem_tables = !getenv("SMB_NO_TMEM_TABLES");
-#define SMB_LAUNCH2048P_R(SQ, MODE, R)                                                         \
-  if (tmem_tables) { SMB_LAUNCH2048P_RT(SQ, MODE, R, true) } else { SMB_LAUNCH2048P_RT(SQ, MODE, R, false) }
+  stft2048p_kernel<SQ, MODE, R><<<grid, kGroups * kGroupThreads, smem, st>>>(p);
   // hop 512 (fft / 4) and 256 (fft / 8) share sample rows between the frames of a pair
 #define SMB_LAUNCH2048P(SQ, MODE)                                                              \
-  if (a.g.hop == 512 && !getenv("SMB_NO_SHARED_ROWS")) { SMB_LAUNCH2048P_R(SQ, MODE, 8) }      \
-  else if (a.g.hop == 256 && !getenv("SMB_NO_SHARED_ROWS")) { SMB_LAUNCH2048P_R(SQ, MODE, 4) } \
+  if (a.g.hop == 512) { SMB_LAUNCH2048P_R(SQ, MODE, 8) }                                       \
+  else if (a.g.hop == 256) { SMB_LAUNCH2048P_R(SQ, MODE, 4) }                                  \
   else { SMB_LAUNCH2048P_R(SQ, MODE, 0) }
-  if (ceiling && getenv("SMB_PAIR_FREERUN")) { SMB_LAUNCH2048P(true, kModeFree) }
-  else if (ceiling) { SMB_LAUNCH2048P(true, kModeCeiling) }
+  if (ceiling) { SMB_LAUNCH2048P(true, kModeCeiling) }
   else if (a.power == 2.0f) { SMB_LAUNCH2048P(true, kModeMel) }
   else { SMB_LAUNCH2048P(false, kModeMel) }
 #undef SMB_LAUNCH2048P
 #undef SMB_LAUNCH2048P_R
-#undef SMB_LAUNCH2048P_RT
   ++g_launch_count;
   return cudaGetLastError();
 }

@@ -43,8 +43,6 @@
 #include "kernels.h"
 
 #include <cstdint>
-#include <cstdio>
-#include <cstdlib>
 #include <cuda_fp16.h>
 
 namespace smb {
@@ -207,7 +205,6 @@ __device__ __forceinline__ float2 unpack_half2(uint32_t h) {
 
 struct Params {
   Stft2048Args a;
-  long long* timing;         // [9] cycle totals (TIMING kernels only)
   int span_cap;              // floats reserved per group for samples (multiple of 4)
   int region_bytes;          // operand / row region per group (multiple of 1024)
   int row_stride;            // floats per output row of a frame
@@ -288,14 +285,9 @@ __device__ __forceinline__ void stage_tile(const Params& p, TileRef t, bool bulk
 }
 
 // STEP1: bin_step == 1 (fft 2048 proper): every bin is kept.
-template <int OUT, bool SQUARE, int kGroups, bool STEP1, bool TIMING = false>
+template <int OUT, bool SQUARE, int kGroups, bool STEP1>
 __global__ void __launch_bounds__(kGroups * kGroupThreads, 1)
 stft2048tc_kernel(const Params p) {
-  // TIMING: per-phase cycle totals of every group's first thread (profiling aid,
-  // SMB_TC_TIMING=1): wait, scale, build, mma1, convert, mma2, split, mel, write
-  long long tacc[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
-  long long tprev = 0;
-#define SMB_TC_MARK(i) if (TIMING) { const long long tnow = clock64(); tacc[i] += tnow - tprev; tprev = tnow; }
   extern __shared__ uint8_t smem_raw[];
   __shared__ __align__(8) uint64_t bars[2 * kMaxGroups];
   __shared__ uint32_t tmem_base_slot;
@@ -417,7 +409,6 @@ stft2048tc_kernel(const Params p) {
     }
     cur = nxt;
 
-    if (TIMING) tprev = clock64();
     if (bulk) {
       mbar_wait(sbar, sphase & 1);
       ++sphase;
@@ -425,7 +416,6 @@ stft2048tc_kernel(const Params p) {
       asm volatile("cp.async.wait_all;" ::: "memory");
     }
     group_sync(group);
-    SMB_TC_MARK(0)
 
     // ---- scale: largest sample magnitude of the tile -> power of two
     float scale, unscale;
@@ -449,7 +439,6 @@ stft2048tc_kernel(const Params p) {
       unscale = __uint_as_float((uint32_t)(254 - sb) << 23);
     }
 
-    SMB_TC_MARK(1)
     // ---- pass-1 operand: rows (f, n2 = lane), this warp's 16 K-columns
     {
       float2 ws[8];
@@ -500,7 +489,6 @@ stft2048tc_kernel(const Params p) {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     group_sync(group);
-    SMB_TC_MARK(2)
 
     if (gtid == 0) {
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -522,7 +510,6 @@ stft2048tc_kernel(const Params p) {
     mbar_wait(bar, phase & 1);
     ++phase;
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    SMB_TC_MARK(3)
 
     // ---- D1 row (f = warp, n2 = lane): twiddle, split, scatter into pass 2's
     // operand, rows (f, k1), K-column (n2, c)
@@ -574,7 +561,6 @@ stft2048tc_kernel(const Params p) {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     group_sync(group);
-    SMB_TC_MARK(4)
 
     if (gtid == 0) {
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -589,7 +575,6 @@ stft2048tc_kernel(const Params p) {
     mbar_wait(bar, phase & 1);
     ++phase;
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    SMB_TC_MARK(5)
 
     // ---- D2 row (f = warp, k1 = lane): a[k2] = s Z'[k1 + 32 k2]; real split as in
     // stft2048.cu.  For the complex spectrum the tile's scale is undone here (it
@@ -681,7 +666,6 @@ stft2048tc_kernel(const Params p) {
       }
     }
     group_sync(group);
-    SMB_TC_MARK(6)
 
     if (OUT == kFastMel) {
       // ---- mel projection over the tile's power rows.  A lane carries one piece
@@ -742,7 +726,6 @@ stft2048tc_kernel(const Params p) {
       }
       group_sync(group);
     }
-    SMB_TC_MARK(7)
 
     // ---- write the tile along the frame axis: [batch, rows, frames]
     {
@@ -782,12 +765,7 @@ stft2048tc_kernel(const Params p) {
       }
     }
     group_sync(group);
-    SMB_TC_MARK(8)
   }
-#undef SMB_TC_MARK
-  if (TIMING && gtid == 0)
-    for (int i = 0; i < 9; ++i) atomicAdd(reinterpret_cast<unsigned long long*>(p.timing) + i, (unsigned long long)tacc[i]);
-
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   if (tid < 32)
@@ -851,7 +829,6 @@ cudaError_t launch_stft2048tc(const Stft2048Args& a, int out_kind, int sm_count,
   }
   Params p;
   p.a = a;
-  p.timing = nullptr;
   if (out_kind != kFastMel) { p.a.nnz = 0; p.a.n_mels = 0; p.a.mel_rounds = 0; p.a.mel_mpad = 0; }
   p.span_cap = span_needed(a.g);
   p.region_bytes = region_needed(out_kind, p.a.mel_mpad);
@@ -859,7 +836,6 @@ cudaError_t launch_stft2048tc(const Stft2048Args& a, int out_kind, int sm_count,
   p.tiles_per_signal = (a.g.frames + kTile - 1) / kTile;
   p.total_tiles = p.tiles_per_signal * a.batch;
   int groups = 4;
-  if (const char* e = getenv("SMB_TC_GROUPS")) groups = atoi(e) >= 2 && atoi(e) <= 4 ? atoi(e) : 4;   // experiments
   auto layout = [&](int gr) {
     return smem_layout(out_kind, p.a.n_mels, p.a.nnz, p.a.mel_rounds, p.a.mel_mpad, p.span_cap, gr);
   };
@@ -881,28 +857,6 @@ cudaError_t launch_stft2048tc(const Stft2048Args& a, int out_kind, int sm_count,
   else if (groups == 3) { SMB_LAUNCHTC_G(OUT, SQ, 3) }                                      \
   else { SMB_LAUNCHTC_G(OUT, SQ, 2) }
   const bool sq = a.power == 2.0f;
-  if (getenv("SMB_TC_TIMING") && out_kind == kFastMel && sq && groups == 4 && a.bin_step == 1) {
-    // profiling aid: per-phase cycle totals, printed per launch
-    static long long* d_timing = nullptr;
-    if (!d_timing) cudaMalloc(&d_timing, 9 * sizeof(long long));
-    cudaMemsetAsync(d_timing, 0, 9 * sizeof(long long), st);
-    p.timing = d_timing;
-    e = cudaFuncSetAttribute(stft2048tc_kernel<kFastMel, true, 4, true, true>,
-                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    stft2048tc_kernel<kFastMel, true, 4, true, true><<<grid, 4 * kGroupThreads, smem, st>>>(p);
-    long long h[9];
-    cudaMemcpyAsync(h, d_timing, sizeof(h), cudaMemcpyDeviceToHost, st);
-    cudaStreamSynchronize(st);
-    static const char* names[9] = {"wait", "scale", "build", "mma1", "convert", "mma2", "split", "mel", "write"};
-    long long tot = 0;
-    for (int i = 0; i < 9; ++i) tot += h[i];
-    for (int i = 0; i < 9; ++i)
-      fprintf(stderr, "tc-timing %-8s %8.1f cycles/tile (%4.1f%%)\n", names[i],
-              (double)h[i] / (double)p.total_tiles, 100.0 * (double)h[i] / (double)tot);
-    ++g_launch_count;
-    return cudaGetLastError();
-  }
   if (out_kind == kFastMel) { if (sq) { SMB_LAUNCHTC(kFastMel, true) } else { SMB_LAUNCHTC(kFastMel, false) } }
   else if (out_kind == kFastPower) { if (sq) { SMB_LAUNCHTC(kFastPower, true) } else { SMB_LAUNCHTC(kFastPower, false) } }
   else { SMB_LAUNCHTC(kFastComplex, true) }

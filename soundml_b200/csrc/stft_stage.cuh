@@ -147,9 +147,9 @@ __device__ __forceinline__ bool stage_tile(const FrameGeom& g, const float* x, c
 // The launcher's side of BulkRule: full tile t reads source samples
 // [t*TILE*hop - left, ... + span): inside the clip, and 16-byte aligned when
 // (x/4 + b*n - left) % 4 == 0 (TILE*hop is a multiple of 4).
-inline BulkRule bulk_rule(const float* x, const FrameGeom& g, int tile, bool enabled) {
+inline BulkRule bulk_rule(const float* x, const FrameGeom& g, int tile) {
   BulkRule r{0, -1, 0u, 0u, 0u};
-  if (!enabled || (g.hop & 3) != 0 || (reinterpret_cast<size_t>(x) & 3) != 0) return r;
+  if ((g.hop & 3) != 0 || (reinterpret_cast<size_t>(x) & 3) != 0) return r;
   const long long th = (long long)tile * g.hop, span = (long long)(tile - 1) * g.hop + 2048;
   const long long lo = (g.left + th - 1) / th;
   long long hi = g.n + g.left - span >= 0 ? (g.n + g.left - span) / th : -1;

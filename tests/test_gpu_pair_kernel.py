@@ -139,13 +139,18 @@ def test_tail_tiles_and_unaligned_clips(sb, frames):
         assert peak_rel_err(got[b], ref[b]) <= FLOAT32_CLASS, (frames, b)
 
 
-def test_bulk_copy_and_cp_async_staging_agree_bitwise(sb, monkeypatch):
-    x = np.stack([_signal(60000, s) for s in range(4)])
+def test_bulk_copy_and_cp_async_staging_agree_bitwise(sb):
+    """Each signal four times over, in clips of n = 1 mod 4 samples: the copies start
+    at every 4-byte phase of a 16-byte line, so the interior tiles of one copy come by
+    bulk copy and those of the other three by cp.async (8-byte requests at one phase,
+    4-byte at two)."""
+    x = np.repeat(np.stack([_signal(60001, s) for s in range(4)]), 4, axis=0)
     c = sb.Stft.Config.create(fft_size=2048, hop=512).set_path("pair")
     mc, _ = _mel(sb)
-    got = sb.mel_spectrogram(c, mc, x)
-    monkeypatch.setenv("SMB_NO_BULK", "1")
-    assert np.array_equal(sb.mel_spectrogram(c, mc, x), got)
+    got = sb.mel_spectrogram(c, mc, x).reshape(4, 4, 128, -1)
+    for s in range(4):
+        for phase in range(1, 4):
+            assert np.array_equal(got[s, phase], got[s, 0]), (s, phase)
 
 
 @pytest.mark.parametrize("window,win_length,scale", [

@@ -36,8 +36,7 @@ pytestmark = pytest.mark.gpu
 
 U = 2.0 ** -24
 TINY = 2.0 ** -126
-SWITCHES = ("SMB_ROWS_SPLIT", "SMB_ROWS_SMEM_A", "SMB_ROWS_TMEM_A", "SMB_GEMM_WINDOWS", "SMB_ROWS_ALIGN",
-            "SMB_ROWS_DEBUG")
+SWITCHES = ("SMB_ROWS_SPLIT", "SMB_ROWS_SMEM_A", "SMB_ROWS_TMEM_A", "SMB_GEMM_WINDOWS")
 
 # (sample_rate, target, quality, the layout Config.layout(0) reports on a B200 under the default
 # switches, one entry per column group).  tools/resample_layouts.py sweeps ~1600 gemm-tagged

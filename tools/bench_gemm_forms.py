@@ -38,20 +38,13 @@ def main():
         os.environ["SMB_GEMM_WINDOWS"] = "1"
         win_ms = run(cfg, x, out)
         os.environ.pop("SMB_GEMM_WINDOWS", None)
-        knobs = {}
-        if "--knobs" in sys.argv:
-            for name, bits in [("no_mma", 1), ("no_b", 2), ("no_a", 4), ("no_epilogue", 8), ("no_mma_no_b", 3),
-                               ("only_epilogue", 7), ("nothing", 15)]:
-                os.environ["SMB_ROWS_DEBUG"] = str(bits)
-                knobs[name] = round(run(cfg, x, out.clone()), 3)
-            os.environ.pop("SMB_ROWS_DEBUG", None)
         diff = float((got - out).abs().max() / out.abs().max())
         gb = (x.numel() + out.numel()) * 4 / 1e9
         print(json.dumps({"pair": f"{sr}->{target}", "clips": clips, "plan": cfg.pp(),
                           "rows_ms": round(rows_ms, 3), "windows_ms": round(win_ms, 3),
                           "rows_hbm_frac": round(gb / (rows_ms * 1e-3) / peak, 3),
                           "windows_hbm_frac": round(gb / (win_ms * 1e-3) / peak, 3),
-                          "max_diff_of_peak": diff, **({"rows_ms_with": knobs} if knobs else {})}), flush=True)
+                          "max_diff_of_peak": diff}), flush=True)
         del x, out, got
 
 

@@ -1,10 +1,9 @@
 """The mel projection as the dense GEMM north_star names (Nx.matmul in mel.ml:231), measured:
 cuBLAS through torch.matmul on a materialised power spectrogram [1024, 1025, 431] -- float32
 and tf32 tensor cores -- beside the library's sparse band product (Mel.apply, standalone) and
-the increment the projection costs inside the fused frame-pair kernel.  One GPU.
+the whole mel spectrogram in the fused frame-pair kernel.  One GPU.
 python tools/bench_mel_gemm.py"""
 import json
-import os
 import sys
 
 import torch
@@ -41,15 +40,12 @@ def main():
     res["cublas_tf32_max_err_of_peak"] = float((out - ref).abs().max() / ref.abs().max())
     res["band_product_ms"] = timed(lambda: sb.Mel.apply(mel, p))
     res["band_product_max_err_of_peak"] = float((sb.Mel.apply(mel, p) - ref).abs().max() / ref.abs().max())
-    # inside the fused kernel: the whole mel spectrogram against the same kernel without its mel phase
+    # the fused kernel: audio to mel spectrogram, the power spectrogram never materialised
     del p, out, ref
     stft = sb.Stft.Config.create(fft_size=2048, hop=512)
     x = torch.rand((clips, 220500), device="cuda") * 2 - 1
     o = torch.empty((clips, n_mels, sb.Stft.frames(stft, 220500)), device="cuda")
     res["fused_mel_spectrogram_ms"] = timed(lambda: sb.mel_spectrogram(stft, mel, x, out=o), 50)
-    os.environ["SMB_PAIR_SKIP_MEL"] = "1"
-    res["fused_without_mel_phase_ms"] = timed(lambda: sb.mel_spectrogram(stft, mel, x, out=o), 50)
-    os.environ.pop("SMB_PAIR_SKIP_MEL")
     res["power_spectrogram_materialised_ms"] = None
     ps = torch.empty((clips, bins, sb.Stft.frames(stft, 220500)), device="cuda")
     res["power_spectrogram_materialised_ms"] = timed(lambda: sb.Stft.power_spectrum(stft, x, out=ps))

@@ -2,7 +2,6 @@ set -x
 # headline bench line (default path) and the tensor-core path beside it
 timeout 300 python bench.py > gpurun_out/bench_line.json 2> gpurun_out/bench_err.log
 timeout 300 python bench.py --path tensor --no-e2e --cpu-seconds 2 > gpurun_out/bench_line_tensor.json 2> gpurun_out/bench_tensor_err.log
-SMB_TC_TIMING=1 timeout 120 python bench.py --path tensor --no-e2e --steps 3 --warmup 3 --cpu-seconds 0.5 2>&1 | grep tc-timing | tail -9 > gpurun_out/tc_phase_cycles.txt
 # launch lists (cold-cache, serialised: shares only)
 timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -k regex:stft2048 -c 20 --csv --log-file gpurun_out/launches.csv python bench.py --steps 10 --warmup 3 --no-e2e --cpu-seconds 0.5 > gpurun_out/launches.log 2>&1
 timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -k regex:stft2048 -c 20 --csv --log-file gpurun_out/launches_tensor.csv python bench.py --path tensor --steps 10 --warmup 3 --no-e2e --cpu-seconds 0.5 > gpurun_out/launches_tensor.log 2>&1

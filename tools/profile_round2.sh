@@ -10,7 +10,6 @@ timeout 120 python bench.py --path tensor --no-e2e --no-secondary --cpu-seconds 
 timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -k regex:'stft2048|to_db|mfcc|resample|ols|fir' -c 60 --csv --log-file $O/r2_launches_bench.csv python bench.py --steps 10 --warmup 3 --no-e2e --no-secondary --cpu-seconds 0.3 > $O/r2_launches.log 2>&1
 # full capture of the headline kernel
 timeout 200 ncu --set full --clock-control none --import-source on -k regex:stft2048p -s 3 -c 1 -o $O/r2_pair python bench.py --steps 3 --warmup 3 --no-e2e --no-secondary --cpu-seconds 0.3 > $O/r2_ncu.log 2>&1
-timeout 100 python tools/bench_pair_variants.py > $O/r2_pair_variants.json 2>> $O/r2_bench_err.log
 timeout 400 python bench_extra.py > $O/r2_bench_extra.jsonl 2>> $O/r2_bench_err.log
 timeout 300 python tools/bench_resample_pairs.py > $O/r2_resample_pairs.jsonl 2>> $O/r2_bench_err.log
 timeout 300 python tools/bench_direct.py > $O/r2_direct_kernel.jsonl 2>> $O/r2_bench_err.log
