@@ -1,7 +1,6 @@
 // C ABI of libsoundml_b200.so (see include/soundml_b200.h).
 //
-// Plans own: the host-side design (window / weights / filter banks, double),
-// its device copies, a CUDA stream, and staging buffers for host-memory calls.
+// Every device table, stream, event and staging buffer is held by a unique_ptr owner.
 // Preconditions are checked in the reference's order and with its messages
 // (SMB_EINVAL = Invalid_argument); CUDA failures are SMB_ECUDA.  There is no
 // CPU execution path in this library.
@@ -13,6 +12,7 @@
 #include <cmath>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/soundml_b200.h"
@@ -61,41 +61,81 @@ void require_device() {
         "soundml_b200: no CUDA device is available (this library has no CPU fallback)");
 }
 
+// Owners of CUDA resources.  The deleters ignore errors: teardown has no one to report to.
+struct DeviceFree {
+  void operator()(void* p) const { cudaFree(p); }
+};
+struct PinnedFree {
+  void operator()(void* p) const { cudaFreeHost(p); }
+};
+struct StreamOrderedFree {                      // cudaMallocAsync scratch, freed on its stream
+  cudaStream_t st = nullptr;
+  void operator()(void* p) const { cudaFreeAsync(p, st); }
+};
+struct StreamDestroy {
+  void operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+};
+struct EventDestroy {
+  void operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+};
+template <typename T>
+using device_ptr = std::unique_ptr<T, DeviceFree>;
+using pinned_ptr = std::unique_ptr<void, PinnedFree>;
+using scratch_ptr = std::unique_ptr<void, StreamOrderedFree>;
+using stream_ptr = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using event_ptr = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+
+template <typename T = void>
+device_ptr<T> device_alloc(size_t bytes) {
+  void* p = nullptr;
+  CK(cudaMalloc(&p, bytes));
+  return device_ptr<T>(static_cast<T*>(p));
+}
+scratch_ptr scratch_alloc(size_t bytes, cudaStream_t st) {
+  void* p = nullptr;
+  CK(cudaMallocAsync(&p, bytes, st));
+  return scratch_ptr(p, StreamOrderedFree{st});
+}
+stream_ptr new_stream() {
+  cudaStream_t s = nullptr;
+  CK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+  return stream_ptr(s);
+}
+event_ptr new_event() {
+  cudaEvent_t e = nullptr;
+  CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  return event_ptr(e);
+}
+
 // A device buffer that only ever grows.
 struct DeviceBuffer {
-  void* ptr = nullptr;
+  device_ptr<void> ptr;
   size_t cap = 0;
   void* ensure(size_t bytes) {
     if (bytes > cap) {
-      if (ptr) cudaFree(ptr);
-      ptr = nullptr;
+      ptr.reset();
       cap = 0;
-      CK(cudaMalloc(&ptr, bytes));
+      ptr = device_alloc(bytes);
       cap = bytes;
     }
-    return ptr;
-  }
-  void release() {
-    if (ptr) cudaFree(ptr);
-    ptr = nullptr;
-    cap = 0;
+    return ptr.get();
   }
 };
 
 template <typename T>
-T* upload(const std::vector<T>& v) {
-  T* d = nullptr;
-  if (v.empty()) return d;
-  CK(cudaMalloc(&d, v.size() * sizeof(T)));
-  CK(cudaMemcpy(d, v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
+device_ptr<T> upload(const std::vector<T>& v) {
+  if (v.empty()) return nullptr;
+  device_ptr<T> d = device_alloc<T>(v.size() * sizeof(T));
+  CK(cudaMemcpy(d.get(), v.data(), v.size() * sizeof(T), cudaMemcpyHostToDevice));
   return d;
 }
 
 struct StreamOwner {
-  cudaStream_t own = nullptr, use = nullptr;
+  stream_ptr own;
+  cudaStream_t use = nullptr;
   void create() {
-    CK(cudaStreamCreateWithFlags(&own, cudaStreamNonBlocking));
-    use = own;
+    own = new_stream();
+    use = own.get();
   }
   // SMB_STREAM_OWN restores the plan's stream; anything else (NULL = the CUDA
   // default stream) is used as given.  Plans own scratch (the generic mel path's power
@@ -106,7 +146,7 @@ struct StreamOwner {
   // been synchronised before it was destroyed (cudaErrorInvalidResourceHandle from a
   // stream already gone is swallowed: nothing can be pending on it).
   void set(void* external) {
-    cudaStream_t next = external == SMB_STREAM_OWN ? own : (cudaStream_t)external;
+    cudaStream_t next = external == SMB_STREAM_OWN ? own.get() : (cudaStream_t)external;
     if (next != use) {
       const cudaError_t e = cudaStreamSynchronize(use);
       if (e != cudaSuccess) {
@@ -116,10 +156,6 @@ struct StreamOwner {
     }
     use = next;
   }
-  void destroy() {
-    if (own) cudaStreamDestroy(own);
-    own = use = nullptr;
-  }
 };
 
 // Host-memory calls stage the batch through the device in slices on three
@@ -128,63 +164,51 @@ struct StreamOwner {
 // With pageable host memory the copies degrade to synchronous staging; pinned
 // memory (smb_host_alloc_pinned) gets the full overlap.
 struct HostPipe {
-  cudaStream_t h2d = nullptr, d2h = nullptr;
-  cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_run[2] = {nullptr, nullptr},
-              ev_out[2] = {nullptr, nullptr};
-  DeviceBuffer in[2], out[2];
-  bool ready = false;
-  void ensure() {
-    if (ready) return;
-    CK(cudaStreamCreateWithFlags(&h2d, cudaStreamNonBlocking));
-    CK(cudaStreamCreateWithFlags(&d2h, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-      CK(cudaEventCreateWithFlags(&ev_in[i], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&ev_run[i], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&ev_out[i], cudaEventDisableTiming));
-    }
-    ready = true;
-  }
-  void release() {
-    for (int i = 0; i < 2; ++i) {      // the buffers may have been used without the streams (smb_mfcc)
-      in[i].release();
-      out[i].release();
-    }
-    if (!ready) return;
-    for (int i = 0; i < 2; ++i) {
-      cudaEventDestroy(ev_in[i]);
-      cudaEventDestroy(ev_run[i]);
-      cudaEventDestroy(ev_out[i]);
-    }
-    cudaStreamDestroy(h2d);
-    cudaStreamDestroy(d2h);
-    ready = false;
-  }
+  struct Streams {
+    stream_ptr h2d, d2h;
+    event_ptr ev_in[2], ev_run[2], ev_out[2];
+  };
+  std::unique_ptr<Streams> streams;  // created by the first host-memory call
+  DeviceBuffer in[2], out[2];        // (smb_mfcc also stages through in[0], without the streams)
   // run(din, dout, items) enqueues the kernels for `items` batch items on `compute`.
   template <typename Run>
   void execute(cudaStream_t compute, const void* x, void* out_host, int64_t batch,
                size_t in_item, size_t out_item, Run&& run) {
-    ensure();
+    if (!streams) {
+      auto s = std::make_unique<Streams>();
+      s->h2d = new_stream();
+      s->d2h = new_stream();
+      for (int i = 0; i < 2; ++i) {
+        s->ev_in[i] = new_event();
+        s->ev_run[i] = new_event();
+        s->ev_out[i] = new_event();
+      }
+      streams = std::move(s);
+    }
+    cudaStream_t h2d = streams->h2d.get(), d2h = streams->d2h.get();
     const size_t slice_bytes = (size_t)64 << 20;
     int64_t per = (int64_t)(slice_bytes / std::max<size_t>(1, in_item + out_item));
     per = std::max<int64_t>(1, std::min<int64_t>(per, batch));
     const int64_t slices = (batch + per - 1) / per;
     for (int64_t i = 0; i < slices; ++i) {
       const int slot = (int)(i & 1);
+      cudaEvent_t ev_in = streams->ev_in[slot].get(), ev_run = streams->ev_run[slot].get(),
+                  ev_out = streams->ev_out[slot].get();
       const int64_t b0 = i * per, nb = std::min<int64_t>(per, batch - b0);
       void* din = in[slot].ensure((size_t)per * in_item);
       void* dout = out[slot].ensure((size_t)per * out_item);
-      if (i >= 2) CK(cudaStreamWaitEvent(h2d, ev_run[slot], 0));      // input slot consumed
+      if (i >= 2) CK(cudaStreamWaitEvent(h2d, ev_run, 0));      // input slot consumed
       CK(cudaMemcpyAsync(din, (const char*)x + (size_t)b0 * in_item, (size_t)nb * in_item,
                          cudaMemcpyHostToDevice, h2d));
-      CK(cudaEventRecord(ev_in[slot], h2d));
-      CK(cudaStreamWaitEvent(compute, ev_in[slot], 0));
-      if (i >= 2) CK(cudaStreamWaitEvent(compute, ev_out[slot], 0));  // output slot drained
+      CK(cudaEventRecord(ev_in, h2d));
+      CK(cudaStreamWaitEvent(compute, ev_in, 0));
+      if (i >= 2) CK(cudaStreamWaitEvent(compute, ev_out, 0));  // output slot drained
       run(din, dout, nb);
-      CK(cudaEventRecord(ev_run[slot], compute));
-      CK(cudaStreamWaitEvent(d2h, ev_run[slot], 0));
+      CK(cudaEventRecord(ev_run, compute));
+      CK(cudaStreamWaitEvent(d2h, ev_run, 0));
       CK(cudaMemcpyAsync((char*)out_host + (size_t)b0 * out_item, dout, (size_t)nb * out_item,
                          cudaMemcpyDeviceToHost, d2h));
-      CK(cudaEventRecord(ev_out[slot], d2h));
+      CK(cudaEventRecord(ev_out, d2h));
     }
     CK(cudaStreamSynchronize(d2h));
     CK(cudaStreamSynchronize(compute));
@@ -218,40 +242,45 @@ void same_device(int bound) {
 struct smb_stft_plan {
   smb::StftGeometry geom;
   std::vector<double> window;        // analysis window, fft doubles
-  bool device_ready = false;
-  int device = 0, sm_count = 0, path = SMB_PATH_AUTO;
-  StreamOwner stream;
-  double* d_window64 = nullptr;
-  double2* d_twiddle64 = nullptr;
-  double* d_folded = nullptr;        // synthesis: folded squared window, one entry per residue
-  float* d_window_inv = nullptr;     // synthesis fast path: window / 2048
-  float* d_window32 = nullptr;       // fast path tables (fft 2048 only)
-  float2* d_tw_pass = nullptr;
-  float2* d_tw_post = nullptr;
-  void* d_dft_images = nullptr;      // tensor-core kernel: split-fp16 images of the 32-point DFT
+  int path = SMB_PATH_AUTO;
+  // Everything the plan has on its device; null until the first device call.
+  struct Device {
+    int device = 0, sm_count = 0;
+    StreamOwner stream;
+    device_ptr<double> d_window64;
+    device_ptr<double2> d_twiddle64;
+    device_ptr<double> d_folded;       // synthesis: folded squared window, one entry per residue
+    device_ptr<float> d_window_inv;    // synthesis fast path: window / 2048
+    device_ptr<float> d_window32;      // fast path tables (fft 2048 only)
+    device_ptr<float2> d_tw_pass;
+    device_ptr<float2> d_tw_post;
+    device_ptr<__half> d_dft_images;   // tensor-core kernel: split-fp16 images of the 32-point DFT
+  };
+  std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   HostPipe pipe;
   DeviceBuffer tmp;        // power spectrogram of the generic mel path
   DeviceBuffer cepstral;   // mel spectrogram (+ host-call output) of the MFCC path
 
   void ensure_device() {
-    if (device_ready) return same_device(device);
+    if (dev) return same_device(dev->device);
     require_device();
-    CK(cudaGetDevice(&device));
-    CK(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, device));
-    stream.create();
-    d_window64 = upload(window);
+    auto d = std::make_unique<Device>();
+    CK(cudaGetDevice(&d->device));
+    CK(cudaDeviceGetAttribute(&d->sm_count, cudaDevAttrMultiProcessorCount, d->device));
+    d->stream.create();
+    d->d_window64 = upload(window);
     const int64_t n = geom.fft;
     std::vector<double2> tw((size_t)n);
     for (int64_t j = 0; j < n; ++j) {
       const double a = kTwoPi * double(j) / double(n);
       tw[(size_t)j] = make_double2(std::cos(a), -std::sin(a));
     }
-    d_twiddle64 = upload(tw);
+    d->d_twiddle64 = upload(tw);
     if (fast_step() > 0) {
       // shorter frames run zero-padded to 2048: the window's tail is zero
       std::vector<float> w32(2048, 0.0f);
       for (int64_t j = 0; j < n; ++j) w32[(size_t)j] = (float)window[(size_t)j];
-      d_window32 = upload(w32);
+      d->d_window32 = upload(w32);
       std::vector<float2> pass(1024), post(512);
       for (int k1 = 0; k1 < 32; ++k1)
         for (int n2 = 0; n2 < 32; ++n2) {
@@ -263,8 +292,8 @@ struct smb_stft_plan {
           const double a = kTwoPi * double(l + 32 * j) / 2048.0;
           post[(size_t)(j * 32 + l)] = make_float2((float)std::cos(a), (float)-std::sin(a));
         }
-      d_tw_pass = upload(pass);
-      d_tw_post = upload(post);
+      d->d_tw_pass = upload(pass);
+      d->d_tw_post = upload(post);
       // The 32-point DFT in real arithmetic, F[n = (k, c')][j = (m, c)] with
       // (re, im) interleaved: out_re = sum in_re cos + in_im sin, out_im = sum
       // in_im cos - in_re sin (angle 2 pi m k / 32).  Two fp16 images (leading 11
@@ -282,9 +311,9 @@ struct smb_stft_plan {
           images[at] = hi;
           images[64 * 64 + at] = lo;
         }
-      d_dft_images = upload(images);
+      d->d_dft_images = upload(images);
     }
-    device_ready = true;
+    dev = std::move(d);
   }
   // stft.ml:712-721: position m receives w[j]^2 for the j congruent to m modulo the hop
   std::vector<double> folded_square_window() const {
@@ -322,25 +351,9 @@ struct smb_stft_plan {
     g.pad_value = geom.pad_value;
     return g;
   }
-  ~smb_stft_plan() {
-    if (!device_ready) return;
-    cudaFree(d_window64);
-    cudaFree(d_twiddle64);
-    cudaFree(d_folded);
-    cudaFree(d_window_inv);
-    cudaFree(d_window32);
-    cudaFree(d_tw_pass);
-    cudaFree(d_tw_post);
-    cudaFree(d_dft_images);
-    pipe.release();
-    tmp.release();
-    cepstral.release();
-    stream.destroy();
-  }
 };
 
 struct smb_mel_plan {
-  int bound_device = 0;              // the device the tables live on (first use)
   int64_t n_mels = 0, fft = 0, bins = 0, sample_rate = 0;
   double f_min = 0, f_max = 0;
   int scale = 0, norm = 0;
@@ -353,12 +366,13 @@ struct smb_mel_plan {
     std::vector<smb::MelPiece> pieces;     // [warps][rounds][32]
     std::vector<unsigned char> pcnt;       // [n_mels]: pieces (= partial sums) of each filter, 1..4
     int rounds = 0, mpad = 0;              // partial-sum slot of (piece j, filter m) = j * mpad + m
-    float* d_vals = nullptr;
-    smb::MelPiece* d_pieces = nullptr;
-    unsigned char* d_pcnt = nullptr;
+    struct Tables {
+      device_ptr<float> d_vals;
+      device_ptr<smb::MelPiece> d_pieces;
+      device_ptr<unsigned char> d_pcnt;
+    };
     void clear() { vals.clear(); pieces.clear(); pcnt.clear(); rounds = mpad = 0; }
-    void to_device() { d_vals = upload(vals); d_pieces = upload(pieces); d_pcnt = upload(pcnt); }
-    void free_device() { cudaFree(d_vals); cudaFree(d_pieces); cudaFree(d_pcnt); }
+    Tables to_device() const { return {upload(vals), upload(pieces), upload(pcnt)}; }
   };
   // Mel schedule of the frame-pair kernel (stft2048p.cu): whole filters, eight per
   // round, a lane = (filter, frame pair); rounds dealt to the group's four warps.
@@ -366,11 +380,12 @@ struct smb_mel_plan {
     std::vector<float> w;                  // [round][step][8 filters] x float4
     std::vector<smb::PairMelItem> items;   // [4 warps][rounds][8]
     int rounds = 0;
-    float* d_w = nullptr;
-    smb::PairMelItem* d_items = nullptr;
+    struct Tables {
+      device_ptr<float> d_w;
+      device_ptr<smb::PairMelItem> d_items;
+    };
     void clear() { w.clear(); items.clear(); rounds = 0; }
-    void to_device() { if (!items.empty()) { d_w = upload(w); d_items = upload(items); } }
-    void free_device() { cudaFree(d_w); cudaFree(d_items); }
+    Tables to_device() const { return items.empty() ? Tables{} : Tables{upload(w), upload(items)}; }
   };
   PairSchedule sched_pair;
   PieceSchedule sched_cc;   // CUDA-core kernel: kFastTile warps, 8 frames per lane
@@ -378,18 +393,24 @@ struct smb_mel_plan {
   // 2048 / fft_size when the fused kernel can carry this filterbank (1 for fft
   // 2048, 2 for 1024, ...), else 0
   int fast_step = 0;
-  bool device_ready = false;
-  StreamOwner stream;
-  double* d_weights = nullptr;
-  int *d_band_lo = nullptr, *d_band_hi = nullptr;
+  // Everything the plan has on its device; null until the first device call.
+  struct Device {
+    int device = 0;
+    StreamOwner stream;
+    device_ptr<double> d_weights;
+    device_ptr<int> d_band_lo, d_band_hi;
+    PairSchedule::Tables pair;
+    PieceSchedule::Tables cc, tc;
+    // MFCC epilogue: DCT table of the last (n_mfcc, lifter) asked for, max scratch
+    device_ptr<double> d_dct;
+    device_ptr<unsigned long long> d_max;
+  };
+  std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   DeviceBuffer in, out;
-  // MFCC epilogue: DCT table of the last (n_mfcc, lifter) asked for, max scratch
-  double* d_dct = nullptr;
-  unsigned long long* d_max = nullptr;
   int64_t dct_n_mfcc = -1;
   double dct_lifter = -1.0;
   const double* dct_table(int64_t n_mfcc, double lifter) {
-    if (d_dct && dct_n_mfcc == n_mfcc && dct_lifter == lifter) return d_dct;
+    if (dev->d_dct && dct_n_mfcc == n_mfcc && dct_lifter == lifter) return dev->d_dct.get();
     // raw DCT-II rows 2 cos(pi k (2m+1) / 2N), orthonormal scales and lifter folded
     // in (soundml.ml:26-43, 84-93), all in double
     std::vector<double> t((size_t)(n_mfcc * n_mels));
@@ -401,11 +422,10 @@ struct smb_mel_plan {
         t[(size_t)(k * n_mels + m)] =
             2.0 * std::cos(pi * double(k) * double(2 * m + 1) / (2.0 * double(n_mels))) * w;
     }
-    cudaFree(d_dct);
-    d_dct = upload(t);
+    dev->d_dct = upload(t);
     dct_n_mfcc = n_mfcc;
     dct_lifter = lifter;
-    return d_dct;
+    return dev->d_dct.get();
   }
 
   void finish_host() {
@@ -651,41 +671,28 @@ struct smb_mel_plan {
     return true;
   }
   void ensure_device() {
-    if (device_ready) return same_device(bound_device);
+    if (dev) return same_device(dev->device);
     require_device();
-    CK(cudaGetDevice(&bound_device));
-    stream.create();
-    d_weights = upload(weights);
-    d_band_lo = upload(band_lo);
-    d_band_hi = upload(band_hi);
-    sched_cc.to_device();
-    sched_tc.to_device();
-    sched_pair.to_device();
-    CK(cudaMalloc(&d_max, sizeof(unsigned long long)));
-    device_ready = true;
-  }
-  ~smb_mel_plan() {
-    if (!device_ready) return;
-    cudaFree(d_weights);
-    cudaFree(d_band_lo);
-    cudaFree(d_band_hi);
-    sched_cc.free_device();
-    sched_tc.free_device();
-    sched_pair.free_device();
-    cudaFree(d_dct);
-    cudaFree(d_max);
-    in.release();
-    out.release();
-    stream.destroy();
+    auto d = std::make_unique<Device>();
+    CK(cudaGetDevice(&d->device));
+    d->stream.create();
+    d->d_weights = upload(weights);
+    d->d_band_lo = upload(band_lo);
+    d->d_band_hi = upload(band_hi);
+    d->cc = sched_cc.to_device();
+    d->tc = sched_tc.to_device();
+    d->pair = sched_pair.to_device();
+    d->d_max = device_alloc<unsigned long long>(sizeof(unsigned long long));
+    dev = std::move(d);
   }
 };
 
 // Device copies of one overlap-save plan.
 struct OlsDevice {
   smb::OlsPlan plan;
-  float2* d_h = nullptr;
-  float2* d_tw = nullptr;
-  float2 *d_tw_pass = nullptr, *d_tw_base = nullptr;   // tables of the N = 2048 kernel
+  device_ptr<float2> d_h;
+  device_ptr<float2> d_tw;
+  device_ptr<float2> d_tw_pass, d_tw_base;             // tables of the N = 2048 kernel
   int sm_count = 0;
   bool fast = true;                                     // the N = 2048 kernel may be used
   void upload_from(const smb::OlsPlan& p) {
@@ -720,13 +727,6 @@ struct OlsDevice {
     }
     d_tw = upload(tw);
   }
-  void release() {
-    cudaFree(d_h);
-    cudaFree(d_tw);
-    cudaFree(d_tw_pass);
-    cudaFree(d_tw_base);
-    d_h = d_tw = d_tw_pass = d_tw_base = nullptr;
-  }
   void run(const float* x, int64_t batch, int64_t n, int64_t n_out, float* out,
            cudaStream_t st) const {
     smb::OlsArgs a{};
@@ -737,11 +737,11 @@ struct OlsDevice {
     a.blocks = plan.blocks_for(n_out);
     a.L = (int)plan.l; a.M = (int)plan.m; a.K = (int)plan.k;
     a.N = (int)plan.n; a.B = (int)plan.b; a.delta = (int)plan.delta; a.W = (int)plan.w;
-    a.H = d_h;
-    a.tw = d_tw;
+    a.H = d_h.get();
+    a.tw = d_tw.get();
     a.polyphase = plan.polyphase ? 1 : 0;
     if (fast && d_tw_pass && smb::ols2048_supports(a))
-      CK(smb::launch_ols2048(a, d_tw_pass, d_tw_base, batch, sm_count, st));
+      CK(smb::launch_ols2048(a, d_tw_pass.get(), d_tw_base.get(), batch, sm_count, st));
     else if (plan.full_inverse || plan.polyphase)
       throw smb::invalid_argument("soundml_b200: this overlap-save plan needs the N = 2048 kernel");
     else
@@ -756,8 +756,8 @@ struct GemmDevice {
   // three accumulators of a group must fit the 512 TMEM columns.
   struct Group {
     int col_begin = 0, width = 0, n_pad = 0, chunk_begin = 0, chunks = 0, tmem_cols = 0;
-    float* d_images = nullptr;
-    int4* d_meta = nullptr;
+    device_ptr<float> d_images;
+    device_ptr<int4> d_meta;
   };
   bool ok = false;
   std::vector<Group> groups;
@@ -767,19 +767,10 @@ struct GemmDevice {
   int rows_sm_count = 0;
   struct RowsGroup {
     smb::GemmRowsArgs a{};
-    float* d_images = nullptr;
-    int4 *d_chunks = nullptr, *d_slices = nullptr;
+    device_ptr<float> d_images;
+    device_ptr<int4> d_chunks, d_slices;
   };
   std::vector<RowsGroup> rows_groups;            // one launch per group of <= 160 columns
-  void release_rows() {
-    for (RowsGroup& g : rows_groups) {
-      cudaFree(g.d_images);
-      cudaFree(g.d_chunks);
-      cudaFree(g.d_slices);
-    }
-    rows_groups.clear();
-    rows_ok = false;
-  }
   // columns [c0, c0 + l) of the stage's L (l_total below)
   // split_main: the row grid is shifted so that every column's filter centre falls into the
   // same shift (qc), and that shift's two small split terms get an accumulator of their own:
@@ -985,11 +976,11 @@ struct GemmDevice {
     g.d_images = upload(img);
     g.d_chunks = upload(chunk_meta);
     g.d_slices = upload(slice_meta);
-    a.b_images = g.d_images;
-    a.chunk_meta = g.d_chunks;
-    a.slice_meta = g.d_slices;
+    a.b_images = g.d_images.get();
+    a.chunk_meta = g.d_chunks.get();
+    a.slice_meta = g.d_slices.get();
     g.a = a;
-    rows_groups.push_back(g);
+    rows_groups.push_back(std::move(g));
     return true;
   }
   void build_rows(const smb::ResampleStage& s) {
@@ -1006,7 +997,7 @@ struct GemmDevice {
         rows_ok = true;
         return;
       }
-      release_rows();
+      rows_groups.clear();
     }
   }
   void build(const smb::ResampleStage& s) {
@@ -1078,56 +1069,52 @@ struct GemmDevice {
       }
       g.d_meta = upload(meta);
       g.d_images = upload(img);
-      groups.push_back(g);
+      groups.push_back(std::move(g));
     }
     ok = true;
-  }
-  void release() {
-    for (Group& g : groups) {
-      cudaFree(g.d_images);
-      cudaFree(g.d_meta);
-    }
-    groups.clear();
-    release_rows();
   }
 };
 
 struct smb_resample_plan {
-  int bound_device = 0;              // the device the tables live on (first use)
   smb::ResamplePlan plan;
-  bool device_ready = false;
-  StreamOwner stream;
-  std::vector<float*> d_bank;        // per stage, [l][2k+1] float32
-  std::vector<double*> d_bank64;     // the same banks uncast, for float64 audio
-  std::vector<OlsDevice> ols;        // per stage; plan.ok only for OLS-tagged power-of-two stages
-  std::vector<GemmDevice> gemm;      // per stage; ok only for GEMM-tagged stages
+  // Everything the plan has on its device; null until the first device call.
+  struct Device {
+    int device = 0;
+    StreamOwner stream;
+    std::vector<device_ptr<float>> d_bank;     // per stage, [l][2k+1] float32
+    std::vector<device_ptr<double>> d_bank64;  // the same banks uncast, for float64 audio
+    std::vector<OlsDevice> ols;        // per stage; plan.ok only for OLS-tagged power-of-two stages
+    std::vector<GemmDevice> gemm;      // per stage; ok only for GEMM-tagged stages
+  };
+  std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   int executor = SMB_EXEC_PLANNED;   // SMB_EXEC_DIRECT forces the dot-product kernel everywhere
   DeviceBuffer in, out, mid;
   HostPipe pipe;                     // host-memory calls: sliced, copies under kernels
   void ensure_device() {
-    if (device_ready) return same_device(bound_device);
+    if (dev) return same_device(dev->device);
     require_device();
-    CK(cudaGetDevice(&bound_device));
-    stream.create();
+    auto d = std::make_unique<Device>();
+    CK(cudaGetDevice(&d->device));
+    d->stream.create();
     for (const auto& s : plan.stages) {
       std::vector<float> b(s.bank.size());
       for (size_t i = 0; i < b.size(); ++i) b[i] = (float)s.bank[i];   // cast at prepare
-      d_bank.push_back(upload(b));
-      d_bank64.push_back(upload(s.bank));
-      ols.emplace_back();
-      ols.back().upload_from(smb::ols_plan_for_stage(s));
-      gemm.emplace_back();
-      gemm.back().build(s);
+      d->d_bank.push_back(upload(b));
+      d->d_bank64.push_back(upload(s.bank));
+      d->ols.emplace_back();
+      d->ols.back().upload_from(smb::ols_plan_for_stage(s));
+      d->gemm.emplace_back();
+      d->gemm.back().build(s);
     }
-    device_ready = true;
+    dev = std::move(d);
   }
   // The kernel run_stage picks for stage i (SMB_FORM_*).
   int form(size_t i) const {
     if (executor == SMB_EXEC_DIRECT) return SMB_FORM_DIRECT;
-    if (ols[i].plan.ok) return SMB_FORM_OLS;
+    if (dev->ols[i].plan.ok) return SMB_FORM_OLS;
     // (SMB_GEMM_WINDOWS=1: the overlapping-window form, for A/B measurement)
-    if (gemm[i].rows_ok && !getenv("SMB_GEMM_WINDOWS")) return SMB_FORM_ROW;
-    if (gemm[i].ok) return SMB_FORM_WINDOW;
+    if (dev->gemm[i].rows_ok && !getenv("SMB_GEMM_WINDOWS")) return SMB_FORM_ROW;
+    if (dev->gemm[i].ok) return SMB_FORM_WINDOW;
     return SMB_FORM_DIRECT;
   }
   // One stage over device buffers: overlap-save where the planner tagged it and
@@ -1138,18 +1125,18 @@ struct smb_resample_plan {
     const smb::ResampleStage& s = plan.stages[i];
     const int f = form(i);
     if (f == SMB_FORM_OLS) {
-      ols[i].run(x, batch, n, n_out, out, st);
+      dev->ols[i].run(x, batch, n, n_out, out, st);
     } else if (f == SMB_FORM_ROW) {
-      for (const GemmDevice::RowsGroup& g : gemm[i].rows_groups) {
+      for (const GemmDevice::RowsGroup& g : dev->gemm[i].rows_groups) {
         smb::GemmRowsArgs a = g.a;
         a.x = x;
         a.out = out;
         a.n = n;
         a.n_out = n_out;
-        CK(smb::launch_resample_rows(a, batch, gemm[i].rows_sm_count, st));
+        CK(smb::launch_resample_rows(a, batch, dev->gemm[i].rows_sm_count, st));
       }
     } else if (f == SMB_FORM_WINDOW) {
-      for (const GemmDevice::Group& g : gemm[i].groups) {
+      for (const GemmDevice::Group& g : dev->gemm[i].groups) {
         smb::GemmResampleArgs a{};
         a.x = x;
         a.out = out;
@@ -1163,57 +1150,39 @@ struct smb_resample_plan {
         a.n_pad = g.n_pad;
         a.chunks = g.chunks;
         a.tmem_cols = g.tmem_cols;
-        a.b_images = g.d_images;
-        a.chunk_meta = g.d_meta;
+        a.b_images = g.d_images.get();
+        a.chunk_meta = g.d_meta.get();
         CK(smb::launch_resample_gemm(a, batch, st));
       }
     } else
-      CK(smb::launch_polyphase_direct(x, batch, n, d_bank[i], (int)s.l, (int)s.m, (int)s.k,
+      CK(smb::launch_polyphase_direct(x, batch, n, dev->d_bank[i].get(), (int)s.l, (int)s.m, (int)s.k,
                                       n_out, out, st));
-  }
-  ~smb_resample_plan() {
-    if (!device_ready) return;
-    for (float* p : d_bank) cudaFree(p);
-    for (double* p : d_bank64) cudaFree(p);
-    for (OlsDevice& o : ols) o.release();
-    for (GemmDevice& g : gemm) g.release();
-    in.release();
-    out.release();
-    mid.release();
-    pipe.release();
-    stream.destroy();
   }
 };
 
 struct smb_fir_plan {
-  int bound_device = 0;              // the device the tables live on (first use)
   std::vector<double> h;
   int64_t k = 0;
-  bool device_ready = false;
-  StreamOwner stream;
-  float* d_bank = nullptr;
-  OlsDevice ols;
-  DeviceBuffer in, out;
+  // Everything the plan has on its device; null until the first device call.
+  struct Device {
+    int device = 0;
+    StreamOwner stream;
+    device_ptr<float> d_bank;
+    OlsDevice ols;
+  };
+  std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   HostPipe pipe;                     // host-memory calls: sliced, copies under kernels
   void ensure_device() {
-    if (device_ready) return same_device(bound_device);
+    if (dev) return same_device(dev->device);
     require_device();
-    CK(cudaGetDevice(&bound_device));
-    stream.create();
+    auto d = std::make_unique<Device>();
+    CK(cudaGetDevice(&d->device));
+    d->stream.create();
     std::vector<float> b(h.size());
     for (size_t s = 0; s < h.size(); ++s) b[s] = (float)h[h.size() - 1 - s];  // row reversed
-    d_bank = upload(b);
-    ols.upload_from(smb::ols_plan_for_fir(h));
-    device_ready = true;
-  }
-  ~smb_fir_plan() {
-    if (!device_ready) return;
-    cudaFree(d_bank);
-    ols.release();
-    in.release();
-    out.release();
-    pipe.release();
-    stream.destroy();
+    d->d_bank = upload(b);
+    d->ols.upload_from(smb::ols_plan_for_fir(h));
+    dev = std::move(d);
   }
 };
 
@@ -1303,7 +1272,7 @@ int smb_stft_plan_destroy(smb_stft_plan* plan) {
   return guarded([&] { delete plan; });
 }
 int smb_stft_plan_set_stream(smb_stft_plan* plan, void* s) {
-  return guarded([&] { plan->ensure_device(); plan->stream.set(s); });
+  return guarded([&] { plan->ensure_device(); plan->dev->stream.set(s); });
 }
 int smb_stft_plan_set_path(smb_stft_plan* plan, int path) {
   return guarded([&] {
@@ -1313,7 +1282,7 @@ int smb_stft_plan_set_path(smb_stft_plan* plan, int path) {
   });
 }
 int smb_stft_plan_sync(smb_stft_plan* plan) {
-  return guarded([&] { if (plan->device_ready) CK(cudaStreamSynchronize(plan->stream.use)); });
+  return guarded([&] { if (plan->dev) CK(cudaStreamSynchronize(plan->dev->stream.use)); });
 }
 int64_t smb_stft_fft_size(const smb_stft_plan* plan) { return plan->geom.fft; }
 int64_t smb_stft_hop(const smb_stft_plan* plan) { return plan->geom.hop; }
@@ -1418,15 +1387,15 @@ smb::Stft2048PairArgs pair_args(const smb_stft_plan* stft, const smb_mel_plan* m
   a.batch = nb;
   a.g = g;
   a.g.fft = 2048;
-  a.window = stft->d_window32;
-  a.tw_pass = stft->d_tw_pass;
-  a.tw_post = stft->d_tw_post;
+  a.window = stft->dev->d_window32.get();
+  a.tw_pass = stft->dev->d_tw_pass.get();
+  a.tw_post = stft->dev->d_tw_post.get();
   a.power = (float)power;
   if (mel) {
     a.n_mels = (int)mel->n_mels;
-    a.mel_w = mel->sched_pair.d_w;
+    a.mel_w = mel->dev->pair.d_w.get();
     a.mel_w_floats = (int)mel->sched_pair.w.size();
-    a.mel_items = mel->sched_pair.d_items;
+    a.mel_items = mel->dev->pair.d_items.get();
     a.mel_rounds = mel->sched_pair.rounds;
   }
   return a;
@@ -1435,7 +1404,8 @@ smb::Stft2048PairArgs pair_args(const smb_stft_plan* stft, const smb_mel_plan* m
 // x (device) -> spectrum (device).  kind: complex or |X|^power.
 void run_spectrum(smb_stft_plan* p, const void* dx, int64_t batch, const smb::FrameGeom& g,
                   int dtype, SpecKind kind, double power, void* dout) {
-  cudaStream_t st = p->stream.use;
+  const smb_stft_plan::Device& d = *p->dev;
+  cudaStream_t st = d.stream.use;
   const int fast_kind = kind == kSpecComplex ? smb::kFastComplex : smb::kFastPower;
   if (const int which = want_fast(p, dtype, g, fast_kind, nullptr)) {
     smb::Stft2048Args a{};
@@ -1445,15 +1415,15 @@ void run_spectrum(smb_stft_plan* p, const void* dx, int64_t batch, const smb::Fr
     a.g = g;
     a.g.fft = 2048;
     a.bin_step = p->fast_step();
-    a.window = p->d_window32;
-    a.tw_pass = p->d_tw_pass;
-    a.tw_post = p->d_tw_post;
+    a.window = d.d_window32.get();
+    a.tw_pass = d.d_tw_pass.get();
+    a.tw_post = d.d_tw_post.get();
     a.power = (float)power;
-    a.dft_images = p->d_dft_images;
-    if (which == SMB_PATH_TENSOR) CK(smb::launch_stft2048tc(a, fast_kind, p->sm_count, st));
-    else CK(smb::launch_stft2048(a, fast_kind, p->sm_count, st));
+    a.dft_images = d.d_dft_images.get();
+    if (which == SMB_PATH_TENSOR) CK(smb::launch_stft2048tc(a, fast_kind, d.sm_count, st));
+    else CK(smb::launch_stft2048(a, fast_kind, d.sm_count, st));
   } else {
-    CK(smb::launch_stft_generic(dx, dtype, batch, g, p->d_window64, p->d_twiddle64,
+    CK(smb::launch_stft_generic(dx, dtype, batch, g, d.d_window64.get(), d.d_twiddle64.get(),
                                 kind == kSpecComplex ? smb::kModeComplex : smb::kModePower,
                                 power, dout, st));
   }
@@ -1481,7 +1451,7 @@ void spectrum_call(const char* op, smb_stft_plan* p, const void* x, int64_t batc
       (size_t)batch * (size_t)p->geom.bins() * (size_t)g.frames * (kind == kSpecComplex ? 2 : 1);
   if (batch == 0 || g.frames == 0) return;       // frameless spectrum: nothing to write
   p->ensure_device();
-  cudaStream_t st = p->stream.use;
+  cudaStream_t st = p->dev->stream.use;
   if (mem == SMB_MEM_DEVICE) {
     run_spectrum(p, x, batch, g, dtype, kind, power, out);
     return;
@@ -1495,8 +1465,8 @@ void spectrum_call(const char* op, smb_stft_plan* p, const void* x, int64_t batc
 
 void run_mel_apply(smb_mel_plan* m, const void* ds, int64_t batch, int64_t frames, int dtype,
                    void* dout, cudaStream_t st) {
-  CK(smb::launch_mel_apply(ds, dtype, batch, (int)m->bins, frames, (int)m->n_mels, m->d_weights,
-                           m->d_band_lo, m->d_band_hi, dout, st));
+  CK(smb::launch_mel_apply(ds, dtype, batch, (int)m->bins, frames, (int)m->n_mels, m->dev->d_weights.get(),
+                           m->dev->d_band_lo.get(), m->dev->d_band_hi.get(), dout, st));
 }
 
 }  // namespace
@@ -1564,8 +1534,9 @@ int smb_stft_invert(smb_stft_plan* plan, const void* z, int64_t batch, int64_t f
     if (has_length) count = std::min(frames, (length + left + hop - 1) / hop);
     if (batch == 0 || out_len == 0) return;
     p->ensure_device();
-    cudaStream_t st = p->stream.use;
-    if (!p->d_folded) p->d_folded = upload(p->folded_square_window());
+    smb_stft_plan::Device& d = *p->dev;
+    cudaStream_t st = d.stream.use;
+    if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
     auto run = [&](const void* dz, void* dout, int64_t nb) {
       if (count == 0) {                                 // nothing reaches the output: zeros
         CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * osz, st));
@@ -1580,9 +1551,9 @@ int smb_stft_invert(smb_stft_plan* plan, const void* z, int64_t batch, int64_t f
       a.fft = (int)p->geom.fft;
       a.hop = (int)hop;
       a.left = (int)left;
-      a.window = p->d_window64;
-      a.twiddle = p->d_twiddle64;
-      a.folded = p->d_folded;
+      a.window = d.d_window64.get();
+      a.twiddle = d.d_twiddle64.get();
+      a.folded = d.d_folded.get();
       a.in_f64 = in_dtype == SMB_F64;
       a.out_f64 = out_dtype == SMB_F64;
       const bool fast = p->path != SMB_PATH_GENERIC && smb::istft2048_supports(a);
@@ -1590,15 +1561,15 @@ int smb_stft_invert(smb_stft_plan* plan, const void* z, int64_t batch, int64_t f
         throw smb::invalid_argument(
             "soundml_b200: the fft-2048 synthesis kernel does not cover this geometry");
       if (fast) {
-        if (!p->d_window_inv) {
+        if (!d.d_window_inv) {
           // 1 / fft of the inverse folded in; frames shorter than 2048 leave a zero tail
           std::vector<float> w(2048, 0.0f);
           for (size_t j = 0; j < (size_t)p->geom.fft; ++j)
             w[j] = (float)(p->window[j] / double(p->geom.fft));
-          p->d_window_inv = upload(w);
+          d.d_window_inv = upload(w);
         }
-        CK(smb::launch_istft2048(a, p->d_window_inv, p->d_tw_pass, p->d_tw_post, nb, p->sm_count,
-                                 st));
+        CK(smb::launch_istft2048(a, d.d_window_inv.get(), d.d_tw_pass.get(), d.d_tw_post.get(), nb,
+                                 d.sm_count, st));
         return;
       }
       CK(smb::launch_istft(a, nb, st));
@@ -1650,36 +1621,33 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
       throw smb::invalid_argument("soundml_b200: unknown memory kind");
     if (frames == 0) {
       if (mem == SMB_MEM_HOST) std::memset(out, 0, (size_t)batch * (size_t)out_len * esz);
-      else { p->ensure_device(); CK(cudaMemsetAsync(out, 0, (size_t)batch * (size_t)out_len * esz, p->stream.use)); }
+      else { p->ensure_device(); CK(cudaMemsetAsync(out, 0, (size_t)batch * (size_t)out_len * esz, p->dev->stream.use)); }
       return;
     }
     p->ensure_device();
-    cudaStream_t st = p->stream.use;
-    if (!p->d_folded) p->d_folded = upload(p->folded_square_window());
+    smb_stft_plan::Device& d = *p->dev;
+    cudaStream_t st = d.stream.use;
+    if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
     const size_t cells = (size_t)batch * (size_t)bins * (size_t)frames;
-    // the whole problem stays resident across the iterations
-    struct Temp {                       // freed when the call returns or throws
-      void* ptr = nullptr;
-      void reserve(size_t bytes) { CK(cudaMalloc(&ptr, bytes ? bytes : 1)); }
-      ~Temp() { if (ptr) cudaFree(ptr); }
-    } d_s, d_phase, d_spec, d_a, d_b, d_y, d_out;
+    // the whole problem stays resident across the iterations; freed when the call returns or throws
+    device_ptr<void> d_s, d_phase, d_out, d_a, d_b, d_y;
     const void* mags = s;
     const void* phase = init_phase;
     void* dout = out;
     if (mem == SMB_MEM_HOST) {
-      d_s.reserve(cells * esz);
-      CK(cudaMemcpyAsync(d_s.ptr, s, cells * esz, cudaMemcpyHostToDevice, st));
-      mags = d_s.ptr;
+      d_s = device_alloc(cells * esz);
+      CK(cudaMemcpyAsync(d_s.get(), s, cells * esz, cudaMemcpyHostToDevice, st));
+      mags = d_s.get();
       if (init_phase) {
-        d_phase.reserve(cells * esz);
-        CK(cudaMemcpyAsync(d_phase.ptr, init_phase, cells * esz, cudaMemcpyHostToDevice, st));
-        phase = d_phase.ptr;
+        d_phase = device_alloc(cells * esz);
+        CK(cudaMemcpyAsync(d_phase.get(), init_phase, cells * esz, cudaMemcpyHostToDevice, st));
+        phase = d_phase.get();
       }
-      d_out.reserve((size_t)batch * (size_t)out_len * esz);
-      dout = d_out.ptr;
+      d_out = device_alloc((size_t)batch * (size_t)out_len * esz);
+      dout = d_out.get();
     }
-    d_spec.reserve(cells * sizeof(double2));
-    double2* spec = (double2*)d_spec.ptr;
+    const device_ptr<double2> d_spec = device_alloc<double2>(cells * sizeof(double2));
+    double2* spec = d_spec.get();
     auto synth = [&](int64_t len, bool named, int out_dtype, void* dst) {
       int64_t count = frames;
       if (named) count = std::min(frames, (len + left + hop - 1) / hop);
@@ -1696,9 +1664,9 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
       a.fft = (int)p->geom.fft;
       a.hop = (int)hop;
       a.left = (int)left;
-      a.window = p->d_window64;
-      a.twiddle = p->d_twiddle64;
-      a.folded = p->d_folded;
+      a.window = d.d_window64.get();
+      a.twiddle = d.d_twiddle64.get();
+      a.folded = d.d_folded.get();
       a.in_f64 = 1;
       a.out_f64 = out_dtype == SMB_F64;
       CK(smb::launch_istft(a, batch, st));
@@ -1708,19 +1676,19 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
     // the loop runs at the natural length, the one geometry that re-analyses to
     // exactly `frames` frames (stft.ml:1000-1008)
     if (natural > 0) {
-      d_a.reserve(cells * sizeof(double2));
-      d_b.reserve(cells * sizeof(double2));
-      d_y.reserve((size_t)batch * (size_t)natural * sizeof(double));
-      double2* rebuilt = (double2*)d_a.ptr;
-      double2* previous = (double2*)d_b.ptr;
+      d_a = device_alloc(cells * sizeof(double2));
+      d_b = device_alloc(cells * sizeof(double2));
+      d_y = device_alloc((size_t)batch * (size_t)natural * sizeof(double));
+      double2* rebuilt = (double2*)d_a.get();
+      double2* previous = (double2*)d_b.get();
       const double beta = momentum / (1.0 + momentum);
       smb::FrameGeom g = p->frame_geom(natural);
       if (g.frames != frames)
         throw smb::invalid_argument("griffin_lim: the natural length does not re-analyse to the "
                                     "given frame count");
       for (int64_t k = 0; k < n_iter; ++k) {
-        synth(natural, false, SMB_F64, d_y.ptr);
-        CK(smb::launch_stft_generic(d_y.ptr, SMB_F64, batch, g, p->d_window64, p->d_twiddle64,
+        synth(natural, false, SMB_F64, d_y.get());
+        CK(smb::launch_stft_generic(d_y.get(), SMB_F64, batch, g, d.d_window64.get(), d.d_twiddle64.get(),
                                     smb::kModeComplex, 1.0, rebuilt, st));
         CK(smb::launch_gl_project(mags, nullptr, dtype == SMB_F64, rebuilt,
                                   k == 0 ? nullptr : previous, beta, 0, (long long)cells, spec, st));
@@ -1785,7 +1753,7 @@ int smb_mel_plan_create_with_weights(smb_mel_plan** plan, int64_t n_mels, int64_
 
 int smb_mel_plan_destroy(smb_mel_plan* plan) { return guarded([&] { delete plan; }); }
 int smb_mel_plan_set_stream(smb_mel_plan* plan, void* s) {
-  return guarded([&] { plan->ensure_device(); plan->stream.set(s); });
+  return guarded([&] { plan->ensure_device(); plan->dev->stream.set(s); });
 }
 int64_t smb_mel_n_mels(const smb_mel_plan* plan) { return plan->n_mels; }
 int64_t smb_mel_bins(const smb_mel_plan* plan) { return plan->bins; }
@@ -1803,7 +1771,7 @@ int smb_mel_apply(smb_mel_plan* plan, const void* s, int64_t batch, int64_t fram
     const size_t esz = dtype_size(dtype);
     if (batch == 0 || frames == 0) return;       // zero-size: nothing to reduce (mel.ml:221-227)
     plan->ensure_device();
-    cudaStream_t st = plan->stream.use;
+    cudaStream_t st = plan->dev->stream.use;
     if (mem == SMB_MEM_DEVICE) {
       run_mel_apply(plan, s, batch, frames, dtype, out, st);
       return;
@@ -1842,14 +1810,15 @@ static bool mel_spectrogram_impl(smb_stft_plan* stft, smb_mel_plan* mel, const v
     if (batch == 0 || g.frames == 0) return false;
     stft->ensure_device();
     mel->ensure_device();
-    cudaStream_t st = stft->stream.use;
+    const smb_stft_plan::Device& sd = *stft->dev;
+    cudaStream_t st = sd.stream.use;
     const int fast = want_fast(stft, dtype, g, smb::kFastMel, mel);
     max_known = fast == SMB_PATH_PAIR && max_slot != nullptr;
     auto run = [&](const void* din, void* dout, int64_t nb) {
       if (fast == SMB_PATH_PAIR) {
         smb::Stft2048PairArgs a = pair_args(stft, mel, din, dout, nb, g, power);
         a.max_slot = max_slot;
-        CK(smb::launch_stft2048p(a, false, stft->sm_count, st));
+        CK(smb::launch_stft2048p(a, false, sd.sm_count, st));
       } else if (fast) {
         smb::Stft2048Args a{};
         a.x = (const float*)din;
@@ -1858,26 +1827,27 @@ static bool mel_spectrogram_impl(smb_stft_plan* stft, smb_mel_plan* mel, const v
         a.g = g;
         a.g.fft = 2048;
         a.bin_step = stft->fast_step();
-        a.window = stft->d_window32;
-        a.tw_pass = stft->d_tw_pass;
-        a.tw_post = stft->d_tw_post;
+        a.window = sd.d_window32.get();
+        a.tw_pass = sd.d_tw_pass.get();
+        a.tw_post = sd.d_tw_post.get();
         a.n_mels = (int)mel->n_mels;
         a.power = (float)power;
-        a.dft_images = stft->d_dft_images;
+        a.dft_images = sd.d_dft_images.get();
         const auto& sc = fast == SMB_PATH_TENSOR ? mel->sched_tc : mel->sched_cc;
+        const auto& tables = fast == SMB_PATH_TENSOR ? mel->dev->tc : mel->dev->cc;
         a.nnz = (int)sc.vals.size();
-        a.vals = sc.d_vals;
-        a.mel_pieces = sc.d_pieces;
-        a.mel_pcnt = sc.d_pcnt;
+        a.vals = tables.d_vals.get();
+        a.mel_pieces = tables.d_pieces.get();
+        a.mel_pcnt = tables.d_pcnt.get();
         a.mel_rounds = sc.rounds;
         a.mel_mpad = sc.mpad;
-        if (fast == SMB_PATH_TENSOR) CK(smb::launch_stft2048tc(a, smb::kFastMel, stft->sm_count, st));
-        else CK(smb::launch_stft2048(a, smb::kFastMel, stft->sm_count, st));
+        if (fast == SMB_PATH_TENSOR) CK(smb::launch_stft2048tc(a, smb::kFastMel, sd.sm_count, st));
+        else CK(smb::launch_stft2048(a, smb::kFastMel, sd.sm_count, st));
       } else {
         // two kernels through a plan-owned power spectrogram
         const size_t spec_bytes = (size_t)nb * stft->geom.bins() * g.frames * esz;
         void* spec = stft->tmp.ensure(spec_bytes);
-        CK(smb::launch_stft_generic(din, dtype, nb, g, stft->d_window64, stft->d_twiddle64,
+        CK(smb::launch_stft_generic(din, dtype, nb, g, sd.d_window64.get(), sd.d_twiddle64.get(),
                                     smb::kModePower, power, spec, st));
         run_mel_apply(mel, spec, nb, g.frames, dtype, dout, st);
       }
@@ -1924,7 +1894,7 @@ int smb_stft_fft_ceiling(smb_stft_plan* stft, const void* x, int64_t batch, int6
     if (batch == 0 || g.frames == 0) return;
     stft->ensure_device();
     CK(smb::launch_stft2048p(pair_args(stft, nullptr, x, scratch, batch, g, 2.0), true,
-                             stft->sm_count, stft->stream.use));
+                             stft->dev->sm_count, stft->dev->stream.use));
   });
 }
 
@@ -1957,36 +1927,25 @@ void to_db_call(const char* fn, double gain, int magnitude, const void* x, int64
   const double offset = scale * std::log(std::max(amin, reference));
   // the maximum's slot and the host call's staging are stream-ordered allocations:
   // no device-wide synchronisation, and a device-memory call stays asynchronous
-  unsigned long long* slot = nullptr;
-  void *din = nullptr, *dout = nullptr;
-  auto release = [&] {
-    if (slot) cudaFreeAsync(slot, st);
-    if (din) cudaFreeAsync(din, st);
-    if (dout) cudaFreeAsync(dout, st);
-  };
-  try {
-    CK(cudaMallocAsync((void**)&slot, sizeof(unsigned long long), st));
-    const void* src = x;
-    void* dst = out;
-    if (mem == SMB_MEM_HOST) {
-      CK(cudaMallocAsync(&din, (size_t)count * esz, st));
-      CK(cudaMallocAsync(&dout, (size_t)count * esz, st));
-      CK(cudaMemcpyAsync(din, x, (size_t)count * esz, cudaMemcpyHostToDevice, st));
-      src = din;
-      dst = dout;
-    } else if (mem != SMB_MEM_DEVICE) {
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    }
-    CK(smb::launch_to_db(src, count, dtype, magnitude, amin, scale, offset, clamp,
-                         clamp ? top_db : 0.0, slot, dst, st));
-    if (mem == SMB_MEM_HOST)
-      CK(cudaMemcpyAsync(out, dout, (size_t)count * esz, cudaMemcpyDeviceToHost, st));
-  } catch (...) {
-    release();
-    throw;
+  const scratch_ptr slot = scratch_alloc(sizeof(unsigned long long), st);
+  scratch_ptr din, dout;
+  const void* src = x;
+  void* dst = out;
+  if (mem == SMB_MEM_HOST) {
+    din = scratch_alloc((size_t)count * esz, st);
+    dout = scratch_alloc((size_t)count * esz, st);
+    CK(cudaMemcpyAsync(din.get(), x, (size_t)count * esz, cudaMemcpyHostToDevice, st));
+    src = din.get();
+    dst = dout.get();
+  } else if (mem != SMB_MEM_DEVICE) {
+    throw smb::invalid_argument("soundml_b200: unknown memory kind");
   }
-  release();
-  if (mem == SMB_MEM_HOST) CK(cudaStreamSynchronize(st));   // the host buffer is the caller's again
+  CK(smb::launch_to_db(src, count, dtype, magnitude, amin, scale, offset, clamp,
+                       clamp ? top_db : 0.0, (unsigned long long*)slot.get(), dst, st));
+  if (mem == SMB_MEM_HOST) {
+    CK(cudaMemcpyAsync(out, dout.get(), (size_t)count * esz, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));   // the host buffer is the caller's again
+  }
 }
 
 }  // namespace
@@ -2031,7 +1990,8 @@ int smb_mfcc(smb_stft_plan* stft, smb_mel_plan* mel, const void* x, int64_t batc
     if (batch == 0 || g.frames == 0) return;
     stft->ensure_device();
     mel->ensure_device();
-    cudaStream_t st = stft->stream.use;
+    cudaStream_t st = stft->dev->stream.use;
+    unsigned long long* d_max = mel->dev->d_max.get();
     // log-mel needs the whole-tensor maximum, so the mel spectrogram is
     // materialised (plan-owned), then reduced, then transformed
     const size_t mel_bytes = (size_t)batch * mel->n_mels * g.frames * esz;
@@ -2042,7 +2002,7 @@ int smb_mfcc(smb_stft_plan* stft, smb_mel_plan* mel, const void* x, int64_t batc
     if (inner_mem != SMB_MEM_HOST && mem != SMB_MEM_DEVICE)
       throw smb::invalid_argument("soundml_b200: unknown memory kind");
     // the frame-pair kernel leaves the mel spectrogram's maximum in the slot as it writes
-    CK(cudaMemsetAsync(mel->d_max, 0, sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
     bool max_known = true;
     if (inner_mem == SMB_MEM_HOST) {
       // host audio goes up in slices of about 64 MB (the whole-tensor maximum needs every
@@ -2056,14 +2016,14 @@ int smb_mfcc(smb_stft_plan* stft, smb_mel_plan* mel, const void* x, int64_t batc
                            cudaMemcpyHostToDevice, st));
         max_known = mel_spectrogram_impl(stft, mel, stage, nb, n, dtype, 2.0,
                                          (char*)dmel + (size_t)b0 * mel->n_mels * g.frames * esz,
-                                         SMB_MEM_DEVICE, mel->d_max) && max_known;
+                                         SMB_MEM_DEVICE, d_max) && max_known;
       }
     } else {
-      max_known = mel_spectrogram_impl(stft, mel, x, batch, n, dtype, 2.0, dmel, SMB_MEM_DEVICE, mel->d_max);
+      max_known = mel_spectrogram_impl(stft, mel, x, batch, n, dtype, 2.0, dmel, SMB_MEM_DEVICE, d_max);
     }
     const double scale = kDecade, offset = scale * std::log(1.0);   // reference 1, amin 1e-10
     CK(smb::launch_mfcc(dmel, dtype, batch, (int)mel->n_mels, g.frames, (int)n_mfcc,
-                        mel->dct_table(n_mfcc, has_lifter ? lifter : 0.0), mel->d_max, max_known,
+                        mel->dct_table(n_mfcc, has_lifter ? lifter : 0.0), d_max, max_known,
                         1e-10, scale, offset, 80.0, dout, st));
     if (mem == SMB_MEM_HOST) {
       CK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
@@ -2100,10 +2060,11 @@ int smb_mel_spectrogram_db(smb_stft_plan* stft, smb_mel_plan* mel, const void* x
     if (batch == 0 || g.frames == 0) return;
     stft->ensure_device();
     mel->ensure_device();
-    cudaStream_t st = stft->stream.use;
+    cudaStream_t st = stft->dev->stream.use;
+    unsigned long long* d_max = mel->dev->d_max.get();
     const int64_t count = batch * mel->n_mels * g.frames;
     void* dmel = mem == SMB_MEM_HOST ? stft->cepstral.ensure((size_t)count * esz) : out;
-    CK(cudaMemsetAsync(mel->d_max, 0, sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
     const void* din = x;
     if (mem == SMB_MEM_HOST) {          // the result stays on the device until it is in decibels
       void* stage = stft->pipe.in[0].ensure((size_t)batch * n * esz);
@@ -2111,15 +2072,15 @@ int smb_mel_spectrogram_db(smb_stft_plan* stft, smb_mel_plan* mel, const void* x
       din = stage;
     }
     const bool max_known = mel_spectrogram_impl(stft, mel, din, batch, n, dtype, power, dmel,
-                                                SMB_MEM_DEVICE, mel->d_max);
+                                                SMB_MEM_DEVICE, d_max);
     const double scale = kDecade;                                   // gain 10: powers
     const double offset = scale * std::log(std::max(amin, reference));
     if (max_known)
       CK(smb::launch_db_known_max(dmel, count, dtype, amin, scale, offset, clamp, clamp ? top_db : 0.0,
-                                  mel->d_max, st));
+                                  d_max, st));
     else
       CK(smb::launch_to_db(dmel, count, dtype, 0, amin, scale, offset, clamp, clamp ? top_db : 0.0,
-                           mel->d_max, dmel, st));
+                           d_max, dmel, st));
     if (mem == SMB_MEM_HOST) {
       CK(cudaMemcpyAsync(out, dmel, (size_t)count * esz, cudaMemcpyDeviceToHost, st));
       CK(cudaStreamSynchronize(st));
@@ -2141,10 +2102,10 @@ int smb_resample_plan_create(smb_resample_plan** plan, int64_t sample_rate, int6
 }
 int smb_resample_plan_destroy(smb_resample_plan* plan) { return guarded([&] { delete plan; }); }
 int smb_resample_plan_set_stream(smb_resample_plan* plan, void* s) {
-  return guarded([&] { plan->ensure_device(); plan->stream.set(s); });
+  return guarded([&] { plan->ensure_device(); plan->dev->stream.set(s); });
 }
 int smb_resample_plan_sync(smb_resample_plan* plan) {
-  return guarded([&] { if (plan->device_ready) CK(cudaStreamSynchronize(plan->stream.use)); });
+  return guarded([&] { if (plan->dev) CK(cudaStreamSynchronize(plan->dev->stream.use)); });
 }
 int smb_resample_plan_set_executor(smb_resample_plan* plan, int exec) {
   return guarded([&] {
@@ -2159,7 +2120,7 @@ int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
     if (stage < 0 || stage >= (int)plan->plan.stages.size())
       throw smb::invalid_argument("stage_layout: no such stage");
     plan->ensure_device();
-    const GemmDevice& gd = plan->gemm[(size_t)stage];
+    const GemmDevice& gd = plan->dev->gemm[(size_t)stage];
     smb_resample_layout r{};
     r.form = plan->form((size_t)stage);
     r.groups = r.form == SMB_FORM_ROW ? (int)gd.rows_groups.size()
@@ -2248,7 +2209,7 @@ int smb_resample_apply(smb_resample_plan* plan, const float* x, int64_t batch, i
     const int64_t total = rp.output_frames(n);
     if (batch == 0 || n == 0 || total == 0) return;
     plan->ensure_device();
-    cudaStream_t st = plan->stream.use;
+    cudaStream_t st = plan->dev->stream.use;
     // signals are independent: a host batch goes through in slices, the copies of one
     // slice under the kernels of its neighbours (HostPipe)
     auto run = [&](const void* din_v, void* dout_v, int64_t nb) {
@@ -2284,7 +2245,7 @@ int smb_resample_apply_f64(smb_resample_plan* plan, const double* x, int64_t bat
     const int64_t total = rp.output_frames(n);
     if (batch == 0 || n == 0 || total == 0) return;
     plan->ensure_device();
-    cudaStream_t st = plan->stream.use;
+    cudaStream_t st = plan->dev->stream.use;
     const size_t in_bytes = (size_t)batch * n * 8, out_bytes = (size_t)batch * total * 8;
     const double* din = x;
     double* dout = out;
@@ -2298,7 +2259,7 @@ int smb_resample_apply_f64(smb_resample_plan* plan, const double* x, int64_t bat
     }
     auto stage_run = [&](size_t i, const double* src, int64_t len, int64_t n_out, double* dst) {
       const smb::ResampleStage& s = rp.stages[i];
-      CK(smb::launch_polyphase_direct_f64(src, batch, len, plan->d_bank64[i], (int)s.l, (int)s.m,
+      CK(smb::launch_polyphase_direct_f64(src, batch, len, plan->dev->d_bank64[i].get(), (int)s.l, (int)s.m,
                                           (int)s.k, n_out, dst, st));
     };
     if (rp.identity()) {
@@ -2357,13 +2318,11 @@ struct smb_resample_kernel {
     DeviceBuffer next;
     next.ensure((size_t)channels * grown * esz);
     if (fed > base)
-      CK(cudaMemcpy2DAsync(next.ptr, (size_t)grown * esz, carry[cur].ptr, (size_t)cap * esz,
+      CK(cudaMemcpy2DAsync(next.ptr.get(), (size_t)grown * esz, carry[cur].ptr.get(), (size_t)cap * esz,
                            (size_t)(fed - base) * esz, (size_t)channels, cudaMemcpyDeviceToDevice, st));
     CK(cudaStreamSynchronize(st));
-    carry[cur].release();
-    carry[cur] = next;
-    carry[1 - cur].release();
-    carry[1 - cur].ensure((size_t)channels * grown * esz);
+    carry[cur] = std::move(next);
+    carry[1 - cur].ensure((size_t)channels * grown * esz);     // (larger than it was: reallocates)
     cap = grown;
   }
   // outputs [emitted, upto) from a window of the retained input, written to `out`
@@ -2375,7 +2334,7 @@ struct smb_resample_kernel {
     const int64_t total_w = plan->plan.output_frames(len);
     char* w = (char*)win.ensure((size_t)channels * len * esz);
     char* r = (char*)res.ensure((size_t)channels * total_w * esz);
-    CK(cudaMemcpy2DAsync(w, (size_t)len * esz, (char*)carry[cur].ptr + (size_t)(a0 - base) * esz,
+    CK(cudaMemcpy2DAsync(w, (size_t)len * esz, (char*)carry[cur].ptr.get() + (size_t)(a0 - base) * esz,
                          (size_t)cap * esz, (size_t)len * esz, (size_t)channels,
                          cudaMemcpyDeviceToDevice, st));
     const int rc = dtype == SMB_F32
@@ -2392,8 +2351,8 @@ struct smb_resample_kernel {
     const int64_t keep = std::max<int64_t>(0, floor_div(emitted * m / l - reach, grain) * grain);
     if (keep > base) {
       if (fed > keep)
-        CK(cudaMemcpy2DAsync(carry[1 - cur].ptr, (size_t)cap * esz,
-                             (char*)carry[cur].ptr + (size_t)(keep - base) * esz, (size_t)cap * esz,
+        CK(cudaMemcpy2DAsync(carry[1 - cur].ptr.get(), (size_t)cap * esz,
+                             (char*)carry[cur].ptr.get() + (size_t)(keep - base) * esz, (size_t)cap * esz,
                              (size_t)(fed - keep) * esz, (size_t)channels, cudaMemcpyDeviceToDevice, st));
       cur = 1 - cur;
       base = keep;
@@ -2440,16 +2399,7 @@ int smb_resample_kernel_create(smb_resample_kernel** kernel, smb_resample_plan* 
     *kernel = k;
   });
 }
-int smb_resample_kernel_destroy(smb_resample_kernel* k) {
-  return guarded([&] {
-    if (!k) return;
-    k->carry[0].release();
-    k->carry[1].release();
-    k->win.release();
-    k->res.release();
-    delete k;
-  });
-}
+int smb_resample_kernel_destroy(smb_resample_kernel* k) { return guarded([&] { delete k; }); }
 int smb_resample_kernel_reset(smb_resample_kernel* k) {
   return guarded([&] {
     k->fed = k->emitted = k->base = 0;
@@ -2481,7 +2431,7 @@ int smb_resample_kernel_step(smb_resample_kernel* k, const void* chunk, int64_t 
       throw smb::invalid_argument("soundml_b200: unknown memory kind");
     if (n == 0) return;
     k->plan->ensure_device();
-    cudaStream_t st = k->plan->stream.use;
+    cudaStream_t st = k->plan->dev->stream.use;
     const cudaMemcpyKind in_kind = mem == SMB_MEM_HOST ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToDevice;
     if (k->l == k->m) {                                   // identity: forward a copy
       CK(cudaMemcpyAsync(out, chunk, (size_t)k->channels * n * k->esz,
@@ -2492,7 +2442,7 @@ int smb_resample_kernel_step(smb_resample_kernel* k, const void* chunk, int64_t 
       return;
     }
     k->ensure_cap(k->fed - k->base + n, st);
-    CK(cudaMemcpy2DAsync((char*)k->carry[k->cur].ptr + (size_t)(k->fed - k->base) * k->esz,
+    CK(cudaMemcpy2DAsync((char*)k->carry[k->cur].ptr.get() + (size_t)(k->fed - k->base) * k->esz,
                          (size_t)k->cap * k->esz, chunk, (size_t)n * k->esz, (size_t)n * k->esz,
                          (size_t)k->channels, in_kind, st));
     k->fed += n;
@@ -2510,7 +2460,7 @@ int smb_resample_kernel_flush(smb_resample_kernel* k, void* out, int mem) {
     const int64_t total = k->fed ? k->plan->plan.output_frames(k->fed) : 0;
     if (total <= k->emitted) return;
     k->plan->ensure_device();
-    cudaStream_t st = k->plan->stream.use;
+    cudaStream_t st = k->plan->dev->stream.use;
     k->window(total, out, mem, st);
     if (mem == SMB_MEM_HOST) CK(cudaStreamSynchronize(st));
   });
@@ -2531,7 +2481,7 @@ int smb_fir_plan_create(smb_fir_plan** plan, const double* h, int64_t taps) {
 }
 int smb_fir_plan_destroy(smb_fir_plan* plan) { return guarded([&] { delete plan; }); }
 int smb_fir_plan_set_stream(smb_fir_plan* plan, void* s) {
-  return guarded([&] { plan->ensure_device(); plan->stream.set(s); });
+  return guarded([&] { plan->ensure_device(); plan->dev->stream.set(s); });
 }
 int smb_fir_apply(smb_fir_plan* plan, const float* x, int64_t batch, int64_t n, float* out,
                   int method, int mem) {
@@ -2543,16 +2493,16 @@ int smb_fir_apply(smb_fir_plan* plan, const float* x, int64_t batch, int64_t n, 
     if (batch == 0 || n == 0) return;
     plan->ensure_device();
     if (method == SMB_EXEC_PLANNED)
-      method = plan->ols.plan.ok && plan->k >= 8 ? SMB_EXEC_OLS : SMB_EXEC_DIRECT;
-    if (method == SMB_EXEC_OLS && !plan->ols.plan.ok)
+      method = plan->dev->ols.plan.ok && plan->k >= 8 ? SMB_EXEC_OLS : SMB_EXEC_DIRECT;
+    if (method == SMB_EXEC_OLS && !plan->dev->ols.plan.ok)
       throw smb::invalid_argument(
           "fir: this filter is too long for the overlap-save kernel (use the direct method)");
-    cudaStream_t st = plan->stream.use;
+    cudaStream_t st = plan->dev->stream.use;
     auto run = [&](const void* din, void* dout, int64_t nb) {
       if (method == SMB_EXEC_OLS)
-        plan->ols.run((const float*)din, nb, n, n, (float*)dout, st);
+        plan->dev->ols.run((const float*)din, nb, n, n, (float*)dout, st);
       else
-        CK(smb::launch_polyphase_direct((const float*)din, nb, n, plan->d_bank, 1, 1, (int)plan->k, n,
+        CK(smb::launch_polyphase_direct((const float*)din, nb, n, plan->dev->d_bank.get(), 1, 1, (int)plan->k, n,
                                         (float*)dout, st));
     };
     if (mem == SMB_MEM_DEVICE) run(x, out, batch);
@@ -2588,10 +2538,17 @@ int smb_ingest_layout(const void* interleaved, int64_t frames, int64_t channels,
     require_device();
     cudaStream_t st = (cudaStream_t)cuda_stream;
     const int64_t width = mode == SMB_INGEST_PLANAR ? channels : 1;
-    static thread_local DeviceBuffer stage_in, stage_out;
+    // staging per thread and per device: kernels only ever see a buffer of the current device
+    static thread_local std::vector<DeviceBuffer> stage_in, stage_out;
+    int device = 0;
+    CK(cudaGetDevice(&device));
+    if ((size_t)device >= stage_in.size()) {
+      stage_in.resize((size_t)device + 1);
+      stage_out.resize((size_t)device + 1);
+    }
     const void* din = interleaved;
     if (mem_in == SMB_MEM_HOST) {
-      void* up = stage_in.ensure((size_t)frames * channels * esz);
+      void* up = stage_in[(size_t)device].ensure((size_t)frames * channels * esz);
       CK(cudaMemcpyAsync(up, interleaved, (size_t)frames * channels * esz, cudaMemcpyHostToDevice, st));
       din = up;
     }
@@ -2600,7 +2557,7 @@ int smb_ingest_layout(const void* interleaved, int64_t frames, int64_t channels,
                                    (char*)out + (size_t)out_off * esz, out_total, st));
       if (mem_in == SMB_MEM_HOST) CK(cudaStreamSynchronize(st));   // the host block may be reused
     } else {
-      void* dn = stage_out.ensure((size_t)frames * width * esz);
+      void* dn = stage_out[(size_t)device].ensure((size_t)frames * width * esz);
       CK(smb::launch_ingest_layout(din, dtype, frames, (int)channels, mode == SMB_INGEST_DOWNMIX, dn,
                                    frames, st));
       CK(cudaMemcpy2DAsync((char*)out + (size_t)out_off * esz, (size_t)out_total * esz, dn,
@@ -2624,17 +2581,24 @@ struct smb_ingest {
   int64_t channels = 0, width = 0, max_block = 0;
   int mode = SMB_INGEST_PLANAR, dtype = SMB_F32;
   size_t esz = 4;
-  smb_resample_plan* plan = nullptr;        // null: native rate
-  smb_resample_kernel* kernel = nullptr;
-  void* staging[2] = {nullptr, nullptr};
+  // streams first: they outlive everything used on them
+  stream_ptr own_compute;                       // native rate: the compute stream
+  stream_ptr copy;
+  std::unique_ptr<smb_resample_plan> plan;      // null: native rate
+  std::unique_ptr<smb_resample_kernel> kernel;  // borrows the plan: declared after it, destroyed first
+  cudaStream_t compute = nullptr;               // own_compute, or the plan's stream
+  pinned_ptr staging[2];
   DeviceBuffer up[2], planar;
-  cudaStream_t copy = nullptr, compute = nullptr;
-  bool own_compute = false;
-  cudaEvent_t copied[2] = {nullptr, nullptr}, consumed[2] = {nullptr, nullptr};
+  event_ptr copied[2], consumed[2];
   bool in_flight[2] = {false, false};
   int cur = 0;
   bool finished = false;
   int64_t frames_in = 0, frames_out = 0;
+  ~smb_ingest() {
+    // an upload in flight may still read a pinned block: drain before anything is freed
+    if (copy) cudaStreamSynchronize(copy.get());
+    if (compute) cudaStreamSynchronize(compute);
+  }
 };
 
 int smb_ingest_create(smb_ingest** reader, int64_t channels, int64_t sample_rate, int64_t target,
@@ -2657,64 +2621,49 @@ int smb_ingest_create(smb_ingest** reader, int64_t channels, int64_t sample_rate
     r->esz = esz;
     r->max_block = max_block > 0 ? max_block : smb_ingest_block_frames(channels, (int64_t)esz, 0);
     if (target > 0 && target != sample_rate) {
-      if (smb_resample_plan_create(&r->plan, sample_rate, target, quality, 0.0, 0.0) != SMB_OK)
+      smb_resample_plan* plan = nullptr;
+      if (smb_resample_plan_create(&plan, sample_rate, target, quality, 0.0, 0.0) != SMB_OK)
         throw smb::invalid_argument(t_error);
-      if (smb_resample_kernel_create(&r->kernel, r->plan, dtype, r->width, r->max_block) != SMB_OK) {
-        const std::string msg = t_error;
-        smb_resample_plan_destroy(r->plan);
-        throw smb::invalid_argument(msg);
-      }
-      r->plan->ensure_device();
-      r->compute = r->plan->stream.use;
+      r->plan.reset(plan);
+      smb_resample_kernel* kernel = nullptr;
+      if (smb_resample_kernel_create(&kernel, plan, dtype, r->width, r->max_block) != SMB_OK)
+        throw smb::invalid_argument(t_error);
+      r->kernel.reset(kernel);
+      plan->ensure_device();
+      r->compute = plan->dev->stream.use;
     } else {
-      CK(cudaStreamCreateWithFlags(&r->compute, cudaStreamNonBlocking));
-      r->own_compute = true;
+      r->own_compute = new_stream();
+      r->compute = r->own_compute.get();
     }
-    CK(cudaStreamCreateWithFlags(&r->copy, cudaStreamNonBlocking));
+    r->copy = new_stream();
     for (int i = 0; i < 2; ++i) {
-      CK(cudaMallocHost(&r->staging[i], (size_t)r->max_block * channels * esz));
+      void* block = nullptr;
+      CK(cudaMallocHost(&block, (size_t)r->max_block * channels * esz));
+      r->staging[i].reset(block);
       r->up[i].ensure((size_t)r->max_block * channels * esz);
-      CK(cudaEventCreateWithFlags(&r->copied[i], cudaEventDisableTiming));
-      CK(cudaEventCreateWithFlags(&r->consumed[i], cudaEventDisableTiming));
+      r->copied[i] = new_event();
+      r->consumed[i] = new_event();
     }
     r->planar.ensure((size_t)r->max_block * r->width * esz);
     *reader = r.release();
   });
 }
-int smb_ingest_destroy(smb_ingest* r) {
-  return guarded([&] {
-    if (!r) return;
-    if (r->copy) cudaStreamSynchronize(r->copy);
-    if (r->compute) cudaStreamSynchronize(r->compute);
-    for (int i = 0; i < 2; ++i) {
-      if (r->staging[i]) cudaFreeHost(r->staging[i]);
-      r->up[i].release();
-      if (r->copied[i]) cudaEventDestroy(r->copied[i]);
-      if (r->consumed[i]) cudaEventDestroy(r->consumed[i]);
-    }
-    r->planar.release();
-    if (r->kernel) smb_resample_kernel_destroy(r->kernel);
-    if (r->plan) smb_resample_plan_destroy(r->plan);
-    if (r->copy) cudaStreamDestroy(r->copy);
-    if (r->own_compute && r->compute) cudaStreamDestroy(r->compute);
-    delete r;
-  });
-}
+int smb_ingest_destroy(smb_ingest* r) { return guarded([&] { delete r; }); }
 int64_t smb_ingest_max_block(const smb_ingest* r) { return r->max_block; }
 int smb_ingest_staging(smb_ingest* r, void** block) {
   return guarded([&] {
     same_device(r->bound_device);
     // the upload that last read this block (two submits ago) must have left the host
     if (r->in_flight[r->cur]) {
-      CK(cudaEventSynchronize(r->copied[r->cur]));
+      CK(cudaEventSynchronize(r->copied[r->cur].get()));
       r->in_flight[r->cur] = false;
     }
-    *block = r->staging[r->cur];
+    *block = r->staging[r->cur].get();
   });
 }
 int64_t smb_ingest_submit_frames(const smb_ingest* r, int64_t frames) {
   if (r->finished || frames <= 0) return 0;
-  return r->kernel ? smb_resample_kernel_step_frames(r->kernel, frames) : frames;
+  return r->kernel ? smb_resample_kernel_step_frames(r->kernel.get(), frames) : frames;
 }
 int smb_ingest_submit(smb_ingest* r, int64_t frames, void* out_device) {
   return guarded([&] {
@@ -2725,24 +2674,26 @@ int smb_ingest_submit(smb_ingest* r, int64_t frames, void* out_device) {
                                               (long long)frames, (long long)r->max_block));
     if (frames == 0) return;
     const int b = r->cur;
+    cudaEvent_t copied = r->copied[b].get(), consumed = r->consumed[b].get();
+    void* up = r->up[b].ptr.get();
     // the layout pass that last read up[b] must be done before the copy overwrites it
-    CK(cudaStreamWaitEvent(r->copy, r->consumed[b], 0));
-    CK(cudaMemcpyAsync(r->up[b].ptr, r->staging[b], (size_t)frames * r->channels * r->esz,
-                       cudaMemcpyHostToDevice, r->copy));
-    CK(cudaEventRecord(r->copied[b], r->copy));
+    CK(cudaStreamWaitEvent(r->copy.get(), consumed, 0));
+    CK(cudaMemcpyAsync(up, r->staging[b].get(), (size_t)frames * r->channels * r->esz,
+                       cudaMemcpyHostToDevice, r->copy.get()));
+    CK(cudaEventRecord(copied, r->copy.get()));
     r->in_flight[b] = true;
-    CK(cudaStreamWaitEvent(r->compute, r->copied[b], 0));
+    CK(cudaStreamWaitEvent(r->compute, copied, 0));
     const int64_t released = smb_ingest_submit_frames(r, frames);
     if (r->kernel) {
-      CK(smb::launch_ingest_layout(r->up[b].ptr, r->dtype, frames, (int)r->channels,
-                                   r->mode == SMB_INGEST_DOWNMIX, r->planar.ptr, frames, r->compute));
-      CK(cudaEventRecord(r->consumed[b], r->compute));
-      if (smb_resample_kernel_step(r->kernel, r->planar.ptr, frames, out_device, SMB_MEM_DEVICE) != SMB_OK)
+      CK(smb::launch_ingest_layout(up, r->dtype, frames, (int)r->channels,
+                                   r->mode == SMB_INGEST_DOWNMIX, r->planar.ptr.get(), frames, r->compute));
+      CK(cudaEventRecord(consumed, r->compute));
+      if (smb_resample_kernel_step(r->kernel.get(), r->planar.ptr.get(), frames, out_device, SMB_MEM_DEVICE) != SMB_OK)
         throw cuda_failure(t_error);
     } else {
-      CK(smb::launch_ingest_layout(r->up[b].ptr, r->dtype, frames, (int)r->channels,
+      CK(smb::launch_ingest_layout(up, r->dtype, frames, (int)r->channels,
                                    r->mode == SMB_INGEST_DOWNMIX, out_device, frames, r->compute));
-      CK(cudaEventRecord(r->consumed[b], r->compute));
+      CK(cudaEventRecord(consumed, r->compute));
     }
     r->frames_in += frames;
     r->frames_out += released;
@@ -2750,7 +2701,7 @@ int smb_ingest_submit(smb_ingest* r, int64_t frames, void* out_device) {
   });
 }
 int64_t smb_ingest_finish_frames(const smb_ingest* r) {
-  return (r->finished || !r->kernel) ? 0 : smb_resample_kernel_flush_frames(r->kernel);
+  return (r->finished || !r->kernel) ? 0 : smb_resample_kernel_flush_frames(r->kernel.get());
 }
 int smb_ingest_finish(smb_ingest* r, void* out_device) {
   return guarded([&] {
@@ -2758,14 +2709,14 @@ int smb_ingest_finish(smb_ingest* r, void* out_device) {
     if (r->finished) return;
     const int64_t tail = smb_ingest_finish_frames(r);
     r->finished = true;
-    if (r->kernel && smb_resample_kernel_flush(r->kernel, out_device, SMB_MEM_DEVICE) != SMB_OK)
+    if (r->kernel && smb_resample_kernel_flush(r->kernel.get(), out_device, SMB_MEM_DEVICE) != SMB_OK)
       throw cuda_failure(t_error);
     r->frames_out += tail;
   });
 }
 int smb_ingest_sync(smb_ingest* r) {
   return guarded([&] {
-    CK(cudaStreamSynchronize(r->copy));
+    CK(cudaStreamSynchronize(r->copy.get()));
     CK(cudaStreamSynchronize(r->compute));
   });
 }

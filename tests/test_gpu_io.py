@@ -41,6 +41,22 @@ def test_layout_is_bit_exact(sb, dtype, channels, mode):
         assert np.array_equal(got_d.cpu().numpy(), ref)
 
 
+def test_layout_staging_is_per_device(sb):
+    """The layout call keeps its staging per thread and per device: after a large block on
+    device 0, a smaller one on device 1 must not reuse device 0's buffer."""
+    import torch
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs two CUDA devices")
+    for device, frames in ((0, 50000), (1, 3000)):
+        b = _block(frames, 2, np.float32, device)
+        ref = io_oracle.layout(b, "planar")
+        with torch.cuda.device(device):
+            got = sb.Io.layout(b, "planar", device=f"cuda:{device}")                      # host -> device
+            assert got.device.index == device and np.array_equal(got.cpu().numpy(), ref)
+            got_h = sb.Io.layout(torch.from_numpy(b).to(f"cuda:{device}"), "planar", device="host")
+            assert np.array_equal(got_h, ref)                                             # device -> host
+
+
 def test_layout_into_a_longer_destination(sb):
     import torch
     b0, b1 = _block(1000, 2, np.float32, 1), _block(500, 2, np.float32, 2)
