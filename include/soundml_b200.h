@@ -13,6 +13,8 @@
  *   smb_mel_*             Mel.Config.create / filterbank / apply
  *                                           soundml/lib/mel.ml:119-164,198-231 (Nx.matmul)
  *   smb_mel_spectrogram   Soundml.mel_spectrogram   soundml/lib/soundml.ml:12-24
+ *   smb_phase_vocoder,    Effects.time_stretch and the phase vocoder it runs
+ *   smb_time_stretch      between Stft.transform and Stft.invert  soundml/lib/effects.ml:296
  *   smb_window_make       Window.make               soundml/lib/window.ml:374-401
  *   smb_resample_*        Resample.Config.create / output_frames / apply
  *                                           soundml/lib/resample.ml:872-1051,1913-1936
@@ -186,6 +188,36 @@ int smb_stft_invert(smb_stft_plan* plan, const void* z, int64_t batch, int64_t f
 int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int64_t frames,
                          int dtype, int64_t n_iter, double momentum, const void* init_phase,
                          int has_length, int64_t length, void* out, int mem);
+
+/* ---- effects (librosa 0.11 effects.py; the reference's soundml/lib/effects.ml) ---- */
+/* phase_vocoder D rate: z [batch, bins, frames] complex (dtype SMB_F32 = complex64,
+ * SMB_F64 = complex128; bins = smb_stft_bins(plan)) -> out [batch, bins, T'] of the
+ * same dtype, T' = ceil(frames / rate) in double (np.arange(0, frames, rate)).  Output
+ * frame t reads source position t * rate in double: magnitudes interpolated linearly
+ * between the two frames around it, phase accumulated from the first frame's, with two
+ * all-zero frames past the end.  The accumulated phase is computed as the sum of the
+ * gap terms of DESIGN.md 4.8 (equal to librosa's recurrence modulo 2 pi), so its error
+ * does not grow with the absolute phase; at rate 1 the output is z to rounding.
+ * Errors, in order: the rate (<= 0, NaN or infinite: "phase_vocoder: cannot stretch by
+ * a rate of %g (...)"), a negative frame or batch count, the dtype. */
+int smb_phase_vocoder(smb_stft_plan* plan, const void* z, int64_t batch, int64_t frames,
+                      int dtype, double rate, void* out, int mem);
+/* time_stretch x rate = invert (phase_vocoder (transform x) rate) ~length:round(n / rate)
+ * (effects.ml:296): x [batch, n] real (dtype) -> out [batch, round(n / rate)] of the
+ * same dtype, rounded half to even as Python's round.  The three stages run on the
+ * plan's stream with both spectra in device scratch the plan owns (freed with the
+ * plan); host memory is staged through the plan's pipeline as smb_stft_invert's is.
+ * Bit for bit the composition of smb_stft_transform, smb_phase_vocoder and
+ * smb_stft_invert (has_length = 1, out_dtype = dtype).  Errors, in order: the rate
+ * ("time_stretch: cannot stretch by a rate of %g (...)"), a negative length or batch,
+ * a non-invertible configuration (smb_stft_invert's message), the dtype. */
+int smb_time_stretch(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
+                     double rate, void* out, int mem);
+/* Sizes for callers that allocate: T' = ceil(frames / rate) of smb_phase_vocoder (the plan
+ * is not read: the count is the same for every configuration) and round(n / rate) of
+ * smb_time_stretch; -1 and the SMB_EINVAL message on a bad rate or a negative count. */
+int64_t smb_time_stretch_frames(const smb_stft_plan* plan, int64_t frames, double rate);
+int64_t smb_time_stretch_length(int64_t n, double rate);
 
 /* ---- mel ----------------------------------------------------------------- */
 /* Mel.Config.create; f_max = NaN means "Nyquist" (the OCaml default). */

@@ -14,6 +14,7 @@
      Resample.apply        resample.ml:1913-1936 -> B200.resample_apply
      Stft.transform_range  stft.ml:652-666   -> B200.transform_range
      Stft.invert           stft.ml:937-939   -> B200.invert
+     Effects.time_stretch  effects.ml:296    -> B200.time_stretch (and B200.phase_vocoder)
      Convert.power_to_db / amplitude_to_db  convert.ml:20-56 -> B200.to_db
      Soundml.mfcc          soundml.ml:50-95  -> B200.mfcc
      Resample.Kernel.prepare / step / flush / reset
@@ -72,6 +73,21 @@ external transform_range_c :
 external invert_c :
   stft_plan -> (Complex.t, 'c) ba -> int -> int -> int -> (float, 'a) ba -> unit
   = "soundml_b200_invert_bc" "soundml_b200_invert"
+
+(* plan -> z -> batch -> frames -> rate -> out *)
+external phase_vocoder_c :
+  stft_plan -> (Complex.t, 'c) ba -> int -> int -> float -> (Complex.t, 'c) ba -> unit
+  = "soundml_b200_phase_vocoder_bc" "soundml_b200_phase_vocoder"
+
+(* plan -> x -> batch -> n -> rate -> out *)
+external time_stretch_c :
+  stft_plan -> (float, 'a) ba -> int -> int -> float -> (float, 'a) ba -> unit
+  = "soundml_b200_time_stretch_bc" "soundml_b200_time_stretch"
+
+external time_stretch_frames : stft_plan -> int -> float -> int
+  = "soundml_b200_time_stretch_frames"
+
+external time_stretch_length : int -> float -> int = "soundml_b200_time_stretch_length"
 
 (* amplitude -> x -> reference -> amin -> top_db (nan = None) -> out *)
 external to_db_c :
@@ -305,6 +321,49 @@ let invert dtype c ?length z =
     invert_c (stft_plan_of c) (array1_of (Nx.contiguous z)) batch frames
       (match length with Some n -> n | None -> -1)
       (array1_of out) ;
+  out
+
+(* Replacement bodies of the phase vocoder and Effects.time_stretch (effects.ml:296):
+   the library checks the rate (positive and finite) and, for time_stretch,
+   invertibility, with the reference's wording. *)
+let phase_vocoder c ~rate z =
+  let rank = Nx.ndim z in
+  if rank < 2 then
+    invalid_arg
+      (Printf.sprintf
+         "phase_vocoder: cannot stretch a rank-%d tensor (the bin and frame axes must exist)"
+         rank) ;
+  let frames = Nx.dim (rank - 1) z in
+  let bins = Nx.dim (rank - 2) z in
+  let lead = Array.sub (Nx.shape z) 0 (rank - 1) in
+  let batch = Array.fold_left ( * ) 1 (Array.sub lead 0 (rank - 2)) in
+  let plan = stft_plan_of c in
+  (* the rate first, then the bin axis, as the Python face orders them *)
+  let out_frames = time_stretch_frames plan frames rate in
+  let want = Stft.Config.bins c in
+  if bins <> want then
+    invalid_arg
+      (Printf.sprintf
+         "phase_vocoder: cannot stretch %d frequency bins of a %d-point transform (the bin \
+          axis must hold fft_size / 2 + 1 = %d values)"
+         bins (Stft.Config.fft_size c) want) ;
+  let out = Nx.zeros (Nx.dtype z) (Array.append lead [|out_frames|]) in
+  if batch > 0 && out_frames > 0 then
+    phase_vocoder_c plan (array1_of (Nx.contiguous z)) batch frames rate (array1_of out) ;
+  out
+
+let time_stretch c ~rate x =
+  let rank = Nx.ndim x in
+  let n = Nx.dim (rank - 1) x in
+  let lead = Array.sub (Nx.shape x) 0 (rank - 1) in
+  let batch = Array.fold_left ( * ) 1 lead in
+  let plan = stft_plan_of c in
+  let length = time_stretch_length n rate in
+  let out = Nx.zeros (Nx.dtype x) (Array.append lead [|length|]) in
+  (* batch 0: the preconditions (invertibility) even when there is nothing to compute *)
+  time_stretch_c plan (array1_of (Nx.contiguous x)) 0 n rate (array1_of out) ;
+  if batch > 0 && length > 0 then
+    time_stretch_c plan (array1_of (Nx.contiguous x)) batch n rate (array1_of out) ;
   out
 
 (* Replacement body of Convert.power_to_db / amplitude_to_db: elementwise over

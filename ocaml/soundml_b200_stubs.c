@@ -318,6 +318,74 @@ CAMLprim value soundml_b200_invert_bc(value *argv, int argn) {
   return soundml_b200_invert(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5]);
 }
 
+/* ---- Effects (effects.ml; librosa 0.11 phase_vocoder / time_stretch) ----------
+ * phase_vocoder: z [batch; bins; frames] complex -> out [batch; bins; T'] of the same
+ * kind, T' = time_stretch_frames plan frames rate.  A bad rate is Invalid_argument with
+ * the reference's wording, raised by the library before any extent is trusted. */
+CAMLprim value soundml_b200_phase_vocoder(value v_plan, value v_z, value v_batch, value v_frames,
+                                          value v_rate, value v_out) {
+  CAMLparam3(v_plan, v_z, v_out);
+  smb_stft_plan *h = live(v_plan);
+  const void *z = Caml_ba_data_val(v_z);
+  void *out = Caml_ba_data_val(v_out);
+  const int dtype = dtype_of(v_z);
+  const int64_t batch = Long_val(v_batch), frames = Long_val(v_frames);
+  const double rate = Double_val(v_rate);
+  const int64_t out_frames = smb_time_stretch_frames(h, frames, rate);
+  if (out_frames >= 0) {
+    need(v_z, batch * smb_stft_bins(h) * frames, "soundml_b200: input extent disagrees with geometry");
+    need(v_out, batch * smb_stft_bins(h) * out_frames,
+         "soundml_b200: output extent disagrees with geometry");
+  }
+  caml_release_runtime_system();
+  int st = smb_phase_vocoder(h, z, batch, frames, dtype, rate, out, SMB_MEM_HOST);
+  caml_acquire_runtime_system();
+  smb_ml_raise(st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value soundml_b200_phase_vocoder_bc(value *argv, int argn) {
+  (void)argn;
+  return soundml_b200_phase_vocoder(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5]);
+}
+
+/* time_stretch: x [batch; n] real -> out [batch; time_stretch_length n rate], same kind. */
+CAMLprim value soundml_b200_time_stretch(value v_plan, value v_x, value v_batch, value v_n,
+                                         value v_rate, value v_out) {
+  CAMLparam3(v_plan, v_x, v_out);
+  smb_stft_plan *h = live(v_plan);
+  const void *x = Caml_ba_data_val(v_x);
+  void *out = Caml_ba_data_val(v_out);
+  const int dtype = dtype_of(v_x);
+  const int64_t batch = Long_val(v_batch), n = Long_val(v_n);
+  const double rate = Double_val(v_rate);
+  const int64_t length = smb_time_stretch_length(n, rate);
+  if (length >= 0) {
+    need(v_x, batch * n, "soundml_b200: input extent disagrees with geometry");
+    need(v_out, batch * length, "soundml_b200: output extent disagrees with geometry");
+  }
+  caml_release_runtime_system();
+  int st = smb_time_stretch(h, x, batch, n, dtype, rate, out, SMB_MEM_HOST);
+  caml_acquire_runtime_system();
+  smb_ml_raise(st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value soundml_b200_time_stretch_bc(value *argv, int argn) {
+  (void)argn;
+  return soundml_b200_time_stretch(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5]);
+}
+
+/* Output sizes, Invalid_argument on a bad rate or a negative count. */
+CAMLprim value soundml_b200_time_stretch_frames(value v_plan, value v_frames, value v_rate) {
+  const int64_t r = smb_time_stretch_frames(live(v_plan), Long_val(v_frames), Double_val(v_rate));
+  if (r < 0) smb_ml_raise(SMB_EINVAL);
+  return Val_long(r);
+}
+CAMLprim value soundml_b200_time_stretch_length(value v_n, value v_rate) {
+  const int64_t r = smb_time_stretch_length(Long_val(v_n), Double_val(v_rate));
+  if (r < 0) smb_ml_raise(SMB_EINVAL);
+  return Val_long(r);
+}
+
 /* Convert.power_to_db / amplitude_to_db (convert.ml:20-56).  top_db = nan stands
  * for None; amplitude selects the 20 log10 form. */
 CAMLprim value soundml_b200_to_db(value v_amplitude, value v_x, value v_reference, value v_amin,

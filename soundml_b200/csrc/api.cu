@@ -260,6 +260,7 @@ struct smb_stft_plan {
   HostPipe pipe;
   DeviceBuffer tmp;        // power spectrogram of the generic mel path
   DeviceBuffer cepstral;   // mel spectrogram (+ host-call output) of the MFCC path
+  DeviceBuffer stretch_spec, stretch_voc;   // time_stretch: the spectrum and its stretched copy
 
   void ensure_device() {
     if (dev) return same_device(dev->device);
@@ -1469,6 +1470,54 @@ void run_mel_apply(smb_mel_plan* m, const void* ds, int64_t batch, int64_t frame
                            m->dev->d_band_lo.get(), m->dev->d_band_hi.get(), dout, st));
 }
 
+// z (device) -> out (device): Stft.invert of `nb` items on the plan's stream (the
+// synthesis kernels of smb_stft_invert; time_stretch's last stage)
+void run_invert(smb_stft_plan* p, const void* dz, void* dout, int64_t nb, int64_t frames,
+                bool has_length, int64_t out_len, int in_dtype, int out_dtype) {
+  smb_stft_plan::Device& d = *p->dev;
+  cudaStream_t st = d.stream.use;
+  const int64_t left = p->geom.left_width(), hop = p->geom.hop;
+  // only the frames the output can reach are inverted (stft.ml:907-915)
+  int64_t count = frames;
+  if (has_length) count = std::min(frames, (out_len + left + hop - 1) / hop);
+  if (count == 0) {                                 // nothing reaches the output: zeros
+    CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * dtype_size(out_dtype), st));
+    return;
+  }
+  if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
+  smb::IstftArgs a{};
+  a.z = dz;
+  a.out = dout;
+  a.frames = frames;
+  a.count = count;
+  a.out_len = out_len;
+  a.fft = (int)p->geom.fft;
+  a.hop = (int)hop;
+  a.left = (int)left;
+  a.window = d.d_window64.get();
+  a.twiddle = d.d_twiddle64.get();
+  a.folded = d.d_folded.get();
+  a.in_f64 = in_dtype == SMB_F64;
+  a.out_f64 = out_dtype == SMB_F64;
+  const bool fast = p->path != SMB_PATH_GENERIC && smb::istft2048_supports(a);
+  if (!fast && p->path == SMB_PATH_FAST)
+    throw smb::invalid_argument(
+        "soundml_b200: the fft-2048 synthesis kernel does not cover this geometry");
+  if (fast) {
+    if (!d.d_window_inv) {
+      // 1 / fft of the inverse folded in; frames shorter than 2048 leave a zero tail
+      std::vector<float> w(2048, 0.0f);
+      for (size_t j = 0; j < (size_t)p->geom.fft; ++j)
+        w[j] = (float)(p->window[j] / double(p->geom.fft));
+      d.d_window_inv = upload(w);
+    }
+    CK(smb::launch_istft2048(a, d.d_window_inv.get(), d.d_tw_pass.get(), d.d_tw_post.get(), nb,
+                             d.sm_count, st));
+    return;
+  }
+  CK(smb::launch_istft(a, nb, st));
+}
+
 }  // namespace
 
 extern "C" {
@@ -1527,52 +1576,12 @@ int smb_stft_invert(smb_stft_plan* plan, const void* z, int64_t batch, int64_t f
           "largest value at every position)",
           (long long)p->geom.win_length, (long long)p->geom.hop, (long long)p->geom.fft));
     const size_t isz = 2 * dtype_size(in_dtype), osz = dtype_size(out_dtype);
-    const int64_t left = p->geom.left_width(), hop = p->geom.hop;
     const int64_t out_len = has_length ? length : p->output_length(frames);
-    // only the frames the output can reach are inverted (stft.ml:907-915)
-    int64_t count = frames;
-    if (has_length) count = std::min(frames, (length + left + hop - 1) / hop);
     if (batch == 0 || out_len == 0) return;
     p->ensure_device();
-    smb_stft_plan::Device& d = *p->dev;
-    cudaStream_t st = d.stream.use;
-    if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
+    cudaStream_t st = p->dev->stream.use;
     auto run = [&](const void* dz, void* dout, int64_t nb) {
-      if (count == 0) {                                 // nothing reaches the output: zeros
-        CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * osz, st));
-        return;
-      }
-      smb::IstftArgs a{};
-      a.z = dz;
-      a.out = dout;
-      a.frames = frames;
-      a.count = count;
-      a.out_len = out_len;
-      a.fft = (int)p->geom.fft;
-      a.hop = (int)hop;
-      a.left = (int)left;
-      a.window = d.d_window64.get();
-      a.twiddle = d.d_twiddle64.get();
-      a.folded = d.d_folded.get();
-      a.in_f64 = in_dtype == SMB_F64;
-      a.out_f64 = out_dtype == SMB_F64;
-      const bool fast = p->path != SMB_PATH_GENERIC && smb::istft2048_supports(a);
-      if (!fast && p->path == SMB_PATH_FAST)
-        throw smb::invalid_argument(
-            "soundml_b200: the fft-2048 synthesis kernel does not cover this geometry");
-      if (fast) {
-        if (!d.d_window_inv) {
-          // 1 / fft of the inverse folded in; frames shorter than 2048 leave a zero tail
-          std::vector<float> w(2048, 0.0f);
-          for (size_t j = 0; j < (size_t)p->geom.fft; ++j)
-            w[j] = (float)(p->window[j] / double(p->geom.fft));
-          d.d_window_inv = upload(w);
-        }
-        CK(smb::launch_istft2048(a, d.d_window_inv.get(), d.d_tw_pass.get(), d.d_tw_post.get(), nb,
-                                 d.sm_count, st));
-        return;
-      }
-      CK(smb::launch_istft(a, nb, st));
+      run_invert(p, dz, dout, nb, frames, has_length != 0, out_len, in_dtype, out_dtype);
     };
     if (mem == SMB_MEM_DEVICE) {
       run(z, out, batch);
@@ -1705,6 +1714,150 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
     }
   });
 }
+
+}  // extern "C"
+
+// ---- effects: phase vocoder, time_stretch (librosa 0.11 effects; DESIGN.md 4.8) ----
+
+namespace {
+
+void check_rate(const char* op, double rate) {
+  if (!(rate > 0.0) || !std::isfinite(rate))
+    throw smb::invalid_argument(smb::format(
+        "%s: cannot stretch by a rate of %g (the rate must be positive and finite)", op, rate));
+}
+
+// ceil(frames / rate) in double: the length of np.arange(0, frames, rate)
+int64_t vocoder_frames(const char* op, int64_t frames, double rate) {
+  check_rate(op, rate);
+  if (frames < 0)
+    throw smb::invalid_argument(smb::format(
+        "%s: cannot stretch %lld frames (frames must be non-negative)", op, (long long)frames));
+  const double q = std::ceil((double)frames / rate);
+  if (!(q <= 9007199254740992.0))
+    throw smb::invalid_argument(smb::format(
+        "%s: cannot stretch %lld frames by a rate of %g (the result would hold more than 2^53 "
+        "frames)", op, (long long)frames, rate));
+  return (int64_t)q;
+}
+
+// round(n / rate), half to even as Python's round (the current rounding mode is the
+// default round-to-nearest-even)
+int64_t stretch_length(int64_t n, double rate) {
+  check_rate("time_stretch", rate);
+  if (n < 0)
+    throw smb::invalid_argument(smb::format(
+        "time_stretch: cannot stretch a signal of length %lld (length must be non-negative)",
+        (long long)n));
+  const double q = std::nearbyint((double)n / rate);
+  if (!(q <= 9007199254740992.0))
+    throw smb::invalid_argument(smb::format(
+        "time_stretch: cannot stretch %lld samples by a rate of %g (the result would hold more "
+        "than 2^53 samples)", (long long)n, rate));
+  return (int64_t)q;
+}
+
+void run_vocoder(smb_stft_plan* p, const void* dz, void* dout, int64_t nb, int64_t frames,
+                 int64_t out_frames, int dtype, double rate) {
+  smb::PhaseVocoderArgs a{};
+  a.z = dz;
+  a.out = dout;
+  a.rows = nb * p->geom.bins();
+  a.frames = frames;
+  a.out_frames = out_frames;
+  a.rate = rate;
+  a.f64 = dtype == SMB_F64;
+  CK(smb::launch_phase_vocoder(a, p->dev->stream.use));
+}
+
+}  // namespace
+
+extern "C" {
+
+int64_t smb_time_stretch_frames(const smb_stft_plan* plan, int64_t frames, double rate) {
+  (void)plan;
+  int64_t r = -1;
+  guarded([&] { r = vocoder_frames("phase_vocoder", frames, rate); });
+  return r;
+}
+
+int64_t smb_time_stretch_length(int64_t n, double rate) {
+  int64_t r = -1;
+  guarded([&] { r = stretch_length(n, rate); });
+  return r;
+}
+
+int smb_phase_vocoder(smb_stft_plan* plan, const void* z, int64_t batch, int64_t frames,
+                      int dtype, double rate, void* out, int mem) {
+  return guarded([&] {
+    smb_stft_plan* p = plan;
+    const int64_t out_frames = vocoder_frames("phase_vocoder", frames, rate);
+    if (batch < 0)
+      throw smb::invalid_argument("phase_vocoder: batch must be non-negative");
+    const size_t csz = 2 * dtype_size(dtype);
+    if (mem != SMB_MEM_DEVICE && mem != SMB_MEM_HOST)
+      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    if (batch == 0 || out_frames == 0) return;
+    p->ensure_device();
+    auto run = [&](const void* dz, void* dout, int64_t nb) {
+      run_vocoder(p, dz, dout, nb, frames, out_frames, dtype, rate);
+    };
+    if (mem == SMB_MEM_DEVICE) {
+      run(z, out, batch);
+      return;
+    }
+    const size_t bins = (size_t)p->geom.bins();
+    p->pipe.execute(p->dev->stream.use, z, out, batch, bins * (size_t)frames * csz,
+                    bins * (size_t)out_frames * csz, run);
+  });
+}
+
+int smb_time_stretch(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
+                     double rate, void* out, int mem) {
+  return guarded([&] {
+    smb_stft_plan* p = plan;
+    check_rate("time_stretch", rate);
+    check_signal("time_stretch", batch, n);
+    if (!p->nola())                                     // Stft.invert's precondition
+      throw smb::invalid_argument(smb::format(
+          "invert: cannot invert a %lld-point window advanced by %lld samples inside a "
+          "%lld-point frame (the overlap-added squared window must stay above 1e-10 of its "
+          "largest value at every position)",
+          (long long)p->geom.win_length, (long long)p->geom.hop, (long long)p->geom.fft));
+    const size_t esz = dtype_size(dtype);
+    if (mem != SMB_MEM_DEVICE && mem != SMB_MEM_HOST)
+      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    const int64_t out_len = stretch_length(n, rate);
+    const smb::FrameGeom g = p->frame_geom(n);
+    const int64_t out_frames = vocoder_frames("time_stretch", g.frames, rate);
+    if (batch == 0 || out_len == 0) return;
+    p->ensure_device();
+    cudaStream_t st = p->dev->stream.use;
+    const size_t bins = (size_t)p->geom.bins();
+    // transform -> vocoder -> invert on the plan's stream; the two spectra stay on the
+    // device in the plan's scratch (reused by the next call on the same stream)
+    auto run = [&](const void* dx, void* dout, int64_t nb) {
+      if (out_frames == 0) {                            // no frame: invert of nothing is zeros
+        CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * esz, st));
+        return;
+      }
+      void* spec = p->stretch_spec.ensure((size_t)nb * bins * (size_t)g.frames * 2 * esz);
+      void* voc = p->stretch_voc.ensure((size_t)nb * bins * (size_t)out_frames * 2 * esz);
+      run_spectrum(p, dx, nb, g, dtype, kSpecComplex, 1.0, spec);
+      run_vocoder(p, spec, voc, nb, g.frames, out_frames, dtype, rate);
+      run_invert(p, voc, dout, nb, out_frames, true, out_len, dtype, dtype);
+    };
+    if (mem == SMB_MEM_DEVICE) {
+      run(x, out, batch);
+      return;
+    }
+    p->pipe.execute(st, x, out, batch, (size_t)n * esz, (size_t)out_len * esz, run);
+  });
+}
+
+}  // extern "C"
+
+extern "C" {
 
 // ---- mel ---------------------------------------------------------------------
 

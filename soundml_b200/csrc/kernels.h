@@ -58,6 +58,19 @@ cudaError_t launch_istft2048(const IstftArgs& a, const float* window_scaled, con
                              const float2* tw_base, long long batch, int sm_count,
                              cudaStream_t st);
 
+// ---- phase vocoder (effects_kernels.cu) ------------------------------------------
+// z [rows, frames] complex -> out [rows, out_frames] complex of the same width; output
+// frame t reads source position t * rate (librosa 0.11 phase_vocoder, DESIGN.md 4.8).
+struct PhaseVocoderArgs {
+  const void* z;            // float2 or double2
+  void* out;
+  long long rows;           // batch * bins
+  long long frames, out_frames;
+  double rate;
+  int f64;
+};
+cudaError_t launch_phase_vocoder(const PhaseVocoderArgs& a, cudaStream_t st);
+
 // ---- fast path: fft 2048, float32, fused frame+window+rFFT+|X|^p(+mel) -------
 // Tile shape of the fused CUDA-core kernel: a group of kFastTile warps transforms
 // kFastTile consecutive frames, one per warp.
