@@ -312,6 +312,30 @@ typedef struct smb_resample_layout {
 } smb_resample_layout;
 int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
                               smb_resample_layout* out);
+/* The overlap-save plan one stage (or FIR) runs when it takes the overlap-save path,
+ * computed on the host (no device state is touched).  Block b transforms the inputs
+ * [index*b - 2k - delta, +n) at length n and inverts at length w; it writes the
+ * outputs after those of the block before it up to hi(index) (resample.ml:1309-1319).
+ * kernel is SMB_OLS_NONE when the stage has no overlap-save plan (it runs on another
+ * executor; every other field is then 0).  For a resampler stage this is the plan of
+ * the planned executor (smb_resample_plan_set_executor may force the direct kernel);
+ * for a FIR it is what SMB_EXEC_OLS runs (SMB_EXEC_PLANNED takes it from 17 taps up). */
+enum { SMB_OLS_NONE = 0, SMB_OLS_2048 = 1, SMB_OLS_STOCKHAM = 2 };
+typedef struct smb_ols_geometry {
+  int kernel;        /* SMB_OLS_*: none, ols2048_kernel (one warp per block, n = 2048) or
+                        ols_kernel (one CTA per block, any power of two n) */
+  int64_t n, b, delta;  /* block length, hop between blocks, input shift */
+  int64_t w;         /* inverse length: n, n / m (alias fold) or n * l (periodic extension) */
+  int64_t l, m, k;   /* stage factors and group delay (l = m = 1 for a FIR) */
+  int polyphase;     /* an xL stage run as its l branches at the input rate (w = n) */
+  int full_inverse;  /* a /m stage inverted at length n, every m-th sample kept (w = n) */
+} smb_ols_geometry;
+int smb_resample_stage_ols(const smb_resample_plan* plan, int stage, smb_ols_geometry* out);
+int smb_fir_ols(const smb_fir_plan* plan, smb_ols_geometry* out);
+/* Blocks the overlap-save executor launches per signal for n_out outputs: the fewest
+ * whose runs cover [0, n_out); -1 (SMB_EINVAL in smb_last_error) for a geometry no plan
+ * reports. */
+int64_t smb_ols_blocks(const smb_ols_geometry* g, int64_t n_out);
 /* Config.pp one-liner, e.g. "resample(44100 -> 16000 Hz, quality=high, ...)". */
 int smb_resample_describe(const smb_resample_plan* plan, char* buf, size_t cap);
 int64_t smb_resample_l(const smb_resample_plan* plan);

@@ -60,6 +60,15 @@ class ResampleLayout(C.Structure):
 
 FORMS = {0: "direct", 1: "ols", 2: "window", 3: "row"}
 
+
+class OlsGeometry(C.Structure):
+    """``smb_ols_geometry`` (include/soundml_b200.h)."""
+    _fields_ = [("kernel", C.c_int)] + [(name, C.c_int64) for name in (
+        "n", "b", "delta", "w", "l", "m", "k")] + [("polyphase", C.c_int), ("full_inverse", C.c_int)]
+
+
+OLS_KERNELS = {0: "direct", 1: "ols2048", 2: "ols"}
+
 SIGNATURES = {
     "smb_last_error": (C.c_char_p, []),
     "smb_version": (C.c_char_p, []),
@@ -120,6 +129,9 @@ SIGNATURES = {
     "smb_resample_plan_sync": (_int, [_vp]),
     "smb_resample_plan_set_executor": (_int, [_vp, _int]),
     "smb_resample_stage_layout": (_int, [_vp, _int, _int, C.POINTER(ResampleLayout)]),
+    "smb_resample_stage_ols": (_int, [_vp, _int, C.POINTER(OlsGeometry)]),
+    "smb_fir_ols": (_int, [_vp, C.POINTER(OlsGeometry)]),
+    "smb_ols_blocks": (_i64, [C.POINTER(OlsGeometry), _i64]),
     "smb_resample_describe": (_int, [_vp, C.c_char_p, _sz]),
     "smb_resample_l": (_i64, [_vp]),
     "smb_resample_m": (_i64, [_vp]),

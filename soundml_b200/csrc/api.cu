@@ -688,6 +688,25 @@ struct smb_mel_plan {
   }
 };
 
+// The geometry fields of plan p's launch arguments (signal pointers and extents unset).
+static smb::OlsArgs ols_args(const smb::OlsPlan& p) {
+  smb::OlsArgs a{};
+  a.L = (int)p.l; a.M = (int)p.m; a.K = (int)p.k;
+  a.N = (int)p.n; a.B = (int)p.b; a.delta = (int)p.delta; a.W = (int)p.w;
+  a.polyphase = p.polyphase ? 1 : 0;
+  return a;
+}
+
+// The kernel that runs plan p (SMB_OLS_*): the warp-per-block kernel wherever it
+// supports the geometry, the Stockham kernel otherwise.
+static int ols_kernel_of(const smb::OlsPlan& p) {
+  if (!p.ok) return SMB_OLS_NONE;
+  if (smb::ols2048_supports(ols_args(p))) return SMB_OLS_2048;
+  if (p.full_inverse || p.polyphase)
+    throw smb::invalid_argument("soundml_b200: this overlap-save plan needs the N = 2048 kernel");
+  return SMB_OLS_STOCKHAM;
+}
+
 // Device copies of one overlap-save plan.
 struct OlsDevice {
   smb::OlsPlan plan;
@@ -695,7 +714,6 @@ struct OlsDevice {
   device_ptr<float2> d_tw;
   device_ptr<float2> d_tw_pass, d_tw_base;             // tables of the N = 2048 kernel
   int sm_count = 0;
-  bool fast = true;                                     // the N = 2048 kernel may be used
   void upload_from(const smb::OlsPlan& p) {
     plan = p;
     if (!p.ok) return;
@@ -730,21 +748,16 @@ struct OlsDevice {
   }
   void run(const float* x, int64_t batch, int64_t n, int64_t n_out, float* out,
            cudaStream_t st) const {
-    smb::OlsArgs a{};
+    smb::OlsArgs a = ols_args(plan);
     a.x = x;
     a.out = out;
     a.n = n;
     a.n_out = n_out;
     a.blocks = plan.blocks_for(n_out);
-    a.L = (int)plan.l; a.M = (int)plan.m; a.K = (int)plan.k;
-    a.N = (int)plan.n; a.B = (int)plan.b; a.delta = (int)plan.delta; a.W = (int)plan.w;
     a.H = d_h.get();
     a.tw = d_tw.get();
-    a.polyphase = plan.polyphase ? 1 : 0;
-    if (fast && d_tw_pass && smb::ols2048_supports(a))
+    if (ols_kernel_of(plan) == SMB_OLS_2048)
       CK(smb::launch_ols2048(a, d_tw_pass.get(), d_tw_base.get(), batch, sm_count, st));
-    else if (plan.full_inverse || plan.polyphase)
-      throw smb::invalid_argument("soundml_b200: this overlap-save plan needs the N = 2048 kernel");
     else
       CK(smb::launch_ols(a, batch, st));
   }
@@ -2299,6 +2312,38 @@ int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
     }
     *out = r;
   });
+}
+static void ols_geometry_of(const smb::OlsPlan& p, smb_ols_geometry* out) {
+  smb_ols_geometry g{};
+  g.kernel = ols_kernel_of(p);
+  if (g.kernel != SMB_OLS_NONE) {
+    g.n = p.n; g.b = p.b; g.delta = p.delta; g.w = p.w;
+    g.l = p.l; g.m = p.m; g.k = p.k;
+    g.polyphase = p.polyphase ? 1 : 0;
+    g.full_inverse = p.full_inverse ? 1 : 0;
+  }
+  *out = g;
+}
+int smb_resample_stage_ols(const smb_resample_plan* plan, int stage, smb_ols_geometry* out) {
+  return guarded([&] {
+    if (stage < 0 || stage >= (int)plan->plan.stages.size())
+      throw smb::invalid_argument("stage_ols: no such stage");
+    ols_geometry_of(smb::ols_plan_for_stage(plan->plan.stages[(size_t)stage]), out);
+  });
+}
+int smb_fir_ols(const smb_fir_plan* plan, smb_ols_geometry* out) {
+  return guarded([&] { ols_geometry_of(smb::ols_plan_for_fir(plan->h), out); });
+}
+int64_t smb_ols_blocks(const smb_ols_geometry* g, int64_t n_out) {
+  int64_t r = -1;
+  guarded([&] {
+    if (g->kernel == SMB_OLS_NONE || g->b < 1 || g->l < 1 || g->m < 1 || (g->l > 1 && g->m != 1))
+      throw smb::invalid_argument("ols_blocks: not an overlap-save geometry");
+    smb::OlsPlan p;
+    p.n = g->n; p.b = g->b; p.delta = g->delta; p.l = g->l; p.m = g->m; p.k = g->k;
+    r = p.blocks_for(n_out);
+  });
+  return r;
 }
 int smb_resample_describe(const smb_resample_plan* plan, char* buf, size_t cap) {
   return guarded([&] {

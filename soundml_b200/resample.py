@@ -95,6 +95,13 @@ class Config:
             groups, g = r.groups, g + 1
         return out
 
+    def ols_geometry(self, i):
+        """The overlap-save plan ``apply`` runs for stage ``i`` under the planned
+        executor; see :func:`ols_geometry_dict`.  Host-only."""
+        g = _lib.OlsGeometry()
+        _lib.check(_lib.lib.smb_resample_stage_ols(self._h, i, C.byref(g)))
+        return ols_geometry_dict(g)
+
     def stage_prototype(self, i):
         n = C.c_int64()
         _lib.check(_lib.lib.smb_resample_stage_prototype(self._h, i, None, C.byref(n)))
@@ -102,6 +109,25 @@ class Config:
         _lib.check(_lib.lib.smb_resample_stage_prototype(
             self._h, i, out.ctypes.data_as(C.POINTER(C.c_double)), C.byref(n)))
         return out
+
+
+def ols_geometry_dict(g):
+    """``smb_ols_geometry`` as a dict: ``kernel`` is "ols2048" (one warp per block,
+    n = 2048), "ols" (one CTA per block, Stockham) or "direct" (no overlap-save plan: the
+    stage runs on another executor; every other field 0); block index j reads the inputs [j b - 2k - delta, +n), is
+    inverted at length w and writes the outputs up to hi(j) (resample.ml:1309-1319).
+    ``blocks_for(n_out)`` is the number of blocks launched per signal."""
+    d = {name: int(getattr(g, name)) for name, _ in g._fields_}
+    d["kernel"] = _lib.OLS_KERNELS[g.kernel]
+    d["polyphase"], d["full_inverse"] = bool(g.polyphase), bool(g.full_inverse)
+
+    def blocks_for(n_out):
+        r = _lib.lib.smb_ols_blocks(C.byref(g), int(n_out))
+        if r < 0:
+            raise ValueError(_lib.last_error())
+        return int(r)
+    d["blocks_for"] = blocks_for
+    return d
 
 
 def _check(op, x, allow_f64=False):
@@ -345,6 +371,13 @@ class Fir:
         h, self._h = getattr(self, "_h", None), None
         if h and getattr(_lib, "lib", None) is not None:      # not during interpreter teardown
             _lib.lib.smb_fir_plan_destroy(h)
+
+    def ols_geometry(self):
+        """The overlap-save plan ``apply(x, "ols")`` runs (``"auto"`` takes it from
+        17 taps up); see :func:`ols_geometry_dict`.  Host-only."""
+        g = _lib.OlsGeometry()
+        _lib.check(_lib.lib.smb_fir_ols(self._h, C.byref(g)))
+        return ols_geometry_dict(g)
 
     def apply(self, x, method="auto", out=None):
         """``method``: ``"auto"`` (overlap-save from 17 taps up, else the direct
