@@ -223,6 +223,34 @@ size_t dtype_size(int dtype) {
 
 const double kTwoPi = 6.283185307179586476925286766559;
 
+// The inter-pass twiddles of the warp FFT 1024 (32 x 32): W_1024^(k1 n2) at [k1][n2].
+std::vector<float2> fft1024_pass_twiddles() {
+  std::vector<float2> pass(1024);
+  for (int k1 = 0; k1 < 32; ++k1)
+    for (int n2 = 0; n2 < 32; ++n2) {
+      const double a = kTwoPi * double(k1 * n2) / 1024.0;
+      pass[(size_t)(k1 * 32 + n2)] = make_float2((float)std::cos(a), (float)-std::sin(a));
+    }
+  return pass;
+}
+
+// Puts weight g at (row r, element k < 32) of a tensor-core resampler B slice that starts
+// at float `base` and holds `rows` rows per split: its tf32 piece hi (the float's leading
+// 10 fraction bits, exact) in the first split and lo = g - hi in the second, each at the
+// K-major SWIZZLE_128B cell (128-byte rows, 16-byte chunk index XOR row mod 8).
+void put_tf32_split(std::vector<float>& img, size_t base, int64_t rows, int64_t r, int64_t k, double g) {
+  const float gf = (float)g;
+  uint32_t bits;
+  std::memcpy(&bits, &gf, 4);
+  bits &= 0xFFFFE000u;
+  float hi;
+  std::memcpy(&hi, &bits, 4);
+  const float lo = (float)(g - (double)hi);
+  const size_t cell = (size_t)(r * 32 + ((((k >> 2) ^ (r & 7)) << 2) | (k & 3)));
+  img[base + cell] = hi;
+  img[base + (size_t)rows * 32 + cell] = lo;
+}
+
 }  // namespace
 
 // A plan's tables, scratch and stream belong to the device that was current when it was
@@ -282,18 +310,13 @@ struct smb_stft_plan {
       std::vector<float> w32(2048, 0.0f);
       for (int64_t j = 0; j < n; ++j) w32[(size_t)j] = (float)window[(size_t)j];
       d->d_window32 = upload(w32);
-      std::vector<float2> pass(1024), post(512);
-      for (int k1 = 0; k1 < 32; ++k1)
-        for (int n2 = 0; n2 < 32; ++n2) {
-          const double a = kTwoPi * double(k1 * n2) / 1024.0;
-          pass[(size_t)(k1 * 32 + n2)] = make_float2((float)std::cos(a), (float)-std::sin(a));
-        }
+      std::vector<float2> post(512);
       for (int j = 0; j < 16; ++j)
         for (int l = 0; l < 32; ++l) {
           const double a = kTwoPi * double(l + 32 * j) / 2048.0;
           post[(size_t)(j * 32 + l)] = make_float2((float)std::cos(a), (float)-std::sin(a));
         }
-      d->d_tw_pass = upload(pass);
+      d->d_tw_pass = upload(fft1024_pass_twiddles());
       d->d_tw_post = upload(post);
       // The 32-point DFT in real arithmetic, F[n = (k, c')][j = (m, c)] with
       // (re, im) interleaved: out_re = sum in_re cos + in_im sin, out_im = sum
@@ -718,17 +741,12 @@ struct OlsDevice {
     plan = p;
     if (!p.ok) return;
     if (p.n == 2048 && (p.l == 1 || p.polyphase)) {
-      std::vector<float2> pass(1024), base(32);
-      for (int k1 = 0; k1 < 32; ++k1)
-        for (int n2 = 0; n2 < 32; ++n2) {
-          const double a = kTwoPi * double(k1 * n2) / 1024.0;
-          pass[(size_t)(k1 * 32 + n2)] = make_float2((float)std::cos(a), (float)-std::sin(a));
-        }
+      std::vector<float2> base(32);
       for (int l = 0; l < 32; ++l) {
         const double a = kTwoPi * double(l) / 2048.0;
         base[(size_t)l] = make_float2((float)std::cos(a), (float)-std::sin(a));
       }
-      d_tw_pass = upload(pass);
+      d_tw_pass = upload(fft1024_pass_twiddles());
       d_tw_base = upload(base);
       int device = 0;
       CK(cudaGetDevice(&device));
@@ -959,19 +977,8 @@ struct GemmDevice {
         const int ri = run_at[(size_t)ch][(size_t)tcol];
         if (ri < 0) return false;                               // (cannot happen: the runs cover every nonzero)
         const Run run = runs[(size_t)ri];
-        const double gv = s.bank[(size_t)(ph * taps + t)];
-        const float gf = (float)gv;
-        uint32_t bits;
-        std::memcpy(&bits, &gf, 4);
-        bits &= 0xFFFFE000u;
-        float hi;
-        std::memcpy(&hi, &bits, 4);
-        const float lo = (float)(gv - (double)hi);
-        const int64_t rr = tcol - run.start;                     // row inside the run
-        const size_t cell = (size_t)(rr * 32 + ((((kk >> 2) ^ (rr & 7)) << 2) | (kk & 3)));
         const size_t base = ((size_t)chunk_meta[(size_t)ch].x + (size_t)run.bytes_at) / 4;
-        img[base + cell] = hi;
-        img[base + (size_t)run.width * 32 + cell] = lo;
+        put_tf32_split(img, base, run.width, tcol - run.start, kk, s.bank[(size_t)(ph * taps + t)]);
       }
     }
     a.slices = (int)slice_meta.size();
@@ -1064,21 +1071,10 @@ struct GemmDevice {
         const int64_t d = (col * m) / l, ph = (col * m) % l;
         for (int64_t t = 0; t < taps; ++t) {
           const int64_t j = d + t;                               // row of G
-          const double gv = s.bank[(size_t)(ph * taps + t)];
-          const float gf = (float)gv;
-          uint32_t bits;
-          std::memcpy(&bits, &gf, 4);
-          bits &= 0xFFFFE000u;                                   // tf32 piece, exact
-          float hi;
-          std::memcpy(&hi, &bits, 4);
-          const float lo = (float)(gv - (double)hi);
           const int64_t ch = j / 32 - g.chunk_begin, kk = j % 32;
           const int4 mt = meta[(size_t)ch];
-          const int64_t rr = r - mt.y;                           // row inside the stored slice
-          const size_t cell = (size_t)(rr * 32 + ((((kk >> 2) ^ (rr & 7)) << 2) | (kk & 3)));
-          const size_t base = (size_t)mt.x / 4;
-          img[base + cell] = hi;
-          img[base + (size_t)mt.z * 32 + cell] = lo;
+          // row r - mt.y of the stored slice
+          put_tf32_split(img, (size_t)mt.x / 4, mt.z, r - mt.y, kk, s.bank[(size_t)(ph * taps + t)]);
         }
       }
       g.d_meta = upload(meta);

@@ -1,7 +1,8 @@
 // 32-point forward complex FFT held entirely in registers (one thread, natural
 // order in and out): n = 8a + b, k = c + 4d -> eight 4-point DFTs over a, twiddle
-// W32^(bc) with compile-time constants, four 8-point DFTs over b.  Shared by the
-// fused STFT kernel and its micro-benchmark.
+// W32^(bc) with compile-time constants, four 8-point DFTs over b.  Also the warp-wide
+// FFT 1024 built from it and the split twiddles of the real FFT 2048.  Shared by the
+// fft-2048 STFT, overlap-save and iSTFT kernels and the micro-benchmark.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -26,6 +27,19 @@ __device__ constexpr float kW32S[32] = {
     0.7071067811865475f, 0.8314696123025452f, 0.9238795325112865f, 0.9807852804032303f,
     1.0f, 0.9807852804032304f, 0.9238795325112866f, 0.8314696123025455f,
     0.7071067811865477f, 0.5555702330196022f, 0.3826834323650904f, 0.19509032201612872f};
+
+// W_64^k2 = exp(-2 pi i k2 / 64), k2 < 16: the split twiddle W_2048^(l + 32 k2) of the
+// real FFT 2048 is the lane's W_2048^l (a 32-entry table) times one of these constants.
+__device__ constexpr float kW64C[16] = {
+    1.0f, 0.9951847266721969f, 0.9807852804032304f, 0.9569403357322088f,
+    0.9238795325112867f, 0.881921264348355f, 0.8314696123025452f, 0.773010453362737f,
+    0.7071067811865476f, 0.6343932841636455f, 0.5555702330196023f, 0.4713967368259978f,
+    0.38268343236508984f, 0.29028467725446233f, 0.19509032201612833f, 0.09801714032956077f};
+__device__ constexpr float kW64S[16] = {
+    0.0f, -0.0980171403295606f, -0.19509032201612825f, -0.2902846772544623f,
+    -0.3826834323650898f, -0.47139673682599764f, -0.5555702330196022f, -0.6343932841636455f,
+    -0.7071067811865475f, -0.773010453362737f, -0.8314696123025452f, -0.8819212643483549f,
+    -0.9238795325112867f, -0.9569403357322089f, -0.9807852804032304f, -0.9951847266721968f};
 
 __device__ __forceinline__ float2 cadd(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
 __device__ __forceinline__ float2 csub(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
@@ -252,6 +266,34 @@ __device__ __forceinline__ void fft32(float2 (&x)[32]) {
 #else
   fft32_scalar(x);
 #endif
+}
+
+// Forward complex FFT of 1024 points spread over a warp, as 32 x 32 with the twiddle
+// W_1024^(k1 n2) and one transposition through the warp's padded buffer `ex`
+// ([32][kFft1024ExStride] complex): in, lane = n mod 32 and register = n div 32; out,
+// lane = k mod 32 and register = k div 32.  tw4 holds the twiddles as
+// [16][32] x (k1, k1 + 1) pairs.
+constexpr int kFft1024ExStride = 34;   // padded transpose row (complex)
+__device__ __forceinline__ void fft1024(float2 (&a)[32], float2* ex, const float4* tw4, int lane) {
+  fft32(a);                                     // a[k1] = Y[n2 = lane][k1]
+#pragma unroll
+  for (int k1 = 0; k1 < 32; k1 += 2) {          // twiddle W_1024^(k1 n2), transpose
+    const float4 t = tw4[(k1 >> 1) * 32 + lane];
+    ex[k1 * kFft1024ExStride + lane] =
+        k1 == 0 ? a[0] : make_float2(a[k1].x * t.x - a[k1].y * t.y, a[k1].x * t.y + a[k1].y * t.x);
+    ex[(k1 + 1) * kFft1024ExStride + lane] = make_float2(a[k1 + 1].x * t.z - a[k1 + 1].y * t.w,
+                                                         a[k1 + 1].x * t.w + a[k1 + 1].y * t.z);
+  }
+  __syncwarp();
+  const float4* e4 = reinterpret_cast<const float4*>(ex + lane * kFft1024ExStride);
+#pragma unroll
+  for (int n2 = 0; n2 < 32; n2 += 2) {
+    const float4 v = e4[n2 >> 1];
+    a[n2] = make_float2(v.x, v.y);
+    a[n2 + 1] = make_float2(v.z, v.w);
+  }
+  __syncwarp();
+  fft32(a);                                     // a[k2] = Z[lane + 32 k2]
 }
 
 }  // namespace fft32impl

@@ -41,48 +41,13 @@ constexpr int kHalf = 1024;
 constexpr int kBins = 1025;
 constexpr int kWarps = 16;
 constexpr int kTileStride = 17;                     // float2 per bin row: 16 frames + 1 pad
-constexpr int kExStride = 34;
-constexpr int kExFloats = 32 * kExStride * 2;
+constexpr int kExFloats = 32 * kFft1024ExStride * 2;
 // shared by the spectrum tile [1025][17] complex and, after it, the 16 transposes
 constexpr int kWorkFloats = ((kBins * kTileStride * 2 + 3) / 4) * 4;
 static_assert(kWorkFloats >= kWarps * kExFloats, "transposes fit the tile space");
 
-__device__ constexpr float kW64C[16] = {
-    1.0f, 0.9951847266721969f, 0.9807852804032304f, 0.9569403357322088f,
-    0.9238795325112867f, 0.881921264348355f, 0.8314696123025452f, 0.773010453362737f,
-    0.7071067811865476f, 0.6343932841636455f, 0.5555702330196023f, 0.4713967368259978f,
-    0.38268343236508984f, 0.29028467725446233f, 0.19509032201612833f, 0.09801714032956077f};
-__device__ constexpr float kW64S[16] = {
-    0.0f, -0.0980171403295606f, -0.19509032201612825f, -0.2902846772544623f,
-    -0.3826834323650898f, -0.47139673682599764f, -0.5555702330196022f, -0.6343932841636455f,
-    -0.7071067811865475f, -0.773010453362737f, -0.8314696123025452f, -0.8819212643483549f,
-    -0.9238795325112867f, -0.9569403357322089f, -0.9807852804032304f, -0.9951847266721968f};
-
 __device__ __forceinline__ long long ceil_div_ll(long long a, long long b) {   // b > 0
   return a >= 0 ? (a + b - 1) / b : -((-a) / b);
-}
-
-// Forward complex FFT of 1024 points spread over a warp (see ols2048.cu).
-__device__ __forceinline__ void fft1024(float2 (&a)[32], float2* ex, const float4* tw4, int lane) {
-  fft32(a);
-#pragma unroll
-  for (int k1 = 0; k1 < 32; k1 += 2) {
-    const float4 t = tw4[(k1 >> 1) * 32 + lane];
-    ex[k1 * kExStride + lane] =
-        k1 == 0 ? a[0] : make_float2(a[k1].x * t.x - a[k1].y * t.y, a[k1].x * t.y + a[k1].y * t.x);
-    ex[(k1 + 1) * kExStride + lane] = make_float2(a[k1 + 1].x * t.z - a[k1 + 1].y * t.w,
-                                                  a[k1 + 1].x * t.w + a[k1 + 1].y * t.z);
-  }
-  __syncwarp();
-  const float4* e4 = reinterpret_cast<const float4*>(ex + lane * kExStride);
-#pragma unroll
-  for (int n2 = 0; n2 < 32; n2 += 2) {
-    const float4 v = e4[n2 >> 1];
-    a[n2] = make_float2(v.x, v.y);
-    a[n2 + 1] = make_float2(v.z, v.w);
-  }
-  __syncwarp();
-  fft32(a);
 }
 
 struct Istft2048Params {

@@ -5,27 +5,13 @@
 // double: mel.ml:228-231).  It is the always-available path; fft 2048 float32
 // dispatches to the fused kernel in stft2048.cu instead.
 #include "kernels.h"
+#include "stft_stage.cuh"
 
 #include <cstdio>
 
 namespace smb {
 
 std::atomic<long long> g_launch_count{0};
-
-__device__ __forceinline__ long long source_index(const FrameGeom& g, long long q) {
-  // padded position q -> source sample, -1 for a constant fill.
-  long long s = q - g.left;
-  if (s >= 0 && s < g.n) return s;
-  if (g.pad == 0) {                       // reflect, stft.ml:300-305
-    if (g.n == 1) return 0;
-    const long long period = 2 * (g.n - 1);
-    long long r = s % period;
-    if (r < 0) r += period;
-    return r < g.n ? r : period - r;
-  }
-  if (g.pad == 2) return s < 0 ? 0 : g.n - 1;   // edge
-  return -1;                                     // constant
-}
 
 template <typename T> struct OutTraits;
 template <> struct OutTraits<float> {
@@ -68,7 +54,7 @@ __global__ void stft_generic_kernel(const T* __restrict__ x, FrameGeom g,
   for (int f = 0; f < nf; ++f) {
     const long long start = (p0 + f) * g.hop;
     for (int j = threadIdx.x; j < N; j += blockDim.x) {
-      const long long s = source_index(g, start + j);
+      const long long s = stage::src_index(g, start + j);
       const double v = s >= 0 ? (double)xs[s] : g.pad_value;
       const double wv = window[j] * v;
       int dst = j;

@@ -38,46 +38,10 @@ using namespace fft32impl;
 constexpr int kN = 2048;
 constexpr int kHalf = 1024;
 constexpr int kWarps = 16;
-constexpr int kExStride = 34;                       // padded transpose row (complex)
-constexpr int kExFloats = 32 * kExStride * 2;       // per-warp transpose buffer
-
-__device__ constexpr float kW64C[16] = {
-    1.0f, 0.9951847266721969f, 0.9807852804032304f, 0.9569403357322088f,
-    0.9238795325112867f, 0.881921264348355f, 0.8314696123025452f, 0.773010453362737f,
-    0.7071067811865476f, 0.6343932841636455f, 0.5555702330196023f, 0.4713967368259978f,
-    0.38268343236508984f, 0.29028467725446233f, 0.19509032201612833f, 0.09801714032956077f};
-__device__ constexpr float kW64S[16] = {
-    0.0f, -0.0980171403295606f, -0.19509032201612825f, -0.2902846772544623f,
-    -0.3826834323650898f, -0.47139673682599764f, -0.5555702330196022f, -0.6343932841636455f,
-    -0.7071067811865475f, -0.773010453362737f, -0.8314696123025452f, -0.8819212643483549f,
-    -0.9238795325112867f, -0.9569403357322089f, -0.9807852804032304f, -0.9951847266721968f};
+constexpr int kExFloats = 32 * kFft1024ExStride * 2;   // per-warp transpose buffer
 
 __device__ __forceinline__ float2 cmulf(float2 a, float2 b) {
   return make_float2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x);
-}
-
-// Forward complex FFT of 1024 points spread over a warp: in, lane = n mod 32 and
-// register = n div 32; out, lane = k mod 32 and register = k div 32.
-__device__ __forceinline__ void fft1024(float2 (&a)[32], float2* ex, const float4* tw4, int lane) {
-  fft32(a);                                     // a[k1] = Y[n2 = lane][k1]
-#pragma unroll
-  for (int k1 = 0; k1 < 32; k1 += 2) {          // twiddle W_1024^(k1 n2), transpose
-    const float4 t = tw4[(k1 >> 1) * 32 + lane];
-    ex[k1 * kExStride + lane] =
-        k1 == 0 ? a[0] : make_float2(a[k1].x * t.x - a[k1].y * t.y, a[k1].x * t.y + a[k1].y * t.x);
-    ex[(k1 + 1) * kExStride + lane] = make_float2(a[k1 + 1].x * t.z - a[k1 + 1].y * t.w,
-                                                  a[k1 + 1].x * t.w + a[k1 + 1].y * t.z);
-  }
-  __syncwarp();
-  const float4* e4 = reinterpret_cast<const float4*>(ex + lane * kExStride);
-#pragma unroll
-  for (int n2 = 0; n2 < 32; n2 += 2) {
-    const float4 v = e4[n2 >> 1];
-    a[n2] = make_float2(v.x, v.y);
-    a[n2 + 1] = make_float2(v.z, v.w);
-  }
-  __syncwarp();
-  fft32(a);                                     // a[k2] = Z[lane + 32 k2]
 }
 
 struct Ols2048Params {

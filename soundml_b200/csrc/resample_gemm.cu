@@ -29,6 +29,7 @@
 //      accumulators, transposed through shared memory so global stores are
 //      row-contiguous (a block-row is L consecutive outputs).
 #include "kernels.h"
+#include "sm100.cuh"
 
 #include <algorithm>
 #include <cstdint>
@@ -47,35 +48,6 @@ constexpr int kRowsPerWarp = kRows / kProducerWarps;
 constexpr int kMmaWarp = kProducerWarps;
 constexpr int kThreads = kProducers + 32;  // producer warps + 1 TMA/MMA warp
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  while (!done) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  }
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes,
-                                         uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-      : "memory");
-}
 // K-major, SWIZZLE_128B shared-memory matrix descriptor (8-row groups 1024 B apart).
 __device__ __forceinline__ uint64_t umma_desc(uint32_t addr) {
   uint64_t d = 0;
@@ -95,11 +67,8 @@ __device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint6
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-               ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
+// loads and waits: the values are ready on return
+__device__ __forceinline__ void tmem_ld16_waited(uint32_t taddr, float (&v)[16]) {
   uint32_t r[16];
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
@@ -111,10 +80,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
   for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
 }
 
 // Warps 0-3: producers (gather + split + swizzled store of A) and, at the end,
@@ -153,11 +118,7 @@ resample_gemm_kernel(const GemmResampleArgs a) {
     mbar_init(bar_done, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == kMmaWarp) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(&tmem_base_slot)), "r"(a.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == kMmaWarp) tmem_alloc(&tmem_base_slot, a.tmem_cols);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -282,9 +243,9 @@ resample_gemm_kernel(const GemmResampleArgs a) {
     const bool two_main = a.chunks > 1;
     for (int col = 0; col < a.n_pad; col += 16) {
       float d0[16], d1[16], dc[16];
-      tmem_ld16(acc_main0 + lane_base + col, d0);
-      tmem_ld16(acc_corr + lane_base + col, dc);
-      if (two_main) tmem_ld16(acc_main1 + lane_base + col, d1);
+      tmem_ld16_waited(acc_main0 + lane_base + col, d0);
+      tmem_ld16_waited(acc_corr + lane_base + col, dc);
+      if (two_main) tmem_ld16_waited(acc_main1 + lane_base + col, d1);
       float4* dst = reinterpret_cast<float4*>(tile + tid * pitch + col);
 #pragma unroll
       for (int e = 0; e < 16; e += 4) {
@@ -327,9 +288,7 @@ resample_gemm_kernel(const GemmResampleArgs a) {
 teardown:
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if (warp == kMmaWarp)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem),
-                 "r"(a.tmem_cols) : "memory");
+  if (warp == kMmaWarp) tmem_dealloc(tmem, a.tmem_cols);
 }
 
 
@@ -407,18 +366,6 @@ __device__ __forceinline__ void umma_tf32_ta(uint32_t tmem_d, uint32_t tmem_a, u
       ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc)
       : "memory");
 }
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]),
-        "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]),
-        "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() {
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 
 __global__ void __launch_bounds__(kRowsThreads, 1)
 resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int total_tiles) {
@@ -461,11 +408,7 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
   }
   for (int i = tid; i < a.chunks; i += kRowsThreads) s_chunk[i] = a.chunk_meta[i];
   for (int i = tid; i < a.slices; i += kRowsThreads) s_slice[i] = a.slice_meta[i];
-  if (warp == kMmaWarp) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(&tmem_base_slot)), "r"(a.tmem_cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == kMmaWarp) tmem_alloc(&tmem_base_slot, a.tmem_cols);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -800,6 +743,8 @@ resample_rows_kernel(const GemmRowsArgs a, const int tiles_per_clip, const int t
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
+  // tmem_dealloc written out: through the wrapper, nvcc 12.9 allocates this kernel's
+  // registers differently (same instructions, other register numbers)
   if (warp == kMmaWarp)
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem),
                  "r"(a.tmem_cols) : "memory");

@@ -48,6 +48,7 @@
 
 #include "fft32.cuh"
 #include "kernels.h"
+#include "stft_stage.cuh"
 
 namespace smb {
 
@@ -67,66 +68,6 @@ constexpr int kMelOutOff = 1032;         // the mel partial sums of a frame sit 
 constexpr int kExStride = 34;            // padded transpose row (complex): 16-byte rows, conflict-free
 
 using namespace fft32impl;
-
-// W_64^k2 = exp(-2 pi i k2 / 64), k2 < 16: the post-split twiddle W_2048^(l + 32 k2)
-// is the lane's W_2048^l (a 32-entry table) times one of these constants.
-__device__ constexpr float kW64C[16] = {
-    1.0f, 0.9951847266721969f, 0.9807852804032304f, 0.9569403357322088f,
-    0.9238795325112867f, 0.881921264348355f, 0.8314696123025452f, 0.773010453362737f,
-    0.7071067811865476f, 0.6343932841636455f, 0.5555702330196023f, 0.4713967368259978f,
-    0.38268343236508984f, 0.29028467725446233f, 0.19509032201612833f, 0.09801714032956077f};
-__device__ constexpr float kW64S[16] = {
-    0.0f, -0.0980171403295606f, -0.19509032201612825f, -0.2902846772544623f,
-    -0.3826834323650898f, -0.47139673682599764f, -0.5555702330196022f, -0.6343932841636455f,
-    -0.7071067811865475f, -0.773010453362737f, -0.8314696123025452f, -0.8819212643483549f,
-    -0.9238795325112867f, -0.9569403357322089f, -0.9807852804032304f, -0.9951847266721968f};
-
-__device__ __forceinline__ long long src_index(const FrameGeom& g, long long q) {
-  long long s = q - g.left;
-  if (s >= 0 && s < g.n) return s;
-  if (g.pad == 0) {
-    if (g.n == 1) return 0;
-    const long long period = 2 * (g.n - 1);
-    long long r = s % period;
-    if (r < 0) r += period;
-    return r < g.n ? r : period - r;
-  }
-  if (g.pad == 2) return s < 0 ? 0 : g.n - 1;
-  return -1;
-}
-
-__device__ __forceinline__ void group_sync(int group) {
-  asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "r"(kGroupThreads) : "memory");
-}
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  while (!done) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  }
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-      : "memory");
-}
 
 struct Params {
   Stft2048Args a;
@@ -178,36 +119,14 @@ __device__ __forceinline__ bool stage_tile(const Params& p, int b, int t, float*
   const int lo = (int)max(0LL, min((long long)span, -s0));
   const int hi = (int)max((long long)lo, min((long long)span, g.n - s0));
   for (int i = gtid; i < lo; i += kGroupThreads) {
-    const long long s = src_index(g, q0 + i);
+    const long long s = stage::src_index(g, q0 + i);
     sSamples[i] = s >= 0 ? __ldg(xs + s) : (float)g.pad_value;
   }
   for (int i = hi + gtid; i < span; i += kGroupThreads) {
-    const long long s = src_index(g, q0 + i);
+    const long long s = stage::src_index(g, q0 + i);
     sSamples[i] = s >= 0 ? __ldg(xs + s) : (float)g.pad_value;
   }
-  const float* src = xs + s0;                       // src + i is valid for i in [lo, hi)
-  const unsigned base = (unsigned)__cvta_generic_to_shared(sSamples);
-  const size_t addr = reinterpret_cast<size_t>(src);
-  if ((addr & 15) == 0) {
-    const int head = min(hi, (lo + 3) & ~3), tail = max(head, hi & ~3);
-    for (int i = lo + gtid; i < head; i += kGroupThreads)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = head + 4 * gtid; i < tail; i += 4 * kGroupThreads)
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = tail + gtid; i < hi; i += kGroupThreads)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  } else if ((addr & 7) == 0) {
-    const int head = min(hi, (lo + 1) & ~1), tail = max(head, hi & ~1);
-    for (int i = lo + gtid; i < head; i += kGroupThreads)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = head + 2 * gtid; i < tail; i += 2 * kGroupThreads)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = tail + gtid; i < hi; i += kGroupThreads)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  } else {
-    for (int i = lo + gtid; i < hi; i += kGroupThreads)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  }
+  stage::copy_real_samples<kGroupThreads>(smem_u32(sSamples), xs + s0, lo, hi, gtid);
   return false;
 }
 
@@ -317,7 +236,7 @@ stft2048_kernel(const Params p) {
     } else {
       asm volatile("cp.async.wait_all;" ::: "memory");
     }
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
 
     if (warp < nf) {
       // ---- pass 1: lane = n2, registers = n1; z[n] = x[2n] + i x[2n+1], n = 32 n1 + n2
@@ -428,7 +347,7 @@ stft2048_kernel(const Params p) {
         }
       }
     }
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
 
     // ---- the sample buffer is free: start fetching the next tile's samples
     // under the mel / write-out phases.
@@ -466,7 +385,7 @@ stft2048_kernel(const Params p) {
 #pragma unroll
         for (int f = 0; f < kTile; ++f) part[f * kRowStride + q.pid] = acc[f];
       }
-      group_sync(group);
+      named_sync(group + 1, kGroupThreads);
     }
 
     // ---- write the tile along the frame axis: [batch, rows, frames].  kTile
@@ -531,7 +450,7 @@ stft2048_kernel(const Params p) {
         if (park) {
           if (w)
             for (int r = r0; r < out_bins; r += kRows, orow += ostep, ld += ldstep) orow[j0] = *ld;
-          group_sync(group);                                  // the old carry has been read
+          named_sync(group + 1, kGroupThreads);                                  // the old carry has been read
           // park the tile's last q frames of every row: carry slot e <-> (row, frame)
           // through the per-period map, dense over the group's threads
           const int r_off = (int)(R0 & (S - 1));

@@ -45,8 +45,8 @@ namespace smb {
 namespace {
 
 using namespace fft32x2;
-using stage::named_sync;
-using stage::smem_u32;
+using fft32impl::kW64C;
+using fft32impl::kW64S;
 
 constexpr int kTile = kPairTile;            // frames per group tile
 constexpr int kGroupWarps = kTile / 2;      // a warp carries two frames
@@ -59,19 +59,6 @@ constexpr int kPowerBins = 1032;            // bins per power row incl. the zero
 static_assert(32 * (kGroupWarps - 1) + kPowerBins * 8 <= kWarpBuf, "power rows fit the transposition buffer");
 
 enum Mode { kModeMel = 0, kModeCeiling = 1 };
-
-// W_64^k2 = exp(-2 pi i k2 / 64), k2 < 16: the split twiddle W_2048^(l + 32 k2) is the
-// lane's W_2048^l times one of these constants.
-__device__ constexpr float kW64C[16] = {
-    1.0f, 0.9951847266721969f, 0.9807852804032304f, 0.9569403357322088f,
-    0.9238795325112867f, 0.881921264348355f, 0.8314696123025452f, 0.773010453362737f,
-    0.7071067811865476f, 0.6343932841636455f, 0.5555702330196023f, 0.4713967368259978f,
-    0.38268343236508984f, 0.29028467725446233f, 0.19509032201612833f, 0.09801714032956077f};
-__device__ constexpr float kW64S[16] = {
-    0.0f, -0.0980171403295606f, -0.19509032201612825f, -0.2902846772544623f,
-    -0.3826834323650898f, -0.47139673682599764f, -0.5555702330196022f, -0.6343932841636455f,
-    -0.7071067811865475f, -0.773010453362737f, -0.8314696123025452f, -0.8819212643483549f,
-    -0.9238795325112867f, -0.9569403357322089f, -0.9807852804032304f, -0.9951847266721968f};
 
 struct Params {
   Stft2048PairArgs a;
@@ -90,27 +77,8 @@ struct Params {
 // the tables live there: columns [0, 64) window, [64, 128) twiddles, one copy per
 // 32-lane quarter (warps w and w + 4 share quarter w % 4).
 constexpr uint32_t kTmemCols = 128;
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-      ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]),
-        "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]),
-        "r"(r[14]), "r"(r[15])
-      : "memory");
-}
-// no "memory" clobber: tensor memory is invisible to C++ loads and stores, so the
-// compiler may move shared-memory traffic across the load; the wait names the
-// registers, which orders their first use behind it
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]),
-        "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]),
-        "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
+// tmem_ld16 (sm100.cuh) leaves the wait to this one: naming the registers orders their
+// first use behind it
 __device__ __forceinline__ void tmem_wait16(uint32_t (&r)[16]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;"
                : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]),
@@ -161,11 +129,7 @@ stft2048p_kernel(const Params p) {
   unsigned char* ex = sBufs + warp * kWarpBuf;                 // this warp's
   float* prow = reinterpret_cast<float*>(ex + 32 * warp);      // its power rows, [bin][2]
 
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(&tmem_slot)), "r"(kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc(&tmem_slot, kTmemCols);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -199,8 +163,8 @@ stft2048p_kernel(const Params p) {
   }
   if (tid == 0) {
     for (int gI = 0; gI < kGroups; ++gI) {
-      stage::mbar_init(smem_u32(&sbars[gI]), 1);
-      stage::mbar_init(smem_u32(&sfree[gI]), kGroupWarps);
+      mbar_init(smem_u32(&sbars[gI]), 1);
+      mbar_init(smem_u32(&sfree[gI]), kGroupWarps);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -237,7 +201,7 @@ stft2048p_kernel(const Params p) {
     // previous tile's mel reads of the power rows against this tile's transposition
     // stores -- is waited for where it matters, just before those stores (sfree)
     if (bulk) {
-      stage::mbar_wait(sbar, sphase & 1);
+      mbar_wait(sbar, sphase & 1);
       ++sphase;
     } else {
       asm volatile("cp.async.wait_all;" ::: "memory");
@@ -286,7 +250,7 @@ stft2048p_kernel(const Params p) {
       }
       fft32(a);                                   // a[k1] = Y[n2 = lane][k1]
       // ---- the previous tile's power rows (this buffer) have been read by all four warps
-      if (tiles_done > 0) stage::mbar_wait(fbar, (tiles_done - 1) & 1);
+      if (tiles_done > 0) mbar_wait(fbar, (tiles_done - 1) & 1);
       // ---- twiddle W1024^(k1 n2), transpose through the warp's padded buffer
       {
         ulonglong2* st = reinterpret_cast<ulonglong2*>(ex) + lane;
@@ -424,15 +388,13 @@ stft2048p_kernel(const Params p) {
     // this warp has read the power rows it needs: count off (the next tile's
     // transposition stores wait for all four warps, see above)
     __syncwarp();
-    if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(fbar) : "memory");
+    if (lane == 0) mbar_arrive(fbar);
     ++tiles_done;
   }
   if (MODE == kModeMel && p.a.max_slot) warp_max_to((double)vmax, p.a.max_slot);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if (tid < 32)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_slot), "r"(kTmemCols)
-                 : "memory");
+  if (tid < 32) tmem_dealloc(tmem_slot, kTmemCols);
 }
 
 }  // namespace

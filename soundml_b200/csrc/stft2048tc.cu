@@ -40,7 +40,9 @@
 //   * The groups of a CTA run out of phase, so one group's MMAs overlap the
 //     CUDA-core phases of the others; operand buffers, the power rows and the
 //     accumulators are private to a group (TMEM columns 128 g .. 128 g + 127).
+#include "fft32.cuh"
 #include "kernels.h"
+#include "stft_stage.cuh"
 
 #include <cstdint>
 #include <cuda_fp16.h>
@@ -48,6 +50,10 @@
 namespace smb {
 
 namespace {
+
+using fft32impl::pk_add;
+using fft32impl::pk_mul;
+using fft32impl::pk_sub;
 
 constexpr int kFft = 2048;
 constexpr int kHalf = 1024;
@@ -60,79 +66,6 @@ constexpr int kABytes = 128 * 128;        // one split of a pass's A operand
 constexpr int kBBytes = 64 * 128;         // one split of F
 constexpr int kMaxGroups = 4;
 
-__device__ __forceinline__ long long src_index(const FrameGeom& g, long long q) {
-  long long s = q - g.left;
-  if (s >= 0 && s < g.n) return s;
-  if (g.pad == 0) {
-    if (g.n == 1) return 0;
-    const long long period = 2 * (g.n - 1);
-    long long r = s % period;
-    if (r < 0) r += period;
-    return r < g.n ? r : period - r;
-  }
-  if (g.pad == 2) return s < 0 ? 0 : g.n - 1;
-  return -1;
-}
-
-__device__ __forceinline__ void group_sync(int group) {
-  asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "r"(kGroupThreads) : "memory");
-}
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  while (!done) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-  }
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-      : "memory");
-}
-// packed float32 pairs (FMUL2 / FADD2 on sm_100): one issue slot for two lanes
-__device__ __forceinline__ float2 mul2(float2 a, float2 b) {
-  unsigned long long ra, rb, rc;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a.x), "f"(a.y));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(rb) : "f"(b.x), "f"(b.y));
-  asm("mul.f32x2 %0, %1, %2;" : "=l"(rc) : "l"(ra), "l"(rb));
-  float2 r;
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(rc));
-  return r;
-}
-__device__ __forceinline__ float2 sub2(float2 a, float2 b) {
-  unsigned long long ra, rb, rc;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a.x), "f"(a.y));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(rb) : "f"(b.x), "f"(b.y));
-  asm("sub.f32x2 %0, %1, %2;" : "=l"(rc) : "l"(ra), "l"(rb));
-  float2 r;
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(rc));
-  return r;
-}
-__device__ __forceinline__ float2 add2(float2 a, float2 b) {
-  unsigned long long ra, rb, rc;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(ra) : "f"(a.x), "f"(a.y));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(rb) : "f"(b.x), "f"(b.y));
-  asm("add.f32x2 %0, %1, %2;" : "=l"(rc) : "l"(ra), "l"(rb));
-  float2 r;
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(r.x), "=f"(r.y) : "l"(rc));
-  return r;
-}
 // tcgen05.mma, K-major SWIZZLE_128B operands (8-row groups 1024 B apart), the descriptors given by their low words (start address field) over the
 // common high word: the K-steps of a batch only move the start address
 __device__ __forceinline__ void umma_f16_lo(uint32_t tmem_d, uint32_t alo, uint32_t blo, uint32_t idesc,
@@ -155,10 +88,6 @@ __device__ __forceinline__ void umma_f16_lo(uint32_t tmem_d, uint32_t alo, uint3
         ::"r"(tmem_d), "r"(alo), "r"(blo), "r"(kDescHi), "r"(idesc)
         : "memory");
 }
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-               ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -170,18 +99,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
         "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]),
         "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
       : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]),
-        "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]),
-        "=r"(r[14]), "=r"(r[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait() {
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c,
                                              uint32_t d) {
@@ -251,37 +168,17 @@ __device__ __forceinline__ void stage_tile(const Params& p, TileRef t, bool bulk
     }
     return;
   }
-  const size_t addr = reinterpret_cast<size_t>(src);
   const int lo = (int)max(0LL, min((long long)span, -s0));
   const int hi = (int)max((long long)lo, min((long long)span, g.n - s0));
   for (int i = lane; i < lo; i += 32) {
-    const long long s = src_index(g, q0 + i);
+    const long long s = stage::src_index(g, q0 + i);
     sSamples[i] = s >= 0 ? __ldg(xs + s) : (float)g.pad_value;
   }
   for (int i = hi + lane; i < span; i += 32) {
-    const long long s = src_index(g, q0 + i);
+    const long long s = stage::src_index(g, q0 + i);
     sSamples[i] = s >= 0 ? __ldg(xs + s) : (float)g.pad_value;
   }
-  if ((addr & 15) == 0) {
-    const int head = min(hi, (lo + 3) & ~3), tail = max(head, hi & ~3);
-    for (int i = lo + lane; i < head; i += 32)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = head + 4 * lane; i < tail; i += 4 * 32)
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = tail + lane; i < hi; i += 32)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  } else if ((addr & 7) == 0) {
-    const int head = min(hi, (lo + 1) & ~1), tail = max(head, hi & ~1);
-    for (int i = lo + lane; i < head; i += 32)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = head + 2 * lane; i < tail; i += 2 * 32)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = tail + lane; i < hi; i += 32)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  } else {
-    for (int i = lo + lane; i < hi; i += 32)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  }
+  stage::copy_real_samples<32>(base, src, lo, hi, lane);
 }
 
 // STEP1: bin_step == 1 (fft 2048 proper): every bin is kept.
@@ -336,11 +233,7 @@ stft2048tc_kernel(const Params p) {
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   constexpr int kTmemCols = kGroups > 2 ? 512 : 256;
-  if (tid < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                 ::"r"(smem_u32(&tmem_base_slot)), "r"(kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (tid < 32) tmem_alloc(&tmem_base_slot, kTmemCols);
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // F images -> async proxy
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
@@ -415,7 +308,7 @@ stft2048tc_kernel(const Params p) {
     } else if (warp == 0) {
       asm volatile("cp.async.wait_all;" ::: "memory");
     }
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
 
     // ---- scale: largest sample magnitude of the tile -> power of two
     float scale, unscale;
@@ -429,7 +322,7 @@ stft2048tc_kernel(const Params p) {
       // non-negative floats order like their bit patterns: one REDUX per warp
       m = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m)));
       if (lane == 0) sMax[group * kTile + warp] = m;
-      group_sync(group);
+      named_sync(group + 1, kGroupThreads);
       const float4 mm = *reinterpret_cast<const float4*>(sMax + group * kTile);
       m = fmaxf(fmaxf(mm.x, mm.y), fmaxf(mm.z, mm.w));
       // m in [2^e, 2^(e+1))  ->  scale = 2^(9 - e): |x| scale < 1024, window/2 <= 1/2
@@ -444,7 +337,7 @@ stft2048tc_kernel(const Params p) {
       float2 ws[8];
       const float2 sc2 = make_float2(scale, scale);
 #pragma unroll
-      for (int i = 0; i < 8; ++i) ws[i] = mul2(wreg[i], sc2);
+      for (int i = 0; i < 8; ++i) ws[i] = pk_mul(wreg[i], sc2);
       const uint32_t sw = (uint32_t)lane & 7u;
       const uint32_t c0 = (((uint32_t)(2 * warp) ^ sw) << 4), c1 = (((uint32_t)(2 * warp + 1) ^ sw) << 4);
       const bool even = (g.hop & 1) == 0;
@@ -465,9 +358,9 @@ stft2048tc_kernel(const Params p) {
         uint32_t hw[8], lw[8];
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-          const float2 u = mul2(v[i], ws[i]);
+          const float2 u = pk_mul(v[i], ws[i]);
           hw[i] = pack_half2(u.x, u.y);
-          const float2 l = sub2(u, unpack_half2(hw[i]));
+          const float2 l = pk_sub(u, unpack_half2(hw[i]));
           lw[i] = pack_half2(l.x, l.y);
         }
         const uint32_t rowoff = (uint32_t)(32 * f + lane) * 128u;
@@ -488,7 +381,7 @@ stft2048tc_kernel(const Params p) {
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
 
     if (gtid == 0) {
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -531,7 +424,7 @@ stft2048tc_kernel(const Params p) {
           const float2 z0 = make_float2(yr0 * t[j].x - yi0 * t[j].y, yr0 * t[j].y + yi0 * t[j].x);
           const float2 z1 = make_float2(yr1 * t[j].z - yi1 * t[j].w, yr1 * t[j].w + yi1 * t[j].z);
           const uint32_t h0 = pack_half2(z0.x, z0.y), h1 = pack_half2(z1.x, z1.y);
-          const float2 l0 = sub2(z0, unpack_half2(h0)), l1 = sub2(z1, unpack_half2(h1));
+          const float2 l0 = pk_sub(z0, unpack_half2(h0)), l1 = pk_sub(z1, unpack_half2(h1));
           const uint32_t o0 = (base_hi ^ ((uint32_t)(2 * j) << 4)) + (uint32_t)k1 * 128u;
           const uint32_t o1 = (base_hi ^ ((uint32_t)(2 * j + 1) << 4)) + (uint32_t)(k1 + 1) * 128u;
           st_shared_b32(o0, h0);
@@ -560,7 +453,7 @@ stft2048tc_kernel(const Params p) {
     if (more && warp == 1 && !bulk) asm volatile("cp.async.wait_all;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
 
     if (gtid == 0) {
       asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -620,13 +513,13 @@ stft2048tc_kernel(const Params p) {
           //   S = Z'[k] + conj Z'[N-k],  D = Z'[k] - conj Z'[N-k],  W = W2048^k
           //   X[k] = S + W (-i D),   X[N-k] = conj(S - W (-i D))
           float2 w = sTwPost[k2 * 32 + lane];
-          if (!late_unscale) w = mul2(w, us2);
-          float2 S = add2(a[k2], r[k2]);
-          const float2 D = sub2(a[k2], r[k2]);
-          if (!late_unscale) S = mul2(S, us2);
+          if (!late_unscale) w = pk_mul(w, us2);
+          float2 S = pk_add(a[k2], r[k2]);
+          const float2 D = pk_sub(a[k2], r[k2]);
+          if (!late_unscale) S = pk_mul(S, us2);
           const float2 T = make_float2(w.x * D.y + w.y * D.x, w.y * D.y - w.x * D.x);
-          const float2 xk = add2(S, T);
-          const float2 xm = sub2(S, T);                     // conj of X[N-k]
+          const float2 xk = pk_add(S, T);
+          const float2 xm = pk_sub(S, T);                     // conj of X[N-k]
           if (OUT == kFastComplex) {
             a[k2] = xk;
             r[k2] = make_float2(xm.x, -xm.y);
@@ -665,7 +558,7 @@ stft2048tc_kernel(const Params p) {
         }
       }
     }
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
 
     if (OUT == kFastMel) {
       // ---- mel projection over the tile's power rows.  A lane carries one piece
@@ -724,7 +617,7 @@ stft2048tc_kernel(const Params p) {
         part[2 * p.row_stride + q.pid] = a2;
         part[3 * p.row_stride + q.pid] = a3;
       }
-      group_sync(group);
+      named_sync(group + 1, kGroupThreads);
     }
 
     // ---- write the tile along the frame axis: [batch, rows, frames]
@@ -764,13 +657,11 @@ stft2048tc_kernel(const Params p) {
         }
       }
     }
-    group_sync(group);
+    named_sync(group + 1, kGroupThreads);
   }
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
-  if (tid < 32)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols)
-                 : "memory");
+  if (tid < 32) tmem_dealloc(tmem, kTmemCols);
 }
 
 }  // namespace

@@ -1,25 +1,30 @@
-// Device helpers shared by the fused fft-2048 kernels: the reference's boundary rule,
-// mbarrier / bulk-copy (TMA) wrappers, named group barriers and the tile staging that
+// Device helpers shared by the STFT kernels: the reference's boundary rule, the
+// cp.async fetch of a tile's real samples and the frame-pair kernel's tile staging that
 // brings a run of overlapping frames into shared memory once.
 #pragma once
 #include <cstdint>
 
 #include "kernels.h"
+#include "sm100.cuh"
 
 namespace smb {
 namespace stage {
 
 // padded stream position q -> source index, or -1 for the constant fill
-// (stft.ml:300-338: reflect_index / edge clamp / constant)
+// (stft.ml:300-338: reflect_index / edge clamp / constant).  kOneReflectionFirst tries
+// the single reflection (every border of a signal longer than the extension) before
+// the division.
+template <bool kOneReflectionFirst = false>
 __device__ __forceinline__ long long src_index(const FrameGeom& g, long long q) {
   long long s = q - g.left;
   if (s >= 0 && s < g.n) return s;
   if (g.pad == 0) {
     if (g.n == 1) return 0;
     const long long period = 2 * (g.n - 1);
-    // one reflection (every border of a signal longer than the extension): no division
-    const long long once = s < 0 ? -s : period - s;
-    if (once >= 0 && once < g.n) return once;
+    if (kOneReflectionFirst) {
+      const long long once = s < 0 ? -s : period - s;
+      if (once >= 0 && once < g.n) return once;
+    }
     long long r = s % period;
     if (r < 0) r += period;
     return r < g.n ? r : period - r;
@@ -28,36 +33,33 @@ __device__ __forceinline__ long long src_index(const FrameGeom& g, long long q) 
   return -1;
 }
 
-__device__ __forceinline__ void named_sync(int id, int threads) {
-  asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
-}
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes)
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-  uint32_t done = 0;
-  while (!done) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
+// cp.async of a tile's real samples, src[i] -> shared address base + 4 i for i in
+// [lo, hi), over THREADS threads of which this is tid: 16-byte requests when src is
+// 16-byte aligned (8 when 8-byte aligned; base is 16-byte aligned), single floats for
+// the unaligned head and tail.  The caller waits with cp.async.wait_all.
+template <int THREADS>
+__device__ __forceinline__ void copy_real_samples(unsigned base, const float* src, int lo, int hi, int tid) {
+  const size_t addr = reinterpret_cast<size_t>(src);
+  if ((addr & 15) == 0) {
+    const int head = min(hi, (lo + 3) & ~3), tail = max(head, hi & ~3);
+    for (int i = lo + tid; i < head; i += THREADS)
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
+    for (int i = head + 4 * tid; i < tail; i += 4 * THREADS)
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
+    for (int i = tail + tid; i < hi; i += THREADS)
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
+  } else if ((addr & 7) == 0) {
+    const int head = min(hi, (lo + 1) & ~1), tail = max(head, hi & ~1);
+    for (int i = lo + tid; i < head; i += THREADS)
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
+    for (int i = head + 2 * tid; i < tail; i += 2 * THREADS)
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
+    for (int i = tail + tid; i < hi; i += THREADS)
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
+  } else {
+    for (int i = lo + tid; i < hi; i += THREADS)
+      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
   }
-}
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-      ::"r"(dst), "l"(src), "r"(bytes), "r"(bar)
-      : "memory");
 }
 
 // Which tiles of which clips are one aligned bulk copy: tiles t in [t_lo, t_hi] of a
@@ -110,7 +112,7 @@ __device__ __forceinline__ bool stage_tile(const FrameGeom& g, const float* x, c
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
         const int i = i0 + k * THREADS;
-        const long long s = i < to ? src_index(g, q0 + i) : -1;
+        const long long s = i < to ? src_index<true>(g, q0 + i) : -1;
         v[k] = s >= 0 ? __ldg(xs + s) : (float)g.pad_value;
       }
 #pragma unroll
@@ -118,29 +120,7 @@ __device__ __forceinline__ bool stage_tile(const FrameGeom& g, const float* x, c
         if (i0 + k * THREADS < to) dst[i0 + k * THREADS] = v[k];
     }
   }
-  const float* src = xs + s0;                       // src + i is valid for i in [lo, hi)
-  const unsigned base = smem_u32(dst);
-  const size_t addr = reinterpret_cast<size_t>(src);
-  if ((addr & 15) == 0) {
-    const int head = min(hi, (lo + 3) & ~3), tail = max(head, hi & ~3);
-    for (int i = lo + gtid; i < head; i += THREADS)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = head + 4 * gtid; i < tail; i += 4 * THREADS)
-      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = tail + gtid; i < hi; i += THREADS)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  } else if ((addr & 7) == 0) {
-    const int head = min(hi, (lo + 1) & ~1), tail = max(head, hi & ~1);
-    for (int i = lo + gtid; i < head; i += THREADS)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = head + 2 * gtid; i < tail; i += 2 * THREADS)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-    for (int i = tail + gtid; i < hi; i += THREADS)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  } else {
-    for (int i = lo + gtid; i < hi; i += THREADS)
-      asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(base + 4u * i), "l"(src + i) : "memory");
-  }
+  copy_real_samples<THREADS>(smem_u32(dst), xs + s0, lo, hi, gtid);
   return false;
 }
 
