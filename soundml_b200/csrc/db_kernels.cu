@@ -62,57 +62,68 @@ __global__ void max_value_kernel(const T* __restrict__ x, long long count,
 constexpr int kMfccFrames = 32;     // frame columns per CTA
 constexpr int kMfccThreads = 256;
 constexpr int kMfccPer = 3;         // coefficients per thread (the log-mel value is loaded once for them)
+constexpr int kMfccGroups = kMfccThreads / kMfccFrames;  // coefficient c = c0 + g + kMfccGroups * j
+constexpr int kMfccCoefs = kMfccGroups * kMfccPer;       // coefficients per CTA
+constexpr int kMfccChunk = 128;     // mel bands staged at once: shared memory stays under 56 KB
 
 // mel [batch, n_mels, frames] (T) -> out [batch, n_mfcc, frames] (T).  One CTA per
-// (32-frame tile, signal): the log-mel tile is built once in shared memory in double
-// (with the 80 dB clamp below the whole-tensor maximum) next to the DCT rows, then
-// thread (coefficient group, frame) walks the mel axis: one log-mel load feeds up to
-// three coefficients.
+// (32-frame tile, signal, group of kMfccCoefs coefficients).  The mel axis is walked
+// in chunks of kMfccChunk bands: each chunk's log-mel tile is built in shared memory in
+// double (with the 80 dB clamp below the whole-tensor maximum) next to that chunk's DCT
+// rows, then thread (coefficient group, frame) continues its fma chains over the chunk:
+// one log-mel load feeds up to three coefficients.  Every coefficient is the same
+// ascending-m fma chain whatever the chunking, so the chunk size does not change a bit.
 template <typename T>
 __global__ void __launch_bounds__(kMfccThreads)
 mfcc_kernel(const T* __restrict__ mel, int n_mels, long long frames, int n_mfcc,
             const double* __restrict__ dct, const unsigned long long* max_mel_slot, double amin,
             double scale, double offset, double range, T* __restrict__ out) {
-  extern __shared__ __align__(8) double sDb[];           // [n_mels][kMfccFrames], then the DCT rows
-  double* sDct = sDb + n_mels * kMfccFrames;              // [n_mfcc][n_mels]
+  extern __shared__ __align__(8) double sDb[];           // [chunk][kMfccFrames], then the DCT rows
   const long long b = blockIdx.y;
   const long long p0 = (long long)blockIdx.x * kMfccFrames;
+  const int c0 = blockIdx.z * kMfccCoefs;
+  const int rows = min(kMfccCoefs, n_mfcc - c0);          // this CTA's coefficients
   const int nf = (int)min((long long)kMfccFrames, frames - p0);
   // the maximum of db is db of the maximum (the map is monotone)
   const double vmax = fmax(value_of(*max_mel_slot), amin);
   const double floor_db = (log(vmax) * scale - offset) - range;
   const T* src = mel + b * n_mels * frames + p0;
-  for (int i = threadIdx.x; i < n_mfcc * n_mels; i += blockDim.x) sDct[i] = __ldg(dct + i);
-  for (int i = threadIdx.x; i < n_mels * kMfccFrames; i += blockDim.x) {
-    const int m = i / kMfccFrames, f = i - m * kMfccFrames;
-    double db = 0.0;
-    if (f < nf) {
-      const double v = fmax((double)src[(long long)m * frames + f], amin);
-      db = fmax(log(v) * scale - offset, floor_db);
-    }
-    sDb[i] = db;
-  }
-  __syncthreads();
   const int f = threadIdx.x & (kMfccFrames - 1);
-  constexpr int kGroups = kMfccThreads / kMfccFrames;     // coefficient c = g + kGroups * j
-  T* dst = out + b * n_mfcc * frames + p0 + f;
-  for (int c0 = threadIdx.x / kMfccFrames; c0 < n_mfcc; c0 += kGroups * kMfccPer) {
-    double acc[kMfccPer];
+  const int g = threadIdx.x / kMfccFrames;
+  double acc[kMfccPer];
+#pragma unroll
+  for (int j = 0; j < kMfccPer; ++j) acc[j] = 0.0;
+  for (int m0 = 0; m0 < n_mels; m0 += kMfccChunk) {
+    const int len = min(kMfccChunk, n_mels - m0);
+    double* sDct = sDb + len * kMfccFrames;               // [rows][len]
+    if (m0 > 0) __syncthreads();                          // the previous chunk is consumed
+    for (int i = threadIdx.x; i < rows * kMfccChunk; i += blockDim.x) {   // (row, band): shifts, no division
+      const int r = i / kMfccChunk, m = i % kMfccChunk;
+      if (m < len) sDct[r * len + m] = __ldg(dct + (long long)(c0 + r) * n_mels + m0 + m);
+    }
+    for (int i = threadIdx.x; i < len * kMfccFrames; i += blockDim.x) {
+      const int m = i / kMfccFrames, ff = i - m * kMfccFrames;
+      double db = 0.0;
+      if (ff < nf) {
+        const double v = fmax((double)src[(long long)(m0 + m) * frames + ff], amin);
+        db = fmax(log(v) * scale - offset, floor_db);
+      }
+      sDb[i] = db;
+    }
+    __syncthreads();
     const double* row[kMfccPer];
 #pragma unroll
-    for (int j = 0; j < kMfccPer; ++j) {
-      acc[j] = 0.0;
-      row[j] = sDct + (long long)min(c0 + kGroups * j, n_mfcc - 1) * n_mels;
-    }
-    for (int m = 0; m < n_mels; ++m) {
+    for (int j = 0; j < kMfccPer; ++j) row[j] = sDct + min(g + kMfccGroups * j, rows - 1) * len;
+    for (int m = 0; m < len; ++m) {
       const double v = sDb[m * kMfccFrames + f];
 #pragma unroll
       for (int j = 0; j < kMfccPer; ++j) acc[j] = fma(row[j][m], v, acc[j]);
     }
-#pragma unroll
-    for (int j = 0; j < kMfccPer; ++j)
-      if (f < nf && c0 + kGroups * j < n_mfcc) dst[(long long)(c0 + kGroups * j) * frames] = (T)acc[j];
   }
+  T* dst = out + b * n_mfcc * frames + p0 + f;
+#pragma unroll
+  for (int j = 0; j < kMfccPer; ++j)
+    if (f < nf && g + kMfccGroups * j < rows) dst[(long long)(c0 + g + kMfccGroups * j) * frames] = (T)acc[j];
 }
 
 // db in place over values whose maximum is already in the slot (the fused mel kernel
@@ -192,12 +203,16 @@ cudaError_t launch_mfcc(const void* mel, int dtype, long long batch, int n_mels,
     else max_value_kernel<double><<<grid_for(count), 256, 0, st>>>((const double*)mel, count, max_slot);
     ++g_launch_count;
   }
-  const size_t smem = (size_t)(n_mels * kMfccFrames + n_mfcc * n_mels) * sizeof(double);
-  if (smem > 200 * 1024) return cudaErrorInvalidConfiguration;
+  // one chunk of the log-mel tile and its DCT rows
+  const int chunk = n_mels < kMfccChunk ? n_mels : kMfccChunk;
+  const int rows = n_mfcc < kMfccCoefs ? n_mfcc : kMfccCoefs;
+  const size_t smem = (size_t)chunk * (kMfccFrames + rows) * sizeof(double);
   const long long tiles = (frames + kMfccFrames - 1) / kMfccFrames;
+  const unsigned groups = (unsigned)((n_mfcc + kMfccCoefs - 1) / kMfccCoefs);
+  if (groups > 65535u) return cudaErrorInvalidConfiguration;
   for (long long b0 = 0; b0 < batch; b0 += 65535) {
     const long long nb = batch - b0 < 65535 ? batch - b0 : 65535;
-    dim3 grid((unsigned)tiles, (unsigned)nb);
+    dim3 grid((unsigned)tiles, (unsigned)nb, groups);
     if (dtype == 0) {
       e = cudaFuncSetAttribute(mfcc_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
       if (e != cudaSuccess) return e;

@@ -51,3 +51,20 @@ def test_pipeline_ptx_has_one_home():
     for asm in SINGLE_HOME_ASM:
         files = sorted(f for f, text in sources.items() if asm in text)
         assert files == ["sm100.cuh"], f"{asm!r} appears in {files}"
+
+
+def test_every_included_file_is_a_build_dependency():
+    """build.py rebuilds when a file in CUDA_SOURCES, HOST_SOURCES or HEADERS is newer than
+    the library: a header it does not list (max_key.cuh once) could change without a rebuild."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("soundml_b200_build", os.path.join(ROOT, "soundml_b200", "build.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    listed = {os.path.normpath(os.path.join(CSRC, f)) for f in b.CUDA_SOURCES + b.HOST_SOURCES + b.HEADERS}
+    for name, text in _sources().items():
+        for inc in re.findall(r'^\s*#\s*include\s+"([^"]+)"', text, re.M):
+            path = os.path.normpath(os.path.join(CSRC, inc))
+            assert os.path.exists(path), f"{name} includes {inc}, which does not exist"
+            assert path in listed, f"{name} includes {inc}, which build.py does not list"
+    for f in listed:
+        assert os.path.exists(f), f"build.py lists {f}, which does not exist"
