@@ -169,7 +169,7 @@ struct HostPipe {
     event_ptr ev_in[2], ev_run[2], ev_out[2];
   };
   std::unique_ptr<Streams> streams;  // created by the first host-memory call
-  DeviceBuffer in[2], out[2];        // (smb_mfcc also stages through in[0], without the streams)
+  DeviceBuffer in[2], out[2];        // (the log-mel calls also stage through in[0], without the streams)
   // run(din, dout, items) enqueues the kernels for `items` batch items on `compute`.
   template <typename Run>
   void execute(cudaStream_t compute, const void* x, void* out_host, int64_t batch,
@@ -214,6 +214,21 @@ struct HostPipe {
     CK(cudaStreamSynchronize(compute));
   }
 };
+
+void check_mem(int mem) {
+  if (mem != SMB_MEM_DEVICE && mem != SMB_MEM_HOST)
+    throw smb::invalid_argument("soundml_b200: unknown memory kind");
+}
+
+// run(din, dout, items) over the caller's device buffers, or over a host batch in
+// slices through `pipe`.
+template <typename Run>
+void dispatch(int mem, HostPipe& pipe, cudaStream_t st, const void* x, void* out, int64_t batch,
+              size_t in_item, size_t out_item, Run&& run) {
+  check_mem(mem);
+  if (mem == SMB_MEM_DEVICE) run(x, out, batch);
+  else pipe.execute(st, x, out, batch, in_item, out_item, run);
+}
 
 size_t dtype_size(int dtype) {
   if (dtype == SMB_F32) return 4;
@@ -360,6 +375,9 @@ struct smb_stft_plan {
     if (frames == 0) return 0;
     return (frames - 1) * geom.hop + geom.fft - geom.left_width() - geom.right_width();
   }
+  int64_t frames_reaching(int64_t len) const {           // stft.ml:907-915
+    return (len + geom.left_width() + geom.hop - 1) / geom.hop;
+  }
   // 2048 / fft when the frame embeds in the fused kernel's 2048-point transform
   int fast_step() const {
     return geom.fft >= 128 && geom.fft <= 2048 && 2048 % geom.fft == 0 ? (int)(2048 / geom.fft) : 0;
@@ -430,7 +448,7 @@ struct smb_mel_plan {
     device_ptr<unsigned long long> d_max;
   };
   std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
-  DeviceBuffer in, out;
+  HostPipe pipe;                     // host-memory calls: sliced, copies under kernels
   int64_t dct_n_mfcc = -1;
   double dct_lifter = -1.0;
   const double* dct_table(int64_t n_mfcc, double lifter) {
@@ -1098,7 +1116,7 @@ struct smb_resample_plan {
   };
   std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   int executor = SMB_EXEC_PLANNED;   // SMB_EXEC_DIRECT forces the dot-product kernel everywhere
-  DeviceBuffer in, out, mid;
+  DeviceBuffer mid;
   HostPipe pipe;                     // host-memory calls: sliced, copies under kernels
   void ensure_device() {
     if (dev) return same_device(dev->device);
@@ -1343,6 +1361,15 @@ void check_signal(const char* op, int64_t batch, int64_t n) {
   if (batch < 0) throw smb::invalid_argument(smb::format("%s: negative batch", op));
 }
 
+void require_nola(const char* op, const smb_stft_plan* p) {     // stft.ml:744-753
+  if (!p->nola())
+    throw smb::invalid_argument(smb::format(
+        "%s: cannot invert a %lld-point window advanced by %lld samples inside a "
+        "%lld-point frame (the overlap-added squared window must stay above 1e-10 of its "
+        "largest value at every position)",
+        op, (long long)p->geom.win_length, (long long)p->geom.hop, (long long)p->geom.fft));
+}
+
 // Which fused kernel takes the call: 0 none (generic path), SMB_PATH_FAST the
 // CUDA-core register-FFT kernel, SMB_PATH_TENSOR the tcgen05 kernel.
 int want_fast(const smb_stft_plan* p, int dtype, const smb::FrameGeom& g, int out_kind,
@@ -1365,14 +1392,12 @@ int want_fast(const smb_stft_plan* p, int dtype, const smb::FrameGeom& g, int ou
     return SMB_PATH_PAIR;
   }
   if (p->path == SMB_PATH_AUTO && ok_pair) return SMB_PATH_PAIR;
-  const bool ok_tc = base && smb::stft2048tc_supports(gk, out_kind, mel ? (int)mel->n_mels : 0,
-                                                      mel ? (int)mel->sched_tc.vals.size() : 0,
-                                                      mel ? mel->sched_tc.rounds : 0,
-                                                      mel ? mel->sched_tc.mpad : 0);
-  const bool ok_cc = base && smb::stft2048_supports(gk, out_kind, mel ? (int)mel->n_mels : 0,
-                                                    mel ? (int)mel->sched_cc.vals.size() : 0,
-                                                    mel ? mel->sched_cc.rounds : 0,
-                                                    mel ? mel->sched_cc.mpad : 0);
+  const smb_mel_plan::PieceSchedule none{};
+  const smb_mel_plan::PieceSchedule& tc = mel ? mel->sched_tc : none;
+  const smb_mel_plan::PieceSchedule& cc = mel ? mel->sched_cc : none;
+  const int n_mels = mel ? (int)mel->n_mels : 0;
+  const bool ok_tc = base && smb::stft2048tc_supports(gk, out_kind, n_mels, (int)tc.vals.size(), tc.rounds, tc.mpad);
+  const bool ok_cc = base && smb::stft2048_supports(gk, out_kind, n_mels, (int)cc.vals.size(), cc.rounds, cc.mpad);
   if (p->path == SMB_PATH_TENSOR) {
     if (!ok_tc)
       throw smb::invalid_argument(
@@ -1411,6 +1436,24 @@ smb::Stft2048PairArgs pair_args(const smb_stft_plan* stft, const smb_mel_plan* m
   return a;
 }
 
+// The launch arguments of the fused kernels (CUDA-core and tensor-core) without a mel schedule.
+smb::Stft2048Args fused_args(const smb_stft_plan* stft, const void* din, void* dout, int64_t nb,
+                             const smb::FrameGeom& g, double power) {
+  smb::Stft2048Args a{};
+  a.x = (const float*)din;
+  a.out = (float*)dout;
+  a.batch = nb;
+  a.g = g;
+  a.g.fft = 2048;
+  a.bin_step = stft->fast_step();
+  a.window = stft->dev->d_window32.get();
+  a.tw_pass = stft->dev->d_tw_pass.get();
+  a.tw_post = stft->dev->d_tw_post.get();
+  a.power = (float)power;
+  a.dft_images = stft->dev->d_dft_images.get();
+  return a;
+}
+
 // x (device) -> spectrum (device).  kind: complex or |X|^power.
 void run_spectrum(smb_stft_plan* p, const void* dx, int64_t batch, const smb::FrameGeom& g,
                   int dtype, SpecKind kind, double power, void* dout) {
@@ -1418,18 +1461,7 @@ void run_spectrum(smb_stft_plan* p, const void* dx, int64_t batch, const smb::Fr
   cudaStream_t st = d.stream.use;
   const int fast_kind = kind == kSpecComplex ? smb::kFastComplex : smb::kFastPower;
   if (const int which = want_fast(p, dtype, g, fast_kind, nullptr)) {
-    smb::Stft2048Args a{};
-    a.x = (const float*)dx;
-    a.out = (float*)dout;
-    a.batch = batch;
-    a.g = g;
-    a.g.fft = 2048;
-    a.bin_step = p->fast_step();
-    a.window = d.d_window32.get();
-    a.tw_pass = d.d_tw_pass.get();
-    a.tw_post = d.d_tw_post.get();
-    a.power = (float)power;
-    a.dft_images = d.d_dft_images.get();
+    const smb::Stft2048Args a = fused_args(p, dx, dout, batch, g, power);
     if (which == SMB_PATH_TENSOR) CK(smb::launch_stft2048tc(a, fast_kind, d.sm_count, st));
     else CK(smb::launch_stft2048(a, fast_kind, d.sm_count, st));
   } else {
@@ -1461,16 +1493,10 @@ void spectrum_call(const char* op, smb_stft_plan* p, const void* x, int64_t batc
       (size_t)batch * (size_t)p->geom.bins() * (size_t)g.frames * (kind == kSpecComplex ? 2 : 1);
   if (batch == 0 || g.frames == 0) return;       // frameless spectrum: nothing to write
   p->ensure_device();
-  cudaStream_t st = p->dev->stream.use;
-  if (mem == SMB_MEM_DEVICE) {
-    run_spectrum(p, x, batch, g, dtype, kind, power, out);
-    return;
-  }
-  if (mem != SMB_MEM_HOST) throw smb::invalid_argument("soundml_b200: unknown memory kind");
-  p->pipe.execute(st, x, out, batch, (size_t)n * esz, out_elems / (size_t)batch * esz,
-                  [&](const void* din, void* dout, int64_t nb) {
-                    run_spectrum(p, din, nb, g, dtype, kind, power, dout);
-                  });
+  dispatch(mem, p->pipe, p->dev->stream.use, x, out, batch, (size_t)n * esz, out_elems / (size_t)batch * esz,
+           [&](const void* din, void* dout, int64_t nb) {
+             run_spectrum(p, din, nb, g, dtype, kind, power, dout);
+           });
 }
 
 void run_mel_apply(smb_mel_plan* m, const void* ds, int64_t batch, int64_t frames, int dtype,
@@ -1479,35 +1505,42 @@ void run_mel_apply(smb_mel_plan* m, const void* ds, int64_t batch, int64_t frame
                            m->dev->d_band_lo.get(), m->dev->d_band_hi.get(), dout, st));
 }
 
+// The synthesis arguments of Stft.invert for `nb` items z (device) -> out (device) on the
+// plan's stream.  Only the frames the output can reach are inverted; when none does, out
+// is zero-filled here and the count is 0: nothing is left to launch.
+smb::IstftArgs istft_args(smb_stft_plan* p, const void* dz, void* dout, int64_t nb, int64_t frames,
+                          bool has_length, int64_t out_len, int in_dtype, int out_dtype) {
+  smb_stft_plan::Device& d = *p->dev;
+  smb::IstftArgs a{};
+  a.count = has_length ? std::min(frames, p->frames_reaching(out_len)) : frames;
+  if (a.count == 0) {
+    CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * dtype_size(out_dtype), d.stream.use));
+    return a;
+  }
+  if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
+  a.z = dz;
+  a.out = dout;
+  a.frames = frames;
+  a.out_len = out_len;
+  a.fft = (int)p->geom.fft;
+  a.hop = (int)p->geom.hop;
+  a.left = (int)p->geom.left_width();
+  a.window = d.d_window64.get();
+  a.twiddle = d.d_twiddle64.get();
+  a.folded = d.d_folded.get();
+  a.in_f64 = in_dtype == SMB_F64;
+  a.out_f64 = out_dtype == SMB_F64;
+  return a;
+}
+
 // z (device) -> out (device): Stft.invert of `nb` items on the plan's stream (the
 // synthesis kernels of smb_stft_invert; time_stretch's last stage)
 void run_invert(smb_stft_plan* p, const void* dz, void* dout, int64_t nb, int64_t frames,
                 bool has_length, int64_t out_len, int in_dtype, int out_dtype) {
   smb_stft_plan::Device& d = *p->dev;
   cudaStream_t st = d.stream.use;
-  const int64_t left = p->geom.left_width(), hop = p->geom.hop;
-  // only the frames the output can reach are inverted (stft.ml:907-915)
-  int64_t count = frames;
-  if (has_length) count = std::min(frames, (out_len + left + hop - 1) / hop);
-  if (count == 0) {                                 // nothing reaches the output: zeros
-    CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * dtype_size(out_dtype), st));
-    return;
-  }
-  if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
-  smb::IstftArgs a{};
-  a.z = dz;
-  a.out = dout;
-  a.frames = frames;
-  a.count = count;
-  a.out_len = out_len;
-  a.fft = (int)p->geom.fft;
-  a.hop = (int)hop;
-  a.left = (int)left;
-  a.window = d.d_window64.get();
-  a.twiddle = d.d_twiddle64.get();
-  a.folded = d.d_folded.get();
-  a.in_f64 = in_dtype == SMB_F64;
-  a.out_f64 = out_dtype == SMB_F64;
+  const smb::IstftArgs a = istft_args(p, dz, dout, nb, frames, has_length, out_len, in_dtype, out_dtype);
+  if (a.count == 0) return;
   const bool fast = p->path != SMB_PATH_GENERIC && smb::istft2048_supports(a);
   if (!fast && p->path == SMB_PATH_FAST)
     throw smb::invalid_argument(
@@ -1578,31 +1611,19 @@ int smb_stft_invert(smb_stft_plan* plan, const void* z, int64_t batch, int64_t f
       throw smb::invalid_argument(smb::format(
           "invert: cannot synthesise a signal of length %lld (length must be non-negative)",
           (long long)length));
-    if (!p->nola())                                     // stft.ml:744-753
-      throw smb::invalid_argument(smb::format(
-          "invert: cannot invert a %lld-point window advanced by %lld samples inside a "
-          "%lld-point frame (the overlap-added squared window must stay above 1e-10 of its "
-          "largest value at every position)",
-          (long long)p->geom.win_length, (long long)p->geom.hop, (long long)p->geom.fft));
+    require_nola("invert", p);
     const size_t isz = 2 * dtype_size(in_dtype), osz = dtype_size(out_dtype);
     const int64_t out_len = has_length ? length : p->output_length(frames);
     if (batch == 0 || out_len == 0) return;
     p->ensure_device();
-    cudaStream_t st = p->dev->stream.use;
-    auto run = [&](const void* dz, void* dout, int64_t nb) {
-      run_invert(p, dz, dout, nb, frames, has_length != 0, out_len, in_dtype, out_dtype);
-    };
-    if (mem == SMB_MEM_DEVICE) {
-      run(z, out, batch);
-      return;
-    }
-    if (mem != SMB_MEM_HOST) throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    if (frames == 0) {
+    if (mem == SMB_MEM_HOST && frames == 0) {
       std::memset(out, 0, (size_t)batch * (size_t)out_len * osz);
       return;
     }
-    p->pipe.execute(st, z, out, batch, (size_t)p->geom.bins() * (size_t)frames * isz,
-                    (size_t)out_len * osz, run);
+    dispatch(mem, p->pipe, p->dev->stream.use, z, out, batch, (size_t)p->geom.bins() * (size_t)frames * isz,
+             (size_t)out_len * osz, [&](const void* dz, void* dout, int64_t nb) {
+               run_invert(p, dz, dout, nb, frames, has_length != 0, out_len, in_dtype, out_dtype);
+             });
   });
 }
 
@@ -1617,12 +1638,7 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
       throw smb::invalid_argument(smb::format(
           "griffin_lim: cannot synthesise a signal of length %lld (length must be non-negative)",
           (long long)length));
-    if (!p->nola())
-      throw smb::invalid_argument(smb::format(
-          "griffin_lim: cannot invert a %lld-point window advanced by %lld samples inside a "
-          "%lld-point frame (the overlap-added squared window must stay above 1e-10 of its "
-          "largest value at every position)",
-          (long long)p->geom.win_length, (long long)p->geom.hop, (long long)p->geom.fft));
+    require_nola("griffin_lim", p);
     if (n_iter < 1)
       throw smb::invalid_argument(smb::format(
           "griffin_lim: cannot run %lld iterations (n_iter must be at least 1)",
@@ -1631,12 +1647,11 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
       throw smb::invalid_argument(smb::format(
           "griffin_lim: cannot use a momentum of %g (momentum must be non-negative)", momentum));
     const size_t esz = dtype_size(dtype);
-    const int64_t bins = p->geom.bins(), left = p->geom.left_width(), hop = p->geom.hop;
+    const int64_t bins = p->geom.bins();
     const int64_t natural = p->output_length(frames);
     const int64_t out_len = has_length ? length : natural;
     if (batch == 0 || out_len == 0) return;
-    if (mem != SMB_MEM_DEVICE && mem != SMB_MEM_HOST)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    check_mem(mem);
     if (frames == 0) {
       if (mem == SMB_MEM_HOST) std::memset(out, 0, (size_t)batch * (size_t)out_len * esz);
       else { p->ensure_device(); CK(cudaMemsetAsync(out, 0, (size_t)batch * (size_t)out_len * esz, p->dev->stream.use)); }
@@ -1645,7 +1660,6 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
     p->ensure_device();
     smb_stft_plan::Device& d = *p->dev;
     cudaStream_t st = d.stream.use;
-    if (!d.d_folded) d.d_folded = upload(p->folded_square_window());
     const size_t cells = (size_t)batch * (size_t)bins * (size_t)frames;
     // the whole problem stays resident across the iterations; freed when the call returns or throws
     device_ptr<void> d_s, d_phase, d_out, d_a, d_b, d_y;
@@ -1667,27 +1681,8 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
     const device_ptr<double2> d_spec = device_alloc<double2>(cells * sizeof(double2));
     double2* spec = d_spec.get();
     auto synth = [&](int64_t len, bool named, int out_dtype, void* dst) {
-      int64_t count = frames;
-      if (named) count = std::min(frames, (len + left + hop - 1) / hop);
-      if (count == 0) {
-        CK(cudaMemsetAsync(dst, 0, (size_t)batch * (size_t)len * dtype_size(out_dtype), st));
-        return;
-      }
-      smb::IstftArgs a{};
-      a.z = spec;
-      a.out = dst;
-      a.frames = frames;
-      a.count = count;
-      a.out_len = len;
-      a.fft = (int)p->geom.fft;
-      a.hop = (int)hop;
-      a.left = (int)left;
-      a.window = d.d_window64.get();
-      a.twiddle = d.d_twiddle64.get();
-      a.folded = d.d_folded.get();
-      a.in_f64 = 1;
-      a.out_f64 = out_dtype == SMB_F64;
-      CK(smb::launch_istft(a, batch, st));
+      const smb::IstftArgs a = istft_args(p, spec, dst, batch, frames, named, len, SMB_F64, out_dtype);
+      if (a.count) CK(smb::launch_istft(a, batch, st));
     };
     CK(smb::launch_gl_project(mags, phase, dtype == SMB_F64, nullptr, nullptr, 0.0, 1,
                               (long long)cells, spec, st));
@@ -1804,20 +1799,14 @@ int smb_phase_vocoder(smb_stft_plan* plan, const void* z, int64_t batch, int64_t
     if (batch < 0)
       throw smb::invalid_argument("phase_vocoder: batch must be non-negative");
     const size_t csz = 2 * dtype_size(dtype);
-    if (mem != SMB_MEM_DEVICE && mem != SMB_MEM_HOST)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    check_mem(mem);
     if (batch == 0 || out_frames == 0) return;
     p->ensure_device();
-    auto run = [&](const void* dz, void* dout, int64_t nb) {
-      run_vocoder(p, dz, dout, nb, frames, out_frames, dtype, rate);
-    };
-    if (mem == SMB_MEM_DEVICE) {
-      run(z, out, batch);
-      return;
-    }
     const size_t bins = (size_t)p->geom.bins();
-    p->pipe.execute(p->dev->stream.use, z, out, batch, bins * (size_t)frames * csz,
-                    bins * (size_t)out_frames * csz, run);
+    dispatch(mem, p->pipe, p->dev->stream.use, z, out, batch, bins * (size_t)frames * csz,
+             bins * (size_t)out_frames * csz, [&](const void* dz, void* dout, int64_t nb) {
+               run_vocoder(p, dz, dout, nb, frames, out_frames, dtype, rate);
+             });
   });
 }
 
@@ -1827,15 +1816,9 @@ int smb_time_stretch(smb_stft_plan* plan, const void* x, int64_t batch, int64_t 
     smb_stft_plan* p = plan;
     check_rate("time_stretch", rate);
     check_signal("time_stretch", batch, n);
-    if (!p->nola())                                     // Stft.invert's precondition
-      throw smb::invalid_argument(smb::format(
-          "invert: cannot invert a %lld-point window advanced by %lld samples inside a "
-          "%lld-point frame (the overlap-added squared window must stay above 1e-10 of its "
-          "largest value at every position)",
-          (long long)p->geom.win_length, (long long)p->geom.hop, (long long)p->geom.fft));
+    require_nola("invert", p);                          // Stft.invert's precondition
     const size_t esz = dtype_size(dtype);
-    if (mem != SMB_MEM_DEVICE && mem != SMB_MEM_HOST)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    check_mem(mem);
     const int64_t out_len = stretch_length(n, rate);
     const smb::FrameGeom g = p->frame_geom(n);
     const int64_t out_frames = vocoder_frames("time_stretch", g.frames, rate);
@@ -1856,11 +1839,7 @@ int smb_time_stretch(smb_stft_plan* plan, const void* x, int64_t batch, int64_t 
       run_vocoder(p, spec, voc, nb, g.frames, out_frames, dtype, rate);
       run_invert(p, voc, dout, nb, out_frames, true, out_len, dtype, dtype);
     };
-    if (mem == SMB_MEM_DEVICE) {
-      run(x, out, batch);
-      return;
-    }
-    p->pipe.execute(st, x, out, batch, (size_t)n * esz, (size_t)out_len * esz, run);
+    dispatch(mem, p->pipe, st, x, out, batch, (size_t)n * esz, (size_t)out_len * esz, run);
   });
 }
 
@@ -1934,23 +1913,23 @@ int smb_mel_apply(smb_mel_plan* plan, const void* s, int64_t batch, int64_t fram
     if (batch == 0 || frames == 0) return;       // zero-size: nothing to reduce (mel.ml:221-227)
     plan->ensure_device();
     cudaStream_t st = plan->dev->stream.use;
-    if (mem == SMB_MEM_DEVICE) {
-      run_mel_apply(plan, s, batch, frames, dtype, out, st);
-      return;
-    }
-    if (mem != SMB_MEM_HOST) throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    const size_t in_bytes = (size_t)batch * plan->bins * frames * esz;
-    const size_t out_bytes = (size_t)batch * plan->n_mels * frames * esz;
-    void* din = plan->in.ensure(in_bytes);
-    void* dout = plan->out.ensure(out_bytes);
-    CK(cudaMemcpyAsync(din, s, in_bytes, cudaMemcpyHostToDevice, st));
-    run_mel_apply(plan, din, batch, frames, dtype, dout, st);
-    CK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
+    dispatch(mem, plan->pipe, st, s, out, batch, (size_t)plan->bins * frames * esz,
+             (size_t)plan->n_mels * frames * esz, [&](const void* din, void* dout, int64_t nb) {
+               run_mel_apply(plan, din, nb, frames, dtype, dout, st);
+             });
   });
 }
 
 }  // extern "C"
+
+// soundml.ml:12-20, 50-70
+static void require_same_fft(const char* op, const smb_stft_plan* stft, const smb_mel_plan* mel) {
+  if (stft->geom.fft != mel->fft)
+    throw smb::invalid_argument(smb::format(
+        "%s: cannot project a %lld-point STFT through a filterbank built for an FFT of size "
+        "%lld (the two configurations must agree on fft_size)",
+        op, (long long)stft->geom.fft, (long long)mel->fft));
+}
 
 // Soundml.mel_spectrogram.  max_slot (device, zeroed by the caller, may be null): where
 // the kernel leaves the maximum of what it writes; the return value says whether it did
@@ -1960,12 +1939,7 @@ static bool mel_spectrogram_impl(smb_stft_plan* stft, smb_mel_plan* mel, const v
                                  unsigned long long* max_slot) {
   bool max_known = false;
   {
-    // soundml.ml:12-20
-    if (stft->geom.fft != mel->fft)
-      throw smb::invalid_argument(smb::format(
-          "mel_spectrogram: cannot project a %lld-point STFT through a filterbank built for "
-          "an FFT of size %lld (the two configurations must agree on fft_size)",
-          (long long)stft->geom.fft, (long long)mel->fft));
+    require_same_fft("mel_spectrogram", stft, mel);
     check_signal("power_spectrum", batch, n);
     const size_t esz = dtype_size(dtype);
     const smb::FrameGeom g = stft->frame_geom(n);
@@ -1982,19 +1956,8 @@ static bool mel_spectrogram_impl(smb_stft_plan* stft, smb_mel_plan* mel, const v
         a.max_slot = max_slot;
         CK(smb::launch_stft2048p(a, false, sd.sm_count, st));
       } else if (fast) {
-        smb::Stft2048Args a{};
-        a.x = (const float*)din;
-        a.out = (float*)dout;
-        a.batch = nb;
-        a.g = g;
-        a.g.fft = 2048;
-        a.bin_step = stft->fast_step();
-        a.window = sd.d_window32.get();
-        a.tw_pass = sd.d_tw_pass.get();
-        a.tw_post = sd.d_tw_post.get();
+        smb::Stft2048Args a = fused_args(stft, din, dout, nb, g, power);
         a.n_mels = (int)mel->n_mels;
-        a.power = (float)power;
-        a.dft_images = sd.d_dft_images.get();
         const auto& sc = fast == SMB_PATH_TENSOR ? mel->sched_tc : mel->sched_cc;
         const auto& tables = fast == SMB_PATH_TENSOR ? mel->dev->tc : mel->dev->cc;
         a.nnz = (int)sc.vals.size();
@@ -2014,14 +1977,36 @@ static bool mel_spectrogram_impl(smb_stft_plan* stft, smb_mel_plan* mel, const v
         run_mel_apply(mel, spec, nb, g.frames, dtype, dout, st);
       }
     };
-    if (mem == SMB_MEM_DEVICE) {
-      run(x, out, batch);
-    } else if (mem == SMB_MEM_HOST) {
-      stft->pipe.execute(st, x, out, batch, (size_t)n * esz,
-                         (size_t)mel->n_mels * g.frames * esz, run);
-    } else {
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    }
+    dispatch(mem, stft->pipe, st, x, out, batch, (size_t)n * esz, (size_t)mel->n_mels * g.frames * esz, run);
+  }
+  return max_known;
+}
+
+// The mel spectrogram of host or device audio into dmel (device), its maximum in the mel
+// plan's slot where the return value says so (mel_spectrogram_impl).  Host audio goes up in
+// slices of about 64 MB: the whole-tensor maximum needs every slice's mel values before the
+// first value in decibels, so those stay on the device -- a quarter of the audio's size --
+// but the audio never does at once.
+static bool mel_spectrogram_to_device(smb_stft_plan* stft, smb_mel_plan* mel, const void* x,
+                                      int64_t batch, int64_t n, int dtype, double power, void* dmel,
+                                      int mem) {
+  const size_t esz = dtype_size(dtype);
+  cudaStream_t st = stft->dev->stream.use;
+  unsigned long long* d_max = mel->dev->d_max.get();
+  CK(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
+  if (mem == SMB_MEM_DEVICE)
+    return mel_spectrogram_impl(stft, mel, x, batch, n, dtype, power, dmel, SMB_MEM_DEVICE, d_max);
+  const size_t mel_item = (size_t)mel->n_mels * stft->geom.frames(n) * esz;
+  const int64_t per = std::max<int64_t>(1, (int64_t)(64u << 20) / std::max<int64_t>(1, n * (int64_t)esz));
+  bool max_known = true;
+  for (int64_t b0 = 0; b0 < batch; b0 += per) {
+    const int64_t nb = std::min(per, batch - b0);
+    void* stage = stft->pipe.in[0].ensure((size_t)std::min(per, batch) * n * esz);
+    CK(cudaMemcpyAsync(stage, (const char*)x + (size_t)b0 * n * esz, (size_t)nb * n * esz,
+                       cudaMemcpyHostToDevice, st));
+    max_known = mel_spectrogram_impl(stft, mel, stage, nb, n, dtype, power,
+                                     (char*)dmel + (size_t)b0 * mel_item, SMB_MEM_DEVICE, d_max) &&
+                max_known;
   }
   return max_known;
 }
@@ -2068,10 +2053,9 @@ namespace {
 
 const double kDecade = 10.0 / std::log(10.0);     // convert.ml:27
 
-void to_db_call(const char* fn, double gain, int magnitude, const void* x, int64_t count,
-                int dtype, double reference, double amin, double top_db, void* out, int mem,
-                void* stream) {
-  // convert.ml:8-22: checks in the reference's order and wording
+// convert.ml:8-22: checks in the reference's order and wording.  Returns whether top_db
+// (NaN: none) clamps.
+bool check_db_args(const char* fn, double reference, double amin, double top_db) {
   if (!(std::isfinite(reference) && reference > 0.0))
     throw smb::invalid_argument(smb::format("Soundml.Convert.%s: reference must be finite and positive", fn));
   if (!(std::isfinite(amin) && amin > 0.0))
@@ -2079,6 +2063,13 @@ void to_db_call(const char* fn, double gain, int magnitude, const void* x, int64
   const bool clamp = !std::isnan(top_db);
   if (clamp && !(std::isfinite(top_db) && top_db >= 0.0))
     throw smb::invalid_argument(smb::format("Soundml.Convert.%s: top_db must be finite and non-negative", fn));
+  return clamp;
+}
+
+void to_db_call(const char* fn, double gain, int magnitude, const void* x, int64_t count,
+                int dtype, double reference, double amin, double top_db, void* out, int mem,
+                void* stream) {
+  const bool clamp = check_db_args(fn, reference, amin, top_db);
   if (count < 0) throw smb::invalid_argument("to_db: negative extent");
   const size_t esz = dtype_size(dtype);
   if (count == 0) return;
@@ -2093,14 +2084,13 @@ void to_db_call(const char* fn, double gain, int magnitude, const void* x, int64
   scratch_ptr din, dout;
   const void* src = x;
   void* dst = out;
+  check_mem(mem);
   if (mem == SMB_MEM_HOST) {
     din = scratch_alloc((size_t)count * esz, st);
     dout = scratch_alloc((size_t)count * esz, st);
     CK(cudaMemcpyAsync(din.get(), x, (size_t)count * esz, cudaMemcpyHostToDevice, st));
     src = din.get();
     dst = dout.get();
-  } else if (mem != SMB_MEM_DEVICE) {
-    throw smb::invalid_argument("soundml_b200: unknown memory kind");
   }
   CK(smb::launch_to_db(src, count, dtype, magnitude, amin, scale, offset, clamp,
                        clamp ? top_db : 0.0, (unsigned long long*)slot.get(), dst, st));
@@ -2131,12 +2121,7 @@ int smb_amplitude_to_db(const void* x, int64_t count, int dtype, double referenc
 int smb_mfcc(smb_stft_plan* stft, smb_mel_plan* mel, const void* x, int64_t batch, int64_t n,
              int dtype, int64_t n_mfcc, double lifter, void* out, int mem) {
   return guarded([&] {
-    // soundml.ml:50-70
-    if (stft->geom.fft != mel->fft)
-      throw smb::invalid_argument(smb::format(
-          "mfcc: cannot project a %lld-point STFT through a filterbank built for an FFT of size "
-          "%lld (the two configurations must agree on fft_size)",
-          (long long)stft->geom.fft, (long long)mel->fft));
+    require_same_fft("mfcc", stft, mel);
     if (n_mfcc < 1 || n_mfcc > mel->n_mels)
       throw smb::invalid_argument(smb::format(
           "mfcc: cannot keep %lld cepstral coefficients of %lld mel bands (n_mfcc must lie in "
@@ -2160,29 +2145,8 @@ int smb_mfcc(smb_stft_plan* stft, smb_mel_plan* mel, const void* x, int64_t batc
     const size_t out_bytes = (size_t)batch * n_mfcc * g.frames * esz;
     void* dmel = stft->cepstral.ensure(mel_bytes + out_bytes);
     void* dout = mem == SMB_MEM_HOST ? (void*)((char*)dmel + mel_bytes) : out;
-    const int inner_mem = mem == SMB_MEM_HOST ? SMB_MEM_HOST : SMB_MEM_DEVICE;
-    if (inner_mem != SMB_MEM_HOST && mem != SMB_MEM_DEVICE)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    // the frame-pair kernel leaves the mel spectrogram's maximum in the slot as it writes
-    CK(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
-    bool max_known = true;
-    if (inner_mem == SMB_MEM_HOST) {
-      // host audio goes up in slices of about 64 MB (the whole-tensor maximum needs every
-      // slice's mel values before the first cepstral coefficient, so those stay on the
-      // device -- a quarter of the audio's size -- but the audio never does at once)
-      const int64_t per = std::max<int64_t>(1, (int64_t)(64u << 20) / std::max<int64_t>(1, n * (int64_t)esz));
-      for (int64_t b0 = 0; b0 < batch; b0 += per) {
-        const int64_t nb = std::min(per, batch - b0);
-        void* stage = stft->pipe.in[0].ensure((size_t)std::min(per, batch) * n * esz);
-        CK(cudaMemcpyAsync(stage, (const char*)x + (size_t)b0 * n * esz, (size_t)nb * n * esz,
-                           cudaMemcpyHostToDevice, st));
-        max_known = mel_spectrogram_impl(stft, mel, stage, nb, n, dtype, 2.0,
-                                         (char*)dmel + (size_t)b0 * mel->n_mels * g.frames * esz,
-                                         SMB_MEM_DEVICE, d_max) && max_known;
-      }
-    } else {
-      max_known = mel_spectrogram_impl(stft, mel, x, batch, n, dtype, 2.0, dmel, SMB_MEM_DEVICE, d_max);
-    }
+    check_mem(mem);
+    const bool max_known = mel_spectrogram_to_device(stft, mel, x, batch, n, dtype, 2.0, dmel, mem);
     const double scale = kDecade, offset = scale * std::log(1.0);   // reference 1, amin 1e-10
     CK(smb::launch_mfcc(dmel, dtype, batch, (int)mel->n_mels, g.frames, (int)n_mfcc,
                         mel->dct_table(n_mfcc, has_lifter ? lifter : 0.0), d_max, max_known,
@@ -2203,20 +2167,11 @@ int smb_mel_spectrogram_db(smb_stft_plan* stft, smb_mel_plan* mel, const void* x
                            int64_t n, int dtype, double power, double reference, double amin,
                            double top_db, void* out, int mem) {
   return guarded([&] {
-    const char* fn = "power_to_db";
-    if (!(std::isfinite(reference) && reference > 0.0))
-      throw smb::invalid_argument(smb::format("Soundml.Convert.%s: reference must be finite and positive", fn));
-    if (!(std::isfinite(amin) && amin > 0.0))
-      throw smb::invalid_argument(smb::format("Soundml.Convert.%s: amin must be finite and positive", fn));
-    const bool clamp = !std::isnan(top_db);
-    if (clamp && !(std::isfinite(top_db) && top_db >= 0.0))
-      throw smb::invalid_argument(smb::format("Soundml.Convert.%s: top_db must be finite and non-negative", fn));
-    if (mem != SMB_MEM_HOST && mem != SMB_MEM_DEVICE)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    if (stft->geom.fft != mel->fft || batch < 0 || n < 0) {   // the composition's first checks, its wording
-      mel_spectrogram_impl(stft, mel, x, batch, n, dtype, power, out, mem, nullptr);
-      return;
-    }
+    const bool clamp = check_db_args("power_to_db", reference, amin, top_db);
+    check_mem(mem);
+    // the composition's first checks, in its wording
+    require_same_fft("mel_spectrogram", stft, mel);
+    check_signal("power_spectrum", batch, n);
     const size_t esz = dtype_size(dtype);
     const smb::FrameGeom g = stft->frame_geom(n);
     if (batch == 0 || g.frames == 0) return;
@@ -2225,16 +2180,9 @@ int smb_mel_spectrogram_db(smb_stft_plan* stft, smb_mel_plan* mel, const void* x
     cudaStream_t st = stft->dev->stream.use;
     unsigned long long* d_max = mel->dev->d_max.get();
     const int64_t count = batch * mel->n_mels * g.frames;
+    // the result stays on the device until it is in decibels
     void* dmel = mem == SMB_MEM_HOST ? stft->cepstral.ensure((size_t)count * esz) : out;
-    CK(cudaMemsetAsync(d_max, 0, sizeof(unsigned long long), st));
-    const void* din = x;
-    if (mem == SMB_MEM_HOST) {          // the result stays on the device until it is in decibels
-      void* stage = stft->pipe.in[0].ensure((size_t)batch * n * esz);
-      CK(cudaMemcpyAsync(stage, x, (size_t)batch * n * esz, cudaMemcpyHostToDevice, st));
-      din = stage;
-    }
-    const bool max_known = mel_spectrogram_impl(stft, mel, din, batch, n, dtype, power, dmel,
-                                                SMB_MEM_DEVICE, d_max);
+    const bool max_known = mel_spectrogram_to_device(stft, mel, x, batch, n, dtype, power, dmel, mem);
     const double scale = kDecade;                                   // gain 10: powers
     const double offset = scale * std::log(std::max(amin, reference));
     if (max_known)
@@ -2276,11 +2224,15 @@ int smb_resample_plan_set_executor(smb_resample_plan* plan, int exec) {
     plan->executor = exec;
   });
 }
+static const smb::ResampleStage& stage_of(const smb_resample_plan* plan, int stage, const char* op) {
+  if (stage < 0 || stage >= (int)plan->plan.stages.size())
+    throw smb::invalid_argument(smb::format("%s: no such stage", op));
+  return plan->plan.stages[(size_t)stage];
+}
 int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
                               smb_resample_layout* out) {
   return guarded([&] {
-    if (stage < 0 || stage >= (int)plan->plan.stages.size())
-      throw smb::invalid_argument("stage_layout: no such stage");
+    const smb::ResampleStage& s = stage_of(plan, stage, "stage_layout");
     plan->ensure_device();
     const GemmDevice& gd = plan->dev->gemm[(size_t)stage];
     smb_resample_layout r{};
@@ -2304,7 +2256,7 @@ int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
       r.col_begin = gd.groups[(size_t)group].col_begin;
       r.chunks = gd.groups[(size_t)group].chunks;
     } else {
-      r.columns = (int)plan->plan.stages[(size_t)stage].l;
+      r.columns = (int)s.l;
     }
     *out = r;
   });
@@ -2322,9 +2274,7 @@ static void ols_geometry_of(const smb::OlsPlan& p, smb_ols_geometry* out) {
 }
 int smb_resample_stage_ols(const smb_resample_plan* plan, int stage, smb_ols_geometry* out) {
   return guarded([&] {
-    if (stage < 0 || stage >= (int)plan->plan.stages.size())
-      throw smb::invalid_argument("stage_ols: no such stage");
-    ols_geometry_of(smb::ols_plan_for_stage(plan->plan.stages[(size_t)stage]), out);
+    ols_geometry_of(smb::ols_plan_for_stage(stage_of(plan, stage, "stage_ols")), out);
   });
 }
 int smb_fir_ols(const smb_fir_plan* plan, smb_ols_geometry* out) {
@@ -2358,9 +2308,7 @@ int smb_resample_stage_info(const smb_resample_plan* plan, int stage, int64_t* l
                             int64_t* k, int* exec, int64_t* ols_n, int64_t* ols_b,
                             int64_t* ols_delta) {
   return guarded([&] {
-    if (stage < 0 || stage >= (int)plan->plan.stages.size())
-      throw smb::invalid_argument("stage_info: no such stage");
-    const smb::ResampleStage& s = plan->plan.stages[(size_t)stage];
+    const smb::ResampleStage& s = stage_of(plan, stage, "stage_info");
     if (l) *l = s.l;
     if (m) *m = s.m;
     if (k) *k = s.k;
@@ -2373,18 +2321,15 @@ int smb_resample_stage_info(const smb_resample_plan* plan, int stage, int64_t* l
 int smb_resample_stage_design(const smb_resample_plan* plan, int stage, double* fc,
                               double* beta) {
   return guarded([&] {
-    if (stage < 0 || stage >= (int)plan->plan.stages.size())
-      throw smb::invalid_argument("stage_design: no such stage");
-    if (fc) *fc = plan->plan.stages[(size_t)stage].fc;
-    if (beta) *beta = plan->plan.stages[(size_t)stage].beta;
+    const smb::ResampleStage& s = stage_of(plan, stage, "stage_design");
+    if (fc) *fc = s.fc;
+    if (beta) *beta = s.beta;
   });
 }
 int smb_resample_stage_prototype(const smb_resample_plan* plan, int stage, double* out,
                                  int64_t* len) {
   return guarded([&] {
-    if (stage < 0 || stage >= (int)plan->plan.stages.size())
-      throw smb::invalid_argument("stage_prototype: no such stage");
-    const std::vector<double>& h = plan->plan.stages[(size_t)stage].proto;
+    const std::vector<double>& h = stage_of(plan, stage, "stage_prototype").proto;
     if (len) *len = (int64_t)h.size();
     if (out) std::memcpy(out, h.data(), h.size() * sizeof(double));
   });
@@ -2395,37 +2340,49 @@ int64_t smb_resample_output_frames(const smb_resample_plan* plan, int64_t n) {
   return r;
 }
 
+}  // extern "C"
+
+// Resample.apply over a batch of independent signals: a copy for the identity, one stage, or
+// a cascade through the plan's hand-off buffer; a host batch goes through in slices, the
+// copies of one slice under the kernels of its neighbours (HostPipe).
+// stage(i, x, nb, n, n_out, out, st) launches stage i over device buffers.
+template <typename T, typename Stage>
+static void resample_call(smb_resample_plan* plan, const T* x, int64_t batch, int64_t n, T* out,
+                          int mem, Stage&& stage) {
+  if (batch < 0) throw smb::invalid_argument("apply: negative batch");
+  const smb::ResamplePlan& rp = plan->plan;
+  const int64_t total = rp.output_frames(n);
+  if (batch == 0 || n == 0 || total == 0) return;
+  plan->ensure_device();
+  cudaStream_t st = plan->dev->stream.use;
+  auto run = [&](const void* din_v, void* dout_v, int64_t nb) {
+    const T* din = (const T*)din_v;
+    T* dout = (T*)dout_v;
+    if (rp.identity()) {
+      CK(cudaMemcpyAsync(dout, din, (size_t)nb * n * sizeof(T), cudaMemcpyDeviceToDevice, st));
+    } else if (rp.stages.size() == 1) {
+      stage(0, din, nb, n, total, dout, st);
+    } else {
+      // cascade (resample.ml:1819-1842): stage 1 emits its exact ceil tail,
+      // stage 2 runs over it with zeros beyond and is cut to output_frames.
+      const smb::ResampleStage& s1 = rp.stages[0];
+      const int64_t n1 = (n * s1.l + s1.m - 1) / s1.m;
+      T* mid = (T*)plan->mid.ensure((size_t)nb * n1 * sizeof(T));
+      stage(0, din, nb, n, n1, mid, st);
+      stage(1, mid, nb, n1, total, dout, st);
+    }
+  };
+  dispatch(mem, plan->pipe, st, x, out, batch, (size_t)n * sizeof(T), (size_t)total * sizeof(T), run);
+}
+
+extern "C" {
+
 int smb_resample_apply(smb_resample_plan* plan, const float* x, int64_t batch, int64_t n,
                        float* out, int mem) {
   return guarded([&] {
-    if (batch < 0) throw smb::invalid_argument("apply: negative batch");
-    const smb::ResamplePlan& rp = plan->plan;
-    const int64_t total = rp.output_frames(n);
-    if (batch == 0 || n == 0 || total == 0) return;
-    plan->ensure_device();
-    cudaStream_t st = plan->dev->stream.use;
-    // signals are independent: a host batch goes through in slices, the copies of one
-    // slice under the kernels of its neighbours (HostPipe)
-    auto run = [&](const void* din_v, void* dout_v, int64_t nb) {
-      const float* din = (const float*)din_v;
-      float* dout = (float*)dout_v;
-      if (rp.identity()) {
-        CK(cudaMemcpyAsync(dout, din, (size_t)nb * n * 4, cudaMemcpyDeviceToDevice, st));
-      } else if (rp.stages.size() == 1) {
-        plan->run_stage(0, din, nb, n, total, dout, st);
-      } else {
-        // cascade (resample.ml:1819-1842): stage 1 emits its exact ceil tail,
-        // stage 2 runs over it with zeros beyond and is cut to output_frames.
-        const smb::ResampleStage& s1 = rp.stages[0];
-        const int64_t n1 = (n * s1.l + s1.m - 1) / s1.m;
-        float* mid = (float*)plan->mid.ensure((size_t)nb * n1 * 4);
-        plan->run_stage(0, din, nb, n, n1, mid, st);
-        plan->run_stage(1, mid, nb, n1, total, dout, st);
-      }
-    };
-    if (mem == SMB_MEM_DEVICE) run(x, out, batch);
-    else if (mem == SMB_MEM_HOST) plan->pipe.execute(st, x, out, batch, (size_t)n * 4, (size_t)total * 4, run);
-    else throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    resample_call(plan, x, batch, n, out, mem,
+                  [&](size_t i, const float* src, int64_t nb, int64_t len, int64_t n_out, float* dst,
+                      cudaStream_t st) { plan->run_stage(i, src, nb, len, n_out, dst, st); });
   });
 }
 
@@ -2434,43 +2391,13 @@ int smb_resample_apply(smb_resample_plan* plan, const float* x, int64_t batch, i
 int smb_resample_apply_f64(smb_resample_plan* plan, const double* x, int64_t batch, int64_t n,
                            double* out, int mem) {
   return guarded([&] {
-    if (batch < 0) throw smb::invalid_argument("apply: negative batch");
-    const smb::ResamplePlan& rp = plan->plan;
-    const int64_t total = rp.output_frames(n);
-    if (batch == 0 || n == 0 || total == 0) return;
-    plan->ensure_device();
-    cudaStream_t st = plan->dev->stream.use;
-    const size_t in_bytes = (size_t)batch * n * 8, out_bytes = (size_t)batch * total * 8;
-    const double* din = x;
-    double* dout = out;
-    if (mem == SMB_MEM_HOST) {
-      double* stage = (double*)plan->in.ensure(in_bytes);
-      dout = (double*)plan->out.ensure(out_bytes);
-      CK(cudaMemcpyAsync(stage, x, in_bytes, cudaMemcpyHostToDevice, st));
-      din = stage;
-    } else if (mem != SMB_MEM_DEVICE) {
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
-    }
-    auto stage_run = [&](size_t i, const double* src, int64_t len, int64_t n_out, double* dst) {
-      const smb::ResampleStage& s = rp.stages[i];
-      CK(smb::launch_polyphase_direct_f64(src, batch, len, plan->dev->d_bank64[i].get(), (int)s.l, (int)s.m,
-                                          (int)s.k, n_out, dst, st));
-    };
-    if (rp.identity()) {
-      CK(cudaMemcpyAsync(dout, din, in_bytes, cudaMemcpyDeviceToDevice, st));
-    } else if (rp.stages.size() == 1) {
-      stage_run(0, din, n, total, dout);
-    } else {
-      const smb::ResampleStage& s1 = rp.stages[0];
-      const int64_t n1 = (n * s1.l + s1.m - 1) / s1.m;
-      double* mid = (double*)plan->mid.ensure((size_t)batch * n1 * 8);
-      stage_run(0, din, n, n1, mid);
-      stage_run(1, mid, n1, total, dout);
-    }
-    if (mem == SMB_MEM_HOST) {
-      CK(cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, st));
-      CK(cudaStreamSynchronize(st));
-    }
+    resample_call(plan, x, batch, n, out, mem,
+                  [&](size_t i, const double* src, int64_t nb, int64_t len, int64_t n_out, double* dst,
+                      cudaStream_t st) {
+                    const smb::ResampleStage& s = plan->plan.stages[i];
+                    CK(smb::launch_polyphase_direct_f64(src, nb, len, plan->dev->d_bank64[i].get(), (int)s.l,
+                                                        (int)s.m, (int)s.k, n_out, dst, st));
+                  });
   });
 }
 
@@ -2621,8 +2548,7 @@ int smb_resample_kernel_step(smb_resample_kernel* k, const void* chunk, int64_t 
       throw smb::invalid_argument(smb::format(
           "step: cannot feed a %lld-sample chunk (max_block is %lld)", (long long)n,
           (long long)k->max_block));
-    if (mem != SMB_MEM_HOST && mem != SMB_MEM_DEVICE)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    check_mem(mem);
     if (n == 0) return;
     k->plan->ensure_device();
     cudaStream_t st = k->plan->dev->stream.use;
@@ -2649,8 +2575,7 @@ int smb_resample_kernel_flush(smb_resample_kernel* k, void* out, int mem) {
   return guarded([&] {
     if (k->drained) return;
     k->drained = true;
-    if (mem != SMB_MEM_HOST && mem != SMB_MEM_DEVICE)
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    check_mem(mem);
     const int64_t total = k->fed ? k->plan->plan.output_frames(k->fed) : 0;
     if (total <= k->emitted) return;
     k->plan->ensure_device();
@@ -2699,9 +2624,7 @@ int smb_fir_apply(smb_fir_plan* plan, const float* x, int64_t batch, int64_t n, 
         CK(smb::launch_polyphase_direct((const float*)din, nb, n, plan->dev->d_bank.get(), 1, 1, (int)plan->k, n,
                                         (float*)dout, st));
     };
-    if (mem == SMB_MEM_DEVICE) run(x, out, batch);
-    else if (mem == SMB_MEM_HOST) plan->pipe.execute(st, x, out, batch, (size_t)n * 4, (size_t)n * 4, run);
-    else throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    dispatch(mem, plan->pipe, st, x, out, batch, (size_t)n * 4, (size_t)n * 4, run);
   });
 }
 // ---- soundml-io device ingest ------------------------------------------------------
@@ -2725,9 +2648,8 @@ int smb_ingest_layout(const void* interleaved, int64_t frames, int64_t channels,
       throw smb::invalid_argument("ingest: the block does not fit the destination "
                                   "(need 0 <= out_off, out_off + frames <= out_total)");
     const size_t esz = dtype_size(dtype);
-    if ((mem_in != SMB_MEM_HOST && mem_in != SMB_MEM_DEVICE) ||
-        (mem_out != SMB_MEM_HOST && mem_out != SMB_MEM_DEVICE))
-      throw smb::invalid_argument("soundml_b200: unknown memory kind");
+    check_mem(mem_in);
+    check_mem(mem_out);
     if (frames == 0) return;
     require_device();
     cudaStream_t st = (cudaStream_t)cuda_stream;
