@@ -293,9 +293,9 @@ int smb_resample_plan_sync(smb_resample_plan* plan);
  * everywhere.  Same designed filter either way. */
 int smb_resample_plan_set_executor(smb_resample_plan* plan, int exec);
 /* Which kernel smb_resample_apply runs for one stage (float32 audio), and how its
- * device tables are laid out.  Read-only; the device tables are built first if no
- * apply has built them yet, so the SMB_ROWS_* and SMB_GEMM_WINDOWS environment
- * switches set at that moment take effect, as they would for a first apply. */
+ * tables are laid out.  Host-only: no device is needed or touched.  The plan's tables
+ * are built by the first layout or apply call, and the SMB_ROWS_* environment switches
+ * are read then; SMB_GEMM_WINDOWS is read at every call. */
 enum { SMB_FORM_DIRECT = 0, SMB_FORM_OLS = 1, SMB_FORM_WINDOW = 2, SMB_FORM_ROW = 3 };
 typedef struct smb_resample_layout {
   int form;          /* SMB_FORM_*: direct kernel, overlap-save, tcgen05 window or row form */

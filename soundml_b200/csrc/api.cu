@@ -4,7 +4,6 @@
 // Preconditions are checked in the reference's order and with its messages
 // (SMB_EINVAL = Invalid_argument); CUDA failures are SMB_ECUDA.  There is no
 // CPU execution path in this library.
-#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <memory>
@@ -17,6 +16,7 @@
 
 #include "../../include/soundml_b200.h"
 #include "host_design.h"
+#include "kernel_tables.h"
 #include "kernels.h"
 
 namespace {
@@ -236,36 +236,6 @@ size_t dtype_size(int dtype) {
   throw smb::invalid_argument("soundml_b200: dtype must be SMB_F32 or SMB_F64");
 }
 
-const double kTwoPi = 6.283185307179586476925286766559;
-
-// The inter-pass twiddles of the warp FFT 1024 (32 x 32): W_1024^(k1 n2) at [k1][n2].
-std::vector<float2> fft1024_pass_twiddles() {
-  std::vector<float2> pass(1024);
-  for (int k1 = 0; k1 < 32; ++k1)
-    for (int n2 = 0; n2 < 32; ++n2) {
-      const double a = kTwoPi * double(k1 * n2) / 1024.0;
-      pass[(size_t)(k1 * 32 + n2)] = make_float2((float)std::cos(a), (float)-std::sin(a));
-    }
-  return pass;
-}
-
-// Puts weight g at (row r, element k < 32) of a tensor-core resampler B slice that starts
-// at float `base` and holds `rows` rows per split: its tf32 piece hi (the float's leading
-// 10 fraction bits, exact) in the first split and lo = g - hi in the second, each at the
-// K-major SWIZZLE_128B cell (128-byte rows, 16-byte chunk index XOR row mod 8).
-void put_tf32_split(std::vector<float>& img, size_t base, int64_t rows, int64_t r, int64_t k, double g) {
-  const float gf = (float)g;
-  uint32_t bits;
-  std::memcpy(&bits, &gf, 4);
-  bits &= 0xFFFFE000u;
-  float hi;
-  std::memcpy(&hi, &bits, 4);
-  const float lo = (float)(g - (double)hi);
-  const size_t cell = (size_t)(r * 32 + ((((k >> 2) ^ (r & 7)) << 2) | (k & 3)));
-  img[base + cell] = hi;
-  img[base + (size_t)rows * 32 + cell] = lo;
-}
-
 }  // namespace
 
 // A plan's tables, scratch and stream belong to the device that was current when it was
@@ -278,6 +248,17 @@ void same_device(int bound) {
     throw smb::invalid_argument(smb::format(
         "soundml_b200: the plan is bound to CUDA device %d but device %d is current "
         "(one plan per device; cudaSetDevice before the call)", bound, now));
+}
+
+// A plan's Device on the current device, with its stream and the device's multiprocessor count.
+template <typename Device>
+std::unique_ptr<Device> new_device() {
+  require_device();
+  auto d = std::make_unique<Device>();
+  CK(cudaGetDevice(&d->device));
+  CK(cudaDeviceGetAttribute(&d->sm_count, cudaDevAttrMultiProcessorCount, d->device));
+  d->stream.create();
+  return d;
 }
 
 // ============================ plan types =====================================
@@ -307,50 +288,17 @@ struct smb_stft_plan {
 
   void ensure_device() {
     if (dev) return same_device(dev->device);
-    require_device();
-    auto d = std::make_unique<Device>();
-    CK(cudaGetDevice(&d->device));
-    CK(cudaDeviceGetAttribute(&d->sm_count, cudaDevAttrMultiProcessorCount, d->device));
-    d->stream.create();
+    auto d = new_device<Device>();
     d->d_window64 = upload(window);
-    const int64_t n = geom.fft;
-    std::vector<double2> tw((size_t)n);
-    for (int64_t j = 0; j < n; ++j) {
-      const double a = kTwoPi * double(j) / double(n);
-      tw[(size_t)j] = make_double2(std::cos(a), -std::sin(a));
-    }
-    d->d_twiddle64 = upload(tw);
+    d->d_twiddle64 = upload(smb::unit_roots<double2>(geom.fft, geom.fft));
     if (fast_step() > 0) {
       // shorter frames run zero-padded to 2048: the window's tail is zero
       std::vector<float> w32(2048, 0.0f);
-      for (int64_t j = 0; j < n; ++j) w32[(size_t)j] = (float)window[(size_t)j];
+      for (int64_t j = 0; j < geom.fft; ++j) w32[(size_t)j] = (float)window[(size_t)j];
       d->d_window32 = upload(w32);
-      std::vector<float2> post(512);
-      for (int j = 0; j < 16; ++j)
-        for (int l = 0; l < 32; ++l) {
-          const double a = kTwoPi * double(l + 32 * j) / 2048.0;
-          post[(size_t)(j * 32 + l)] = make_float2((float)std::cos(a), (float)-std::sin(a));
-        }
-      d->d_tw_pass = upload(fft1024_pass_twiddles());
-      d->d_tw_post = upload(post);
-      // The 32-point DFT in real arithmetic, F[n = (k, c')][j = (m, c)] with
-      // (re, im) interleaved: out_re = sum in_re cos + in_im sin, out_im = sum
-      // in_im cos - in_re sin (angle 2 pi m k / 32).  Two fp16 images (leading 11
-      // bits, remainder) in the K-major SWIZZLE_128B operand layout: row n is
-      // 128 bytes, its 16-byte chunk q sits at position q ^ (n mod 8).
-      std::vector<__half> images(2 * 64 * 64);
-      for (int n = 0; n < 64; ++n)
-        for (int j = 0; j < 64; ++j) {
-          const int k = n >> 1, co = n & 1, m = j >> 1, ci = j & 1;
-          const double a = kTwoPi * double((m * k) % 32) / 32.0;
-          const double v = ci == co ? std::cos(a) : (ci == 1 ? std::sin(a) : -std::sin(a));
-          const __half hi = __float2half_rn((float)v);
-          const __half lo = __float2half_rn((float)(v - (double)__half2float(hi)));
-          const size_t at = (size_t)n * 64 + (size_t)((((j >> 3) ^ (n & 7)) << 3) | (j & 7));
-          images[at] = hi;
-          images[64 * 64 + at] = lo;
-        }
-      d->d_dft_images = upload(images);
+      d->d_tw_pass = upload(smb::fft1024_pass_twiddles());
+      d->d_tw_post = upload(smb::unit_roots<float2>(512, 2048));   // W_2048^(l + 32 j) at [j][l]
+      d->d_dft_images = upload(smb::dft32_split_images());
     }
     dev = std::move(d);
   }
@@ -401,48 +349,25 @@ struct smb_mel_plan {
   int scale = 0, norm = 0;
   std::vector<double> weights;       // [n_mels][bins]
   std::vector<int> band_lo, band_hi;
-  // Mel schedule of a fused kernel: every filter's band cut into pieces of at most
-  // `ps` float4 steps, a lane carries one piece for all the frames of the tile.
-  struct PieceSchedule {
-    std::vector<float> vals;               // [round][step][lane] float4 weights
-    std::vector<smb::MelPiece> pieces;     // [warps][rounds][32]
-    std::vector<unsigned char> pcnt;       // [n_mels]: pieces (= partial sums) of each filter, 1..4
-    int rounds = 0, mpad = 0;              // partial-sum slot of (piece j, filter m) = j * mpad + m
-    struct Tables {
-      device_ptr<float> d_vals;
-      device_ptr<smb::MelPiece> d_pieces;
-      device_ptr<unsigned char> d_pcnt;
-    };
-    void clear() { vals.clear(); pieces.clear(); pcnt.clear(); rounds = mpad = 0; }
-    Tables to_device() const { return {upload(vals), upload(pieces), upload(pcnt)}; }
-  };
-  // Mel schedule of the frame-pair kernel (stft2048p.cu): whole filters, eight per
-  // round, a lane = (filter, frame pair); rounds dealt to the group's four warps.
-  struct PairSchedule {
-    std::vector<float> w;                  // [round][step][8 filters] x float4
-    std::vector<smb::PairMelItem> items;   // [4 warps][rounds][8]
-    int rounds = 0;
-    struct Tables {
-      device_ptr<float> d_w;
-      device_ptr<smb::PairMelItem> d_items;
-    };
-    void clear() { w.clear(); items.clear(); rounds = 0; }
-    Tables to_device() const { return items.empty() ? Tables{} : Tables{upload(w), upload(items)}; }
-  };
-  PairSchedule sched_pair;
-  PieceSchedule sched_cc;   // CUDA-core kernel: kFastTile warps, 8 frames per lane
-  PieceSchedule sched_tc;   // tensor-core kernel: kTcTile warps, 4 frames per lane
+  smb::PairSchedule sched_pair;
+  smb::PieceSchedule sched_cc;   // CUDA-core kernel: kFastTile warps, 8 frames per lane
+  smb::PieceSchedule sched_tc;   // tensor-core kernel: kTcTile warps, 4 frames per lane
   // 2048 / fft_size when the fused kernel can carry this filterbank (1 for fft
   // 2048, 2 for 1024, ...), else 0
   int fast_step = 0;
   // Everything the plan has on its device; null until the first device call.
   struct Device {
-    int device = 0;
+    int device = 0, sm_count = 0;
     StreamOwner stream;
     device_ptr<double> d_weights;
     device_ptr<int> d_band_lo, d_band_hi;
-    PairSchedule::Tables pair;
-    PieceSchedule::Tables cc, tc;
+    struct PieceTables {
+      device_ptr<float> d_vals;
+      device_ptr<smb::MelPiece> d_pieces;
+      device_ptr<unsigned char> d_pcnt;
+    } cc, tc;
+    device_ptr<float> d_pair_w;
+    device_ptr<smb::PairMelItem> d_pair_items;
     // MFCC epilogue: DCT table of the last (n_mfcc, lifter) asked for, max scratch
     device_ptr<double> d_dct;
     device_ptr<unsigned long long> d_max;
@@ -490,240 +415,26 @@ struct smb_mel_plan {
     // (shorter frames run zero-padded and keep every step-th bin in the power row)
     if (bins < 65 || bins > 1025 || 1024 % (bins - 1) != 0) return;
     const int step = (int)(1024 / (bins - 1));
-    if (step == 1 && !build_pair_schedule(sched_pair)) sched_pair.clear();
+    if (step == 1) sched_pair = smb::pair_schedule(weights, band_lo, band_hi, n_mels, bins);
     // the CUDA-core kernel trades a few padded steps for conflict-free octets
     // (whole list as the window); the tensor-core kernel has no shared memory to
     // spare for longer weight tables and keeps the strict longest-first rounds
-    if (!build_schedule(sched_cc, smb::kFastTile, smb::kFastPieceSteps, 1 << 30) ||
-        !build_schedule(sched_tc, smb::kTcTile, smb::kTcPieceSteps, 32)) {
-      sched_cc.clear();
-      sched_tc.clear();
-      return;
-    }
-    fast_step = step;
-  }
-  // Mel schedule of the frame-pair kernel.  Filter m's band [band_lo, band_hi) is read
-  // in 4-bin steps from an even bin b0 <= band_lo; eight consecutive filters make a
-  // round (neighbouring bands have similar lengths), lane (i, j) of the round's warp
-  // carries filter i for frame pair j.  The two filters of a quarter-warp start on
-  // 16-byte groups of opposite parity (b0 / 2 odd against even; one of them moves two
-  // bins down, weights zero there) so that the eight 16-byte loads of a quarter-warp,
-  // whose four frame pairs sit 32 bytes apart, fall in eight distinct bank groups.
-  // Weights are stored [round][step][filter] x float4 = one 128-byte run per warp
-  // load.  Rounds go longest-first onto the lightest of the four warps.
-  bool build_pair_schedule(PairSchedule& sc) const {
-    sc.clear();
-    const int kBins = 1032;                                  // power row incl. zeroed tail (stft2048p.cu)
-    if (bins != 1025 || n_mels > 32767) return false;
-    constexpr int F = smb::kPairFilters;                     // filters per round (lane = filter, frame pair)
-    const int rounds_total = (int)((n_mels + F - 1) / F);
-    struct Round { int steps; size_t base; int b0[F]; int m[F]; };
-    std::vector<Round> built((size_t)rounds_total);
-    for (int q = 0; q < rounds_total; ++q) {
-      Round& rd = built[(size_t)q];
-      int hi[F];
-      for (int i = 0; i < F; ++i) {
-        const int64_t m = (int64_t)q * F + i;
-        rd.m[i] = m < n_mels ? (int)m : -1;
-        rd.b0[i] = m < n_mels ? band_lo[(size_t)m] & ~1 : 0;
-        hi[i] = m < n_mels ? std::max(band_hi[(size_t)m], rd.b0[i]) : 0;
-      }
-      for (int i = 0; i < F; i += 2) {
-        if (rd.m[i] < 0 || rd.m[i + 1] < 0) continue;
-        if ((((rd.b0[i] >> 1) + (rd.b0[i + 1] >> 1)) & 1) != 0) continue;
-        if (rd.b0[i + 1] >= 2) rd.b0[i + 1] -= 2;
-        else if (rd.b0[i] >= 2) rd.b0[i] -= 2;
-      }
-      rd.steps = 1;                                        // 0 marks an idle round in the kernel
-      for (int i = 0; i < F; ++i)
-        if (rd.m[i] >= 0) rd.steps = std::max(rd.steps, (hi[i] - rd.b0[i] + 3) / 4);
-      rd.steps = (rd.steps + 1) & ~1;                      // the kernel runs two steps per iteration
-      if (rd.steps > 510 || 4 * rd.steps > kBins) return false;
-      // every lane runs the round's step count: keep its reads inside the row
-      for (int i = 0; i < F; ++i) rd.b0[i] = std::min(rd.b0[i], (kBins - 4 * rd.steps) & ~1);
-      rd.base = sc.w.size();
-      sc.w.resize(rd.base + (size_t)rd.steps * F * 4, 0.0f);
-      for (int i = 0; i < F; ++i) {
-        if (rd.m[i] < 0) continue;
-        for (int k = band_lo[(size_t)rd.m[i]]; k < band_hi[(size_t)rd.m[i]]; ++k) {
-          const int u = k - rd.b0[i];
-          sc.w[rd.base + ((size_t)(u >> 2) * F + (size_t)i) * 4 + (size_t)(u & 3)] =
-              (float)weights[(size_t)((int64_t)rd.m[i] * bins + k)];
-        }
-      }
-    }
-    sc.w.resize(sc.w.size() + F * 4, 0.0f);                // the kernel's prefetch reads one step ahead
-    if (sc.w.size() >= (1u << 24)) return false;
-    const int warps = smb::kPairTile / 2;
-    std::vector<int> by_len((size_t)rounds_total);
-    for (int q = 0; q < rounds_total; ++q) by_len[(size_t)q] = q;
-    std::stable_sort(by_len.begin(), by_len.end(),
-                     [&](int a, int b) { return built[(size_t)a].steps > built[(size_t)b].steps; });
-    std::vector<std::vector<int>> lists((size_t)warps);
-    std::vector<long long> load((size_t)warps, 0);
-    for (int q : by_len) {
-      const size_t wi = (size_t)(std::min_element(load.begin(), load.end()) - load.begin());
-      lists[wi].push_back(q);
-      load[wi] += built[(size_t)q].steps * 10 + 30;
-    }
-    sc.rounds = 0;
-    for (const auto& l : lists) sc.rounds = std::max(sc.rounds, (int)l.size());
-    sc.items.assign((size_t)(warps * sc.rounds * F), smb::PairMelItem{0, 0, -1});   // idle: no steps
-    for (int wi = 0; wi < warps; ++wi)
-      for (size_t r = 0; r < lists[(size_t)wi].size(); ++r) {
-        const Round& rd = built[(size_t)lists[(size_t)wi][r]];
-        for (int i = 0; i < F; ++i) {
-          smb::PairMelItem& it = sc.items[((size_t)wi * (size_t)sc.rounds + r) * F + (size_t)i];
-          it.w4_steps = (int)(rd.base / 4 + (size_t)i) | ((rd.steps / 2) << 24);
-          it.h0 = (unsigned short)(rd.b0[i] >> 1);
-          it.m = (short)rd.m[i];
-        }
-      }
-    return true;
-  }
-  // Mel schedule of the fused kernels.  Every filter's band, starting on a float4
-  // of the power row, is cut into pieces of at most `ps` float4 steps; a lane
-  // carries one piece for all the frames of its tile (one weight load feeds 4 FMAs
-  // per frame) and leaves a partial sum in slot `pid` = j * mpad + m for the j-th
-  // piece of filter m (at most four per filter: `ps` grows with the longest band;
-  // the write-out adds the pcnt[m] of them up).  Rounds of 32 lanes share one
-  // step count.  They are filled longest pieces first out of a window of
-  // candidates, so that the lanes of a quarter-warp get distinct start residues
-  // (start / 4 mod 8) where the window allows: their 16-byte power-row loads then
-  // fall in distinct bank groups.  Weights are stored
-  // [round][step][lane] x float4, a contiguous run per warp-wide load.  Rounds go
-  // to the group's warps longest-first onto the lightest warp.
-  bool build_schedule(PieceSchedule& sc, int warps, int ps, int window) const {
-    sc.clear();
-    const int row_floats = (int)((bins + 3) / 4 * 4);        // the kernel zeroes the row tail
-    struct Piece { int m, start, steps, pid; };
-    std::vector<Piece> pieces;
-    sc.pcnt.assign((size_t)n_mels, 1);
-    sc.mpad = (int)((n_mels + 7) / 8 * 8);
-    int longest = 1;
-    for (int64_t m = 0; m < n_mels; ++m) {
-      const int lo = band_lo[(size_t)m] & ~3, hi = std::max(band_hi[(size_t)m], lo + 1);
-      longest = std::max(longest, (hi - lo + 3) / 4);
-    }
-    ps = std::max(ps, (longest + 3) / 4);                // no filter in more than four pieces
-    if (ps > 255) return false;
-    for (int64_t m = 0; m < n_mels; ++m) {
-      const int lo = band_lo[(size_t)m] & ~3, hi = std::max(band_hi[(size_t)m], lo + 1);
-      const int total = (hi - lo + 3) / 4;
-      int j = 0;
-      for (int s0 = 0; s0 < total; s0 += ps, ++j)
-        pieces.push_back(Piece{(int)m, lo + 4 * s0, std::min(ps, total - s0), j * sc.mpad + (int)m});
-      sc.pcnt[(size_t)m] = (unsigned char)j;
-    }
-    const int scratch = 4 * sc.mpad;                     // idle lanes drop their zeros here
-    // pieces longest first; a round is picked from the first `window` of them
-    std::vector<int> rest(pieces.size());
-    for (size_t i = 0; i < rest.size(); ++i) rest[i] = (int)i;
-    std::stable_sort(rest.begin(), rest.end(),
-                     [&](int a, int b) { return pieces[(size_t)a].steps > pieces[(size_t)b].steps; });
-    struct Round { int steps; size_t base; int member[32]; int start[32]; };
-    std::vector<Round> built;
-    while (!rest.empty()) {
-      Round rd;
-      for (int t = 0; t < 32; ++t) rd.member[t] = -1;
-      const size_t nc = std::min(rest.size(), (size_t)window);
-      std::vector<char> used(nc, 0);
-      // four octets, each scanning the candidates for eight distinct residues ...
-      for (int o = 0; o < 4; ++o) {
-        unsigned seen = 0;
-        int lane = o * 8;
-        for (size_t c = 0; c < nc && lane < o * 8 + 8; ++c) {
-          if (used[c]) continue;
-          const unsigned r = (unsigned)((pieces[(size_t)rest[c]].start >> 2) & 7);
-          if (seen & (1u << r)) continue;
-          seen |= 1u << r;
-          used[c] = 1;
-          rd.member[lane++] = rest[c];
-        }
-      }
-      // ... then the free lanes take the longest candidates left
-      for (int t = 0; t < 32; ++t) {
-        if (rd.member[t] >= 0) continue;
-        size_t c = 0;
-        while (c < nc && used[c]) ++c;
-        if (c == nc) break;
-        used[c] = 1;
-        rd.member[t] = rest[c];
-      }
-      std::vector<int> keep;
-      for (size_t c = 0; c < rest.size(); ++c)
-        if (c >= nc || !used[c]) keep.push_back(rest[c]);
-      rest.swap(keep);
-      rd.steps = 1;
-      for (int t = 0; t < 32; ++t)
-        if (rd.member[t] >= 0) rd.steps = std::max(rd.steps, pieces[(size_t)rd.member[t]].steps);
-      if (rd.steps * 4 > row_floats) return false;
-      rd.base = sc.vals.size();
-      sc.vals.resize(rd.base + (size_t)rd.steps * 32 * 4, 0.0f);
-      for (int t = 0; t < 32; ++t) {
-        const int id = rd.member[t];
-        rd.start[t] = 0;
-        if (id < 0) continue;
-        const Piece& pc = pieces[(size_t)id];
-        // the stored run [start, start + 4 steps) must stay inside the row
-        rd.start[t] = std::min(pc.start, row_floats - 4 * rd.steps);
-        // the piece's own bins [pc.start, pc.start + 4 pc.steps), clipped to the band
-        for (int k = pc.start; k < pc.start + 4 * pc.steps; ++k) {
-          if (k >= bins || k < band_lo[(size_t)pc.m] || k >= band_hi[(size_t)pc.m]) continue;
-          const int u = k - rd.start[t];
-          sc.vals[rd.base + ((size_t)(u >> 2) * 32 + (size_t)t) * 4 + (size_t)(u & 3)] =
-              (float)weights[(size_t)((int64_t)pc.m * bins + k)];
-        }
-      }
-      built.push_back(rd);
-    }
-    const int rounds_total = (int)built.size();
-    std::vector<int> by_len((size_t)rounds_total);
-    for (int q = 0; q < rounds_total; ++q) by_len[(size_t)q] = q;
-    std::stable_sort(by_len.begin(), by_len.end(),
-                     [&](int a, int b) { return built[(size_t)a].steps > built[(size_t)b].steps; });
-    std::vector<std::vector<int>> lists((size_t)warps);
-    std::vector<long long> load((size_t)warps, 0);
-    for (int q : by_len) {
-      const size_t w = (size_t)(std::min_element(load.begin(), load.end()) - load.begin());
-      lists[w].push_back(q);
-      load[w] += built[(size_t)q].steps * 21 + 20;
-    }
-    sc.rounds = 0;
-    for (const auto& l : lists) sc.rounds = std::max(sc.rounds, (int)l.size());
-    const size_t zero_off = sc.vals.size();            // idle rounds: one step over zero weights
-    sc.vals.insert(sc.vals.end(), (size_t)(32 * 4), 0.0f);
-    if (sc.vals.size() >= (1u << 24)) return false;
-    sc.pieces.assign((size_t)(warps * sc.rounds * 32), smb::MelPiece{});
-    for (int w = 0; w < warps; ++w)
-      for (int r = 0; r < sc.rounds; ++r)
-        for (int t = 0; t < 32; ++t) {
-          smb::MelPiece& out = sc.pieces[((size_t)w * (size_t)sc.rounds + (size_t)r) * 32 + (size_t)t];
-          if ((size_t)r < lists[(size_t)w].size()) {
-            const Round& rd = built[(size_t)lists[(size_t)w][(size_t)r]];
-            out.off = (int)(rd.base + (size_t)t * 4) | (rd.steps << 24);
-            out.lo = (short)rd.start[t];
-            out.pid = (unsigned short)(rd.member[t] >= 0 ? pieces[(size_t)rd.member[t]].pid : scratch);
-          } else {
-            out.off = (int)(zero_off + (size_t)t * 4) | (1 << 24);
-            out.lo = 0;
-            out.pid = (unsigned short)scratch;
-          }
-        }
-    return true;
+    sched_cc = smb::piece_schedule(weights, band_lo, band_hi, n_mels, bins, smb::kFastTile, smb::kFastPieceSteps,
+                                   1 << 30);
+    sched_tc = smb::piece_schedule(weights, band_lo, band_hi, n_mels, bins, smb::kTcTile, smb::kTcPieceSteps, 32);
+    if (sched_cc.pieces.empty() || sched_tc.pieces.empty()) sched_cc = sched_tc = {};
+    else fast_step = step;
   }
   void ensure_device() {
     if (dev) return same_device(dev->device);
-    require_device();
-    auto d = std::make_unique<Device>();
-    CK(cudaGetDevice(&d->device));
-    d->stream.create();
+    auto d = new_device<Device>();
     d->d_weights = upload(weights);
     d->d_band_lo = upload(band_lo);
     d->d_band_hi = upload(band_hi);
-    d->cc = sched_cc.to_device();
-    d->tc = sched_tc.to_device();
-    d->pair = sched_pair.to_device();
+    d->cc = {upload(sched_cc.vals), upload(sched_cc.pieces), upload(sched_cc.pcnt)};
+    d->tc = {upload(sched_tc.vals), upload(sched_tc.pieces), upload(sched_tc.pcnt)};
+    d->d_pair_w = upload(sched_pair.w);
+    d->d_pair_items = upload(sched_pair.items);
     d->d_max = device_alloc<unsigned long long>(sizeof(unsigned long long));
     dev = std::move(d);
   }
@@ -748,42 +459,26 @@ static int ols_kernel_of(const smb::OlsPlan& p) {
   return SMB_OLS_STOCKHAM;
 }
 
-// Device copies of one overlap-save plan.
+// Device copies of one overlap-save plan's tables.
 struct OlsDevice {
-  smb::OlsPlan plan;
   device_ptr<float2> d_h;
   device_ptr<float2> d_tw;
   device_ptr<float2> d_tw_pass, d_tw_base;             // tables of the N = 2048 kernel
-  int sm_count = 0;
   void upload_from(const smb::OlsPlan& p) {
-    plan = p;
     if (!p.ok) return;
     if (p.n == 2048 && (p.l == 1 || p.polyphase)) {
-      std::vector<float2> base(32);
-      for (int l = 0; l < 32; ++l) {
-        const double a = kTwoPi * double(l) / 2048.0;
-        base[(size_t)l] = make_float2((float)std::cos(a), (float)-std::sin(a));
-      }
-      d_tw_pass = upload(fft1024_pass_twiddles());
-      d_tw_base = upload(base);
-      int device = 0;
-      CK(cudaGetDevice(&device));
-      CK(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, device));
+      d_tw_pass = upload(smb::fft1024_pass_twiddles());
+      d_tw_base = upload(smb::unit_roots<float2>(32, 2048));
     }
     std::vector<float2> h(p.spectrum_re.size());
     for (size_t i = 0; i < h.size(); ++i)
       h[i] = make_float2((float)p.spectrum_re[i], (float)p.spectrum_im[i]);
     d_h = upload(h);
     const int64_t tn = std::max(p.n, p.w);
-    std::vector<float2> tw((size_t)(tn / 2));
-    for (int64_t j = 0; j < tn / 2; ++j) {
-      const double a = kTwoPi * double(j) / double(tn);
-      tw[(size_t)j] = make_float2((float)std::cos(a), (float)-std::sin(a));
-    }
-    d_tw = upload(tw);
+    d_tw = upload(smb::unit_roots<float2>(tn / 2, tn));
   }
-  void run(const float* x, int64_t batch, int64_t n, int64_t n_out, float* out,
-           cudaStream_t st) const {
+  void run(const smb::OlsPlan& plan, const float* x, int64_t batch, int64_t n, int64_t n_out, float* out,
+           int sm_count, cudaStream_t st) const {
     smb::OlsArgs a = ols_args(plan);
     a.x = x;
     a.out = out;
@@ -799,350 +494,65 @@ struct OlsDevice {
   }
 };
 
-// Device image of G for the tensor-core executor of one phase-rich stage.
-struct GemmDevice {
-  // L <= 160 is one launch; wider stages (L = 320, 441, 640: the 44.1 k <-> 48 k
-  // family) are cut into column groups of <= 160, one launch each, because the
-  // three accumulators of a group must fit the 512 TMEM columns.
-  struct Group {
-    int col_begin = 0, width = 0, n_pad = 0, chunk_begin = 0, chunks = 0, tmem_cols = 0;
-    device_ptr<float> d_images;
-    device_ptr<int4> d_meta;
-  };
-  bool ok = false;
-  std::vector<Group> groups;
-  // Row form (resample_rows_kernel): stages whose L columns are one launch and whose
-  // shift accumulators fit tensor memory.
-  bool rows_ok = false;
-  int rows_sm_count = 0;
-  struct RowsGroup {
-    smb::GemmRowsArgs a{};
-    device_ptr<float> d_images;
-    device_ptr<int4> d_chunks, d_slices;
-  };
-  std::vector<RowsGroup> rows_groups;            // one launch per group of <= 160 columns
-  // columns [c0, c0 + l) of the stage's L (l_total below)
-  // split_main: the row grid is shifted so that every column's filter centre falls into the
-  // same shift (qc), and that shift's two small split terms get an accumulator of their own:
-  // its main accumulator then is a chain of exact hi x hi products only (4 per chunk).  With
-  // everything in one accumulator per shift, a 14-chunk stage (44.1 -> 16 kHz) measured
-  // -121.9 dB THD+N in float32 against the reference's -125 dB gate (resample_quality.ml
-  // Q1/Q2); the window form, which separates the small terms, -132.5 dB.
-  bool build_rows_group(const smb::ResampleStage& s, int64_t c0, int64_t l, bool single_group, bool split_main) {
-    const int64_t l_total = s.l, m = s.m, taps = 2 * s.k + 1;
-    if (l > 160 || m < 32) return false;
-    std::vector<int64_t> d((size_t)l);
-    int64_t k;
-    int qc = 0;
-    if (split_main) {
-      // row j of G for (column r, tap t) is d_r + t; the centre tap of the group's first column
-      // is moved onto a multiple of M, so every centre (they span less than M rows) lies in shift qc
-      const int64_t d_first = (c0 * m) / l_total, shift = (m - s.k % m) % m;
-      for (int64_t r = 0; r < l; ++r) d[(size_t)r] = ((c0 + r) * m) / l_total - d_first + shift;
-      k = s.k + shift - d_first;
-      qc = (int)((s.k + shift) / m);
-    } else {
-      // the group's first column starts q0 whole input rows in: fold them into the delay
-      const int64_t q0 = ((c0 * m) / l_total) / m;
-      k = s.k - q0 * m;
-      for (int64_t r = 0; r < l; ++r) d[(size_t)r] = ((c0 + r) * m) / l_total - q0 * m;
-    }
-    const int64_t p_len = taps + d[(size_t)(l - 1)];
-    const int shifts = (int)((p_len + m - 1) / m);
-    const int chunks = (int)((m + 31) / 32);
-    const int n_pad = (int)((l + 15) / 16 * 16);
-    if (shifts > 4) return false;
-    // columns of G_q with a nonzero in rows [j0, j1] of the shift's block: d_r <= q m + j <= d_r + taps - 1
-    auto active = [&](int q, int64_t j0, int64_t j1, int* lo, int* hi) {
-      *lo = n_pad;
-      *hi = -1;
-      for (int64_t r = 0; r < l; ++r) {
-        const int64_t first = d[(size_t)r] - (int64_t)q * m, last = first + taps - 1;
-        if (first <= j1 && last >= j0) {
-          *lo = std::min(*lo, (int)r);
-          *hi = std::max(*hi, (int)r);
-        }
-      }
-      return *hi >= 0;
-    };
-    smb::GemmRowsArgs a{};
-    int total_cols = 0;
-    // accumulators side by side in DESCENDING q: the active columns of D_q are a suffix
-    // and those of D_(q-1) a prefix, so a chunk's nonzeros form one run of TMEM columns
-    // (split_main: the outer shifts first, then the main shift, then its small-term accumulator:
-    // the main shift and the tails are dealt to different issuing threads)
-    std::vector<int> order;
-    for (int q = shifts - 1; q >= 0; --q)
-      if (!split_main || q != qc) order.push_back(q);
-    if (split_main && qc >= shifts) return false;
-    if (split_main) order.push_back(qc);
-    int tails_cols = 0;
-    for (int q : order) {
-      int lo, hi;
-      if (!active(q, 0, m - 1, &lo, &hi)) return false;
-      if (split_main && q == qc) tails_cols = total_cols;
-      a.acc_shift[q] = q;
-      a.acc_lo[q] = (q == 0 && !split_main) ? 0 : lo / 16 * 16;
-      a.acc_w[q] = (q == 0 && !split_main) ? n_pad : (hi + 1 - a.acc_lo[q] + 15) / 16 * 16;
-      a.acc_col[q] = total_cols;
-      total_cols += a.acc_w[q];
-    }
-    const int d_cols = total_cols;                                // the shifts' accumulators: what a run may cover
-    a.n_acc = shifts;
-    if (split_main) {
-      a.acc_shift[shifts] = qc;
-      a.acc_lo[shifts] = a.acc_lo[qc];
-      a.acc_w[shifts] = a.acc_w[qc];
-      a.acc_col[shifts] = total_cols;
-      total_cols += a.acc_w[qc];
-      a.n_acc = shifts + 1;
-    }
-    if (total_cols > 512 || chunks > 32 || chunks < 3) return false;   // (chunks >= stages: the loader's scratch hand-over)
-    // the A tiles go to tensor memory when two stages of 64 columns fit beside the accumulators
-    // (the products then read only B from shared memory: 1.99 -> 1.90 ms on configs[3]); a stage
-    // cut into column groups gathers A once per group and is better off with the cheaper
-    // shared-memory producers (44.1 -> 32 kHz: 0.88 against 0.93 ms).  SMB_ROWS_SMEM_A=1 /
-    // SMB_ROWS_TMEM_A=1 force either.
-    const bool a_tmem = total_cols + 128 <= 512 && !getenv("SMB_ROWS_SMEM_A") &&
-                        (single_group || getenv("SMB_ROWS_TMEM_A"));
-    int tmem_alloc = 32;
-    while (tmem_alloc < total_cols + (a_tmem ? 128 : 0)) tmem_alloc *= 2;
-    const int kSliceAlign = 8;
-    std::vector<int4> chunk_meta((size_t)chunks), slice_meta;
-    struct Run { int bytes_at, start, width; };                  // a chunk's stored rows: [hi | lo][width][32]
-    std::vector<Run> runs;
-    // per chunk: TMEM column -> run, -1 where nothing is stored
-    std::vector<std::vector<int>> run_at((size_t)chunks, std::vector<int>((size_t)d_cols, -1));
-    size_t total_bytes = 0;
-    int stage_bytes = 0;
-    for (int ch = 0; ch < chunks; ++ch) {
-      // exact active columns (TMEM coordinates); a run may start on any column -- only its
-      // width is a multiple of 16 -- so a chunk stores ceil16(band) columns, not the
-      // band widened to 16-column boundaries on both sides
-      std::vector<char> on((size_t)d_cols, 0);
-      for (int q = 0; q < shifts; ++q) {
-        int lo, hi;
-        if (!active(q, 32 * (int64_t)ch, std::min<int64_t>(32 * (int64_t)ch + 31, m - 1), &lo, &hi)) continue;
-        for (int cc = lo; cc <= hi; ++cc) on[(size_t)(a.acc_col[q] + cc - a.acc_lo[q])] = 1;
-      }
-      const int first_slice = (int)slice_meta.size();
-      int bytes = 0;
-      for (int t0 = 0; t0 < d_cols;) {
-        if (!on[(size_t)t0]) { ++t0; continue; }
-        int t1 = t0 + 1;                                          // one past the run's last active column
-        const int t_end = split_main && t0 < tails_cols ? tails_cols : d_cols;   // a run stays with one owner
-        for (int t = t0 + 1; t < t_end && t - t0 < 256; ++t) {
-          if (on[(size_t)t]) t1 = t + 1;
-          else if (t - t1 >= 16) break;                           // a gap of 16 columns ends the run
-        }
-        int start = t0 / kSliceAlign * kSliceAlign;              // the accumulator address of a product
-        int width = (t1 - start + 15) / 16 * 16;
-        if (width > 256) { width = 256; t1 = start + 256; }
-        if (start + width > d_cols) start = d_cols - width;      // (never past the shifts' accumulators)
-        if (split_main && t0 < tails_cols && start + width > tails_cols) start = tails_cols - width;
-        if (split_main && t0 >= tails_cols && start < tails_cols) start = tails_cols;   // (a 16-column boundary)
-        if (start < 0) return false;
-        for (int t = start; t < start + width; ++t) run_at[(size_t)ch][(size_t)t] = (int)runs.size();
-        runs.push_back(Run{bytes, start, width});
-        const int lo_delta = width * 128;                         // from a row's hi image to its lo image
-        if (!split_main) {
-          slice_meta.push_back(make_int4(bytes, start, width, 0 | (lo_delta << 3)));
-        } else if (start < tails_cols) {
-          // the outer shifts: all three products in their own accumulators, second issuer
-          slice_meta.push_back(make_int4(bytes, start, width, 0 | 4 | (lo_delta << 3)));
-        } else {
-          // the main shift: hi x hi into its accumulator, the small terms into the extra one
-          slice_meta.push_back(make_int4(bytes, start, width, 1 | (lo_delta << 3)));
-          slice_meta.push_back(make_int4(bytes, a.acc_col[shifts] + (start - a.acc_col[qc]), width, 2 | (lo_delta << 3)));
-        }
-        bytes += 2 * width * 128;
-        t0 = std::max(t1, start + width);
-      }
-      chunk_meta[(size_t)ch] = make_int4((int)total_bytes, bytes, first_slice, (int)slice_meta.size() - first_slice);
-      total_bytes += (size_t)bytes;
-      stage_bytes = std::max(stage_bytes, bytes);
-    }
-    if (slice_meta.size() > 80) return false;
-    stage_bytes = (stage_bytes + 1023) / 1024 * 1024;
-    // static shared memory of the kernel (barriers, metadata) comes out of the same 227 KB
-    const size_t budget = 227 * 1024 - 2048;
-    a.a_tmem = a_tmem ? 1 : 0;
-    a.a_tmem_col = total_cols;
-    if (a_tmem) {
-      a.a_stages = 2;
-      // no more B stages than chunks: the B loader takes back the stage the epilogue borrowed
-      // at chunk b_stages - 1 of the next tile, a chunk a 3-chunk tile does not have
-      a.b_stages = std::min(4, chunks);
-      const size_t turn = 8 * 32 * 17 * 4;                      // the producers' transposition tiles
-      while (a.b_stages > 2 && smb::resample_rows_smem_bytes(0, a.b_stages, stage_bytes) + turn > budget) --a.b_stages;
-      if (smb::resample_rows_smem_bytes(0, a.b_stages, stage_bytes) + turn > budget) return false;
-    } else if (smb::resample_rows_smem_bytes(2, 3, stage_bytes) <= budget) { a.a_stages = 2; a.b_stages = 3; }
-    else if (smb::resample_rows_smem_bytes(3, 2, stage_bytes) <= budget) { a.a_stages = 3; a.b_stages = 2; }
-    else if (smb::resample_rows_smem_bytes(2, 2, stage_bytes) <= budget) { a.a_stages = 2; a.b_stages = 2; }
-    else return false;
-    int device = 0;
-    CK(cudaGetDevice(&device));
-    CK(cudaDeviceGetAttribute(&rows_sm_count, cudaDevAttrMultiProcessorCount, device));
-    std::vector<float> img(total_bytes / 4, 0.0f);
-    for (int64_t r = 0; r < l; ++r) {
-      const int64_t ph = ((c0 + r) * m) % l_total;
-      for (int64_t t = 0; t < taps; ++t) {
-        const int64_t j = d[(size_t)r] + t;
-        const int q = (int)(j / m);
-        const int64_t jj = j % m;
-        const int ch = (int)(jj / 32), kk = (int)(jj % 32);
-        const int tcol = a.acc_col[q] + (int)r - a.acc_lo[q];
-        const int ri = run_at[(size_t)ch][(size_t)tcol];
-        if (ri < 0) return false;                               // (cannot happen: the runs cover every nonzero)
-        const Run run = runs[(size_t)ri];
-        const size_t base = ((size_t)chunk_meta[(size_t)ch].x + (size_t)run.bytes_at) / 4;
-        put_tf32_split(img, base, run.width, tcol - run.start, kk, s.bank[(size_t)(ph * taps + t)]);
-      }
-    }
-    a.slices = (int)slice_meta.size();
-    a.two_issuers = split_main ? 1 : 0;
-    a.l = (int)l;
-    a.m = (int)m;
-    a.k = (int)k;
-    a.n_pad = n_pad;
-    a.shifts = shifts;
-    a.chunks = chunks;
-    a.tmem_cols = tmem_alloc;
-    a.b_stage_bytes = stage_bytes;
-    a.l_total = (int)l_total;
-    a.col_begin = (int)c0;
-    RowsGroup g;
-    g.d_images = upload(img);
-    g.d_chunks = upload(chunk_meta);
-    g.d_slices = upload(slice_meta);
-    a.b_images = g.d_images.get();
-    a.chunk_meta = g.d_chunks.get();
-    a.slice_meta = g.d_slices.get();
-    g.a = a;
-    rows_groups.push_back(std::move(g));
-    return true;
-  }
-  void build_rows(const smb::ResampleStage& s) {
-    const int n_groups = (int)((s.l + 159) / 160);
-    const int64_t base_width = ((s.l + n_groups - 1) / n_groups + 15) / 16 * 16;
-    // long stages (many K-chunks = long accumulation chains) separate the small terms of the
-    // main shift when tensor memory has room for the extra accumulator; SMB_ROWS_SPLIT=0/1 forces
-    const bool want_split = getenv("SMB_ROWS_SPLIT") ? atoi(getenv("SMB_ROWS_SPLIT")) != 0 : (s.m + 31) / 32 >= 8;
-    for (int attempt = want_split ? 0 : 1; attempt < 2; ++attempt) {
-      bool ok = true;
-      for (int64_t c0 = 0; c0 < s.l && ok; c0 += base_width)
-        ok = build_rows_group(s, c0, std::min<int64_t>(base_width, s.l - c0), n_groups == 1, attempt == 0);
-      if (ok) {
-        rows_ok = true;
-        return;
-      }
-      rows_groups.clear();
-    }
-  }
-  void build(const smb::ResampleStage& s) {
-    const int64_t l = s.l, m = s.m, k = s.k, taps = 2 * k + 1;
-    if (s.exec != smb::kExecGemm || l > 1024) return;
-    build_rows(s);
-    const int n_groups = (int)((l + 159) / 160);
-    const int base_width = (int)(((l + n_groups - 1) / n_groups + 15) / 16 * 16);
-    for (int c0 = 0; c0 < l; c0 += base_width) {
-      Group g;
-      g.col_begin = c0;
-      g.width = (int)std::min<int64_t>(base_width, l - c0);
-      g.n_pad = (g.width + 15) / 16 * 16;
-      // rows of G (K index) this group's columns touch: d(r) = floor(r M / L) .. + taps - 1
-      const int64_t d_first = ((int64_t)c0 * m) / l;
-      const int64_t d_last = ((int64_t)(c0 + g.width - 1) * m) / l + taps - 1;
-      g.chunk_begin = (int)(d_first / 32);
-      g.chunks = (int)(d_last / 32) - g.chunk_begin + 1;
-      g.tmem_cols = 32;
-      while (g.tmem_cols < 3 * g.n_pad) g.tmem_cols *= 2;
-      // G is banded: chunk ch only has nonzeros in a run of columns.  Store and
-      // multiply just that run, widened to multiples of 16 columns; the group's
-      // first two chunks keep the full width because their first products
-      // zero-initialise the accumulators.
-      std::vector<int> cmin((size_t)g.chunks, g.n_pad), cmax((size_t)g.chunks, -1);
-      for (int r = 0; r < g.width; ++r) {
-        const int64_t d = ((int64_t)(c0 + r) * m) / l;
-        for (int64_t ch = d / 32; ch <= (d + taps - 1) / 32; ++ch) {
-          const size_t rel = (size_t)(ch - g.chunk_begin);
-          cmin[rel] = std::min(cmin[rel], r);
-          cmax[rel] = std::max(cmax[rel], r);
-        }
-      }
-      std::vector<int4> meta((size_t)g.chunks);
-      size_t total_floats = 0;
-      for (int ch = 0; ch < g.chunks; ++ch) {
-        int col0 = 0, ncols = g.n_pad;
-        if (ch >= 2 && cmax[(size_t)ch] >= 0) {
-          col0 = cmin[(size_t)ch] / 16 * 16;
-          ncols = (cmax[(size_t)ch] + 1 - col0 + 15) / 16 * 16;
-        } else if (ch >= 2) {
-          ncols = 16;                                          // empty chunk: a zero slice
-        }
-        meta[(size_t)ch] = make_int4((int)(total_floats * 4), col0, ncols, 0);
-        total_floats += (size_t)2 * ncols * 32;
-      }
-      std::vector<float> img(total_floats, 0.0f);
-      for (int r = 0; r < g.width; ++r) {
-        const int64_t col = c0 + r;
-        const int64_t d = (col * m) / l, ph = (col * m) % l;
-        for (int64_t t = 0; t < taps; ++t) {
-          const int64_t j = d + t;                               // row of G
-          const int64_t ch = j / 32 - g.chunk_begin, kk = j % 32;
-          const int4 mt = meta[(size_t)ch];
-          // row r - mt.y of the stored slice
-          put_tf32_split(img, (size_t)mt.x / 4, mt.z, r - mt.y, kk, s.bank[(size_t)(ph * taps + t)]);
-        }
-      }
-      g.d_meta = upload(meta);
-      g.d_images = upload(img);
-      groups.push_back(std::move(g));
-    }
-    ok = true;
-  }
+// Device copies of one column group's tcgen05 resampler images (smb::GemmLayout).
+struct GemmImages {
+  device_ptr<float> d_images;
+  device_ptr<int4> d_meta, d_slices;   // chunk meta; slice meta (row form only)
 };
 
 struct smb_resample_plan {
   smb::ResamplePlan plan;
+  // Host tables per stage, built by the first layout() or device call (the SMB_ROWS_*
+  // switches are read then); once uploaded, the host keeps the launch arguments only.
+  struct StageTables { smb::OlsPlan ols; smb::GemmLayout gemm; };
+  std::vector<StageTables> tables;
   // Everything the plan has on its device; null until the first device call.
   struct Device {
-    int device = 0;
+    int device = 0, sm_count = 0;
     StreamOwner stream;
-    std::vector<device_ptr<float>> d_bank;     // per stage, [l][2k+1] float32
-    std::vector<device_ptr<double>> d_bank64;  // the same banks uncast, for float64 audio
-    std::vector<OlsDevice> ols;        // per stage; plan.ok only for OLS-tagged power-of-two stages
-    std::vector<GemmDevice> gemm;      // per stage; ok only for GEMM-tagged stages
+    struct Stage {
+      device_ptr<float> d_bank;                // [l][2k+1] float32
+      device_ptr<double> d_bank64;             // the same bank uncast, for float64 audio
+      OlsDevice ols;
+      std::vector<GemmImages> rows, windows;   // per column group of the stage's GemmLayout
+    };
+    std::vector<Stage> stages;
   };
   std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   int executor = SMB_EXEC_PLANNED;   // SMB_EXEC_DIRECT forces the dot-product kernel everywhere
   DeviceBuffer mid;
   HostPipe pipe;                     // host-memory calls: sliced, copies under kernels
+  void build_tables() {
+    for (size_t i = tables.size(); i < plan.stages.size(); ++i)
+      tables.push_back({smb::ols_plan_for_stage(plan.stages[i]), smb::gemm_layout(plan.stages[i])});
+  }
   void ensure_device() {
     if (dev) return same_device(dev->device);
-    require_device();
-    auto d = std::make_unique<Device>();
-    CK(cudaGetDevice(&d->device));
-    d->stream.create();
-    for (const auto& s : plan.stages) {
-      std::vector<float> b(s.bank.size());
-      for (size_t i = 0; i < b.size(); ++i) b[i] = (float)s.bank[i];   // cast at prepare
-      d->d_bank.push_back(upload(b));
-      d->d_bank64.push_back(upload(s.bank));
-      d->ols.emplace_back();
-      d->ols.back().upload_from(smb::ols_plan_for_stage(s));
-      d->gemm.emplace_back();
-      d->gemm.back().build(s);
+    build_tables();
+    auto d = new_device<Device>();
+    for (size_t i = 0; i < plan.stages.size(); ++i) {
+      const std::vector<double>& bank = plan.stages[i].bank;
+      Device::Stage& ds = d->stages.emplace_back();
+      ds.d_bank = upload(std::vector<float>(bank.begin(), bank.end()));   // cast at prepare
+      ds.d_bank64 = upload(bank);
+      ds.ols.upload_from(tables[i].ols);
+      for (const auto& g : tables[i].gemm.rows)
+        ds.rows.push_back({upload(g.images), upload(g.chunk_meta), upload(g.slice_meta)});
+      for (const auto& g : tables[i].gemm.windows) ds.windows.push_back({upload(g.images), upload(g.chunk_meta)});
+    }
+    for (StageTables& t : tables) {
+      for (auto& g : t.gemm.rows) g = {g.a};
+      for (auto& g : t.gemm.windows) g = {g.a};
     }
     dev = std::move(d);
   }
-  // The kernel run_stage picks for stage i (SMB_FORM_*).
+  // The kernel run_stage picks for stage i (SMB_FORM_*); the host tables must be built.
   int form(size_t i) const {
     if (executor == SMB_EXEC_DIRECT) return SMB_FORM_DIRECT;
-    if (dev->ols[i].plan.ok) return SMB_FORM_OLS;
+    if (tables[i].ols.ok) return SMB_FORM_OLS;
     // (SMB_GEMM_WINDOWS=1: the overlapping-window form, for A/B measurement)
-    if (dev->gemm[i].rows_ok && !getenv("SMB_GEMM_WINDOWS")) return SMB_FORM_ROW;
-    if (dev->gemm[i].ok) return SMB_FORM_WINDOW;
+    if (!tables[i].gemm.rows.empty() && !getenv("SMB_GEMM_WINDOWS")) return SMB_FORM_ROW;
+    if (!tables[i].gemm.windows.empty()) return SMB_FORM_WINDOW;
     return SMB_FORM_DIRECT;
   }
   // One stage over device buffers: overlap-save where the planner tagged it and
@@ -1151,40 +561,32 @@ struct smb_resample_plan {
   void run_stage(size_t i, const float* x, int64_t batch, int64_t n, int64_t n_out, float* out,
                  cudaStream_t st) {
     const smb::ResampleStage& s = plan.stages[i];
+    const smb::GemmLayout& gl = tables[i].gemm;
+    const Device::Stage& ds = dev->stages[i];
+    // the launch arguments of a tcgen05 column group over x -> out
+    auto bind = [&](auto a, const GemmImages& im) {
+      a.x = x;
+      a.out = out;
+      a.n = n;
+      a.n_out = n_out;
+      a.b_images = im.d_images.get();
+      a.chunk_meta = im.d_meta.get();
+      return a;
+    };
     const int f = form(i);
     if (f == SMB_FORM_OLS) {
-      dev->ols[i].run(x, batch, n, n_out, out, st);
+      ds.ols.run(tables[i].ols, x, batch, n, n_out, out, dev->sm_count, st);
     } else if (f == SMB_FORM_ROW) {
-      for (const GemmDevice::RowsGroup& g : dev->gemm[i].rows_groups) {
-        smb::GemmRowsArgs a = g.a;
-        a.x = x;
-        a.out = out;
-        a.n = n;
-        a.n_out = n_out;
-        CK(smb::launch_resample_rows(a, batch, dev->gemm[i].rows_sm_count, st));
+      for (size_t g = 0; g < gl.rows.size(); ++g) {
+        smb::GemmRowsArgs a = bind(gl.rows[g].a, ds.rows[g]);
+        a.slice_meta = ds.rows[g].d_slices.get();
+        CK(smb::launch_resample_rows(a, batch, dev->sm_count, st));
       }
     } else if (f == SMB_FORM_WINDOW) {
-      for (const GemmDevice::Group& g : dev->gemm[i].groups) {
-        smb::GemmResampleArgs a{};
-        a.x = x;
-        a.out = out;
-        a.n = n;
-        a.n_out = n_out;
-        a.l = g.width;
-        a.m = (int)s.m;
-        a.k = (int)s.k - 32 * g.chunk_begin;          // the group's first K-chunk is chunk 0
-        a.l_total = (int)s.l;
-        a.col_begin = g.col_begin;
-        a.n_pad = g.n_pad;
-        a.chunks = g.chunks;
-        a.tmem_cols = g.tmem_cols;
-        a.b_images = g.d_images.get();
-        a.chunk_meta = g.d_meta.get();
-        CK(smb::launch_resample_gemm(a, batch, st));
-      }
+      for (size_t g = 0; g < gl.windows.size(); ++g)
+        CK(smb::launch_resample_gemm(bind(gl.windows[g].a, ds.windows[g]), batch, st));
     } else
-      CK(smb::launch_polyphase_direct(x, batch, n, dev->d_bank[i].get(), (int)s.l, (int)s.m, (int)s.k,
-                                      n_out, out, st));
+      CK(smb::launch_polyphase_direct(x, batch, n, ds.d_bank.get(), (int)s.l, (int)s.m, (int)s.k, n_out, out, st));
   }
 };
 
@@ -1193,23 +595,20 @@ struct smb_fir_plan {
   int64_t k = 0;
   // Everything the plan has on its device; null until the first device call.
   struct Device {
-    int device = 0;
+    int device = 0, sm_count = 0;
     StreamOwner stream;
     device_ptr<float> d_bank;
+    smb::OlsPlan ols_plan;
     OlsDevice ols;
   };
   std::unique_ptr<Device> dev;       // declared before the buffers used on its stream
   HostPipe pipe;                     // host-memory calls: sliced, copies under kernels
   void ensure_device() {
     if (dev) return same_device(dev->device);
-    require_device();
-    auto d = std::make_unique<Device>();
-    CK(cudaGetDevice(&d->device));
-    d->stream.create();
-    std::vector<float> b(h.size());
-    for (size_t s = 0; s < h.size(); ++s) b[s] = (float)h[h.size() - 1 - s];  // row reversed
-    d->d_bank = upload(b);
-    d->ols.upload_from(smb::ols_plan_for_fir(h));
+    auto d = new_device<Device>();
+    d->d_bank = upload(std::vector<float>(h.rbegin(), h.rend()));   // row reversed
+    d->ols_plan = smb::ols_plan_for_fir(h);
+    d->ols.upload_from(d->ols_plan);
     dev = std::move(d);
   }
 };
@@ -1350,9 +749,6 @@ namespace {
 
 enum SpecKind { kSpecComplex, kSpecPower };
 
-// SMB_PATH_AUTO: the tensor-core kernel when it covers the call
-constexpr bool kAutoPrefersTensor = false;
-
 void check_signal(const char* op, int64_t batch, int64_t n) {
   if (n < 0)
     throw smb::invalid_argument(smb::format(
@@ -1392,9 +788,9 @@ int want_fast(const smb_stft_plan* p, int dtype, const smb::FrameGeom& g, int ou
     return SMB_PATH_PAIR;
   }
   if (p->path == SMB_PATH_AUTO && ok_pair) return SMB_PATH_PAIR;
-  const smb_mel_plan::PieceSchedule none{};
-  const smb_mel_plan::PieceSchedule& tc = mel ? mel->sched_tc : none;
-  const smb_mel_plan::PieceSchedule& cc = mel ? mel->sched_cc : none;
+  const smb::PieceSchedule none{};
+  const smb::PieceSchedule& tc = mel ? mel->sched_tc : none;
+  const smb::PieceSchedule& cc = mel ? mel->sched_cc : none;
   const int n_mels = mel ? (int)mel->n_mels : 0;
   const bool ok_tc = base && smb::stft2048tc_supports(gk, out_kind, n_mels, (int)tc.vals.size(), tc.rounds, tc.mpad);
   const bool ok_cc = base && smb::stft2048_supports(gk, out_kind, n_mels, (int)cc.vals.size(), cc.rounds, cc.mpad);
@@ -1410,13 +806,15 @@ int want_fast(const smb_stft_plan* p, int dtype, const smb::FrameGeom& g, int ou
           "soundml_b200: the fused fft-2048 kernel does not cover this geometry");
     return SMB_PATH_FAST;
   }
-  if (ok_tc && kAutoPrefersTensor) return SMB_PATH_TENSOR;
   return ok_cc ? SMB_PATH_FAST : (ok_tc ? SMB_PATH_TENSOR : 0);
 }
 
-smb::Stft2048PairArgs pair_args(const smb_stft_plan* stft, const smb_mel_plan* mel, const void* din,
-                                void* dout, int64_t nb, const smb::FrameGeom& g, double power) {
-  smb::Stft2048PairArgs a{};
+// The launch arguments of a fused fft-2048 kernel without a mel schedule: Stft2048Args for the
+// CUDA-core and tensor-core kernels, Stft2048PairArgs for the frame-pair kernel.
+template <typename Args = smb::Stft2048Args>
+Args fused_args(const smb_stft_plan* stft, const void* din, void* dout, int64_t nb, const smb::FrameGeom& g,
+                double power) {
+  Args a{};
   a.x = (const float*)din;
   a.out = (float*)dout;
   a.batch = nb;
@@ -1426,31 +824,23 @@ smb::Stft2048PairArgs pair_args(const smb_stft_plan* stft, const smb_mel_plan* m
   a.tw_pass = stft->dev->d_tw_pass.get();
   a.tw_post = stft->dev->d_tw_post.get();
   a.power = (float)power;
-  if (mel) {
-    a.n_mels = (int)mel->n_mels;
-    a.mel_w = mel->dev->pair.d_w.get();
-    a.mel_w_floats = (int)mel->sched_pair.w.size();
-    a.mel_items = mel->dev->pair.d_items.get();
-    a.mel_rounds = mel->sched_pair.rounds;
+  if constexpr (std::is_same_v<Args, smb::Stft2048Args>) {
+    a.bin_step = stft->fast_step();
+    a.dft_images = stft->dev->d_dft_images.get();
   }
   return a;
 }
 
-// The launch arguments of the fused kernels (CUDA-core and tensor-core) without a mel schedule.
-smb::Stft2048Args fused_args(const smb_stft_plan* stft, const void* din, void* dout, int64_t nb,
-                             const smb::FrameGeom& g, double power) {
-  smb::Stft2048Args a{};
-  a.x = (const float*)din;
-  a.out = (float*)dout;
-  a.batch = nb;
-  a.g = g;
-  a.g.fft = 2048;
-  a.bin_step = stft->fast_step();
-  a.window = stft->dev->d_window32.get();
-  a.tw_pass = stft->dev->d_tw_pass.get();
-  a.tw_post = stft->dev->d_tw_post.get();
-  a.power = (float)power;
-  a.dft_images = stft->dev->d_dft_images.get();
+smb::Stft2048PairArgs pair_args(const smb_stft_plan* stft, const smb_mel_plan* mel, const void* din,
+                                void* dout, int64_t nb, const smb::FrameGeom& g, double power) {
+  auto a = fused_args<smb::Stft2048PairArgs>(stft, din, dout, nb, g, power);
+  if (mel) {
+    a.n_mels = (int)mel->n_mels;
+    a.mel_w = mel->dev->d_pair_w.get();
+    a.mel_w_floats = (int)mel->sched_pair.w.size();
+    a.mel_items = mel->dev->d_pair_items.get();
+    a.mel_rounds = mel->sched_pair.rounds;
+  }
   return a;
 }
 
@@ -2233,15 +1623,15 @@ int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
                               smb_resample_layout* out) {
   return guarded([&] {
     const smb::ResampleStage& s = stage_of(plan, stage, "stage_layout");
-    plan->ensure_device();
-    const GemmDevice& gd = plan->dev->gemm[(size_t)stage];
+    plan->build_tables();
+    const smb::GemmLayout& gl = plan->tables[(size_t)stage].gemm;
     smb_resample_layout r{};
     r.form = plan->form((size_t)stage);
-    r.groups = r.form == SMB_FORM_ROW ? (int)gd.rows_groups.size()
-             : r.form == SMB_FORM_WINDOW ? (int)gd.groups.size() : 1;
+    r.groups = r.form == SMB_FORM_ROW ? (int)gl.rows.size()
+             : r.form == SMB_FORM_WINDOW ? (int)gl.windows.size() : 1;
     if (group < 0 || group >= r.groups) throw smb::invalid_argument("stage_layout: no such column group");
     if (r.form == SMB_FORM_ROW) {
-      const smb::GemmRowsArgs& a = gd.rows_groups[(size_t)group].a;
+      const smb::GemmRowsArgs& a = gl.rows[(size_t)group].a;
       r.columns = a.l;
       r.col_begin = a.col_begin;
       r.two_issuers = a.two_issuers;
@@ -2252,9 +1642,10 @@ int smb_resample_stage_layout(smb_resample_plan* plan, int stage, int group,
       r.chunks = a.chunks;
       r.slices = a.slices;
     } else if (r.form == SMB_FORM_WINDOW) {
-      r.columns = gd.groups[(size_t)group].width;
-      r.col_begin = gd.groups[(size_t)group].col_begin;
-      r.chunks = gd.groups[(size_t)group].chunks;
+      const smb::GemmResampleArgs& a = gl.windows[(size_t)group].a;
+      r.columns = a.l;
+      r.col_begin = a.col_begin;
+      r.chunks = a.chunks;
     } else {
       r.columns = (int)s.l;
     }
@@ -2395,7 +1786,7 @@ int smb_resample_apply_f64(smb_resample_plan* plan, const double* x, int64_t bat
                   [&](size_t i, const double* src, int64_t nb, int64_t len, int64_t n_out, double* dst,
                       cudaStream_t st) {
                     const smb::ResampleStage& s = plan->plan.stages[i];
-                    CK(smb::launch_polyphase_direct_f64(src, nb, len, plan->dev->d_bank64[i].get(), (int)s.l,
+                    CK(smb::launch_polyphase_direct_f64(src, nb, len, plan->dev->stages[i].d_bank64.get(), (int)s.l,
                                                         (int)s.m, (int)s.k, n_out, dst, st));
                   });
   });
@@ -2612,14 +2003,15 @@ int smb_fir_apply(smb_fir_plan* plan, const float* x, int64_t batch, int64_t n, 
     if (batch == 0 || n == 0) return;
     plan->ensure_device();
     if (method == SMB_EXEC_PLANNED)
-      method = plan->dev->ols.plan.ok && plan->k >= 8 ? SMB_EXEC_OLS : SMB_EXEC_DIRECT;
-    if (method == SMB_EXEC_OLS && !plan->dev->ols.plan.ok)
+      method = plan->dev->ols_plan.ok && plan->k >= 8 ? SMB_EXEC_OLS : SMB_EXEC_DIRECT;
+    if (method == SMB_EXEC_OLS && !plan->dev->ols_plan.ok)
       throw smb::invalid_argument(
           "fir: this filter is too long for the overlap-save kernel (use the direct method)");
     cudaStream_t st = plan->dev->stream.use;
     auto run = [&](const void* din, void* dout, int64_t nb) {
       if (method == SMB_EXEC_OLS)
-        plan->dev->ols.run((const float*)din, nb, n, n, (float*)dout, st);
+        plan->dev->ols.run(plan->dev->ols_plan, (const float*)din, nb, n, n, (float*)dout, plan->dev->sm_count,
+                           st);
       else
         CK(smb::launch_polyphase_direct((const float*)din, nb, n, plan->dev->d_bank.get(), 1, 1, (int)plan->k, n,
                                         (float*)dout, st));

@@ -93,7 +93,7 @@ struct Stft2048Args {
   const float* window;     // [2048]
   const float2* tw_pass;   // [32][32]  W_1024^(k1*n2), index k1*32 + n2
   const float2* tw_post;   // [16][32]  W_2048^(l + 32 j), index j*32 + l
-  // piece-wise mel schedule (kFastMel only; one per kernel, see api.cu build_schedule)
+  // piece-wise mel schedule (kFastMel only; one per kernel, see kernel_tables.cpp piece_schedule)
   int n_mels, nnz;
   const float* vals;               // [nnz] weights, [round][step][lane] x float4
   const MelPiece* mel_pieces;      // [warps of a group][mel_rounds][32 lanes]

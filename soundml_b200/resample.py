@@ -81,9 +81,10 @@ class Config:
     def layout(self, i):
         """How ``apply`` runs stage ``i`` on float32 audio: one dict per column group
         (launch) with the kernel ``form`` ("row", "window", "ols" or "direct") and the
-        tcgen05 layout fields of ``smb_resample_layout``.  Builds the plan's device
-        tables if no ``apply`` has yet (the ``SMB_ROWS_*`` / ``SMB_GEMM_WINDOWS``
-        switches are read then)."""
+        tcgen05 layout fields of ``smb_resample_layout``.  Host-only: needs no GPU.
+        The plan's tables are built by the first ``layout`` or ``apply`` (the
+        ``SMB_ROWS_*`` switches are read then); ``SMB_GEMM_WINDOWS`` is read at
+        every call."""
         out, g, groups = [], 0, 1
         while g < groups:
             r = _lib.ResampleLayout()

@@ -3,8 +3,8 @@
 Every plan the planner tags "gemm" is one stage, so the float64 reference of an output is
 ``oracle.resample_oracle.stage_apply(x, h, L, M, K, n_out)`` with ``h`` the stage's
 prototype, and its magnitude ``mag = stage_apply(|x|, |h|, ...)``.  The geometry table
-below reaches every layout the device planner (``GemmDevice`` in csrc/api.cu) builds;
-``Config.layout`` reports which one ran.
+(resample_geometries.py) reaches every layout the planner (``gemm_layout`` in
+csrc/kernel_tables.cpp) builds; ``Config.layout`` reports which one ran.
 
 Bounds, with u = 2^-24 (float32 unit roundoff):
 
@@ -31,85 +31,12 @@ import numpy as np
 import pytest
 
 from oracle import resample_oracle as R
+from resample_geometries import FORCED, GEOM_IDS, GEOMETRIES, env, geometry, plan, summary  # noqa: F401 (env)
 
 pytestmark = pytest.mark.gpu
 
 U = 2.0 ** -24
 TINY = 2.0 ** -126
-SWITCHES = ("SMB_ROWS_SPLIT", "SMB_ROWS_SMEM_A", "SMB_ROWS_TMEM_A", "SMB_GEMM_WINDOWS")
-
-# (sample_rate, target, quality, the layout Config.layout(0) reports on a B200 under the default
-# switches, one entry per column group).  tools/resample_layouts.py sweeps ~1600 gemm-tagged
-# plans; these rows reach every branch of the planner (test_table_covers_every_layout_branch).
-GEOMETRIES = [
-    # configs[3]: one group, split main shift (14 chunks >= 8), shared-memory A at (3, 2)
-    # (the stage's 53 KB B stages leave no room for (2, 3)), runs split by the split
-    (44100, 16000, "high",
-     "row 160 split smem-A 3/2 shifts 3 chunks 14 slices 42"),
-    # split wanted but its extra accumulator does not fit: the fall back to unsplit; (2, 2)
-    (44100, 16000, "best",
-     "row 160 unsplit smem-A 2/2 shifts 3 chunks 14 slices 28"),
-    # one group with A in tensor memory, B at 3 stages; L mod 4 = 0
-    (44100, 48000, "high",
-     "row 160 unsplit tmem-A 2/3 shifts 3 chunks 5 slices 5"),
-    # L mod 4 = 3 (the epilogue's transposed stores)
-    (48000, 44100, "high",
-     "row 147 unsplit tmem-A 2/3 shifts 3 chunks 5 slices 5"),
-    # no row layout fits (five shifts): a gemm stage on the window form
-    (48000, 44100, "best",
-     "window 147 chunks 15"),
-    # two column groups, split, (2, 3)
-    (44100, 32000, "high",
-     "row 160 split smem-A 2/3 shifts 2 chunks 14 slices 27 | "
-     "row 160 split smem-A 2/3 shifts 2 chunks 14 slices 27"),
-    # three groups, L mod 4 = 1, (2, 2) and (3, 2) in one stage, runs split at gaps (6 and 7
-    # slices over 5 chunks, unsplit)
-    (16000, 44100, "high",
-     "row 160 unsplit smem-A 2/2 shifts 2 chunks 5 slices 6 | "
-     "row 160 unsplit smem-A 2/2 shifts 2 chunks 5 slices 7 | "
-     "row 121 unsplit smem-A 3/2 shifts 3 chunks 5 slices 5"),
-    # four groups, split
-    (11025, 16000, "high",
-     "row 160 split smem-A 2/3 shifts 2 chunks 14 slices 18 | "
-     "row 160 split smem-A 2/3 shifts 2 chunks 14 slices 18 | "
-     "row 160 split smem-A 2/3 shifts 2 chunks 14 slices 18 | "
-     "row 160 split smem-A 2/3 shifts 2 chunks 14 slices 18"),
-    # 10 chunks wants split, which does not fit with A in tensor memory: unsplit, tensor-memory A
-    (48000, 22050, "high",
-     "row 147 unsplit tmem-A 2/3 shifts 3 chunks 10 slices 10"),
-    # a standard pair on the window form (row layout fails), three window groups
-    (8000, 44100, "high",
-     "window 160 chunks 7 | window 160 chunks 8 | window 121 chunks 8"),
-    # L mod 4 = 2, four shifts, 3 chunks, tensor-memory A at (2, 2), a run split
-    (6500, 9800, "fast",
-     "row 98 unsplit tmem-A 2/2 shifts 4 chunks 3 slices 6"),
-    # 3 chunks with tensor-memory A: the B stages capped at 3 (with 4, the B loader never took
-    # back the stage lent to the epilogue and overwrote it: wrong outputs on misaligned clips)
-    (6500, 6400, ("custom", 80.0, 0.8),
-     "row 64 unsplit tmem-A 2/3 shifts 2 chunks 3 slices 3"),
-    # a column group whose taps stay inside one shift
-    (9700, 44100, ("custom", 80.0, 0.8),
-     "row 160 unsplit smem-A 2/3 shifts 1 chunks 4 slices 3 | "
-     "row 160 unsplit smem-A 2/3 shifts 2 chunks 4 slices 4 | "
-     "row 121 unsplit smem-A 2/3 shifts 2 chunks 4 slices 4"),
-    # M = 20 < 32: window form
-    (12000, 88200, ("custom", 80.0, 0.8),
-     "window 147 chunks 3"),
-    # M = 40: two K-chunks per row, below the row form's three: window form
-    (12000, 44100, ("custom", 80.0, 0.8),
-     "window 147 chunks 3"),
-    # split with A in tensor memory (four B stages), L mod 4 = 3
-    (25600, 12700, ("custom", 80.0, 0.8),
-     "row 127 split tmem-A 2/4 shifts 3 chunks 8 slices 20"),
-    # gemm-tagged but L = 1280 > 1024: no tcgen05 tables, the direct kernel
-    (11025, 96000, ("custom", 80.0, 0.8),
-     "direct 1280"),
-]
-GEOM_IDS = [f"{g[0]}-{g[1]}-{g[2] if isinstance(g[2], str) else 'custom%g-%g' % g[2][1:]}" for g in GEOMETRIES]
-
-
-def geometry(sr, target, quality="high"):
-    return next(g for g in GEOMETRIES if g[:3] == (sr, target, quality))
 
 
 @pytest.fixture(scope="module")
@@ -117,26 +44,6 @@ def sb(lib):
     import torch
     assert torch.cuda.is_available()
     return lib
-
-
-@pytest.fixture
-def env(monkeypatch):
-    """The layout switches cleared; a test sets the ones it forces.  They are read when a
-    plan's device tables are built (its first layout() or apply), SMB_GEMM_WINDOWS at
-    every apply."""
-    for k in SWITCHES:
-        monkeypatch.delenv(k, raising=False)
-    return monkeypatch
-
-
-def plan(sb, geom, executor="planned"):
-    """A fresh Config with its device tables built now, under the current switches."""
-    sr, target, quality = geom[:3]
-    cfg = sb.Resample.Config.create(sample_rate=sr, target=target, quality=quality)
-    st = cfg.stages()
-    assert len(st) == 1 and st[0]["exec"] == "gemm", cfg.pp()
-    cfg.set_executor(executor)
-    return cfg, st[0], cfg.layout(0), cfg.stage_prototype(0)
 
 
 def run(sb, cfg, x, reps=1):
@@ -254,19 +161,6 @@ def assert_dense_bound(got, ref, bound, what):
     return worst
 
 
-def summary(layout):
-    """Config.layout as one line per column group, the table's notation."""
-    parts = []
-    for g in layout:
-        if g["form"] != "row":
-            parts.append(f'{g["form"]} {g["columns"]}' + (f' chunks {g["chunks"]}' if g["form"] == "window" else ""))
-        else:
-            parts.append(f'row {g["columns"]} {"split" if g["two_issuers"] else "unsplit"} '
-                         f'{"tmem" if g["a_tmem"] else "smem"}-A {g["a_stages"]}/{g["b_stages"]} '
-                         f'shifts {g["shifts"]} chunks {g["chunks"]} slices {g["slices"]}')
-    return " | ".join(parts)
-
-
 def check_impulses(sb, cfg, s, layout, h, seed, scale=1.0):
     """(b): sparse impulses through one batch large enough that every persistent CTA walks
     several tiles across clip boundaries (the P distinct clips repeated), each output within
@@ -309,42 +203,6 @@ def check_dense(sb, cfg, s, layout, h, seed):
     return assert_dense_bound(got, ref, bound, f"{cfg.pp()} {summary(layout)}")
 
 
-def test_table_covers_every_layout_branch(sb, env):
-    """Each row still builds the layout its comment describes, and together the rows reach
-    every branch of the row-form planner and its fall backs."""
-    layouts = []
-    for g in GEOMETRIES:
-        cfg, s, layout, _ = plan(sb, g)
-        assert summary(layout) == g[3], (g[:3], summary(layout))
-        layouts += [(s, x) for x in layout]
-    rows = [(s, x) for s, x in layouts if x["form"] == "row"]
-    want = {
-        "row form, one column group": any(x["groups"] == 1 for _, x in rows),
-        "row form, several column groups": any(x["groups"] > 1 for _, x in rows),
-        "split main shift (two issuers)": any(x["two_issuers"] for _, x in rows),
-        "unsplit": any(not x["two_issuers"] for _, x in rows),
-        "A tiles in tensor memory": any(x["a_tmem"] for _, x in rows),
-        "A tiles in shared memory": any(not x["a_tmem"] for _, x in rows),
-        "one K-chunk count of 3": any(x["chunks"] == 3 for _, x in rows),
-        "14 or more K-chunks": any(x["chunks"] >= 14 for _, x in rows),
-        "a run split (slices > chunks, unsplit)": any(not x["two_issuers"] and x["slices"] > x["chunks"]
-                                                      for _, x in rows),
-        "a gemm stage on the window form": any(x["form"] == "window" for _, x in layouts),
-        "a gemm stage on the direct kernel (L > 1024)": any(x["form"] == "direct" for _, x in layouts),
-    }
-    # every staging depth the planner can pick: tensor-memory A at B = 4, 3, 2, shared-memory
-    # A at (2, 3), (3, 2), (2, 2)
-    for tmem, a_st, b_st in [(True, 2, 4), (True, 2, 3), (True, 2, 2), (False, 2, 3), (False, 3, 2), (False, 2, 2)]:
-        want[f"{'tensor' if tmem else 'shared'}-memory A, stages ({a_st}, {b_st})"] = any(
-            x["a_tmem"] == tmem and (x["a_stages"], x["b_stages"]) == (a_st, b_st) for _, x in rows)
-    for q in range(1, 5):
-        want[f"{q} shifts"] = any(x["shifts"] == q for _, x in rows)
-    for r in range(4):
-        want[f"L mod 4 = {r}"] = any(s["l"] % 4 == r for s, _ in rows)
-    missing = [k for k, ok in want.items() if not ok]
-    assert not missing, missing
-
-
 @pytest.mark.parametrize("geom", GEOMETRIES, ids=GEOM_IDS)
 def test_impulses_exact_per_element(sb, env, geom):
     cfg, s, layout, h = plan(sb, geom)
@@ -357,22 +215,6 @@ def test_dense_per_element_bound(sb, env, geom):
     cfg, s, layout, h = plan(sb, geom)
     worst = check_dense(sb, cfg, s, layout, h, seed=geom[0] * 3 + geom[1])
     print(f"dense {geom[:3]}: largest err / bound {worst:.3g}")
-
-
-# (switch, value or the executor, geometry): each switch on geometries where it changes the layout
-FORCED = [
-    ("SMB_ROWS_SMEM_A", "1", (44100, 48000, "high")),          # tensor-memory A -> shared (3, 2)
-    ("SMB_ROWS_SMEM_A", "1", (6500, 9800, "fast")),            # ... no shared-memory staging fits: window form
-    ("SMB_ROWS_TMEM_A", "1", (16000, 44100, "high")),          # three groups, shared -> tensor-memory A
-    ("SMB_ROWS_SPLIT", "0", (44100, 16000, "high")),           # split -> unsplit (tensor-memory A)
-    ("SMB_ROWS_SPLIT", "0", (44100, 32000, "high")),
-    ("SMB_ROWS_SPLIT", "1", (16000, 44100, "high")),           # unsplit -> split, five chunks
-    ("SMB_ROWS_SPLIT", "1", (6500, 6400, ("custom", 80.0, 0.8))),   # ... three chunks
-    ("SMB_GEMM_WINDOWS", "1", (44100, 16000, "high")),         # row -> window form
-    ("SMB_GEMM_WINDOWS", "1", (16000, 44100, "high")),
-    ("executor", "direct", (44100, 16000, "high")),            # the blocked direct float32 kernel
-    ("executor", "direct", (48000, 44100, "high")),
-]
 
 
 @pytest.mark.parametrize("switch,value,geom", FORCED,

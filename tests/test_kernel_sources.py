@@ -68,3 +68,12 @@ def test_every_included_file_is_a_build_dependency():
             assert path in listed, f"{name} includes {inc}, which build.py does not list"
     for f in listed:
         assert os.path.exists(f), f"build.py lists {f}, which does not exist"
+
+
+def test_kernel_tables_make_no_cuda_runtime_calls():
+    """kernel_tables.{h,cpp} decide and fill the kernels' tables on the host; api.cu uploads
+    and owns them.  A CUDA runtime call there would make a layout query need a device."""
+    sources = _sources()
+    for name in ("kernel_tables.h", "kernel_tables.cpp"):
+        calls = sorted(set(re.findall(r"\bcuda[A-Z]\w*\s*\(", sources[name])))
+        assert not calls, f"{name} calls {calls}"

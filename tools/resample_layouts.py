@@ -1,11 +1,11 @@
-"""Which tcgen05 layout the resampler's device plan builds, over a sweep of rate pairs
-and qualities (needs a GPU: the layout is decided when the device tables are built).
+"""Which tcgen05 layout the resampler's plan builds, over a sweep of rate pairs and
+qualities (host-only: the layouts are host tables, no GPU is needed).
 
     python tools/resample_layouts.py [out.jsonl]
 
 One JSON line per plan whose single stage the planner tags "gemm": the stage's L, M, K
 and ``Config.layout(0)`` under the default switches and under each of SMB_ROWS_SPLIT=0/1,
-SMB_ROWS_SMEM_A=1, SMB_ROWS_TMEM_A=1.  tests/test_gpu_resample_bounds.py picks its
+SMB_ROWS_SMEM_A=1, SMB_ROWS_TMEM_A=1.  tests/resample_geometries.py picks its
 geometry table from this output."""
 import json
 import math
