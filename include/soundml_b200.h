@@ -15,6 +15,8 @@
  *   smb_mel_spectrogram   Soundml.mel_spectrogram   soundml/lib/soundml.ml:12-24
  *   smb_phase_vocoder,    Effects.time_stretch and the phase vocoder it runs
  *   smb_time_stretch      between Stft.transform and Stft.invert  soundml/lib/effects.ml:296
+ *   smb_hpss,             harmonic-percussive separation (librosa 0.11 decompose.hpss
+ *   smb_hpss_audio        and effects.hpss; the reference's hpss.ml)
  *   smb_window_make       Window.make               soundml/lib/window.ml:374-401
  *   smb_resample_*        Resample.Config.create / output_frames / apply
  *                                           soundml/lib/resample.ml:872-1051,1913-1936
@@ -218,6 +220,61 @@ int smb_time_stretch(smb_stft_plan* plan, const void* x, int64_t batch, int64_t 
  * smb_time_stretch; -1 and the SMB_EINVAL message on a bad rate or a negative count. */
 int64_t smb_time_stretch_frames(const smb_stft_plan* plan, int64_t frames, double rate);
 int64_t smb_time_stretch_length(int64_t n, double rate);
+
+/* Harmonic-percussive separation, librosa 0.11 decompose.hpss (DESIGN.md 4.9).
+ * harm = median of win_harm frames along the frame axis, perc = median of win_perc bins
+ * along the bin axis, both under scipy's mode="reflect" rule (half-sample symmetric,
+ * wrapping as often as a window longer than its axis needs); the median of w values is
+ * element floor(w / 2) of the sorted window (the upper median for even w), so it is
+ * exact.  The masks are librosa.util.softmask in the input's precision:
+ * mask_harm = softmask(harm, perc * margin_harm), mask_perc = softmask(perc, harm *
+ * margin_perc), split_zeros when both margins are 1; power = +inf gives the hard masks
+ * (1 where harm > perc * margin_harm, else 0).
+ *
+ * `what` selects the outputs; the outputs of one item are adjacent:
+ *   SMB_HPSS_BOTH        out [batch, 2, bins, frames]: harmonic then percussive
+ *   SMB_HPSS_HARMONIC    out [batch, 1, bins, frames]
+ *   SMB_HPSS_PERCUSSIVE  out [batch, 1, bins, frames]
+ *   SMB_HPSS_MASKS       out [batch, 2, bins, frames] real: mask_harm, mask_perc
+ * A harmonic or percussive part is S * mask for real input S (a non-negative magnitude or
+ * power spectrogram) and (|D| * mask) * phase for complex input D, with librosa
+ * magphase's phase (1 where |D| = 0).
+ *
+ * Windows of up to 32 on both axes run on a fused tile kernel that keeps each window
+ * sorted in registers; longer windows run on an exact counting kernel.  Both give the
+ * same bits.
+ *
+ * Medians order values as np.sort does (every NaN above +inf), so a NaN input gives what
+ * librosa gives, on both kernels.  Unlike librosa, a NaN power or margin is an error.
+ * Errors, in order: a window below 1 ("hpss: cannot take a median over %lld values
+ * (kernel sizes must be at least 1)"), a margin below 1 or not finite, a power <= 0 or
+ * NaN, a negative extent, the dtype, the memory kind, an unknown `what`. */
+#define SMB_HPSS_BOTH 0
+#define SMB_HPSS_HARMONIC 1
+#define SMB_HPSS_PERCUSSIVE 2
+#define SMB_HPSS_MASKS 3
+/* smb_hpss: s [batch, bins, frames] real (dtype), or complex (complex_in = 1: complex64
+ * for SMB_F32, complex128 for SMB_F64) -> out as above.  No plan: runs on `cuda_stream`
+ * (NULL or SMB_STREAM_OWN = the default stream); a host-memory call stages through
+ * stream-ordered device scratch and returns when the result is in `out`, a device-memory
+ * call is asynchronous on the stream. */
+int smb_hpss(const void* s, int64_t batch, int64_t bins, int64_t frames, int dtype, int complex_in,
+             int64_t win_harm, int64_t win_perc, double power, double margin_harm,
+             double margin_perc, int what, void* out, int mem, void* cuda_stream);
+/* librosa effects.hpss over the plan: x [batch, n] real (dtype) -> out [batch, 2, n]
+ * (SMB_HPSS_BOTH: harmonic then percussive) or [batch, 1, n] (SMB_HPSS_HARMONIC,
+ * SMB_HPSS_PERCUSSIVE), each invert(hpss(transform(x)), length = n) with the plan's own
+ * padding.  transform, hpss and invert run on the plan's stream (3 launches on the
+ * fused fft-2048 float32 path); the spectrum and its separated parts stay in device
+ * scratch the plan owns, 2 * esz * bins * frames * (1 + parts) bytes per clip (esz = 4
+ * for SMB_F32, 8 for SMB_F64; parts = 2 for SMB_HPSS_BOTH, else 1), freed with the
+ * plan.  Host memory is staged through the plan's pipeline in slices.  Errors, in order:
+ * the window, margin and power errors of smb_hpss, a negative length or batch, a
+ * non-invertible configuration (smb_stft_invert's message), the dtype, the memory kind,
+ * an unknown `what` (SMB_HPSS_MASKS included: audio has no masks). */
+int smb_hpss_audio(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
+                   int64_t win_harm, int64_t win_perc, double power, double margin_harm,
+                   double margin_perc, int what, void* out, int mem);
 
 /* ---- mel ----------------------------------------------------------------- */
 /* Mel.Config.create; f_max = NaN means "Nyquist" (the OCaml default). */

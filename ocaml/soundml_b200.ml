@@ -15,6 +15,7 @@
      Stft.transform_range  stft.ml:652-666   -> B200.transform_range
      Stft.invert           stft.ml:937-939   -> B200.invert
      Effects.time_stretch  effects.ml:296    -> B200.time_stretch (and B200.phase_vocoder)
+     hpss / effects.hpss   hpss.ml           -> B200.Hpss
      Convert.power_to_db / amplitude_to_db  convert.ml:20-56 -> B200.to_db
      Soundml.mfcc          soundml.ml:50-95  -> B200.mfcc
      Resample.Kernel.prepare / step / flush / reset
@@ -88,6 +89,20 @@ external time_stretch_frames : stft_plan -> int -> float -> int
   = "soundml_b200_time_stretch_frames"
 
 external time_stretch_length : int -> float -> int = "soundml_b200_time_stretch_length"
+
+(* s -> batch -> bins -> frames -> win_harm -> win_perc -> power -> margin_harm
+   -> margin_perc -> what -> out; s real or complex, out of s's kind or real masks *)
+external hpss_c :
+  ('a, 'b) ba -> int -> int -> int -> int -> int -> float -> float -> float -> int
+  -> ('c, 'd) ba -> unit
+  = "soundml_b200_hpss_bc" "soundml_b200_hpss"
+
+(* plan -> x -> batch -> n -> win_harm -> win_perc -> power -> margin_harm -> margin_perc
+   -> what -> out *)
+external hpss_audio_c :
+  stft_plan -> (float, 'a) ba -> int -> int -> int -> int -> float -> float -> float -> int
+  -> (float, 'a) ba -> unit
+  = "soundml_b200_hpss_audio_bc" "soundml_b200_hpss_audio"
 
 (* amplitude -> x -> reference -> amin -> top_db (nan = None) -> out *)
 external to_db_c :
@@ -365,6 +380,77 @@ let time_stretch c ~rate x =
   if batch > 0 && length > 0 then
     time_stretch_c plan (array1_of (Nx.contiguous x)) batch n rate (array1_of out) ;
   out
+
+(* Harmonic-percussive separation, librosa 0.11 decompose.hpss and effects.hpss /
+   harmonic / percussive (the reference's hpss.ml).  kernel_size and margin are
+   (harmonic, percussive) pairs; power = infinity gives hard masks.  The library checks
+   the parameters (and, for audio, invertibility) with its own wording. *)
+module Hpss = struct
+  let both = 0 and harmonic_only = 1 and percussive_only = 2 and masks_only = 3
+
+  (* [lead; parts; rest] -> the part's [lead; rest] *)
+  let part t lead rest i =
+    let batch = Array.fold_left ( * ) 1 lead in
+    let flat = Nx.reshape (Array.append [|batch; 2|] rest) t in
+    Nx.reshape (Array.append lead rest) (Nx.slice [Nx.A; Nx.R (i, i + 1)] flat)
+
+  let run ~what ~kernel_size ~power ~margin dtype s =
+    let rank = Nx.ndim s in
+    if rank < 2 then
+      invalid_arg
+        (Printf.sprintf
+           "hpss: cannot separate a rank-%d tensor (the bin and frame axes must exist)" rank) ;
+    let frames = Nx.dim (rank - 1) s and bins = Nx.dim (rank - 2) s in
+    let lead = Array.sub (Nx.shape s) 0 (rank - 2) in
+    let batch = Array.fold_left ( * ) 1 lead in
+    let win_harm, win_perc = kernel_size and margin_harm, margin_perc = margin in
+    let out = Nx.zeros dtype (Array.append lead [|2; bins; frames|]) in
+    let s = Nx.contiguous s in
+    (* batch 0: the parameter checks even when there is nothing to compute *)
+    hpss_c (array1_of s) 0 bins frames win_harm win_perc power margin_harm margin_perc what
+      (array1_of out) ;
+    if batch * bins * frames > 0 then
+      hpss_c (array1_of s) batch bins frames win_harm win_perc power margin_harm margin_perc
+        what (array1_of out) ;
+    (part out lead [|bins; frames|] 0, part out lead [|bins; frames|] 1)
+
+  (* (harmonic, percussive) of a real or complex spectrogram [...; bins; frames] *)
+  let hpss ?(kernel_size = (31, 31)) ?(power = 2.) ?(margin = (1., 1.)) s =
+    run ~what:both ~kernel_size ~power ~margin (Nx.dtype s) s
+
+  (* (mask_harm, mask_perc) in the real dtype [dtype] of s *)
+  let masks ?(kernel_size = (31, 31)) ?(power = 2.) ?(margin = (1., 1.)) dtype s =
+    run ~what:masks_only ~kernel_size ~power ~margin dtype s
+
+  let audio ~what ~kernel_size ~power ~margin c x =
+    let n = Nx.dim (Nx.ndim x - 1) x in
+    let lead = leading_shape x in
+    let batch = Array.fold_left ( * ) 1 lead in
+    let parts = if what = both then 2 else 1 in
+    let win_harm, win_perc = kernel_size and margin_harm, margin_perc = margin in
+    let plan = stft_plan_of c in
+    let out = Nx.zeros (Nx.dtype x) (Array.append lead [|parts; n|]) in
+    let x = Nx.contiguous x in
+    hpss_audio_c plan (array1_of x) 0 n win_harm win_perc power margin_harm margin_perc what
+      (array1_of out) ;
+    if batch > 0 && n > 0 then
+      hpss_audio_c plan (array1_of x) batch n win_harm win_perc power margin_harm margin_perc
+        what (array1_of out) ;
+    (out, lead, n)
+
+  (* effects.hpss: (harmonic, percussive) signals of x [...; n] *)
+  let separate ?(kernel_size = (31, 31)) ?(power = 2.) ?(margin = (1., 1.)) c x =
+    let out, lead, n = audio ~what:both ~kernel_size ~power ~margin c x in
+    (part out lead [|n|] 0, part out lead [|n|] 1)
+
+  let harmonic ?(kernel_size = (31, 31)) ?(power = 2.) ?(margin = (1., 1.)) c x =
+    let out, lead, n = audio ~what:harmonic_only ~kernel_size ~power ~margin c x in
+    Nx.reshape (Array.append lead [|n|]) out
+
+  let percussive ?(kernel_size = (31, 31)) ?(power = 2.) ?(margin = (1., 1.)) c x =
+    let out, lead, n = audio ~what:percussive_only ~kernel_size ~power ~margin c x in
+    Nx.reshape (Array.append lead [|n|]) out
+end
 
 (* Replacement body of Convert.power_to_db / amplitude_to_db: elementwise over
    the flat storage, the top_db clamp is one whole-tensor maximum on the GPU. *)

@@ -386,6 +386,75 @@ CAMLprim value soundml_b200_time_stretch_length(value v_n, value v_rate) {
   return Val_long(r);
 }
 
+/* ---- Hpss (librosa 0.11 decompose.hpss / effects.hpss; the reference's hpss.ml) ----
+ * Outputs per item: 2 for SMB_HPSS_BOTH and SMB_HPSS_MASKS, 1 for one part; an unknown
+ * `what` is left to the library, which names it after the parameters' errors. */
+static int64_t hpss_parts(int what) {
+  return what == SMB_HPSS_BOTH || what == SMB_HPSS_MASKS ? 2 : 1;
+}
+
+/* hpss: s [batch; bins; frames] real or complex -> out [batch; parts; bins; frames], of
+ * s's kind, or real masks for SMB_HPSS_MASKS. */
+CAMLprim value soundml_b200_hpss(value v_s, value v_batch, value v_bins, value v_frames,
+                                 value v_win_harm, value v_win_perc, value v_power,
+                                 value v_margin_harm, value v_margin_perc, value v_what, value v_out) {
+  CAMLparam2(v_s, v_out);
+  const void *s = Caml_ba_data_val(v_s);
+  void *out = Caml_ba_data_val(v_out);
+  const int kind = Caml_ba_array_val(v_s)->flags & CAML_BA_KIND_MASK;
+  const int complex_in = kind == CAML_BA_COMPLEX32 || kind == CAML_BA_COMPLEX64;
+  const int dtype = dtype_of(v_s);
+  const int64_t batch = Long_val(v_batch), bins = Long_val(v_bins), frames = Long_val(v_frames);
+  const int what = Int_val(v_what);
+  if (batch >= 0 && bins >= 0 && frames >= 0) {
+    need(v_s, batch * bins * frames, "soundml_b200: input extent disagrees with geometry");
+    need(v_out, batch * hpss_parts(what) * bins * frames,
+         "soundml_b200: output extent disagrees with geometry");
+  }
+  caml_release_runtime_system();
+  int st = smb_hpss(s, batch, bins, frames, dtype, complex_in, Long_val(v_win_harm), Long_val(v_win_perc),
+                    Double_val(v_power), Double_val(v_margin_harm), Double_val(v_margin_perc), what, out,
+                    SMB_MEM_HOST, SMB_STREAM_OWN);
+  caml_acquire_runtime_system();
+  smb_ml_raise(st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value soundml_b200_hpss_bc(value *argv, int argn) {
+  (void)argn;
+  return soundml_b200_hpss(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5], argv[6], argv[7],
+                           argv[8], argv[9], argv[10]);
+}
+
+/* hpss_audio: x [batch; n] real -> out [batch; parts; n], same kind. */
+CAMLprim value soundml_b200_hpss_audio(value v_plan, value v_x, value v_batch, value v_n,
+                                       value v_win_harm, value v_win_perc, value v_power,
+                                       value v_margin_harm, value v_margin_perc, value v_what,
+                                       value v_out) {
+  CAMLparam3(v_plan, v_x, v_out);
+  smb_stft_plan *h = live(v_plan);
+  const void *x = Caml_ba_data_val(v_x);
+  void *out = Caml_ba_data_val(v_out);
+  const int dtype = dtype_of(v_x);
+  const int64_t batch = Long_val(v_batch), n = Long_val(v_n);
+  const int what = Int_val(v_what);
+  if (batch >= 0 && n >= 0) {
+    need(v_x, batch * n, "soundml_b200: input extent disagrees with geometry");
+    need(v_out, batch * hpss_parts(what) * n, "soundml_b200: output extent disagrees with geometry");
+  }
+  caml_release_runtime_system();
+  int st = smb_hpss_audio(h, x, batch, n, dtype, Long_val(v_win_harm), Long_val(v_win_perc),
+                          Double_val(v_power), Double_val(v_margin_harm), Double_val(v_margin_perc),
+                          what, out, SMB_MEM_HOST);
+  caml_acquire_runtime_system();
+  smb_ml_raise(st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value soundml_b200_hpss_audio_bc(value *argv, int argn) {
+  (void)argn;
+  return soundml_b200_hpss_audio(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5], argv[6],
+                                 argv[7], argv[8], argv[9], argv[10]);
+}
+
 /* Convert.power_to_db / amplitude_to_db (convert.ml:20-56).  top_db = nan stands
  * for None; amplitude selects the 20 log10 form. */
 CAMLprim value soundml_b200_to_db(value v_amplitude, value v_x, value v_reference, value v_amin,

@@ -284,7 +284,9 @@ struct smb_stft_plan {
   HostPipe pipe;
   DeviceBuffer tmp;        // power spectrogram of the generic mel path
   DeviceBuffer cepstral;   // mel spectrogram (+ host-call output) of the MFCC path
-  DeviceBuffer stretch_spec, stretch_voc;   // time_stretch: the spectrum and its stretched copy
+  // the effects' spectra: the input's (effect_in) and the effect's result (effect_out):
+  // time_stretch's stretched copy, hpss_audio's separated parts
+  DeviceBuffer effect_in, effect_out;
 
   void ensure_device() {
     if (dev) return same_device(dev->device);
@@ -1111,7 +1113,7 @@ int smb_stft_griffin_lim(smb_stft_plan* plan, const void* s, int64_t batch, int6
 
 }  // extern "C"
 
-// ---- effects: phase vocoder, time_stretch (librosa 0.11 effects; DESIGN.md 4.8) ----
+// ---- effects: phase vocoder, time_stretch (librosa 0.11 effects; DESIGN.md 4.8) and hpss (4.9) ----
 
 namespace {
 
@@ -1223,13 +1225,142 @@ int smb_time_stretch(smb_stft_plan* plan, const void* x, int64_t batch, int64_t 
         CK(cudaMemsetAsync(dout, 0, (size_t)nb * (size_t)out_len * esz, st));
         return;
       }
-      void* spec = p->stretch_spec.ensure((size_t)nb * bins * (size_t)g.frames * 2 * esz);
-      void* voc = p->stretch_voc.ensure((size_t)nb * bins * (size_t)out_frames * 2 * esz);
+      void* spec = p->effect_in.ensure((size_t)nb * bins * (size_t)g.frames * 2 * esz);
+      void* voc = p->effect_out.ensure((size_t)nb * bins * (size_t)out_frames * 2 * esz);
       run_spectrum(p, dx, nb, g, dtype, kSpecComplex, 1.0, spec);
       run_vocoder(p, spec, voc, nb, g.frames, out_frames, dtype, rate);
       run_invert(p, voc, dout, nb, out_frames, true, out_len, dtype, dtype);
     };
     dispatch(mem, p->pipe, st, x, out, batch, (size_t)n * esz, (size_t)out_len * esz, run);
+  });
+}
+
+}  // extern "C"
+
+namespace {
+
+// hpss's parameters in the documented order (include/soundml_b200.h); librosa lets a NaN
+// power or margin through, which would only make every mask NaN
+void check_hpss(int64_t win_harm, int64_t win_perc, double power, double margin_harm,
+                double margin_perc) {
+  for (int64_t w : {win_harm, win_perc})
+    if (w < 1)
+      throw smb::invalid_argument(smb::format(
+          "hpss: cannot take a median over %lld values (kernel sizes must be at least 1)", (long long)w));
+  for (double m : {margin_harm, margin_perc})
+    if (!(m >= 1.0) || !std::isfinite(m))
+      throw smb::invalid_argument(smb::format(
+          "hpss: cannot use a margin of %g (margins must be finite and at least 1)", m));
+  if (!(power > 0.0))
+    throw smb::invalid_argument(smb::format(
+        "hpss: cannot raise the masks to a power of %g (the power must be positive; +inf gives "
+        "hard masks)", power));
+}
+
+// outputs per item: 2 for SMB_HPSS_BOTH and SMB_HPSS_MASKS, else 1
+int hpss_parts(int what, bool masks_allowed) {
+  if (what == SMB_HPSS_HARMONIC || what == SMB_HPSS_PERCUSSIVE) return 1;
+  if (what == SMB_HPSS_BOTH || (masks_allowed && what == SMB_HPSS_MASKS)) return 2;
+  throw smb::invalid_argument(smb::format(
+      "hpss: cannot return output kind %d (what must be SMB_HPSS_BOTH, SMB_HPSS_HARMONIC, "
+      "SMB_HPSS_PERCUSSIVE%s)", what, masks_allowed ? " or SMB_HPSS_MASKS" : ""));
+}
+
+smb::HpssArgs hpss_args(const void* s, void* out, int64_t batch, int64_t bins, int64_t frames, int dtype,
+                        bool complex_in, int64_t win_harm, int64_t win_perc, double power,
+                        double margin_harm, double margin_perc, int what) {
+  smb::HpssArgs a{};
+  a.s = s;
+  a.out = out;
+  a.batch = batch;
+  a.bins = bins;
+  a.frames = frames;
+  a.win_harm = win_harm;
+  a.win_perc = win_perc;
+  a.power = power;
+  a.margin_harm = margin_harm;
+  a.margin_perc = margin_perc;
+  a.what = what;
+  a.f64 = dtype == SMB_F64;
+  a.complex_in = complex_in;
+  return a;
+}
+
+}  // namespace
+
+extern "C" {
+
+int smb_hpss(const void* s, int64_t batch, int64_t bins, int64_t frames, int dtype, int complex_in,
+             int64_t win_harm, int64_t win_perc, double power, double margin_harm,
+             double margin_perc, int what, void* out, int mem, void* cuda_stream) {
+  return guarded([&] {
+    check_hpss(win_harm, win_perc, power, margin_harm, margin_perc);
+    if (batch < 0 || bins < 0 || frames < 0)
+      throw smb::invalid_argument(smb::format(
+          "hpss: cannot separate a [%lld, %lld, %lld] spectrogram (extents must be non-negative)",
+          (long long)batch, (long long)bins, (long long)frames));
+    const size_t esz = dtype_size(dtype);
+    check_mem(mem);
+    const int parts = hpss_parts(what, true);
+    const size_t cells = (size_t)batch * (size_t)bins * (size_t)frames;
+    if (cells == 0) return;
+    require_device();
+    // no plan, hence no plan stream: SMB_STREAM_OWN means the default stream
+    cudaStream_t st = cuda_stream == SMB_STREAM_OWN ? nullptr : (cudaStream_t)cuda_stream;
+    const size_t in_bytes = cells * esz * (complex_in ? 2 : 1);
+    const size_t out_bytes = cells * (size_t)parts * esz * (complex_in && what != SMB_HPSS_MASKS ? 2 : 1);
+    // a host call stages through stream-ordered scratch, as the dB conversions do
+    scratch_ptr din, dout;
+    const void* src = s;
+    void* dst = out;
+    if (mem == SMB_MEM_HOST) {
+      din = scratch_alloc(in_bytes, st);
+      dout = scratch_alloc(out_bytes, st);
+      CK(cudaMemcpyAsync(din.get(), s, in_bytes, cudaMemcpyHostToDevice, st));
+      src = din.get();
+      dst = dout.get();
+    }
+    CK(smb::launch_hpss(hpss_args(src, dst, batch, bins, frames, dtype, complex_in != 0, win_harm, win_perc,
+                                  power, margin_harm, margin_perc, what), st));
+    if (mem == SMB_MEM_HOST) {
+      CK(cudaMemcpyAsync(out, dout.get(), out_bytes, cudaMemcpyDeviceToHost, st));
+      CK(cudaStreamSynchronize(st));   // the host buffer is the caller's again
+    }
+  });
+}
+
+int smb_hpss_audio(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
+                   int64_t win_harm, int64_t win_perc, double power, double margin_harm,
+                   double margin_perc, int what, void* out, int mem) {
+  return guarded([&] {
+    smb_stft_plan* p = plan;
+    check_hpss(win_harm, win_perc, power, margin_harm, margin_perc);
+    check_signal("hpss", batch, n);
+    require_nola("invert", p);                          // Stft.invert's precondition
+    const size_t esz = dtype_size(dtype);
+    check_mem(mem);
+    const int parts = hpss_parts(what, false);
+    if (batch == 0 || n == 0) return;
+    p->ensure_device();
+    cudaStream_t st = p->dev->stream.use;
+    const smb::FrameGeom g = p->frame_geom(n);
+    const size_t bins = (size_t)p->geom.bins();
+    // transform -> hpss -> one invert over the nb * parts separated spectra, whose
+    // [nb, parts, bins, frames] layout makes the output [nb, parts, n]
+    auto run = [&](const void* dx, void* dout, int64_t nb) {
+      if (g.frames == 0) {                              // no frame: invert of nothing is zeros
+        CK(cudaMemsetAsync(dout, 0, (size_t)nb * parts * (size_t)n * esz, st));
+        return;
+      }
+      const size_t spectrum = bins * (size_t)g.frames * 2 * esz;
+      void* spec = p->effect_in.ensure((size_t)nb * spectrum);
+      void* sep = p->effect_out.ensure((size_t)nb * parts * spectrum);
+      run_spectrum(p, dx, nb, g, dtype, kSpecComplex, 1.0, spec);
+      CK(smb::launch_hpss(hpss_args(spec, sep, nb, (int64_t)bins, g.frames, dtype, true, win_harm, win_perc,
+                                    power, margin_harm, margin_perc, what), st));
+      run_invert(p, sep, dout, nb * parts, g.frames, true, n, dtype, dtype);
+    };
+    dispatch(mem, p->pipe, st, x, out, batch, (size_t)n * esz, (size_t)parts * (size_t)n * esz, run);
   });
 }
 

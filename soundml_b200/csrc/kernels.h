@@ -71,6 +71,26 @@ struct PhaseVocoderArgs {
 };
 cudaError_t launch_phase_vocoder(const PhaseVocoderArgs& a, cudaStream_t st);
 
+// ---- harmonic-percussive separation (hpss_kernels.cu) ------------------------------
+// s [batch, bins, frames] real or complex -> the masked spectra or the masks of librosa
+// 0.11 decompose.hpss (DESIGN.md 4.9).  `what` is SMB_HPSS_*; out is [batch, 2 | 1, bins,
+// frames], complex for complex input unless the masks are asked for.
+struct HpssArgs {
+  const void* s;
+  void* out;
+  long long batch, bins, frames;
+  long long win_harm, win_perc;
+  double power;             // > 0, +inf for the hard mask
+  double margin_harm, margin_perc;
+  int what;
+  int f64, complex_in;
+};
+// The fused tile kernel keeps each window sorted in registers: it takes windows of up to
+// kHpssFastWindow; the exact counting kernel takes the rest.
+constexpr long long kHpssFastWindow = 32;
+bool hpss_fast_supports(long long win_harm, long long win_perc);
+cudaError_t launch_hpss(const HpssArgs& a, cudaStream_t st);
+
 // ---- fast path: fft 2048, float32, fused frame+window+rFFT+|X|^p(+mel) -------
 // Tile shape of the fused CUDA-core kernel: a group of kFastTile warps transforms
 // kFastTile consecutive frames, one per warp.
