@@ -17,6 +17,8 @@
  *   smb_time_stretch      between Stft.transform and Stft.invert  soundml/lib/effects.ml:296
  *   smb_hpss,             harmonic-percussive separation (librosa 0.11 decompose.hpss
  *   smb_hpss_audio        and effects.hpss; the reference's hpss.ml)
+ *   smb_spectral,         per-frame spectral descriptors (librosa 0.11 feature.spectral_*;
+ *   smb_spectral_audio    the reference's spectral.ml)
  *   smb_window_make       Window.make               soundml/lib/window.ml:374-401
  *   smb_resample_*        Resample.Config.create / output_frames / apply
  *                                           soundml/lib/resample.ml:872-1051,1913-1936
@@ -275,6 +277,50 @@ int smb_hpss(const void* s, int64_t batch, int64_t bins, int64_t frames, int dty
 int smb_hpss_audio(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
                    int64_t win_harm, int64_t win_perc, double power, double margin_harm,
                    double margin_perc, int what, void* out, int mem);
+
+/* Spectral descriptors, librosa 0.11 feature.spectral_centroid / _bandwidth / _rolloff /
+ * _flatness (DESIGN.md 4.10), of a non-negative magnitude spectrogram S [batch, bins,
+ * frames].  f_k = k * (1 / (n_fft * (1 / sample_rate))) in double (numpy rfftfreq), and
+ * L = sum_k S_k, taken as 1 when below the smallest normal number of S's type (librosa
+ * util.normalize with fill=None: a silent frame gives 0):
+ *   SMB_SPECTRAL_CENTROID   c = sum_k f_k S_k / L
+ *   SMB_SPECTRAL_BANDWIDTH  (sum_k S'_k |f_k - c|^p)^(1/p), S' = S / L if norm, else S
+ *   SMB_SPECTRAL_ROLLOFF    f_k of the first k with !(cum_k < thr), cum_k = S_0 + ... + S_k
+ *                           added in order in S's precision, thr = roll_percent * cum_last
+ *                           in the same precision (np.cumsum; a NaN or silent frame gives 0)
+ *   SMB_SPECTRAL_FLATNESS   exp(mean_k ln m_k) / mean_k m_k, m_k = max(amin, S_k^power)
+ * Sums accumulate in double; outputs have S's type.  Nothing checks S on the device:
+ * a NaN stays in its own frame, and negative values are outside the domain (rolloff may
+ * then miss the first crossing, and gives NaN for a frame that never reaches it).
+ * Errors, in order, also for an empty batch: a `what` that is 0 or has unknown bits, a
+ * sample rate that is not positive and finite, a p that is not positive and finite, a
+ * roll_percent outside (0, 1), an amin <= 0, a power <= 0, a negative extent, an n_fft
+ * that is not positive or whose n_fft / 2 + 1 is not `bins`, the dtype, the memory kind.
+ * Every parameter is checked whichever descriptors `what` selects. */
+#define SMB_SPECTRAL_CENTROID 1
+#define SMB_SPECTRAL_BANDWIDTH 2
+#define SMB_SPECTRAL_ROLLOFF 4
+#define SMB_SPECTRAL_FLATNESS 8
+/* smb_spectral: s [batch, bins, frames] real (dtype) -> out [batch, popcount(what), frames],
+ * the rows of `what` in flag order, of s's dtype.  n_fft = SMB_DEFAULT means 2 (bins - 1).
+ * No plan: runs on `cuda_stream` (NULL or SMB_STREAM_OWN = the default stream); a
+ * host-memory call stages through stream-ordered device scratch and returns when the
+ * result is in `out`, a device-memory call is asynchronous on the stream. */
+int smb_spectral(const void* s, int64_t batch, int64_t bins, int64_t frames, int dtype,
+                 int64_t n_fft, double sample_rate, int what, double p, int norm,
+                 double roll_percent, double amin, double power, void* out, int mem,
+                 void* cuda_stream);
+/* The descriptors of the plan's magnitude spectrogram: x [batch, n] real (dtype) ->
+ * out [batch, popcount(what), frames] with frames = smb_stft_frames(plan, n) and n_fft the
+ * plan's fft size.  The spectrum (smb_stft_power_spectrum at power 1) stays in device
+ * scratch the plan owns, esz * bins * frames bytes per clip, freed with the plan; both
+ * steps run on the plan's stream (2 launches on the fused fft-2048 float32 path).  Host
+ * memory is staged through the plan's pipeline in slices.  Errors, in order: the
+ * parameter errors of smb_spectral, a negative length or batch, the dtype, the memory
+ * kind. */
+int smb_spectral_audio(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
+                       double sample_rate, int what, double p, int norm, double roll_percent,
+                       double amin, double power, void* out, int mem);
 
 /* ---- mel ----------------------------------------------------------------- */
 /* Mel.Config.create; f_max = NaN means "Nyquist" (the OCaml default). */

@@ -16,6 +16,7 @@
      Stft.invert           stft.ml:937-939   -> B200.invert
      Effects.time_stretch  effects.ml:296    -> B200.time_stretch (and B200.phase_vocoder)
      hpss / effects.hpss   hpss.ml           -> B200.Hpss
+     spectral.ml                             -> B200.Spectral
      Convert.power_to_db / amplitude_to_db  convert.ml:20-56 -> B200.to_db
      Soundml.mfcc          soundml.ml:50-95  -> B200.mfcc
      Resample.Kernel.prepare / step / flush / reset
@@ -103,6 +104,20 @@ external hpss_audio_c :
   stft_plan -> (float, 'a) ba -> int -> int -> int -> int -> float -> float -> float -> int
   -> (float, 'a) ba -> unit
   = "soundml_b200_hpss_audio_bc" "soundml_b200_hpss_audio"
+
+(* s -> batch -> bins -> frames -> n_fft -> sample_rate -> what -> p -> norm -> roll_percent
+   -> amin -> power -> out; out [batch; popcount what; frames] of s's kind *)
+external spectral_c :
+  (float, 'a) ba -> int -> int -> int -> int -> float -> int -> float -> bool -> float -> float
+  -> float -> (float, 'a) ba -> unit
+  = "soundml_b200_spectral_bc" "soundml_b200_spectral"
+
+(* plan -> x -> batch -> n -> sample_rate -> what -> p -> norm -> roll_percent -> amin
+   -> power -> out *)
+external spectral_audio_c :
+  stft_plan -> (float, 'a) ba -> int -> int -> float -> int -> float -> bool -> float -> float
+  -> float -> (float, 'a) ba -> unit
+  = "soundml_b200_spectral_audio_bc" "soundml_b200_spectral_audio"
 
 (* amplitude -> x -> reference -> amin -> top_db (nan = None) -> out *)
 external to_db_c :
@@ -450,6 +465,65 @@ module Hpss = struct
   let percussive ?(kernel_size = (31, 31)) ?(power = 2.) ?(margin = (1., 1.)) c x =
     let out, lead, n = audio ~what:percussive_only ~kernel_size ~power ~margin c x in
     Nx.reshape (Array.append lead [|n|]) out
+end
+
+(* Per-frame spectral descriptors, librosa 0.11 feature.spectral_centroid / _bandwidth /
+   _rolloff / _flatness (the reference's spectral.ml).  [which] lists SMB_SPECTRAL_* flags;
+   the result holds one [...; 1; frames] tensor per flag, in flag order.  n_fft = None
+   means 2 (bins - 1); the library checks every parameter with its own wording. *)
+module Spectral = struct
+  let centroid = 1 and bandwidth = 2 and rolloff = 4 and flatness = 8
+
+  let what_of which = List.fold_left ( lor ) 0 which
+
+  let rows what = List.length (List.filter (fun f -> what land f <> 0) [centroid; bandwidth; rolloff; flatness])
+
+  (* [lead; rows; frames] -> one [lead; 1; frames] tensor per row *)
+  let split out lead frames what =
+    let batch = Array.fold_left ( * ) 1 lead and k = rows what in
+    let flat = Nx.reshape [|batch; k; frames|] out in
+    List.init k (fun i ->
+        Nx.reshape (Array.append lead [|1; frames|]) (Nx.slice [Nx.A; Nx.R (i, i + 1)] flat))
+
+  let features ?(sample_rate = 22050.) ?n_fft ?(p = 2.) ?(norm = true) ?(roll_percent = 0.85)
+      ?(amin = 1e-10) ?(power = 2.) which s =
+    let rank = Nx.ndim s in
+    if rank < 2 then
+      invalid_arg
+        (Printf.sprintf
+           "spectral: cannot describe a rank-%d tensor (the bin and frame axes must exist)" rank) ;
+    let frames = Nx.dim (rank - 1) s and bins = Nx.dim (rank - 2) s in
+    let lead = Array.sub (Nx.shape s) 0 (rank - 2) in
+    let batch = Array.fold_left ( * ) 1 lead in
+    let what = what_of which in
+    let n_fft = match n_fft with Some n -> n | None -> 2 * (bins - 1) in
+    let out = Nx.zeros (Nx.dtype s) (Array.append lead [|rows what; frames|]) in
+    let s = Nx.contiguous s in
+    (* batch 0: the parameter checks even when there is nothing to compute *)
+    spectral_c (array1_of s) 0 bins frames n_fft sample_rate what p norm roll_percent amin power
+      (array1_of out) ;
+    if batch * frames > 0 then
+      spectral_c (array1_of s) batch bins frames n_fft sample_rate what p norm roll_percent amin
+        power (array1_of out) ;
+    split out lead frames what
+
+  let features_audio ?(sample_rate = 22050.) ?(p = 2.) ?(norm = true) ?(roll_percent = 0.85)
+      ?(amin = 1e-10) ?(power = 2.) c which x =
+    let n = Nx.dim (Nx.ndim x - 1) x in
+    let lead = leading_shape x in
+    let batch = Array.fold_left ( * ) 1 lead in
+    let what = what_of which in
+    let plan = stft_plan_of c in
+    let x = Nx.contiguous x in
+    let probe = Nx.zeros (Nx.dtype x) [|0|] in
+    spectral_audio_c plan (array1_of x) 0 n sample_rate what p norm roll_percent amin power
+      (array1_of probe) ;
+    let frames = Stft.frames c ~n in
+    let out = Nx.zeros (Nx.dtype x) (Array.append lead [|rows what; frames|]) in
+    if batch > 0 && frames > 0 then
+      spectral_audio_c plan (array1_of x) batch n sample_rate what p norm roll_percent amin power
+        (array1_of out) ;
+    split out lead frames what
 end
 
 (* Replacement body of Convert.power_to_db / amplitude_to_db: elementwise over

@@ -455,6 +455,71 @@ CAMLprim value soundml_b200_hpss_audio_bc(value *argv, int argn) {
                                  argv[7], argv[8], argv[9], argv[10]);
 }
 
+/* ---- Spectral (librosa 0.11 feature.spectral_*; the reference's spectral.ml) ----
+ * Rows per item: one per bit of `what`; unknown bits are left to the library, which names
+ * them first. */
+static int64_t spectral_rows(int what) {
+  return __builtin_popcount((unsigned)what & 15u);
+}
+
+/* spectral: s [batch; bins; frames] real -> out [batch; rows; frames], same kind. */
+CAMLprim value soundml_b200_spectral(value v_s, value v_batch, value v_bins, value v_frames, value v_n_fft,
+                                     value v_sample_rate, value v_what, value v_p, value v_norm,
+                                     value v_roll_percent, value v_amin, value v_power, value v_out) {
+  CAMLparam2(v_s, v_out);
+  const void *s = Caml_ba_data_val(v_s);
+  void *out = Caml_ba_data_val(v_out);
+  const int dtype = dtype_of(v_s);
+  const int64_t batch = Long_val(v_batch), bins = Long_val(v_bins), frames = Long_val(v_frames);
+  const int what = Int_val(v_what);
+  if (batch >= 0 && bins >= 0 && frames >= 0) {
+    need(v_s, batch * bins * frames, "soundml_b200: input extent disagrees with geometry");
+    need(v_out, batch * spectral_rows(what) * frames, "soundml_b200: output extent disagrees with geometry");
+  }
+  caml_release_runtime_system();
+  int st = smb_spectral(s, batch, bins, frames, dtype, Long_val(v_n_fft), Double_val(v_sample_rate), what,
+                        Double_val(v_p), Bool_val(v_norm), Double_val(v_roll_percent), Double_val(v_amin),
+                        Double_val(v_power), out, SMB_MEM_HOST, SMB_STREAM_OWN);
+  caml_acquire_runtime_system();
+  smb_ml_raise(st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value soundml_b200_spectral_bc(value *argv, int argn) {
+  (void)argn;
+  return soundml_b200_spectral(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5], argv[6], argv[7],
+                               argv[8], argv[9], argv[10], argv[11], argv[12]);
+}
+
+/* spectral_audio: x [batch; n] real -> out [batch; rows; frames], same kind. */
+CAMLprim value soundml_b200_spectral_audio(value v_plan, value v_x, value v_batch, value v_n,
+                                           value v_sample_rate, value v_what, value v_p, value v_norm,
+                                           value v_roll_percent, value v_amin, value v_power, value v_out) {
+  CAMLparam3(v_plan, v_x, v_out);
+  smb_stft_plan *h = live(v_plan);
+  const void *x = Caml_ba_data_val(v_x);
+  void *out = Caml_ba_data_val(v_out);
+  const int dtype = dtype_of(v_x);
+  const int64_t batch = Long_val(v_batch), n = Long_val(v_n);
+  const int what = Int_val(v_what);
+  if (batch >= 0 && n >= 0) {
+    need(v_x, batch * n, "soundml_b200: input extent disagrees with geometry");
+    need(v_out, batch * spectral_rows(what) * smb_stft_frames(h, n),
+         "soundml_b200: output extent disagrees with geometry");
+  }
+  caml_release_runtime_system();
+  int st = smb_spectral_audio(h, x, batch, n, dtype, Double_val(v_sample_rate), what, Double_val(v_p),
+                              Bool_val(v_norm), Double_val(v_roll_percent), Double_val(v_amin),
+                              Double_val(v_power), out, SMB_MEM_HOST);
+  caml_acquire_runtime_system();
+  smb_ml_raise(st);
+  CAMLreturn(Val_unit);
+}
+CAMLprim value soundml_b200_spectral_audio_bc(value *argv, int argn) {
+  (void)argn;
+  return soundml_b200_spectral_audio(argv[0], argv[1], argv[2], argv[3], argv[4], argv[5], argv[6], argv[7],
+                                     argv[8], argv[9], argv[10], argv[11]);
+}
+
 /* Convert.power_to_db / amplitude_to_db (convert.ml:20-56).  top_db = nan stands
  * for None; amplitude selects the 20 log10 form. */
 CAMLprim value soundml_b200_to_db(value v_amplitude, value v_x, value v_reference, value v_amin,

@@ -1,15 +1,15 @@
 """soundml_b200 — B200-native spectral hot path of SoundML.
 
 The flat API mirrors ``soundml/lib/soundml.ml``: ``mel_spectrogram`` and
-``resample``, with the ``stft``, ``mel``, ``window``, ``resample``, ``effects`` and
-``hpss`` modules underneath.  All arithmetic runs in ``libsoundml_b200.so`` (hand-written CUDA
+``resample``, with the ``stft``, ``mel``, ``window``, ``resample``, ``effects``,
+``hpss`` and ``spectral`` modules underneath.  All arithmetic runs in ``libsoundml_b200.so`` (hand-written CUDA
 for sm_100a behind the C ABI in ``include/soundml_b200.h``).
 """
 import numpy as np
 
 import math
 
-from . import _lib, convert, effects, hpss, io, mel, stft, window
+from . import _lib, convert, effects, hpss, io, mel, spectral, stft, window
 from . import resample as _resample_mod
 from ._lib import SoundmlError
 
@@ -22,8 +22,9 @@ Fir = _resample_mod.Fir
 Io = io
 Effects = effects
 Hpss = hpss
+Spectral = spectral
 
-__all__ = ["Stft", "Mel", "Window", "Convert", "Resample", "Fir", "Io", "Effects", "Hpss", "mel_spectrogram",
+__all__ = ["Stft", "Mel", "Window", "Convert", "Resample", "Fir", "Io", "Effects", "Hpss", "Spectral", "mel_spectrogram",
            "log_mel_spectrogram", "mfcc",
            "resample",
            "kernel_launch_count", "SoundmlError"]

@@ -109,6 +109,9 @@ SIGNATURES = {
     "smb_time_stretch_length": (_i64, [_i64, _dbl]),
     "smb_hpss": (_int, [_vp, _i64, _i64, _i64, _int, _int, _i64, _i64, _dbl, _dbl, _dbl, _int, _vp, _int, _vp]),
     "smb_hpss_audio": (_int, [_vp, _vp, _i64, _i64, _int, _i64, _i64, _dbl, _dbl, _dbl, _int, _vp, _int]),
+    "smb_spectral": (_int, [_vp, _i64, _i64, _i64, _int, _i64, _dbl, _int, _dbl, _int, _dbl, _dbl, _dbl, _vp, _int,
+                            _vp]),
+    "smb_spectral_audio": (_int, [_vp, _vp, _i64, _i64, _int, _dbl, _int, _dbl, _int, _dbl, _dbl, _dbl, _vp, _int]),
     "smb_mel_plan_create": (_int, [_pvp, _i64, _i64, _i64, _dbl, _dbl, _int, _int]),
     "smb_mel_plan_create_with_weights": (_int, [_pvp, _i64, _i64, _pd]),
     "smb_mel_plan_destroy": (_int, [_vp]),

@@ -17,7 +17,7 @@ LIB = os.path.join(HERE, "libsoundml_b200.so")
 
 CUDA_SOURCES = ["api.cu", "kernels_generic.cu", "stft2048.cu", "stft2048p.cu", "stft2048tc.cu", "resample_kernels.cu",
                 "ols_kernels.cu", "ols2048.cu", "resample_gemm.cu", "db_kernels.cu", "istft_kernels.cu", "istft2048.cu", "ingest_kernels.cu",
-                "effects_kernels.cu", "hpss_kernels.cu"]
+                "effects_kernels.cu", "hpss_kernels.cu", "spectral_kernels.cu"]
 HOST_SOURCES = ["host_design.cpp", "kernel_tables.cpp"]
 HEADERS = ["host_design.h", "kernel_tables.h", "kernels.h", "fft32.cuh", "fft32x2.cuh", "max_key.cuh", "sm100.cuh", "stft_stage.cuh",
            os.path.join("..", "..", "include", "soundml_b200.h")]

@@ -230,6 +230,21 @@ void dispatch(int mem, HostPipe& pipe, cudaStream_t st, const void* x, void* out
   else pipe.execute(st, x, out, batch, in_item, out_item, run);
 }
 
+// A call without a plan: run(src, dst) on the caller's device buffers, or, for host
+// memory, through stream-ordered scratch (as the dB conversions stage), returning once the
+// result is in `out`.
+template <typename Run>
+void on_stream(int mem, cudaStream_t st, const void* x, size_t in_bytes, void* out, size_t out_bytes,
+               Run&& run) {
+  if (mem == SMB_MEM_DEVICE) return run(x, out);
+  scratch_ptr din = scratch_alloc(in_bytes, st);
+  scratch_ptr dout = scratch_alloc(out_bytes, st);
+  CK(cudaMemcpyAsync(din.get(), x, in_bytes, cudaMemcpyHostToDevice, st));
+  run(din.get(), dout.get());
+  CK(cudaMemcpyAsync(out, dout.get(), out_bytes, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));   // the host buffer is the caller's again
+}
+
 size_t dtype_size(int dtype) {
   if (dtype == SMB_F32) return 4;
   if (dtype == SMB_F64) return 8;
@@ -1309,23 +1324,10 @@ int smb_hpss(const void* s, int64_t batch, int64_t bins, int64_t frames, int dty
     cudaStream_t st = cuda_stream == SMB_STREAM_OWN ? nullptr : (cudaStream_t)cuda_stream;
     const size_t in_bytes = cells * esz * (complex_in ? 2 : 1);
     const size_t out_bytes = cells * (size_t)parts * esz * (complex_in && what != SMB_HPSS_MASKS ? 2 : 1);
-    // a host call stages through stream-ordered scratch, as the dB conversions do
-    scratch_ptr din, dout;
-    const void* src = s;
-    void* dst = out;
-    if (mem == SMB_MEM_HOST) {
-      din = scratch_alloc(in_bytes, st);
-      dout = scratch_alloc(out_bytes, st);
-      CK(cudaMemcpyAsync(din.get(), s, in_bytes, cudaMemcpyHostToDevice, st));
-      src = din.get();
-      dst = dout.get();
-    }
-    CK(smb::launch_hpss(hpss_args(src, dst, batch, bins, frames, dtype, complex_in != 0, win_harm, win_perc,
-                                  power, margin_harm, margin_perc, what), st));
-    if (mem == SMB_MEM_HOST) {
-      CK(cudaMemcpyAsync(out, dout.get(), out_bytes, cudaMemcpyDeviceToHost, st));
-      CK(cudaStreamSynchronize(st));   // the host buffer is the caller's again
-    }
+    on_stream(mem, st, s, in_bytes, out, out_bytes, [&](const void* src, void* dst) {
+      CK(smb::launch_hpss(hpss_args(src, dst, batch, bins, frames, dtype, complex_in != 0, win_harm, win_perc,
+                                    power, margin_harm, margin_perc, what), st));
+    });
   });
 }
 
@@ -1361,6 +1363,121 @@ int smb_hpss_audio(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n,
       run_invert(p, sep, dout, nb * parts, g.frames, true, n, dtype, dtype);
     };
     dispatch(mem, p->pipe, st, x, out, batch, (size_t)n * esz, (size_t)parts * (size_t)n * esz, run);
+  });
+}
+
+}  // extern "C"
+
+// ---- spectral descriptors (librosa 0.11 feature.spectral_*; DESIGN.md 4.10) ----
+
+namespace {
+
+constexpr int kSpectralAll = SMB_SPECTRAL_CENTROID | SMB_SPECTRAL_BANDWIDTH | SMB_SPECTRAL_ROLLOFF |
+                             SMB_SPECTRAL_FLATNESS;
+
+// the descriptors' parameters in the documented order (include/soundml_b200.h); returns the
+// rows per item
+int check_spectral(int what, double sample_rate, double p, double roll_percent, double amin,
+                   double power) {
+  if (what == 0 || (what & ~kSpectralAll))
+    throw smb::invalid_argument(smb::format(
+        "spectral: cannot compute descriptor set %d (what must be a nonzero combination of "
+        "SMB_SPECTRAL_CENTROID, SMB_SPECTRAL_BANDWIDTH, SMB_SPECTRAL_ROLLOFF and "
+        "SMB_SPECTRAL_FLATNESS)", what));
+  if (!(sample_rate > 0.0) || !std::isfinite(sample_rate))
+    throw smb::invalid_argument(smb::format(
+        "spectral: cannot use a sample rate of %g (it must be positive and finite)", sample_rate));
+  if (!(p > 0.0) || !std::isfinite(p))
+    throw smb::invalid_argument(smb::format(
+        "spectral: cannot take the bandwidth at p = %g (p must be positive and finite)", p));
+  if (!(roll_percent > 0.0 && roll_percent < 1.0))
+    throw smb::invalid_argument(smb::format(
+        "spectral: cannot roll off at %g of the energy (roll_percent must lie in (0, 1))", roll_percent));
+  if (!(amin > 0.0))
+    throw smb::invalid_argument(smb::format(
+        "spectral: cannot floor the spectrum at amin = %g (amin must be positive)", amin));
+  if (!(power > 0.0))
+    throw smb::invalid_argument(smb::format(
+        "spectral: cannot raise the spectrum to a power of %g (the power must be positive)", power));
+  return __builtin_popcount((unsigned)what);
+}
+
+smb::SpectralArgs spectral_args(const void* s, void* out, int64_t batch, int64_t bins, int64_t frames,
+                                int dtype, int64_t n_fft, double sample_rate, int what, double p,
+                                int norm, double roll_percent, double amin, double power) {
+  smb::SpectralArgs a{};
+  a.s = s;
+  a.out = out;
+  a.batch = batch;
+  a.bins = bins;
+  a.frames = frames;
+  a.bin_hz = 1.0 / ((double)n_fft * (1.0 / sample_rate));   // numpy rfftfreq's 1 / (n d)
+  a.what = what;
+  a.p = p;
+  a.norm = norm != 0;
+  a.roll_percent = roll_percent;
+  a.amin = amin;
+  a.power = power;
+  a.f64 = dtype == SMB_F64;
+  return a;
+}
+
+}  // namespace
+
+extern "C" {
+
+int smb_spectral(const void* s, int64_t batch, int64_t bins, int64_t frames, int dtype,
+                 int64_t n_fft, double sample_rate, int what, double p, int norm,
+                 double roll_percent, double amin, double power, void* out, int mem,
+                 void* cuda_stream) {
+  return guarded([&] {
+    const int rows = check_spectral(what, sample_rate, p, roll_percent, amin, power);
+    if (batch < 0 || bins < 0 || frames < 0)
+      throw smb::invalid_argument(smb::format(
+          "spectral: cannot describe a [%lld, %lld, %lld] spectrogram (extents must be non-negative)",
+          (long long)batch, (long long)bins, (long long)frames));
+    if (n_fft == SMB_DEFAULT) n_fft = 2 * (bins - 1);
+    if (n_fft <= 0 || n_fft / 2 + 1 != bins)
+      throw smb::invalid_argument(smb::format(
+          "spectral: cannot read %lld bins as the spectrum of a %lld-point transform (n_fft must "
+          "be positive, with n_fft / 2 + 1 bins)", (long long)bins, (long long)n_fft));
+    const size_t esz = dtype_size(dtype);
+    check_mem(mem);
+    if (batch == 0 || frames == 0) return;
+    require_device();
+    // no plan, hence no plan stream: SMB_STREAM_OWN means the default stream
+    cudaStream_t st = cuda_stream == SMB_STREAM_OWN ? nullptr : (cudaStream_t)cuda_stream;
+    const size_t in_bytes = (size_t)batch * (size_t)bins * (size_t)frames * esz;
+    const size_t out_bytes = (size_t)batch * (size_t)rows * (size_t)frames * esz;
+    on_stream(mem, st, s, in_bytes, out, out_bytes, [&](const void* src, void* dst) {
+      CK(smb::launch_spectral(spectral_args(src, dst, batch, bins, frames, dtype, n_fft, sample_rate, what,
+                                            p, norm, roll_percent, amin, power), st));
+    });
+  });
+}
+
+int smb_spectral_audio(smb_stft_plan* plan, const void* x, int64_t batch, int64_t n, int dtype,
+                       double sample_rate, int what, double p, int norm, double roll_percent,
+                       double amin, double power, void* out, int mem) {
+  return guarded([&] {
+    smb_stft_plan* pl = plan;
+    const int rows = check_spectral(what, sample_rate, p, roll_percent, amin, power);
+    check_signal("spectral", batch, n);
+    const size_t esz = dtype_size(dtype);
+    check_mem(mem);
+    const smb::FrameGeom g = pl->frame_geom(n);
+    if (batch == 0 || g.frames == 0) return;          // no frame: nothing to write
+    pl->ensure_device();
+    cudaStream_t st = pl->dev->stream.use;
+    const int64_t bins = pl->geom.bins();
+    // |transform| into the plan's scratch, then the descriptors
+    auto run = [&](const void* dx, void* dout, int64_t nb) {
+      void* mag = pl->effect_in.ensure((size_t)nb * (size_t)bins * (size_t)g.frames * esz);
+      run_spectrum(pl, dx, nb, g, dtype, kSpecPower, 1.0, mag);
+      CK(smb::launch_spectral(spectral_args(mag, dout, nb, bins, g.frames, dtype, pl->geom.fft, sample_rate,
+                                            what, p, norm, roll_percent, amin, power), st));
+    };
+    dispatch(mem, pl->pipe, st, x, out, batch, (size_t)n * esz, (size_t)rows * (size_t)g.frames * esz, run);
   });
 }
 

@@ -91,6 +91,23 @@ constexpr long long kHpssFastWindow = 32;
 bool hpss_fast_supports(long long win_harm, long long win_perc);
 cudaError_t launch_hpss(const HpssArgs& a, cudaStream_t st);
 
+// ---- spectral descriptors (spectral_kernels.cu) ---------------------------------
+// s [batch, bins, frames] real -> out [batch, popcount(what), frames] of s's type: the
+// SMB_SPECTRAL_* rows of `what` in flag order (librosa 0.11; DESIGN.md 4.10).
+struct SpectralArgs {
+  const void* s;
+  void* out;
+  long long batch, bins, frames;
+  double bin_hz;            // f_k = k * bin_hz
+  int what;
+  double p;                 // bandwidth: > 0, finite
+  int norm;
+  double roll_percent;      // in (0, 1)
+  double amin, power;       // flatness: > 0
+  int f64;
+};
+cudaError_t launch_spectral(const SpectralArgs& a, cudaStream_t st);
+
 // ---- fast path: fft 2048, float32, fused frame+window+rFFT+|X|^p(+mel) -------
 // Tile shape of the fused CUDA-core kernel: a group of kFastTile warps transforms
 // kFastTile consecutive frames, one per warp.
